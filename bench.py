@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W          (N>1: launched under torch.distributed.run)
     python bench.py --impl reference ...                   (the CPU path of the reference algorithm)
+    python bench.py ... --dump-outputs DIR                 (+ what the last timed step computed, as DIR/<name>.npy)
 
 One JSON line on stdout (rank 0).  A "step" is one ``QLearner.train()`` on one synthetic 2s3z-shaped
 episode batch (BASELINE.json configs[1]: 5 agents, 11 actions, T=120, batch 32 per GPU).
@@ -175,7 +176,7 @@ def run_reference(opt):
     if rank != 0:
         return
     import torch
-    steps, warm = max(1, min(opt.steps, 30)), max(1, min(opt.warmup, 3))
+    steps, warm = opt.steps, max(1, min(opt.warmup, 3))
     r = time_reference(steps, warm)
     sample = (f"{steps} train steps (after {warm} warm-up) of one B=32 synthetic 2s3z-shaped batch through "
               + ("the UNMODIFIED reference QLearner.train (oracle/_ref), args.cuda=False" if r["kind"] == "reference"
@@ -337,6 +338,7 @@ def run_ours(opt):
 
     args = make_args()
     learner = make_learner(SHAPE)
+    seeded = [t.clone() for t in learner_state(learner)] if opt.dump_outputs else None
     if world > 1:
         learner.enable_data_parallel()
 
@@ -379,6 +381,7 @@ def run_ours(opt):
     # ---- value: device-resident batches ---------------------------------------------------------------------------------
     ms_dev, ms_dev_median = tm.run(K, lambda i: train(dev_batches[i % NB]))
     dev_max = float(max(tm.last_per_step))
+    last = (dev_batches[(K - 1) % NB], state["step"] - 1)        # batch and train_step of the last timed step
 
     # ---- e2e (headline): the reference's own loop, runner.py:92-97 -- one freshly generated HOST episode is stored
     # (pinned float64 -> read over PCIe by the cast kernel -> fp32 ring row), a batch of 32 is sampled, train() returns the loss ----
@@ -464,7 +467,7 @@ def run_ours(opt):
 
     for i in range(6):
         cfg5_step(i)
-    ms5, ms5_med = tm.run(max(K, 20), lambda i: cfg5_step(6 + i))
+    ms5, ms5_med = tm.run(K, lambda i: cfg5_step(6 + i))
     cfg5 = {"workload": "4096 matrix-game envs sharded over the ranks (one env launch per rank) -> QMIX train step on the "
                         "emitted device batch, gradients exchanged like config 2",
             "envs_per_gpu": n5, "ms_per_iteration": ms5, "ms_per_iteration_median": ms5_med,
@@ -484,6 +487,16 @@ def run_ours(opt):
     learner._use_graph = True
     env_small = bench_env(torch, dist, world, 4096, 200, hbm_peak)
     env_big = bench_env(torch, dist, world, 1 << 24, 20, hbm_peak)
+    outputs = None
+    if opt.dump_outputs:
+        # The last timed step once more, through the same captured graph of the default path, from the learner's seeded state.
+        # The timed loop's own state differs from run to run: its weight gradients meet in fp32 atomics, and the training steps
+        # grow those last-bit differences.  From the seeded state the step's inputs are identical every run.  (Untimed, after
+        # every measurement: the numbers above are those of a run without --dump-outputs.)
+        for t, s0 in zip(learner_state(learner), seeded):
+            t.copy_(s0)
+        loss = learner.train(last[0], last[1])
+        outputs = snapshot_outputs(torch, learner, loss) if rank == 0 else None
     if rank != 0:
         if world > 1:
             dist.destroy_process_group()
@@ -661,9 +674,40 @@ def run_ours(opt):
         "cpu_baseline": cpu,
         "gpu_baseline": gpu_base,
     }
+    if outputs is not None:
+        write_outputs(opt.dump_outputs, outputs)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
+
+
+def learner_state(learner):
+    """What a train() step reads besides its batch and then updates: parameters, target parameters, optimiser state."""
+    return [learner._flat.data, learner._tflat.data] + list(learner.optimizer.state_dict().values())
+
+
+def snapshot_outputs(torch, learner, loss):
+    """Device copies of what a caller of QLearner.train holds after a step: the returned loss, the clipped gradients left
+    in p.grad, the state_dicts of the trained and target networks, and the hidden states left in the two controllers."""
+    out = {"loss": torch.tensor([loss], dtype=torch.float64)}
+    for prefix, module in (("agent", learner.eval_net.agent), ("mixer", learner.mixer)):
+        for k, p in module.named_parameters():
+            out[f"grad.{prefix}.{k}"] = p.grad.detach().clone()
+    for prefix, module in (("agent", learner.eval_net.agent), ("mixer", learner.mixer),
+                           ("target_agent", learner.target_net.agent), ("target_mixer", learner.target_mixer)):
+        for k, v in module.state_dict().items():
+            out[f"{prefix}.{k}"] = v.detach().clone()
+    out["hidden_states"] = learner.eval_net.hidden_states.detach().clone()
+    out["target_hidden_states"] = learner.target_net.hidden_states.detach().clone()
+    return out
+
+
+def write_outputs(path, outputs):
+    """One DIR/<name>.npy per array: float64 stays float64, everything else is written as float32 (~0.6 MB in all)."""
+    os.makedirs(path, exist_ok=True)
+    for name, t in outputs.items():
+        a = t.cpu().numpy()
+        np.save(os.path.join(path, name + ".npy"), a if a.dtype == np.float64 else a.astype(np.float32))
 
 
 def pin_to_gpu_numa(local):
@@ -687,13 +731,28 @@ def pin_to_gpu_numa(local):
         pass
 
 
+def positive(v):
+    n = int(v)
+    if n < 1:
+        raise argparse.ArgumentTypeError(f"must be >= 1, got {n}")
+    return n
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=positive, default=50,
+                    help="timed train() steps of the headline, end-to-end and env+learner loops (the batch sweep, the other "
+                         "configs, the per-kernel profile and the baselines time fixed counts)")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-sweep", dest="no_sweep", action="store_true", help="skip the B=256/1024 legs")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR",
+                    help="after the measurements, restore the learner's seeded state, run the last timed step of the "
+                         "headline (device-resident batch) loop once more through the same captured graph, and write what "
+                         "it leaves a caller (loss, clipped gradients, networks, hidden states) to DIR/<name>.npy: the "
+                         "step's inputs are identical every run, so two runs or two builds can be compared output for "
+                         "output; the timings are those of a run without this option")
     opt = ap.parse_args()
     if opt.impl == "reference":
         run_reference(opt)

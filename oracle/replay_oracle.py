@@ -3,8 +3,8 @@
 Follows ``common/replaybuffer.py:5-80`` of the reference: eleven float64 numpy rings
 ``[buffer_size, episode_limit, ...]`` (``:19-30``), ``store_episode`` (``:35-51``), uniform sampling with
 replacement through ``np.random.randint`` (``:54-60``) and the ring cursor of ``_get_storage_idx``
-(``:63-80``).  Pinned against the reference itself by ``tests/test_replay_cpu.py`` when ``/root/reference``
-is present.  Only tests may import this module; the product's buffer is ``marl_b200/common/replaybuffer.py``.
+(``:63-80``).  Pinned against the reference itself by ``tests/test_replay_cpu.py`` when it is staged in
+``oracle/_ref``.  Only tests may import this module; the product's buffer is ``marl_b200/common/replaybuffer.py``.
 """
 import numpy as np
 

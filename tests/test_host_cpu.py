@@ -84,7 +84,7 @@ def test_gradient_buffer_can_move_to_caller_memory():
     learner = QLearner(SharedMAC(a), a)
     fl = learner._flat
     assert fl.numel % 4 == 0 and fl.numel <= (1 << 18) and fl.grad_full.numel() == fl.numel + 2
-    new = torch.full((fl.numel + 2,), 7.0)
+    new = torch.full((fl.numel + 2,), 7.0, device=fl.grad_full.device)      # the learner packs on CUDA when there is one
     fl.adopt_grad_storage(new)
     assert float(new.abs().max()) == 0.0                       # zeroed on adoption
     assert fl.grad.data_ptr() == new.data_ptr() and fl.tail.data_ptr() == new.data_ptr() + 4 * fl.numel
@@ -188,3 +188,32 @@ def test_ctypes_structs_have_the_headers_layout(tmp_path):
         assert int(got[cname]) == ctypes.sizeof(cls), cname
         for fname, _ in cls._fields_:
             assert int(got[f"{cname}.{fname}"]) == getattr(cls, fname).offset, (cname, fname)
+
+
+def test_bench_dump_outputs_file_layout(tmp_path):
+    """bench.py --dump-outputs, file layout only (on hand-made hidden states; which step is dumped is bench.py's business):
+    one <name>.npy per array a caller of QLearner.train holds after a step -- loss, clipped gradients, trained and target
+    networks, the two controllers' hidden states -- float64 for the loss and float32 otherwise, far below 64 MB."""
+    import bench
+    a = bench.make_args()
+    learner = QLearner(SharedMAC(a), a)
+    rows = bench.SHAPE["B"] * bench.SHAPE["N"]
+    learner.eval_net.hidden_states = torch.randn(rows, 64)            # as train() leaves them: [B*N, H]
+    learner.target_net.hidden_states = torch.randn(rows, 64)
+    bench.write_outputs(str(tmp_path), bench.snapshot_outputs(torch, learner, 1.5))
+    got = {p.name[:-4]: np.load(p) for p in tmp_path.iterdir()}
+    want = {"loss", "hidden_states", "target_hidden_states"}
+    for prefix, module in (("agent", learner.eval_net.agent), ("mixer", learner.mixer)):
+        for k, p in module.named_parameters():
+            want.add(f"grad.{prefix}.{k}")
+            assert np.array_equal(got[f"grad.{prefix}.{k}"], p.grad.cpu().numpy()), (prefix, k)
+    for prefix, module in (("agent", learner.eval_net.agent), ("mixer", learner.mixer),
+                           ("target_agent", learner.target_net.agent), ("target_mixer", learner.target_mixer)):
+        for k, v in module.state_dict().items():
+            want.add(f"{prefix}.{k}")
+            assert np.array_equal(got[f"{prefix}.{k}"], v.cpu().numpy()), (prefix, k)
+    assert set(got) == want
+    assert got["loss"].dtype == np.float64 and got["loss"].tolist() == [1.5]
+    assert all(v.dtype == np.float32 for k, v in got.items() if k != "loss")
+    assert np.array_equal(got["hidden_states"], learner.eval_net.hidden_states.numpy())
+    assert sum(p.stat().st_size for p in tmp_path.iterdir()) < 64 << 20

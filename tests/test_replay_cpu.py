@@ -1,6 +1,5 @@
 """Host logic of the device replay buffer (run on CPU tensors) against the oracle restatement and, when the
-reference is mounted, against the reference's own ReplayBuffer (common/replaybuffer.py)."""
-import os
+reference is staged in oracle/_ref (oracle/fetch_ref.py), against the reference's own ReplayBuffer (common/replaybuffer.py)."""
 import sys
 from types import SimpleNamespace
 
@@ -10,6 +9,7 @@ import torch
 
 from marl_b200.common.replaybuffer import ReplayBuffer, DeviceEpisodeBatch, KEYS
 from marl_b200.synthetic import synthetic_batch
+from oracle import fetch_ref as FR
 from oracle.replay_oracle import OracleReplayBuffer
 
 DIMS = dict(T=6, N=2, A=3, O=4, S=5)
@@ -33,13 +33,13 @@ def test_ring_cursor_matches_oracle_over_many_wraps():
         assert (mine.current_idx, mine.current_size) == (orc.cursor, orc.filled)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference not mounted")
+@pytest.mark.skipif(not FR.available(), reason="reference not staged in oracle/_ref")
 def test_ring_cursor_matches_reference():
-    sys.path.insert(0, "/root/reference")
+    sys.path.insert(0, FR.DST)
     try:
         from common.replaybuffer import ReplayBuffer as Ref
     finally:
-        sys.path.remove("/root/reference")
+        sys.path.remove(FR.DST)
     ref, mine = Ref(_args(5)), ReplayBuffer(_args(5), device="cpu")
     rng = np.random.RandomState(1)
     for _ in range(300):

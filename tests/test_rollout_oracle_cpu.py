@@ -1,6 +1,6 @@
 """Pins oracle/rollout_oracle.py against the UNMODIFIED reference (RolloutWorker + SharedMAC.choose_action +
-TwoAgentsMatrixGame) when it is mounted; the GPU tests then hold the batched rollout to the oracle."""
-import os
+TwoAgentsMatrixGame) when it is staged in oracle/_ref (oracle/fetch_ref.py); the GPU tests then hold the batched
+rollout to the oracle."""
 import sys
 import types
 from types import SimpleNamespace
@@ -9,15 +9,16 @@ import numpy as np
 import pytest
 import torch
 
+from oracle import fetch_ref as FR
 from oracle import rollout_oracle as RO
 
 PAYOFF1 = [[8, -12, -12], [-12, 0, 0], [-12, 0, 0]]
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference not mounted")
+@pytest.mark.skipif(not FR.available(), reason="reference not staged in oracle/_ref")
 @pytest.mark.parametrize("scale", ["step", "episode"])
 def test_rollout_oracle_matches_reference(scale, capsys):
-    sys.path.insert(0, "/root/reference")
+    sys.path.insert(0, FR.DST)
     saved_gym = sys.modules.get("gym")
     sys.modules["gym"] = types.SimpleNamespace(Env=object)          # env/single_state_matrix_game.py:3,123
     if not hasattr(np, "float"):
@@ -48,7 +49,7 @@ def test_rollout_oracle_matches_reference(scale, capsys):
         params = {k: v.detach().clone() for k, v in mac.agent.state_dict().items()}
         u, r, eps = RO.generate_episodes(params, PAYOFF1, 40, 0.5, 0.01, 0.05, scale)
     finally:
-        sys.path.remove("/root/reference")
+        sys.path.remove(FR.DST)
         if saved_gym is not None:
             sys.modules["gym"] = saved_gym
         else:
