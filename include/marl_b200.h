@@ -186,6 +186,44 @@ int marl_q_select(const marl_dims* d, const float* q_evals, const long long* u, 
 int marl_epsgreedy_select(int rows, int A, const float* q, const float* avail, const unsigned char* explore,
                           const long long* random_action, long long* action, float* onehot, void* stream);
 
+/* One epsilon-greedy step of the shared agent for every row r = e*N + n of n_envs instances, in ONE launch:
+ *   in = [obs[r] (O) | last_onehot[r] (A) | eye(N)[n]]  (share_params.py:84-112, never materialised)
+ *   x = relu(fc1 in + b1);  h' = GRUCell(x, h_in[r]) (gate order r, z, n);  q = fc2 h' + b2
+ *   greedy = first maximum of q masked to -inf where avail[r, a] == 0 (every action masked -> 0).
+ * Exploration, at most one form (both given -> MARL_EINVAL):
+ *   flag form:    explore[r] (uint8) != 0 takes random_action[r] (int64), drawn on the host in the reference's RNG order;
+ *   uniform form: explore_u[r] < eps (float64 compare) takes the min(floor(choice_u[r] * cnt), cnt - 1)-th available
+ *                 action (float64), cnt = number of available actions; cnt = 0 gives action 0.
+ * obs [rows, O], last_onehot [rows, A], avail [rows, A] (NULL: all available), h_in / h_out [rows, H] (may alias: the
+ * hidden state is advanced in place).  Outputs: action [rows] int64; nullable onehot [rows, A] fp32 of the action and
+ * q [rows, A], the network's output before the mask.  gate (nullable, device int): when *gate == 0 the launch does
+ * nothing (a rollout step after every instance has finished).  All weights are staged on chip: a shape whose
+ * fc1 / GRU / fc2 weights do not fit in one block's shared memory returns MARL_EINVAL. */
+int marl_agent_act(int n_envs, int N, int A, int O, const marl_agent_params* p, const float* obs,
+                   const float* last_onehot, const float* avail, const float* h_in, float* h_out,
+                   const unsigned char* explore, const long long* random_action, const double* explore_u,
+                   const double* choice_u, double eps, const int* gate, long long* action, float* onehot, float* q,
+                   void* stream);
+
+/* Bookkeeping of the batched multi-step rollout (rollout.py:52-149), one launch per environment step.
+ * d: B = n instances, L = T (episode_limit), N, A, O, S; ep: the [n, T, ...] episode buffers (padding pre-filled by the
+ * caller: zeros, padded = terminated = 1).  Phase t (1 <= t <= T), for every instance e that was active in step t-1:
+ * u, u_onehot, r, terminated, padded = 0 of step t-1 (action / onehot of that step, reward / terminated as env.step
+ * returned them), o_next / s_next / avail_u_next of step t-1 = obs / state / avail (the getters read after that step),
+ * reward_sum[e] += reward (float64), last[e] = onehot[e], active[e] = !terminated[e].  Then, for t < T, every instance
+ * still active gets o / s / avail_u of step t from the same getters, and counters[t] (instances active at the start of
+ * step t) and counters[T] (their running sum: the environment steps) grow by the active count.  Phase 0 only opens
+ * step 0 (action, onehot, reward, terminated may be NULL).  counters: device int [T + 2], counters[T + 1] is the
+ * launch's scratch word (zero between launches).  active_host (nullable): page-locked host int that receives
+ * counters[t] once the phase's count is complete, so the host can stop stepping without a synchronisation (the count
+ * never increases, so a stale read only costs steps that do nothing).
+ * obs [n, N, O], state [n, S], avail [n, N, A] fp32; action [n, N] int64; onehot / last [n, N, A] fp32; reward [n]
+ * float64; terminated / active [n] uint8 (0 / 1). */
+int marl_rollout_record(const marl_dims* d, int t, const marl_episode_f32* ep, const float* obs, const float* state,
+                        const float* avail, const long long* action, const float* onehot, const double* reward,
+                        const unsigned char* terminated, unsigned char* active, float* last, double* reward_sum,
+                        int* counters, int* active_host, void* stream);
+
 /* ---- TD target + masked MSE: algorithm/q_learner.py:165-168 ----
  * y = r + gamma*q_tot_target*(1-terminated); d = (1-padded)*(y - q_tot);
  * scalars[0] += sum d^2, scalars[1] += sum (1-padded); dq_tot = -2*(1-padded)*d  (UN-normalised:

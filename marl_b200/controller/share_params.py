@@ -9,11 +9,13 @@ input rows [obs | last_action | agent_id] (share_params.py:84-112) are never mat
 """
 from __future__ import annotations
 
+import ctypes as C
+
 import numpy as np
 import torch as th
 
 from .. import _lib as L
-from ..network.q_network import RNNQNet
+from ..network.q_network import RNNQNet, agent_param_struct
 
 
 def _as_f32_cuda(x, device):
@@ -129,6 +131,57 @@ class SharedMAC:
         else:
             action = th.argmax(q_value)
         return action
+
+    def choose_actions(self, obs, last_action, avail_actions, epsilon, evaluate=False, draws=None):
+        """Epsilon-greedy actions of every agent of every instance in ONE ``marl_agent_act`` launch: the batched
+        counterpart of ``choose_action``.
+
+        obs [n, N, O], last_action [n, N, A], avail_actions [n, N, A] or None (all available); numpy arrays or tensors.
+        Agent a of instance e explores iff explore_u[e, a] < epsilon and then takes the
+        min(floor(choice_u[e, a] * cnt), cnt - 1)-th of its cnt available actions (action 0 when it has none);
+        ``draws=(explore_u, choice_u)`` ([n, N] uniforms in [0, 1)) supplies them, None draws them on the device from
+        torch's generator.  ``evaluate=True`` is greedy.  Advances ``self.hidden_states`` (n * N rows, e.g. after
+        ``init_hidden(n)``) in place and keeps its shape.  Returns the int64 CUDA actions [n, N]; nothing waits for the GPU."""
+        dev = self.device
+        if dev.type != "cuda":
+            raise L.MarlLibraryError("SharedMAC needs a CUDA device: marl_b200 has no CPU path")
+        N, A, O, H = self.n_agents, self.n_actions, self.obs_shape, self.args.rnn_hidden_dim
+        obs = _as_f32_cuda(obs, dev)
+        n = obs.shape[0]
+        last = _as_f32_cuda(last_action, dev)
+        avail = None if avail_actions is None else _as_f32_cuda(avail_actions, dev)
+        for name, t, want in (("obs", obs, (n, N, O)), ("last_action", last, (n, N, A)), ("avail_actions", avail, (n, N, A))):
+            if t is not None and tuple(t.shape) != want:
+                raise ValueError(f"{name} has shape {tuple(t.shape)}, expected {want}")
+        h = self.hidden_states
+        if h is None or h.numel() != n * N * H:
+            raise ValueError(f"hidden_states must hold {n} x {N} rows: call init_hidden({n}) first")
+        work = h if (h.is_cuda and h.dtype == th.float32 and h.is_contiguous()) else h.to(dev, th.float32).contiguous()
+        explore_u = choice_u = None
+        if not evaluate:
+            if draws is None:
+                explore_u = th.rand(n, N, dtype=th.float64, device=dev)
+                choice_u = th.rand(n, N, dtype=th.float64, device=dev)
+            else:
+                explore_u, choice_u = (th.as_tensor(d, dtype=th.float64).to(dev).reshape(n, N).contiguous() for d in draws)
+        with th.no_grad():
+            actions = self.act(n, obs, last, avail, work, explore_u=explore_u, choice_u=choice_u, eps=float(epsilon))
+            if work is not h:
+                h.copy_(work.view_as(h))
+        return actions
+
+    def act(self, n, obs, last, avail, hidden, explore=None, random_action=None, explore_u=None, choice_u=None, eps=0.0,
+            gate=None, actions=None, onehot=None, q=None):
+        """One ``marl_agent_act`` launch over n instances: contiguous device tensors, ``hidden`` [n * N, H] advanced in
+        place (include/marl_b200.h documents every argument).  Returns ``actions`` [n, N] int64."""
+        if actions is None:
+            actions = th.empty(n, self.n_agents, dtype=th.int64, device=self.device)
+        p = agent_param_struct(self.agent.param_addresses())
+        L.call("marl_agent_act", n, self.n_agents, self.n_actions, self.obs_shape, C.byref(p), obs.data_ptr(),
+               last.data_ptr(), L.ptr(avail), hidden.data_ptr(), hidden.data_ptr(), L.ptr(explore), L.ptr(random_action),
+               L.ptr(explore_u), L.ptr(choice_u), float(eps), L.ptr(gate), actions.data_ptr(), L.ptr(onehot), L.ptr(q),
+               L.stream_ptr())
+        return actions
 
 
 class SeparatedMAC:

@@ -3,8 +3,8 @@
 The reference's ``RolloutWorker.generate_episodes`` plays ONE environment, asks ``mac.choose_action`` for one
 agent at a time (a batch-1 network forward each, ``rollout.py:60-76``) and concatenates episodes with
 ``np.concatenate``.  ``BatchedRolloutWorker`` plays every instance of a batched environment
-(``BatchedMatrixGame``) at once: one agent forward for all (env, agent) rows, one epsilon-greedy selection
-launch, one environment step launch; the episode batch comes out on the device in the ReplayBuffer layout
+(``BatchedMatrixGame``) at once: one ``marl_agent_act`` launch (agent network and epsilon-greedy selection) for all
+(env, agent) rows, one environment step launch; the episode batch comes out on the device in the ReplayBuffer layout
 (``rollout.py:135-149``) and can go straight into ``marl_b200.common.replaybuffer.ReplayBuffer``.
 
 RNG contract.  ``rng="numpy"`` draws, on the host, exactly what the reference would draw and in its order --
@@ -15,6 +15,8 @@ Q-values, which is what makes hoisting them out of the per-agent loop exact.  ``
 schedule (``rollout.py:47-49, 103-104, 166-167``): annealed per step or per episode, carried across calls.
 """
 from __future__ import annotations
+
+import ctypes as C
 
 import numpy as np
 import torch as th
@@ -38,6 +40,12 @@ class BatchedRolloutWorker:
         # one-step matrix game: the fused record-writing env kernel; anything else that speaks the batched protocol
         # (reset / get_obs / get_state / get_avail_actions / step(actions, active)) goes through the generic multi-step loop
         self._generic = not (hasattr(env, "payoff_table") and self.episode_limit == 1)
+        self._active_host = None             # page-locked word: instances still active, stored by marl_rollout_record
+
+    def _record(self, dims, t, ep_s, obs, state, avail, actions, onehot, reward, term, active, last, rewards, counters):
+        L.call("marl_rollout_record", C.byref(dims), t, C.byref(ep_s), obs.data_ptr(), state.data_ptr(), avail.data_ptr(),
+               actions.data_ptr(), onehot.data_ptr(), L.ptr(reward), L.ptr(term), active.data_ptr(), last.data_ptr(),
+               rewards.data_ptr(), counters.data_ptr(), self._active_host.data_ptr(), L.stream_ptr())
 
     def _epsilons(self, n, evaluate):
         """Per-episode epsilon, advanced exactly like n sequential episodes of the reference would."""
@@ -82,15 +90,13 @@ class BatchedRolloutWorker:
             explore_d = (th.rand(n, N, device=dev) < eps_d).to(th.uint8).contiguous()
             rand_d = th.randint(0, A, (n, N), device=dev, dtype=th.int64)
         # the worker's view of the game at the only step: obs = get_obs() (zeros), no last action, fresh hidden state
-        obs = th.zeros(n, 1, N, self.obs_shape, device=dev)
-        last = th.zeros(n, 1, N, A, device=dev)
-        self.mac.init_hidden(n)
-        q, _ = self.mac.get_current_q_values({"o": obs, "u_onehot": last}, 1)          # [n, 1, N, A]
-        actions = th.empty(n, N, dtype=th.int64, device=dev)
-        L.call("marl_epsgreedy_select", n * N, A, q.contiguous().data_ptr(), None, explore_d.data_ptr(), rand_d.data_ptr(),
-               actions.data_ptr(), None, L.stream_ptr())
+        obs = th.zeros(n, N, self.obs_shape, device=dev)
+        last = th.zeros(n, N, A, device=dev)
+        hidden = th.zeros(n * N, self.args.rnn_hidden_dim, device=dev)
+        actions = self.mac.act(n, obs, last, None, hidden, explore=explore_d, random_action=rand_d)
+        self.mac.hidden_states = hidden                                                 # [n*N, H], as an unroll leaves it
         episodes = self.env.step(actions)
-        self._keep = (explore_d, rand_d, q)
+        self._keep = (explore_d, rand_d)
         if not evaluate:
             self.epsilon = eps_after
         rewards = episodes["r"].reshape(n)
@@ -100,9 +106,14 @@ class BatchedRolloutWorker:
     def _generate_multistep(self, evaluate, random_select, draws):
         """All env.n_envs instances step together until each has terminated or hit ``episode_limit``.
 
-        Per step: ONE agent forward over the (instance, agent) rows with the carried hidden state and the last actions
-        (share_params.py:37-60), ONE ``marl_epsgreedy_select`` launch with the availability mask (``-inf``, first
-        maximum; share_params.py:62-72), one ``env.step``.  Finished instances are frozen and their remaining steps are
+        Per step: ONE ``marl_agent_act`` launch over the (instance, agent) rows -- agent forward with the carried hidden
+        state and the last actions (share_params.py:37-60), availability mask (``-inf``, first maximum) and exploration
+        (share_params.py:62-72) -- then ``env.step``, then ONE ``marl_rollout_record`` launch that writes what the step
+        produced into the episode buffers.  Nothing in the step loop waits for the GPU: the record kernel stores the
+        number of instances still active into a page-locked host word that the loop polls, a step issued after
+        every instance has finished does nothing on the device, and the one synchronisation of the call reads the
+        device step counter at the end.  Every hidden-state row advances on every step in which some instance is
+        active (finished instances feed their frozen observation and last action).  Finished instances are frozen and their remaining steps are
         the reference's padding (rollout.py:122-133): zeros everywhere, ``padded = 1``, ``terminated = 1``; the trailing
         observation / state / availability read after an instance's last step fill ``o_next`` / ``s_next`` /
         ``avail_u_next`` (rollout.py:106-120).
@@ -130,6 +141,7 @@ class BatchedRolloutWorker:
         eps = 0.0 if evaluate else float(self.epsilon)
         if self.args.epsilon_anneal_scale == 'episode':
             eps = eps - self.anneal_epsilon if eps > self.min_epsilon else eps
+        explore_u, choice_u = explore_u.transpose(0, 1).contiguous(), choice_u.transpose(0, 1).contiguous()   # [T, n, N]
         env.reset()
         hidden = th.zeros(n * N, self.args.rnn_hidden_dim, device=dev)
         last = f(n, N, A)
@@ -137,44 +149,41 @@ class BatchedRolloutWorker:
         rewards = th.zeros(n, dtype=th.float64, device=dev)
         actions = th.empty(n, N, dtype=th.int64, device=dev)
         onehot = th.empty(n, N, A, dtype=th.float32, device=dev)
-        steps_tot, prev_active = 0, None
+        counters = th.zeros(T + 2, dtype=th.int32, device=dev)      # [t]: active at the start of step t, [T]: their sum
+        counters[0:1].fill_(n)              # fills, not scalar copies: no host synchronisation
+        counters[T:T + 1].fill_(n)
+        if self._active_host is None:
+            self._active_host = th.zeros(1, dtype=th.int32).pin_memory()
+        host = self._active_host.numpy()
+        host[0] = n                          # the previous call ended with a synchronisation: no launch still writes it
+        dims = L.Dims(n, T, N, A, O, S)
+        ep_s = L.EpisodeF32(*(ep[k].data_ptr() for k in L.EPISODE_KEYS))
+        grab = lambda: tuple(x.to(dev, th.float32).contiguous() for x in (env.get_obs(), env.get_state(), env.get_avail_actions()))
+        reward = term = None
+        t = 0
         with th.no_grad():
-            for t in range(T + 1):
-                obs, state, avail = env.get_obs(), env.get_state(), env.get_avail_actions()
-                if prev_active is not None:          # what the instances that acted at t-1 see afterwards
-                    m = prev_active
-                    ep["o_next"][:, t - 1] = th.where(m.view(n, 1, 1), obs, ep["o_next"][:, t - 1])
-                    ep["s_next"][:, t - 1] = th.where(m.view(n, 1), state, ep["s_next"][:, t - 1])
-                    ep["avail_u_next"][:, t - 1] = th.where(m.view(n, 1, 1), avail, ep["avail_u_next"][:, t - 1])
-                if t == T:
+            for t in range(T):
+                if host[0] == 0:             # every instance has finished (a stale read only adds steps that do nothing)
                     break
-                n_active = int(active.sum().item())
-                if n_active == 0:
-                    break
-                q, _, hidden = mac.agent.unroll(obs.unsqueeze(1).contiguous(), last.unsqueeze(1).contiguous(), hidden, 0)
-                explore = (explore_u[:, t] < eps).to(th.uint8).contiguous()
-                cnt = avail.sum(-1).to(th.float64)
-                kth = th.minimum((choice_u[:, t] * cnt).floor(), cnt - 1)
-                rand_a = ((avail.cumsum(-1).to(th.float64) == (kth + 1).unsqueeze(-1)) & (avail > 0)).to(th.uint8).argmax(-1)
-                L.call("marl_epsgreedy_select", n * N, A, q.reshape(n * N, A).contiguous().data_ptr(), avail.contiguous().data_ptr(),
-                       explore.data_ptr(), rand_a.contiguous().data_ptr(), actions.data_ptr(), onehot.data_ptr(), L.stream_ptr())
+                obs, state, avail = grab()
+                if t == 0:                   # every instance is active: step 0 opens with the first observation
+                    ep["o"][:, 0] = obs
+                    ep["s"][:, 0] = state
+                    ep["avail_u"][:, 0] = avail
+                else:                        # close step t-1, open step t (the getters are consumed before env.step)
+                    self._record(dims, t, ep_s, obs, state, avail, actions, onehot, reward, term, active, last, rewards, counters)
+                mac.act(n, obs, last, avail, hidden, explore_u=explore_u[t], choice_u=choice_u[t], eps=eps,
+                        gate=counters[t:], actions=actions, onehot=onehot)
                 reward, term = env.step(actions, active)
-                a3, a2 = active.view(n, 1, 1), active.view(n, 1)
-                ep["o"][:, t] = th.where(a3, obs, ep["o"][:, t])
-                ep["s"][:, t] = th.where(a2, state, ep["s"][:, t])
-                ep["avail_u"][:, t] = th.where(a3, avail, ep["avail_u"][:, t])
-                ep["u"][:, t] = th.where(a3, actions.unsqueeze(-1), ep["u"][:, t])
-                ep["u_onehot"][:, t] = th.where(a3, onehot, ep["u_onehot"][:, t])
-                ep["r"][:, t] = th.where(a2, reward.to(th.float32).view(n, 1), ep["r"][:, t])
-                ep["terminated"][:, t] = th.where(a2, term.to(th.float32).view(n, 1), ep["terminated"][:, t])
-                ep["padded"][:, t] = th.where(a2, th.zeros_like(ep["padded"][:, t]), ep["padded"][:, t])
-                rewards += th.where(active, reward.to(th.float64), th.zeros_like(rewards))
-                last = th.where(a3, onehot, last)
-                steps_tot += n_active
-                prev_active = active
-                active = active & ~term
+                reward = reward.to(dev, th.float64).contiguous()
+                term = term.to(dev, th.bool).contiguous()
                 if self.args.epsilon_anneal_scale == 'step':
                     eps = eps - self.anneal_epsilon if eps > self.min_epsilon else eps
+            else:
+                t = T
+            obs, state, avail = grab()       # what the instances that acted last see afterwards
+            self._record(dims, t, ep_s, obs, state, avail, actions, onehot, reward, term, active, last, rewards, counters)
+            steps_tot = int(counters[T].item())          # the call's one synchronisation
         if not evaluate:
             cur = float(self.epsilon)
             if self.args.epsilon_anneal_scale == 'step':
