@@ -205,6 +205,20 @@ int marl_agent_act(int n_envs, int N, int A, int O, const marl_agent_params* p, 
                    const double* choice_u, double eps, const int* gate, long long* action, float* onehot, float* q,
                    void* stream);
 
+/* marl_agent_act with one network per agent (SeparatedMAC, share_params.py:389-610): row r = e*N + n uses p[n], an
+ * array of N parameter sets, and its input is
+ *   in = [obs[r] (O) | last_onehot[r] (A, only if last_action) | eye(N)[n] (N, only if agent_id)]  (share_params.py:467-506)
+ * so p[n].fc1_w is [64, O + A*last_action + N*agent_id].  Every other argument, the row layout, the exploration forms,
+ * gate and the outputs are those of marl_agent_act; last_onehot may be NULL when last_action is 0.  A tile holds up to
+ * 32 instances of one agent, so the launch stages each agent's weights in shared memory once per CTA that serves it.
+ * MARL_EINVAL when N > 128, when any of the N parameter sets has a NULL pointer, when last_action is set and last_onehot
+ * is NULL, or when one agent's weights do not fit in one block's shared memory. */
+int marl_agent_act_separated(int n_envs, int N, int A, int O, int last_action, int agent_id, const marl_agent_params* p,
+                             const float* obs, const float* last_onehot, const float* avail, const float* h_in,
+                             float* h_out, const unsigned char* explore, const long long* random_action,
+                             const double* explore_u, const double* choice_u, double eps, const int* gate,
+                             long long* action, float* onehot, float* q, void* stream);
+
 /* Bookkeeping of the batched multi-step rollout (rollout.py:52-149), one launch per environment step.
  * d: B = n instances, L = T (episode_limit), N, A, O, S; ep: the [n, T, ...] episode buffers (padding pre-filled by the
  * caller: zeros, padded = terminated = 1).  Phase t (1 <= t <= T), for every instance e that was active in step t-1:

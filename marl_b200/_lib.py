@@ -167,6 +167,7 @@ _SIGNATURES = {
     "marl_qtran_losses_fwd_bwd": ([_P(Dims)] + [c_ptr] * 12 + [C.c_float] * 3 + [c_ptr] * 5 + [c_ptr], C.c_int),
     "marl_epsgreedy_select": ([C.c_int, C.c_int] + [c_ptr] * 6 + [c_ptr], C.c_int),
     "marl_agent_act": ([C.c_int] * 4 + [_P(AgentParams)] + [c_ptr] * 9 + [C.c_double] + [c_ptr] * 5, C.c_int),
+    "marl_agent_act_separated": ([C.c_int] * 6 + [_P(AgentParams)] + [c_ptr] * 9 + [C.c_double] + [c_ptr] * 5, C.c_int),
     "marl_rollout_record": ([_P(Dims), C.c_int, _P(EpisodeF32)] + [c_ptr] * 12 + [c_ptr], C.c_int),
     "marl_select_fits": ([C.c_int] * 4, C.c_int),
     "marl_episode_lengths": ([c_ptr, C.c_int, C.c_int, c_ptr, c_ptr], C.c_int),

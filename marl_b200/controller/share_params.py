@@ -26,6 +26,41 @@ def _as_f32_cuda(x, device):
     return x.to(device=device, dtype=th.float32, non_blocking=True).contiguous()
 
 
+def _choose_actions(mac, obs, last_action, avail_actions, epsilon, evaluate, draws):
+    """The body of ``SharedMAC.choose_actions`` / ``SeparatedMAC.choose_actions``: checks shapes, draws the exploration
+    uniforms and calls ``mac.act`` on the carried hidden state.  ``last_action`` may be None when ``args.last_action``
+    is False."""
+    dev = mac.device
+    if dev.type != "cuda":
+        raise L.MarlLibraryError(f"{type(mac).__name__} needs a CUDA device: marl_b200 has no CPU path")
+    N, A, O, H = mac.n_agents, mac.n_actions, mac.obs_shape, mac.args.rnn_hidden_dim
+    obs = _as_f32_cuda(obs, dev)
+    n = obs.shape[0]
+    if last_action is None and mac.args.last_action:
+        raise ValueError("last_action is required: the network reads the last action")
+    last = None if last_action is None else _as_f32_cuda(last_action, dev)
+    avail = None if avail_actions is None else _as_f32_cuda(avail_actions, dev)
+    for name, t, want in (("obs", obs, (n, N, O)), ("last_action", last, (n, N, A)), ("avail_actions", avail, (n, N, A))):
+        if t is not None and tuple(t.shape) != want:
+            raise ValueError(f"{name} has shape {tuple(t.shape)}, expected {want}")
+    h = mac.hidden_states
+    if h is None or h.numel() != n * N * H:
+        raise ValueError(f"hidden_states must hold {n} x {N} rows: call init_hidden({n}) first")
+    work = h if (h.is_cuda and h.dtype == th.float32 and h.is_contiguous()) else h.to(dev, th.float32).contiguous()
+    explore_u = choice_u = None
+    if not evaluate:
+        if draws is None:
+            explore_u = th.rand(n, N, dtype=th.float64, device=dev)
+            choice_u = th.rand(n, N, dtype=th.float64, device=dev)
+        else:
+            explore_u, choice_u = (th.as_tensor(d, dtype=th.float64).to(dev).reshape(n, N).contiguous() for d in draws)
+    with th.no_grad():
+        actions = mac.act(n, obs, last, avail, work, explore_u=explore_u, choice_u=choice_u, eps=float(epsilon))
+        if work is not h:
+            h.copy_(work.view_as(h))
+    return actions
+
+
 class SharedMAC:
     """All agents share one RNNQNet; the agent id travels as a one-hot input."""
 
@@ -142,33 +177,7 @@ class SharedMAC:
         ``draws=(explore_u, choice_u)`` ([n, N] uniforms in [0, 1)) supplies them, None draws them on the device from
         torch's generator.  ``evaluate=True`` is greedy.  Advances ``self.hidden_states`` (n * N rows, e.g. after
         ``init_hidden(n)``) in place and keeps its shape.  Returns the int64 CUDA actions [n, N]; nothing waits for the GPU."""
-        dev = self.device
-        if dev.type != "cuda":
-            raise L.MarlLibraryError("SharedMAC needs a CUDA device: marl_b200 has no CPU path")
-        N, A, O, H = self.n_agents, self.n_actions, self.obs_shape, self.args.rnn_hidden_dim
-        obs = _as_f32_cuda(obs, dev)
-        n = obs.shape[0]
-        last = _as_f32_cuda(last_action, dev)
-        avail = None if avail_actions is None else _as_f32_cuda(avail_actions, dev)
-        for name, t, want in (("obs", obs, (n, N, O)), ("last_action", last, (n, N, A)), ("avail_actions", avail, (n, N, A))):
-            if t is not None and tuple(t.shape) != want:
-                raise ValueError(f"{name} has shape {tuple(t.shape)}, expected {want}")
-        h = self.hidden_states
-        if h is None or h.numel() != n * N * H:
-            raise ValueError(f"hidden_states must hold {n} x {N} rows: call init_hidden({n}) first")
-        work = h if (h.is_cuda and h.dtype == th.float32 and h.is_contiguous()) else h.to(dev, th.float32).contiguous()
-        explore_u = choice_u = None
-        if not evaluate:
-            if draws is None:
-                explore_u = th.rand(n, N, dtype=th.float64, device=dev)
-                choice_u = th.rand(n, N, dtype=th.float64, device=dev)
-            else:
-                explore_u, choice_u = (th.as_tensor(d, dtype=th.float64).to(dev).reshape(n, N).contiguous() for d in draws)
-        with th.no_grad():
-            actions = self.act(n, obs, last, avail, work, explore_u=explore_u, choice_u=choice_u, eps=float(epsilon))
-            if work is not h:
-                h.copy_(work.view_as(h))
-        return actions
+        return _choose_actions(self, obs, last_action, avail_actions, epsilon, evaluate, draws)
 
     def act(self, n, obs, last, avail, hidden, explore=None, random_action=None, explore_u=None, choice_u=None, eps=0.0,
             gate=None, actions=None, onehot=None, q=None):
@@ -312,3 +321,24 @@ class SeparatedMAC:
         else:
             action = th.argmax(q_value)
         return action
+
+    def choose_actions(self, obs, last_action, avail_actions, epsilon, evaluate=False, draws=None):
+        """``SharedMAC.choose_actions`` with each agent's own network, in ONE ``marl_agent_act_separated`` launch: the
+        batched counterpart of ``choose_action``.  Same arguments, exploration rule, hidden-state handling and result;
+        ``last_action`` may be None when ``args.last_action`` is False."""
+        return _choose_actions(self, obs, last_action, avail_actions, epsilon, evaluate, draws)
+
+    def act(self, n, obs, last, avail, hidden, explore=None, random_action=None, explore_u=None, choice_u=None, eps=0.0,
+            gate=None, actions=None, onehot=None, q=None):
+        """``SharedMAC.act`` with each agent's own network: one ``marl_agent_act_separated`` launch over n instances,
+        ``hidden`` [n * N, H] advanced in place, ``last`` may be None without a last-action input.  Returns ``actions``
+        [n, N] int64."""
+        if actions is None:
+            actions = th.empty(n, self.n_agents, dtype=th.int64, device=self.device)
+        # rebuilt on every call: a learner's flat buffer or .cuda() re-packs the agents and moves their addresses
+        p = (L.AgentParams * self.n_agents)(*(agent_param_struct(net.param_addresses()) for net in self.agent))
+        L.call("marl_agent_act_separated", n, self.n_agents, self.n_actions, self.obs_shape, int(self.args.last_action),
+               int(self.args.reuse_network), p, obs.data_ptr(), L.ptr(last), L.ptr(avail), hidden.data_ptr(),
+               hidden.data_ptr(), L.ptr(explore), L.ptr(random_action), L.ptr(explore_u), L.ptr(choice_u), float(eps),
+               L.ptr(gate), actions.data_ptr(), L.ptr(onehot), L.ptr(q), L.stream_ptr())
+        return actions

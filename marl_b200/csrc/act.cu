@@ -1,4 +1,5 @@
-// Batched acting (controller/share_params.py:37-72 for every (env, agent) row in one launch) and the per-step
+// Batched acting (controller/share_params.py:37-72 for every (env, agent) row in one launch, with the shared network
+// or, as SeparatedMAC does at :419-453, with each agent's own network) and the per-step
 // bookkeeping of the batched multi-step rollout (rollout.py:52-149 for all instances at once).
 #include <math.h>
 
@@ -39,8 +40,8 @@ inline ActLayout act_layout(int I, int A) {
 }
 
 struct ActArgs {
-    int rows, N, A, O;
-    marl_agent_params p;
+    int rows, n_envs, N, A, O;
+    int last_action, agent_id;                              // input blocks present (the shared agent has both)
     const float* obs; const float* last; const float* avail;
     const float* h_in; float* h_out;                       // may alias
     const unsigned char* explore; const long long* random_action;
@@ -49,7 +50,18 @@ struct ActArgs {
     long long* action; float* onehot; float* q;
 };
 
-__global__ void __launch_bounds__(kActThreads) agent_act_kernel(ActArgs a, ActLayout l) {
+constexpr int kActMaxAgents = 128;  // parameter sets one separated launch carries (8 KB of kernel parameters)
+
+template <int kSets>
+struct ActParams { marl_agent_params p[kSets]; };
+
+// kSets == 1: the shared agent; a tile is 32 consecutive rows, tiles dealt round-robin.
+// kSets > 1: agent n's own weights; a tile is up to 32 instances of ONE agent (rows e*N + n), tiles are agent-major and
+// every CTA takes a contiguous range of them, so it restages weights only when its agent changes.
+template <int kSets>
+__global__ void __launch_bounds__(kActThreads) agent_act_kernel(const __grid_constant__ ActParams<kSets> ps, ActArgs a,
+                                                                ActLayout l) {
+    constexpr bool kSep = kSets > 1;
     if (a.gate && *(volatile const int*)a.gate == 0) return;
     extern __shared__ float sm[];
     __shared__ int act_s[kActRows];
@@ -57,26 +69,48 @@ __global__ void __launch_bounds__(kActThreads) agent_act_kernel(ActArgs a, ActLa
     float *w2 = sm + l.w2, *b2 = sm + l.b2, *ins = sm + l.in, *xq = sm + l.xq, *hs = sm + l.h;
     const int tid = threadIdx.x, A = a.A, O = a.O, I = l.I, Ip = l.Ip;
 
-    for (int i = tid; i < MARL_H * I; i += kActThreads) { const int j = i / I; w1[j * Ip + (i - j * I)] = __ldg(a.p.fc1_w + i); }
-    for (int i = tid; i < MARL_G * MARL_H; i += kActThreads) {
-        const int g = i >> 6, k = i & 63;
-        wih[g * kHP + k] = __ldg(a.p.w_ih + i);
-        whh[g * kHP + k] = __ldg(a.p.w_hh + i);
-    }
-    for (int i = tid; i < A * MARL_H; i += kActThreads) w2[(i >> 6) * kHP + (i & 63)] = __ldg(a.p.fc2_w + i);
-    for (int i = tid; i < MARL_H; i += kActThreads) b1[i] = __ldg(a.p.fc1_b + i);
-    for (int i = tid; i < MARL_G; i += kActThreads) { bih[i] = __ldg(a.p.b_ih + i); bhh[i] = __ldg(a.p.b_hh + i); }
-    for (int i = tid; i < A; i += kActThreads) b2[i] = __ldg(a.p.fc2_b + i);
+    auto stage = [&](const marl_agent_params& p) {
+        for (int i = tid; i < MARL_H * I; i += kActThreads) { const int j = i / I; w1[j * Ip + (i - j * I)] = __ldg(p.fc1_w + i); }
+        for (int i = tid; i < MARL_G * MARL_H; i += kActThreads) {
+            const int g = i >> 6, k = i & 63;
+            wih[g * kHP + k] = __ldg(p.w_ih + i);
+            whh[g * kHP + k] = __ldg(p.w_hh + i);
+        }
+        for (int i = tid; i < A * MARL_H; i += kActThreads) w2[(i >> 6) * kHP + (i & 63)] = __ldg(p.fc2_w + i);
+        for (int i = tid; i < MARL_H; i += kActThreads) b1[i] = __ldg(p.fc1_b + i);
+        for (int i = tid; i < MARL_G; i += kActThreads) { bih[i] = __ldg(p.b_ih + i); bhh[i] = __ldg(p.b_hh + i); }
+        for (int i = tid; i < A; i += kActThreads) b2[i] = __ldg(p.fc2_b + i);
+    };
 
     const int jg = tid & 15, rg = tid >> 4;
-    const int K = O + A;                  // [obs | last action]; the agent-id block is one column, added below
-    const int ntiles = (a.rows + kActRows - 1) / kActRows;
-    for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
-        const int r0 = tile * kActRows;
+    const int K = O + (a.last_action ? A : 0);   // [obs | last action]; the agent-id block is one column, added below
+    const int per_agent = (a.n_envs + kActRows - 1) / kActRows;
+    const int ntiles = kSep ? per_agent * a.N : (a.rows + kActRows - 1) / kActRows;
+    const int t_begin = kSep ? (int)((long long)ntiles * blockIdx.x / gridDim.x) : blockIdx.x;
+    const int t_end = kSep ? (int)((long long)ntiles * (blockIdx.x + 1) / gridDim.x) : ntiles;
+    const int t_step = kSep ? 1 : gridDim.x;
+    int staged = -1;
+    if (!kSep) stage(ps.p[0]);
+    for (int tile = t_begin; tile < t_end; tile += t_step) {
+        // tile row r is global row base + r * stride, r < cnt; the tile's agent is n_tile (separated) or row % N
+        int n_tile = 0, stride = 1, cnt;
+        long long base;
+        if (kSep) {
+            n_tile = tile / per_agent;
+            const int e0 = (tile - n_tile * per_agent) * kActRows;
+            base = (long long)e0 * a.N + n_tile; stride = a.N; cnt = min(kActRows, a.n_envs - e0);
+            if (n_tile != staged) {
+                __syncthreads();          // the previous agent's weights are no longer read
+                stage(ps.p[n_tile]);
+                staged = n_tile;
+            }
+        } else {
+            base = (long long)tile * kActRows; cnt = min(kActRows, a.rows - (int)base);
+        }
         __syncthreads();                  // weights staged / the previous tile's q tile consumed
         for (int i = tid; i < kActRows * MARL_H; i += kActThreads) {
-            const int r = i >> 6, k = i & 63, row = r0 + r;
-            hs[r * kHP + k] = row < a.rows ? a.h_in[(long long)row * MARL_H + k] : 0.f;
+            const int r = i >> 6, k = i & 63;
+            hs[r * kHP + k] = r < cnt ? a.h_in[(base + (long long)r * stride) * MARL_H + k] : 0.f;
         }
         // ---- x = relu(fc1 [obs | last | eye(N)[n]] + b1)
         float acc[2][4];
@@ -86,10 +120,11 @@ __global__ void __launch_bounds__(kActThreads) agent_act_kernel(ActArgs a, ActLa
             const int kc = min(kActKC, K - k0);
             __syncthreads();
             for (int i = tid; i < kActRows * kActKC; i += kActThreads) {
-                const int r = i / kActKC, kk = i % kActKC, row = r0 + r, k = k0 + kk;
+                const int r = i / kActKC, kk = i % kActKC, k = k0 + kk;
+                const long long row = base + (long long)r * stride;
                 float v = 0.f;
-                if (row < a.rows && kk < kc)
-                    v = k < O ? __ldg(a.obs + (long long)row * O + k) : __ldg(a.last + (long long)row * A + (k - O));
+                if (r < cnt && kk < kc)
+                    v = k < O ? __ldg(a.obs + row * O + k) : __ldg(a.last + row * A + (k - O));
                 ins[r * (kActKC + 1) + kk] = v;
             }
             __syncthreads();
@@ -105,11 +140,11 @@ __global__ void __launch_bounds__(kActThreads) agent_act_kernel(ActArgs a, ActLa
         }
 #pragma unroll
         for (int rr = 0; rr < 2; ++rr) {
-            const int r = rg + 16 * rr, n = (r0 + r) % a.N;
+            const int r = rg + 16 * rr, n = kSep ? n_tile : ((int)base + r) % a.N;
 #pragma unroll
             for (int c = 0; c < 4; ++c) {
                 const int j = jg + 16 * c;
-                xq[r * kHP + j] = fmaxf(acc[rr][c] + w1[j * Ip + K + n], 0.f);
+                xq[r * kHP + j] = fmaxf(a.agent_id ? acc[rr][c] + w1[j * Ip + K + n] : acc[rr][c], 0.f);
             }
         }
         __syncthreads();
@@ -153,8 +188,8 @@ __global__ void __launch_bounds__(kActThreads) agent_act_kernel(ActArgs a, ActLa
             for (int c = 0; c < 4; ++c) hs[(rg + 16 * rr) * kHP + jg + 16 * c] = hn[rr][c];
         __syncthreads();
         for (int i = tid; i < kActRows * MARL_H; i += kActThreads) {
-            const int r = i >> 6, k = i & 63, row = r0 + r;
-            if (row < a.rows) a.h_out[(long long)row * MARL_H + k] = hs[r * kHP + k];
+            const int r = i >> 6, k = i & 63;
+            if (r < cnt) a.h_out[(base + (long long)r * stride) * MARL_H + k] = hs[r * kHP + k];
         }
         // ---- q = fc2 h' + b2 (the q tile reuses the x tile)
         for (int i = tid; i < kActRows * A; i += kActThreads) {
@@ -163,27 +198,27 @@ __global__ void __launch_bounds__(kActThreads) agent_act_kernel(ActArgs a, ActLa
 #pragma unroll 8
             for (int k = 0; k < MARL_H; ++k) s = fmaf(w2[act * kHP + k], hs[r * kHP + k], s);
             xq[r * A + act] = s;
-            if (a.q && r0 + r < a.rows) a.q[(long long)(r0 + r) * A + act] = s;
+            if (a.q && r < cnt) a.q[(base + (long long)r * stride) * A + act] = s;
         }
         __syncthreads();
         // ---- masked first maximum, then the exploration forms
-        if (tid < kActRows && r0 + tid < a.rows) {
-            const long long row = r0 + tid;
+        if (tid < cnt) {
+            const long long row = base + (long long)tid * stride;
             const float* av = a.avail ? a.avail + row * A : nullptr;
-            int best = 0, cnt = 0;
+            int best = 0, cnt_av = 0;
             float bv = -INFINITY;
             for (int k = 0; k < A; ++k) {
                 const bool ok = !av || av[k] != 0.0f;
                 const float v = ok ? xq[tid * A + k] : -INFINITY;
                 if (v > bv) { bv = v; best = k; }          // strict: first maximum; all masked -> 0 like th.argmax
-                cnt += ok;
+                cnt_av += ok;
             }
             if (a.explore) {
                 if (a.explore[row]) best = (int)a.random_action[row];
             } else if (a.explore_u && a.explore_u[row] < a.eps) {
                 best = 0;                                   // no available action: action 0
-                if (cnt > 0) {
-                    const double c = (double)cnt;
+                if (cnt_av > 0) {
+                    const double c = (double)cnt_av;
                     const int kth = (int)fmin(floor(a.choice_u[row] * c), c - 1.0);
                     for (int k = 0, seen = 0; k < A; ++k)
                         if (!av || av[k] != 0.0f) {
@@ -198,8 +233,8 @@ __global__ void __launch_bounds__(kActThreads) agent_act_kernel(ActArgs a, ActLa
         if (a.onehot) {
             __syncthreads();
             for (int i = tid; i < kActRows * A; i += kActThreads) {
-                const int r = i / A;
-                if (r0 + r < a.rows) a.onehot[(long long)r0 * A + i] = (i - r * A) == act_s[r] ? 1.0f : 0.0f;
+                const int r = i / A, act = i - r * A;
+                if (r < cnt) a.onehot[(base + (long long)r * stride) * A + act] = act == act_s[r] ? 1.0f : 0.0f;
             }
         }
     }
@@ -277,17 +312,10 @@ __global__ void __launch_bounds__(kRecWarps * 32) rollout_record_kernel(RecArgs 
 
 using namespace marl;
 
-extern "C" int marl_agent_act(int n_envs, int N, int A, int O, const marl_agent_params* p, const float* obs,
-                              const float* last_onehot, const float* avail, const float* h_in, float* h_out,
-                              const unsigned char* explore, const long long* random_action, const double* explore_u,
-                              const double* choice_u, double eps, const int* gate, long long* action, float* onehot,
-                              float* q, void* stream) {
-    if (n_envs < 0 || N <= 0 || A <= 0 || O < 0 || !p || !obs || !last_onehot || !h_in || !h_out || !action) return MARL_EINVAL;
-    if (!p->fc1_w || !p->fc1_b || !p->w_ih || !p->w_hh || !p->b_ih || !p->b_hh || !p->fc2_w || !p->fc2_b) return MARL_EINVAL;
-    if (!explore != !random_action || !explore_u != !choice_u || (explore && explore_u)) return MARL_EINVAL;
-    const long long rows = (long long)n_envs * N;
-    if (rows > 0x7fffffffLL) return MARL_EINVAL;
-    const ActLayout l = act_layout(O + A + N, A);
+// Validates the on-chip footprint of one parameter set of input width I and launches agent_act_kernel<kSets>.
+template <int kSets>
+static int act_launch(const char* name, const ActParams<kSets>& ps, const ActArgs& a, int I, long long tiles, void* stream) {
+    const ActLayout l = act_layout(I, a.A);
     const size_t smem = (size_t)l.total * sizeof(float);
     int dev = 0, sms = 0, optin = 0;
     cudaError_t e = cudaGetDevice(&dev);
@@ -295,29 +323,69 @@ extern "C" int marl_agent_act(int n_envs, int N, int A, int O, const marl_agent_
     if (e == cudaSuccess) e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
     if (e != cudaSuccess) return (int)e;
     if (smem + kActRows * sizeof(int) > (size_t)optin) return MARL_EINVAL;      // weights of this shape do not fit on chip
-    if (rows == 0) return MARL_OK;
+    if (tiles == 0) return MARL_OK;
     static size_t smem_set[64] = {};
     static int blocks_per_sm[64] = {};
     static size_t blocks_for[64] = {};
     const int slot = dev & 63;
     if (smem_set[slot] < smem) {
-        e = cudaFuncSetAttribute(agent_act_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        e = cudaFuncSetAttribute(agent_act_kernel<kSets>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return (int)e;
         smem_set[slot] = smem;
     }
     if (blocks_for[slot] != smem) {
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm[slot], agent_act_kernel, kActThreads, smem);
+        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm[slot], agent_act_kernel<kSets>, kActThreads, smem);
         if (e != cudaSuccess) return (int)e;
         blocks_for[slot] = smem;
     }
-    const long long tiles = (rows + kActRows - 1) / kActRows;
     const long long cap = (long long)sms * (blocks_per_sm[slot] > 0 ? blocks_per_sm[slot] : 1);
-    ActArgs a{(int)rows, N, A, O, *p, obs, last_onehot, avail, h_in, h_out, explore, random_action, explore_u, choice_u, eps,
-              gate, action, onehot, q};
-    { ProfScope ps_("agent_act_kernel", (cudaStream_t)stream);
-      agent_act_kernel<<<(int)(tiles < cap ? tiles : cap), kActThreads, smem, (cudaStream_t)stream>>>(a, l); }
+    { ProfScope ps_(name, (cudaStream_t)stream);
+      agent_act_kernel<kSets><<<(int)(tiles < cap ? tiles : cap), kActThreads, smem, (cudaStream_t)stream>>>(ps, a, l); }
     MARL_LAUNCH_CHECK();
     return MARL_OK;
+}
+
+static bool params_complete(const marl_agent_params& p) {
+    return p.fc1_w && p.fc1_b && p.w_ih && p.w_hh && p.b_ih && p.b_hh && p.fc2_w && p.fc2_b;
+}
+
+extern "C" int marl_agent_act(int n_envs, int N, int A, int O, const marl_agent_params* p, const float* obs,
+                              const float* last_onehot, const float* avail, const float* h_in, float* h_out,
+                              const unsigned char* explore, const long long* random_action, const double* explore_u,
+                              const double* choice_u, double eps, const int* gate, long long* action, float* onehot,
+                              float* q, void* stream) {
+    if (n_envs < 0 || N <= 0 || A <= 0 || O < 0 || !p || !obs || !last_onehot || !h_in || !h_out || !action) return MARL_EINVAL;
+    if (!params_complete(*p)) return MARL_EINVAL;
+    if (!explore != !random_action || !explore_u != !choice_u || (explore && explore_u)) return MARL_EINVAL;
+    const long long rows = (long long)n_envs * N;
+    if (rows > 0x7fffffffLL) return MARL_EINVAL;
+    const ActParams<1> ps{{*p}};
+    const ActArgs a{(int)rows, n_envs, N, A, O, 1, 1, obs, last_onehot, avail, h_in, h_out, explore, random_action, explore_u,
+                    choice_u, eps, gate, action, onehot, q};
+    return act_launch("agent_act_kernel", ps, a, O + A + N, (rows + kActRows - 1) / kActRows, stream);
+}
+
+extern "C" int marl_agent_act_separated(int n_envs, int N, int A, int O, int last_action, int agent_id,
+                                        const marl_agent_params* p, const float* obs, const float* last_onehot,
+                                        const float* avail, const float* h_in, float* h_out, const unsigned char* explore,
+                                        const long long* random_action, const double* explore_u, const double* choice_u,
+                                        double eps, const int* gate, long long* action, float* onehot, float* q,
+                                        void* stream) {
+    if (n_envs < 0 || N <= 0 || N > kActMaxAgents || A <= 0 || O < 0 || !p || !obs || !h_in || !h_out || !action)
+        return MARL_EINVAL;
+    if (last_action && !last_onehot) return MARL_EINVAL;
+    ActParams<kActMaxAgents> ps{};
+    for (int n = 0; n < N; ++n) {
+        if (!params_complete(p[n])) return MARL_EINVAL;
+        ps.p[n] = p[n];
+    }
+    if (!explore != !random_action || !explore_u != !choice_u || (explore && explore_u)) return MARL_EINVAL;
+    const long long rows = (long long)n_envs * N;
+    if (rows > 0x7fffffffLL) return MARL_EINVAL;
+    const ActArgs a{(int)rows, n_envs, N, A, O, last_action ? 1 : 0, agent_id ? 1 : 0, obs, last_onehot, avail, h_in, h_out,
+                    explore, random_action, explore_u, choice_u, eps, gate, action, onehot, q};
+    const int I = O + (last_action ? A : 0) + (agent_id ? N : 0);
+    return act_launch("agent_act_separated_kernel", ps, a, I, (long long)N * ((n_envs + kActRows - 1) / kActRows), stream);
 }
 
 extern "C" int marl_rollout_record(const marl_dims* d, int t, const marl_episode_f32* ep, const float* obs, const float* state,

@@ -3,9 +3,11 @@
 The reference's ``RolloutWorker.generate_episodes`` plays ONE environment, asks ``mac.choose_action`` for one
 agent at a time (a batch-1 network forward each, ``rollout.py:60-76``) and concatenates episodes with
 ``np.concatenate``.  ``BatchedRolloutWorker`` plays every instance of a batched environment
-(``BatchedMatrixGame``) at once: one ``marl_agent_act`` launch (agent network and epsilon-greedy selection) for all
-(env, agent) rows, one environment step launch; the episode batch comes out on the device in the ReplayBuffer layout
-(``rollout.py:135-149``) and can go straight into ``marl_b200.common.replaybuffer.ReplayBuffer``.
+(``BatchedMatrixGame``) at once: one act launch (agent network and epsilon-greedy selection) for all (env, agent)
+rows, one environment step launch; the episode batch comes out on the device in the ReplayBuffer layout
+(``rollout.py:135-149``) and can go straight into ``marl_b200.common.replaybuffer.ReplayBuffer``.  The act launch is
+``mac.act``: ``marl_agent_act`` for a ``SharedMAC``, ``marl_agent_act_separated`` (each agent on its own network) for the
+``SeparatedMAC`` that ``runner.py:24-26`` builds when ``reuse_network`` is False.
 
 RNG contract.  ``rng="numpy"`` draws, on the host, exactly what the reference would draw and in its order --
 per episode, per agent: one ``np.random.uniform()``, then ``np.random.choice(available)`` only when exploring
@@ -106,7 +108,7 @@ class BatchedRolloutWorker:
     def _generate_multistep(self, evaluate, random_select, draws):
         """All env.n_envs instances step together until each has terminated or hit ``episode_limit``.
 
-        Per step: ONE ``marl_agent_act`` launch over the (instance, agent) rows -- agent forward with the carried hidden
+        Per step: ONE act launch (``mac.act``) over the (instance, agent) rows -- agent forward with the carried hidden
         state and the last actions (share_params.py:37-60), availability mask (``-inf``, first maximum) and exploration
         (share_params.py:62-72) -- then ``env.step``, then ONE ``marl_rollout_record`` launch that writes what the step
         produced into the episode buffers.  Nothing in the step loop waits for the GPU: the record kernel stores the
