@@ -22,6 +22,7 @@ from __future__ import annotations
 import copy
 import ctypes as C
 import os
+from collections import namedtuple
 
 import numpy as np
 import torch as th
@@ -30,11 +31,21 @@ from .. import _lib as L
 from ..flat import FlatBuffer, prefixed
 from ..parallel import shard_bounds, allreduce_flat, PeerGradients
 from ..common.replaybuffer import DeviceEpisodeBatch
-from ..network.mixer import VDNMixer, QMixMixer, qmix_struct, qmix2_struct, qmix_tail_struct, QMIX2_FLAT_ORDER
-from ..network.q_network import agent_param_struct, AGENT_FLAT_ORDER
+from ..network.mixer import VDNMixer, QMixMixer, qmix_struct, qmix2_struct, qmix_tail_struct
+from ..network.q_network import agent_param_struct
 
 H = 64
 BATCH_KEYS = ("o", "u", "s", "r", "o_next", "s_next", "avail_u", "avail_u_next", "u_onehot", "padded", "terminated")
+
+
+# One stream of marl_agent_unroll_fwd: batch key of the input; shift of the last-action one-hot (1: u_onehot one step back, for
+# o; 0: for o_next); target net's weights (else the eval net's); stream whose final hidden state it starts from (-1: zeros); keep
+# the gates and W_ih^T for the BPTT
+_Unroll = namedtuple("_Unroll", "obs shift target h0_from keep")
+_EVAL_O = _Unroll("o", 1, False, -1, True)                # eval net on o          (q_learner.py:96-97)
+_TARGET_O_NEXT = _Unroll("o_next", 0, True, -1, False)    # target net on o_next   (:103-104)
+_EVAL_O_NEXT = _Unroll("o_next", 0, False, 0, False)      # eval net on o_next, hidden carried (:110)
+_Fusion = namedtuple("_Fusion", "select heads dhext")       # QLearner._fusion
 
 
 def host_max_episode_len(terminated, episode_limit):
@@ -95,7 +106,7 @@ class QLearner:
         self._use_graph = bool(getattr(args, "cuda_graph", True))
         self._dist = None
         self._peer = None
-        self._side = None
+        self._side = []
         self._copy_stream, self._prefetched, self._slot_free, self._prefetch_seq = None, {}, {}, 0
         self.last = {}
         self.launches_per_step = 0
@@ -148,12 +159,10 @@ class QLearner:
         self._graph_key = None
         self._inplace_cache = {}
         self._ring_structs = {}
-        self._loss_host = th.zeros(2, dtype=th.float32).pin_memory() if dev.type == "cuda" else th.zeros(2)
         # (loss, gradient norm) of a step: the optimiser kernel stores them straight into the page-locked host buffer (the host
         # pointer is the device pointer), so the read-back the reference's loss.item() implies is two posted PCIe writes at the end
-        # of the step's last kernel instead of a copy queued behind it; MARL_B200_LOSS_ZEROCOPY=0 keeps the device buffer + copy
-        zero_copy = dev.type == "cuda" and os.environ.get("MARL_B200_LOSS_ZEROCOPY", "1") != "0"
-        self._loss_out = self._loss_host if zero_copy else th.zeros(2, dtype=th.float32, device=dev)
+        # of the step's last kernel instead of a copy queued behind it (317 -> 308 us per step, profiles/r2c_ab_loss_zerocopy.txt)
+        self._loss_host = th.zeros(2, dtype=th.float32).pin_memory() if dev.type == "cuda" else th.zeros(2)
         self._ws, self._graphs = {}, {}
 
     def _build_extra(self, args):
@@ -421,205 +430,227 @@ class QLearner:
         return shard_bounds(B_glob, dist.get_world_size(group), dist.get_rank(group))
 
     # ---- the device step -----------------------------------------------------------------------------
-    def _agent_structs(self, flat, prefix="agent."):
-        return agent_param_struct({n: flat.ptr(prefix + n) for n in AGENT_FLAT_ORDER})
+    def _agent_plan(self, B, Lq):
+        """The step's agent unrolls (stream i writes ws["q" / "hidden" / "h_last" / "x" / "gi"][i]), and whether the
+        recurrences stop at each episode's end.
 
-    def _launch_forward_backward(self, bt, ws, B, Lq):
-        """Everything between the staged batch and the flat un-normalised gradient."""
+        SURVEY 8(f) N3: args.early_exit: True / False, or None (default) = on from 640 agent rows when there is a time axis to
+        cut.  Measured on ragged batches (lengths U{T/2..T}, tools/early_exit_bench.py, profiles/r2c_early_exit.txt): the QMIX
+        step is 7 % / 5.5 % / 6 % shorter at B = 128 / 256 / 1024 (640 / 1280 / 5120 rows); at config 2 (160 rows, one or two
+        per CTA) the kernels still end with the CTA that holds the longest episode and the shorter chains of the others (-4 us
+        forward, -4 us BPTT in isolation) do not show in the step: 317.6 us either way"""
         a = self.args
-        d = self._dims(B, Lq)
-        sp = L.stream_ptr()
-        self._flat.grad_full.zero_()
-        n_launch = 1
-        pe, pt = self._agent_structs(self._flat), self._agent_structs(self._tflat)
-        double_q = bool(a.double_q)
-        cur = th.cuda.current_stream()
-        if a.alg == "qmix":
-            # the hyper-networks only read the states: run them beside the (latency-bound) agent unrolls
-            if self._side is None:
-                self._side = th.cuda.Stream()
-            two = bool(getattr(a, "two_hyper_layers", False))
-            if two:
-                hh = a.hyper_hidden_dim
-                qp = qmix_tail_struct({n: self._flat.ptr("mixer." + n) for n in ("hyper_b2.2.weight", "hyper_b2.2.bias")})
-                qpt = qmix_tail_struct({n: self._tflat.ptr("mixer." + n) for n in ("hyper_b2.2.weight", "hyper_b2.2.bias")})
-                qg = qmix_tail_struct({n: self._flat.ptr("mixer." + n, self._flat.grad) for n in
-                                       ("hyper_b2.2.weight", "hyper_b2.2.bias")}, L.QmixGrads)
-                q2 = qmix2_struct({n: self._flat.ptr("mixer." + n) for n in QMIX2_FLAT_ORDER}, hh)
-                q2t = qmix2_struct({n: self._tflat.ptr("mixer." + n) for n in QMIX2_FLAT_ORDER}, hh)
-                g2 = qmix2_struct({n: self._flat.ptr("mixer." + n, self._flat.grad) for n in QMIX2_FLAT_ORDER}, None,
-                                  L.QmixHyper2Grads)
-            else:
-                qp = qmix_struct({n: self._flat.ptr("mixer." + n) for n in ("hyper_w1.weight", "hyper_w1.bias",
-                                                                            "hyper_b2.2.weight", "hyper_b2.2.bias")})
-                qpt = qmix_struct({n: self._tflat.ptr("mixer." + n) for n in ("hyper_w1.weight", "hyper_w1.bias",
-                                                                              "hyper_b2.2.weight", "hyper_b2.2.bias")})
-                qg = qmix_struct({n: self._flat.ptr("mixer." + n, self._flat.grad) for n in
-                                  ("hyper_w1.weight", "hyper_w1.bias", "hyper_b2.2.weight", "hyper_b2.2.bias")}, L.QmixGrads)
-            self._side.wait_stream(cur)
-            with th.cuda.stream(self._side):
-                ssp = L.stream_ptr()
-                if two:
-                    L.call("marl_qmix_hyper2_fwd", B * Lq, a.n_agents, a.state_shape, C.byref(q2), bt["s"].data_ptr(),
-                           ws["hh"].data_ptr(), ws["hy"].data_ptr(), ssp)
-                    L.call("marl_qmix_hyper2_fwd", B * Lq, a.n_agents, a.state_shape, C.byref(q2t), bt["s_next"].data_ptr(),
-                           ws["hh_t"].data_ptr(), ws["hy_t"].data_ptr(), ssp)
-                else:
-                    L.call("marl_qmix_hyper_fwd", B * Lq, a.n_agents, a.state_shape, C.byref(qp), bt["s"].data_ptr(),
-                           ws["hy"].data_ptr(), ssp)
-                    L.call("marl_qmix_hyper_fwd", B * Lq, a.n_agents, a.state_shape, C.byref(qpt), bt["s_next"].data_ptr(),
-                           ws["hy_t"].data_ptr(), ssp)
-        n_streams = 3 if double_q else 2
-        arr = (L.UnrollStream * 3)()
-        # VDN / QMIX: the mixing kernel gathers / arg-maxes its own sample (the [N, A] slabs of a warp's sample staged in
-        # shared memory), evaluates the agents' heads q = fc2(h) on the way (no head GEMMs after the unroll) and, dq having
-        # one non-zero per agent row, writes dq . fc2_w itself: no q_select, no dgrad launch
-        NA = a.n_agents * a.n_actions
+        ee = getattr(a, "early_exit", None)
+        early = (B * a.n_agents >= 640 and Lq >= 16) if ee is None else bool(ee)
+        return ((_EVAL_O, _TARGET_O_NEXT, _EVAL_O_NEXT) if a.double_q else (_EVAL_O, _TARGET_O_NEXT)), early
+
+    def _agent_structs(self, flat, grad=False):
+        return agent_param_struct(flat.addrs("agent.", flat.grad if grad else None), L.AgentGrads if grad else L.AgentParams)
+
+    def _side_streams(self, n):
+        self._side += [th.cuda.Stream() for _ in range(n - len(self._side))]
+        return self._side[:n]
+
+    def _fusion(self):
+        """What the VDN / QMIX mixing kernel takes over: the greedy selection (it gathers / arg-maxes its own sample, the [N, A]
+        slabs of a warp's sample staged in shared memory), the agents' heads q = fc2(h) (no head GEMMs after the unroll) and,
+        dq having one non-zero per agent row, dq . fc2_w (no dgrad launch in the BPTT)."""
+        a = self.args
         fc2_w, fc2_wt = self._flat.ptr("agent.fc2.weight"), self._tflat.ptr("agent.fc2.weight")
         fuse = a.alg in ("vdn", "qmix") and bool(getattr(a, "fused_mixer_kernel", True))   # False: one kernel per stage
         fits = lambda heads: bool(L.load().marl_select_fits(int(a.alg == "qmix"), a.n_agents, a.n_actions, heads))
-        fused_select = fuse and fits(0)
-        fused_heads = fused_select and fits(1) and fc2_w % 16 == 0 and fc2_wt % 16 == 0
-        dhext_fused = fuse and fc2_w % 8 == 0
+        select = fuse and fits(0)
+        return _Fusion(select, select and fits(1) and fc2_w % 16 == 0 and fc2_wt % 16 == 0, fuse and fc2_w % 8 == 0)
 
-        # SURVEY 8(f) N3: per-episode early exit of the recurrences.  The eval unroll on `o` must run to L when the double-Q
-        # unroll continues from its final hidden state (the reference carries it through the padded steps, q_learner.py:96,110)
-        # args.early_exit: True / False, or None (default) = on from 640 agent rows when there is a time axis to cut.  Measured on
-        # ragged batches (lengths U{T/2..T}, tools/early_exit_bench.py, profiles/r2c_early_exit.txt): the QMIX step is 7 % / 5.5 % / 6 %
-        # shorter at B = 128 / 256 / 1024 (640 / 1280 / 5120 rows); at config 2 (160 rows, one or two per CTA) the kernels still end
-        # with the CTA that holds the longest episode and the shorter chains of the others (-4 us forward, -4 us BPTT in isolation)
-        # do not show in the step: 317.6 us either way
-        ee = getattr(a, "early_exit", None)
-        early = (B * a.n_agents >= 640 and Lq >= 16) if ee is None else bool(ee)
-        if early:
-            n_launch += 2      # episode lengths + row orders, launched by marl_agent_unroll_fwd beside the input layers
-        ep_len = ws["ep_len"].data_ptr() if early else None
+    def _launch_forward_backward(self, bt, ws, B, Lq):
+        """Everything between the staged batch and the flat un-normalised gradient: zero it, the mixer's prologue, every agent
+        unroll in one launch, the mixer stage, the BPTT.  Each stage returns the launches it issues; this returns their sum."""
+        d = self._dims(B, Lq)
+        plan, early = self._agent_plan(B, Lq)
+        fused = self._fusion()
+        self._flat.grad_full.zero_()
+        n = 1 + self._mixer_prologue(bt, ws, d)
+        n += self._agent_forward(bt, ws, d, plan, early, heads=not fused.heads)
+        n_mix, bptt = self._mixer_stage(bt, ws, d, fused)
+        return n + n_mix + self._agent_backward(bt, ws, d, early, dhext_ready=fused.dhext, **bptt)
 
-        def fill(i, obs, shift, params, h0_from, gates):
+    def _agent_forward(self, bt, ws, d, plan, early, heads):
+        """Every unroll of `plan` in one launch; `heads`: they also evaluate q = fc2(h) into ws["q"]."""
+        pe, pt = self._agent_structs(self._flat), self._agent_structs(self._tflat)
+        continued = {u.h0_from for u in plan}
+        arr = (L.UnrollStream * len(plan))()
+        for i, u in enumerate(plan):
             s = arr[i]
-            s.ep_len = ep_len if (i > 0 or not double_q) else None      # stream 0 is continued by stream 2 under double-Q
-            s.padded = bt["padded"].data_ptr() if (early and s.ep_len) else None
-            s.row_order = ws["row_order"][i].data_ptr() if (early and s.ep_len) else None
-            s.row_order_bwd = ws["row_order"][3].data_ptr() if (early and i == 1) else None     # (stream 1 always has ep_len)
-            s.obs, s.onehot, s.shift_onehot, s.full_input = obs.data_ptr(), bt["u_onehot"].data_ptr(), shift, 0
-            s.h0_from, s.h0, s.params = h0_from, None, params
-            s.q = None if fused_heads else ws["q"][i].data_ptr()
+            # an unroll that another one continues from runs to L (the reference carries the hidden state through the padded
+            # steps, q_learner.py:96,110); stream 1, the target unroll, computes the BPTT's row order
+            cut = early and i not in continued
+            s.ep_len = ws["ep_len"].data_ptr() if cut else None
+            s.padded = bt["padded"].data_ptr() if cut else None
+            s.row_order = ws["row_order"][i].data_ptr() if cut else None
+            s.row_order_bwd = ws["row_order"][3].data_ptr() if (early and i == 1) else None
+            s.obs, s.onehot, s.shift_onehot, s.full_input = bt[u.obs].data_ptr(), bt["u_onehot"].data_ptr(), u.shift, 0
+            s.h0_from, s.h0, s.params = u.h0_from, None, pt if u.target else pe
+            s.q = ws["q"][i].data_ptr() if heads else None
             s.hidden, s.h_last = ws["hidden"][i].data_ptr(), ws["h_last"][i].data_ptr()
-            s.x, s.gi, s.gates = ws["x"][i].data_ptr(), ws["gi"][i].data_ptr(), gates
-            s.w_ih_t = ws["w_ih_t"].data_ptr() if gates else None       # W_ih^T for the backward's data gradient (same step)
+            s.x, s.gi = ws["x"][i].data_ptr(), ws["gi"][i].data_ptr()
+            s.gates = ws["gates"].data_ptr() if u.keep else None
+            s.w_ih_t = ws["w_ih_t"].data_ptr() if u.keep else None       # W_ih^T for the backward's data gradient (same step)
+        L.call("marl_agent_unroll_fwd", C.byref(d), arr, len(plan), L.stream_ptr())
+        # + episode lengths and row orders, launched by marl_agent_unroll_fwd beside the input layers
+        return (3 if heads else 2) * len(plan) + 1 + (2 if early else 0)
 
-        fill(0, bt["o"], 1, pe, -1, ws["gates"].data_ptr())          # eval net on o          (q_learner.py:96-97)
-        fill(1, bt["o_next"], 0, pt, -1, None)                        # target net on o_next   (:103-104)
-        if double_q:
-            fill(2, bt["o_next"], 0, pe, 0, None)                     # eval net on o_next, hidden carried (:110)
-        L.call("marl_agent_unroll_fwd", C.byref(d), arr, n_streams, sp)
-        n_launch += (2 if fused_heads else 3) * n_streams + 1
+    def _agent_backward(self, bt, ws, d, early, dhidden=None, dhext_ready=False, join=None):
+        """BPTT through stream 0 (which kept its gates) from ws["dq"] and `dhidden`.  `dhext_ready`: the mixing kernel wrote
+        dq . fc2_w into ws["dhext"].  `join`: a side stream with work beside the BPTT, waited for after it."""
+        bw = L.UnrollBwd()
+        bw.obs, bw.onehot, bw.shift_onehot, bw.full_input = bt["o"].data_ptr(), bt["u_onehot"].data_ptr(), 1, 0
+        bw.params = self._agent_structs(self._flat)
+        bw.hidden, bw.x, bw.gates = ws["hidden"][0].data_ptr(), ws["x"][0].data_ptr(), ws["gates"].data_ptr()
+        bw.h0, bw.dq, bw.dhidden = None, ws["dq"].data_ptr(), dhidden
+        bw.dhext, bw.dgi, bw.dgh, bw.dx = (ws[k].data_ptr() for k in ("dhext", "dgi", "dgh", "dx"))
+        bw.dh0 = None
+        bw.dhext_ready = int(dhext_ready)
+        bw.w_ih_t = ws["w_ih_t"].data_ptr()
+        bw.ep_len = ws["ep_len"].data_ptr() if early else None
+        bw.row_order = ws["row_order"][3].data_ptr() if early else None
+        bw.grads = self._agent_structs(self._flat, grad=True)
+        L.call("marl_agent_unroll_bwd", C.byref(d), C.byref(bw), L.stream_ptr())
+        if join is not None:
+            th.cuda.current_stream().wait_stream(join)
+        return 7 - int(dhext_ready)
+
+    def _mixer_prologue(self, bt, ws, d):
+        """Mixer work that does not wait for the agent unrolls, issued ahead of them; returns its launches."""
+        if self.args.alg != "qmix":
+            return 0
+        # QMIX: the hyper-networks only read the states: run them beside the (latency-bound) agent unrolls
+        a, M = self.args, d.B * d.L
+        (p, p2), (pt, pt2) = self._qmix_structs(self._flat), self._qmix_structs(self._tflat)
+        side = self._side_streams(1)[0]
+        side.wait_stream(th.cuda.current_stream())
+        with th.cuda.stream(side):
+            sp = L.stream_ptr()
+            if p2 is not None:
+                L.call("marl_qmix_hyper2_fwd", M, a.n_agents, a.state_shape, C.byref(p2), bt["s"].data_ptr(),
+                       ws["hh"].data_ptr(), ws["hy"].data_ptr(), sp)
+                L.call("marl_qmix_hyper2_fwd", M, a.n_agents, a.state_shape, C.byref(pt2), bt["s_next"].data_ptr(),
+                       ws["hh_t"].data_ptr(), ws["hy_t"].data_ptr(), sp)
+                return 2 * 5
+            L.call("marl_qmix_hyper_fwd", M, a.n_agents, a.state_shape, C.byref(p), bt["s"].data_ptr(), ws["hy"].data_ptr(), sp)
+            L.call("marl_qmix_hyper_fwd", M, a.n_agents, a.state_shape, C.byref(pt), bt["s_next"].data_ptr(),
+                   ws["hy_t"].data_ptr(), sp)
+            return 2
+
+    def _mixer_stage(self, bt, ws, d, fused):
+        """Selection, mixers, TD loss and their gradient down to ws["dq"]; returns (launches, options of _agent_backward)."""
+        stage = {"vdn": self._vdn_stage, "qmix": self._qmix_stage, "qplex": self._qplex_stage}[self.args.alg]
+        return stage(bt, ws, d, fused)
+
+    def _select(self, bt, ws, d, fused):
+        """Chosen and target agent Q-values: in the VDN / QMIX mixing kernel, or one marl_q_select.  Returns (launches,
+        the mixing kernel's trailing arguments)."""
+        a, double_q = self.args, bool(self.args.double_q)
         qplex = a.alg == "qplex"
-        if fused_select:
+        n, sel = 0, None
+        fc2_w = self._flat.ptr("agent.fc2.weight")
+        if fused.select:
             sel = L.SelectFused()
             sel.q_evals, sel.q_targets = ws["q"][0].data_ptr(), ws["q"][1].data_ptr()
             sel.q_evals_next = ws["q"][2].data_ptr() if double_q else None
             sel.avail_u_next, sel.a_star = bt["avail_u_next"].data_ptr(), ws["a_star"].data_ptr()
-            if fused_heads:
+            if fused.heads:
                 sel.hidden_evals, sel.hidden_targets = ws["hidden"][0].data_ptr(), ws["hidden"][1].data_ptr()
                 sel.hidden_evals_next = ws["hidden"][2].data_ptr() if double_q else None
                 sel.fc2_w, sel.fc2_b = fc2_w, self._flat.ptr("agent.fc2.bias")
-                sel.fc2_w_target, sel.fc2_b_target = fc2_wt, self._tflat.ptr("agent.fc2.bias")
+                sel.fc2_w_target, sel.fc2_b_target = self._tflat.ptr("agent.fc2.weight"), self._tflat.ptr("agent.fc2.bias")
         else:
             L.call("marl_q_select", C.byref(d), ws["q"][0].data_ptr(), bt["u"].data_ptr(),
                    ws["q"][2].data_ptr() if double_q else None, ws["q"][1].data_ptr(), bt["avail_u_next"].data_ptr(),
                    bt["avail_u"].data_ptr() if qplex else None, ws["q_chosen"].data_ptr(), ws["a_star"].data_ptr(),
                    ws["q_tc"].data_ptr(), ws["max_q"].data_ptr() if qplex else None,
-                   ws["qt_max"].data_ptr() if qplex else None, ws["oh_star"].data_ptr() if qplex else None, sp)
-            n_launch += 1
-        fused_tail = (fc2_w if dhext_fused else None, ws["dhext"].data_ptr() if dhext_fused else None,
-                      C.byref(sel) if fused_select else None)
-        scalars = self._flat.tail.data_ptr()
-        if a.alg == "vdn":
-            L.call("marl_vdn_td_fwd_bwd", C.byref(d), ws["q_chosen"].data_ptr(), ws["q_tc"].data_ptr(), bt["u"].data_ptr(),
-                   bt["r"].data_ptr(), bt["terminated"].data_ptr(), bt["padded"].data_ptr(), float(self.gamma),
-                   ws["q_tot"].data_ptr(), ws["q_tot_t"].data_ptr(), ws["dq"].data_ptr(), scalars, *fused_tail, sp)
-            n_launch += 1
-        elif a.alg == "qmix":
-            p, ptg, g = qp, qpt, qg
-            cur.wait_stream(self._side)
-            L.call("marl_qmix_td_fwd_bwd", C.byref(d), C.byref(p), C.byref(ptg), bt["s"].data_ptr(), bt["s_next"].data_ptr(),
-                   ws["q_chosen"].data_ptr(), ws["q_tc"].data_ptr(), bt["u"].data_ptr(), bt["r"].data_ptr(),
-                   bt["terminated"].data_ptr(), bt["padded"].data_ptr(), float(self.gamma), ws["hy"].data_ptr(),
-                   ws["hy_t"].data_ptr(), ws["dhy"].data_ptr(), ws["q_tot"].data_ptr(), ws["q_tot_t"].data_ptr(),
-                   ws["dq"].data_ptr(), C.byref(g), scalars, 3, *fused_tail, sp)
-            # ... and their weight gradient beside the BPTT (see _hyper_wgrad below)
-            n_launch += 18 if two else 4
-        elif a.alg == "qplex":
-            from ..network.qplex import qplex_struct, qplex_dims, ws_struct
-            M = B * Lq
-            qd = qplex_dims(a)
-            K = a.num_kernel
-            nl = int(getattr(a, "adv_hypernet_layers", 1))
-            p = qplex_struct(lambda n: self._flat.ptr("mixer." + n), K, layers=nl)
-            ptg = qplex_struct(lambda n: self._tflat.ptr("mixer." + n), K, layers=nl)
-            g = qplex_struct(lambda n: self._flat.ptr("mixer." + n, self._flat.grad), K, L.QplexGrads, layers=nl)
-            wse, wst, dws = ws_struct(ws["qp"]), ws_struct(ws["qp_t"]), ws_struct(ws["dqp"])
-            # q_tot = v_tot + a_tot (q_learner.py:120-135); target likewise with the eval net's argmax (:138-158)
-            # the target mixer only shares the selection's outputs with the eval mixer: its chain of products runs beside it
-            if self._side is None:
-                self._side = th.cuda.Stream()
-            self._side.wait_stream(cur)
-            with th.cuda.stream(self._side):
-                sps = L.stream_ptr()
-                if double_q:
-                    L.call("marl_qplex_fwd", M, C.byref(qd), C.byref(ptg), ws["q_tc"].data_ptr(), bt["s_next"].data_ptr(),
-                           ws["oh_star"].data_ptr(), ws["qt_max"].data_ptr(), C.byref(wst), None, None,
-                           ws["q_tot_t"].data_ptr(), sps)
-                else:
-                    L.call("marl_qplex_fwd", M, C.byref(qd), C.byref(ptg), ws["q_tc"].data_ptr(), bt["s_next"].data_ptr(),
-                           None, None, C.byref(wst), ws["q_tot_t"].data_ptr(), None, None, sps)
-            L.call("marl_qplex_fwd", M, C.byref(qd), C.byref(p), ws["q_chosen"].data_ptr(), bt["s"].data_ptr(),
-                   bt["u_onehot"].data_ptr(), ws["max_q"].data_ptr(), C.byref(wse), None, None, ws["q_tot"].data_ptr(), sp)
-            cur.wait_stream(self._side)
-            L.call("marl_td_loss", M, ws["q_tot"].data_ptr(), ws["q_tot_t"].data_ptr(), bt["r"].data_ptr(),
-                   bt["terminated"].data_ptr(), bt["padded"].data_ptr(), float(self.gamma), ws["dq_tot"].data_ptr(),
-                   scalars, sp)
-            L.call("marl_qplex_bwd", M, C.byref(qd), C.byref(p), ws["q_chosen"].data_ptr(), bt["s"].data_ptr(),
-                   bt["u_onehot"].data_ptr(), ws["max_q"].data_ptr(), C.byref(wse), ws["dq_tot"].data_ptr(),
-                   ws["dq_tot"].data_ptr(), C.byref(dws), ws["dq_small"].data_ptr(), C.byref(g), sp)
-            L.call("marl_scatter_dq", C.byref(d), ws["dq_small"].data_ptr(), bt["u"].data_ptr(), ws["dq"].data_ptr(), sp)
-            n_launch += 7 + (7 if double_q else 2) + 1 + 12 + 1
-        else:
-            raise NotImplementedError(a.alg)
-        bw = L.UnrollBwd()
-        bw.obs, bw.onehot, bw.shift_onehot, bw.full_input = bt["o"].data_ptr(), bt["u_onehot"].data_ptr(), 1, 0
-        bw.params = pe
-        bw.hidden, bw.x, bw.gates = ws["hidden"][0].data_ptr(), ws["x"][0].data_ptr(), ws["gates"].data_ptr()
-        bw.h0, bw.dq, bw.dhidden = None, ws["dq"].data_ptr(), None
-        bw.dhext, bw.dgi, bw.dgh, bw.dx = (ws[k].data_ptr() for k in ("dhext", "dgi", "dgh", "dx"))
-        bw.dh0 = None
-        bw.dhext_ready = int(dhext_fused)
-        bw.w_ih_t = ws["w_ih_t"].data_ptr()
-        bw.ep_len = ep_len
-        bw.row_order = ws["row_order"][3].data_ptr() if early else None
-        bw.grads = agent_param_struct({n: self._flat.ptr("agent." + n, self._flat.grad) for n in AGENT_FLAT_ORDER},
-                                      L.AgentGrads)
-        if a.alg == "qmix":
-            # the hyper-network weight gradient runs beside the BPTT (whose kernel is launched at a higher priority)
-            self._hyper_wgrad(cur, two, B * Lq, bt, ws, qg, q2 if two else None, g2 if two else None)
-        L.call("marl_agent_unroll_bwd", C.byref(d), C.byref(bw), sp)
-        if a.alg == "qmix":
-            cur.wait_stream(self._side)
-        n_launch += 7 - int(dhext_fused)
-        return n_launch
+                   ws["qt_max"].data_ptr() if qplex else None, ws["oh_star"].data_ptr() if qplex else None, L.stream_ptr())
+            n = 1
+        return n, (fc2_w if fused.dhext else None, ws["dhext"].data_ptr() if fused.dhext else None,
+                   C.byref(sel) if fused.select else None)
 
-    def _hyper_wgrad(self, cur, two, M, bt, ws, g, q2, g2):
-        """QMIX hyper-network weight gradient on the side stream, after what `cur` holds so far."""
-        a = self.args
-        self._side.wait_stream(cur)
-        with th.cuda.stream(self._side):
-            if two:
-                L.call("marl_qmix_hyper2_bwd", M, a.n_agents, a.state_shape, C.byref(q2), bt["s"].data_ptr(),
+    def _vdn_stage(self, bt, ws, d, fused):
+        n, fused_tail = self._select(bt, ws, d, fused)
+        L.call("marl_vdn_td_fwd_bwd", C.byref(d), ws["q_chosen"].data_ptr(), ws["q_tc"].data_ptr(), bt["u"].data_ptr(),
+               bt["r"].data_ptr(), bt["terminated"].data_ptr(), bt["padded"].data_ptr(), float(self.gamma),
+               ws["q_tot"].data_ptr(), ws["q_tot_t"].data_ptr(), ws["dq"].data_ptr(), self._flat.tail.data_ptr(), *fused_tail,
+               L.stream_ptr())
+        return n + 1, {}
+
+    def _qmix_structs(self, flat, grad=False):
+        """(mixing kernel, two-layer hyper-networks or None) structs of the QMIX mixer in `flat` or its gradient."""
+        addr = flat.addrs("mixer.", flat.grad if grad else None)
+        if not getattr(self.args, "two_hyper_layers", False):
+            return qmix_struct(addr, L.QmixGrads if grad else L.QmixParams), None
+        if grad:
+            return qmix_tail_struct(addr, L.QmixGrads), qmix2_struct(addr, None, L.QmixHyper2Grads)
+        return qmix_tail_struct(addr), qmix2_struct(addr, self.args.hyper_hidden_dim)
+
+    def _qmix_stage(self, bt, ws, d, fused):
+        a, M, sp = self.args, d.B * d.L, L.stream_ptr()
+        (p, p2), (pt, _), (g, g2) = (self._qmix_structs(self._flat), self._qmix_structs(self._tflat),
+                                     self._qmix_structs(self._flat, grad=True))
+        n, fused_tail = self._select(bt, ws, d, fused)
+        cur, side = th.cuda.current_stream(), self._side_streams(1)[0]
+        cur.wait_stream(side)
+        L.call("marl_qmix_td_fwd_bwd", C.byref(d), C.byref(p), C.byref(pt), bt["s"].data_ptr(), bt["s_next"].data_ptr(),
+               ws["q_chosen"].data_ptr(), ws["q_tc"].data_ptr(), bt["u"].data_ptr(), bt["r"].data_ptr(),
+               bt["terminated"].data_ptr(), bt["padded"].data_ptr(), float(self.gamma), ws["hy"].data_ptr(),
+               ws["hy_t"].data_ptr(), ws["dhy"].data_ptr(), ws["q_tot"].data_ptr(), ws["q_tot_t"].data_ptr(),
+               ws["dq"].data_ptr(), C.byref(g), self._flat.tail.data_ptr(), 3, *fused_tail, sp)
+        # the hyper-network weight gradient runs beside the BPTT (whose kernel is launched at a higher priority)
+        side.wait_stream(cur)
+        with th.cuda.stream(side):
+            if p2 is not None:
+                L.call("marl_qmix_hyper2_bwd", M, a.n_agents, a.state_shape, C.byref(p2), bt["s"].data_ptr(),
                        ws["hh"].data_ptr(), ws["dhy"].data_ptr(), ws["dhh"].data_ptr(), C.byref(g2), L.stream_ptr())
+                n += 7
             else:
                 L.call("marl_qmix_hyper_wgrad", M, a.n_agents, a.state_shape, bt["s"].data_ptr(), ws["dhy"].data_ptr(),
                        C.byref(g), L.stream_ptr())
+                n += 1
+        return n + 1, dict(join=side)
+
+    def _qplex_stage(self, bt, ws, d, fused):
+        from ..network.qplex import qplex_struct, qplex_dims, ws_struct
+        a, M, sp = self.args, d.B * d.L, L.stream_ptr()
+        n, _ = self._select(bt, ws, d, fused)
+        qd, K, nl = qplex_dims(a), a.num_kernel, int(getattr(a, "adv_hypernet_layers", 1))
+        p = qplex_struct(self._flat.addrs("mixer.").__getitem__, K, layers=nl)
+        ptg = qplex_struct(self._tflat.addrs("mixer.").__getitem__, K, layers=nl)
+        g = qplex_struct(self._flat.addrs("mixer.", self._flat.grad).__getitem__, K, L.QplexGrads, layers=nl)
+        wse, wst, dws = ws_struct(ws["qp"]), ws_struct(ws["qp_t"]), ws_struct(ws["dqp"])
+        # q_tot = v_tot + a_tot (q_learner.py:120-135); target likewise with the eval net's argmax (:138-158)
+        # the target mixer only shares the selection's outputs with the eval mixer: its chain of products runs beside it
+        cur, side = th.cuda.current_stream(), self._side_streams(1)[0]
+        side.wait_stream(cur)
+        with th.cuda.stream(side):
+            if a.double_q:
+                L.call("marl_qplex_fwd", M, C.byref(qd), C.byref(ptg), ws["q_tc"].data_ptr(), bt["s_next"].data_ptr(),
+                       ws["oh_star"].data_ptr(), ws["qt_max"].data_ptr(), C.byref(wst), None, None,
+                       ws["q_tot_t"].data_ptr(), L.stream_ptr())
+                n += 7
+            else:
+                L.call("marl_qplex_fwd", M, C.byref(qd), C.byref(ptg), ws["q_tc"].data_ptr(), bt["s_next"].data_ptr(),
+                       None, None, C.byref(wst), ws["q_tot_t"].data_ptr(), None, None, L.stream_ptr())
+                n += 2
+        L.call("marl_qplex_fwd", M, C.byref(qd), C.byref(p), ws["q_chosen"].data_ptr(), bt["s"].data_ptr(),
+               bt["u_onehot"].data_ptr(), ws["max_q"].data_ptr(), C.byref(wse), None, None, ws["q_tot"].data_ptr(), sp)
+        n += 7
+        cur.wait_stream(side)
+        L.call("marl_td_loss", M, ws["q_tot"].data_ptr(), ws["q_tot_t"].data_ptr(), bt["r"].data_ptr(),
+               bt["terminated"].data_ptr(), bt["padded"].data_ptr(), float(self.gamma), ws["dq_tot"].data_ptr(),
+               self._flat.tail.data_ptr(), sp)
+        L.call("marl_qplex_bwd", M, C.byref(qd), C.byref(p), ws["q_chosen"].data_ptr(), bt["s"].data_ptr(),
+               bt["u_onehot"].data_ptr(), ws["max_q"].data_ptr(), C.byref(wse), ws["dq_tot"].data_ptr(),
+               ws["dq_tot"].data_ptr(), C.byref(dws), ws["dq_small"].data_ptr(), C.byref(g), sp)
+        n += 1 + 12
+        L.call("marl_scatter_dq", C.byref(d), ws["dq_small"].data_ptr(), bt["u"].data_ptr(), ws["dq"].data_ptr(), sp)
+        return n + 1, {}
 
     def _launch_optimizer(self):
         a, fl, opt, sp = self.args, self._flat, self.optimizer, L.stream_ptr()
@@ -628,17 +659,17 @@ class QLearner:
             L.call("marl_clip_step_peer", int(adam), fl.data.data_ptr(), fl.grad.data_ptr(),
                    (opt.exp_avg if adam else opt.square_avg).data_ptr(), opt.exp_avg_sq.data_ptr() if adam else None,
                    fl.numel, float(a.grad_norm_clip), float(self.lr), 0.9 if adam else 0.99, 0.999 if adam else 0.0, 1e-8,
-                   opt.step_counter.data_ptr() if adam else None, self._loss_out.data_ptr(), C.byref(self._peer.struct), sp)
+                   opt.step_counter.data_ptr() if adam else None, self._loss_host.data_ptr(), C.byref(self._peer.struct), sp)
             return 1
         if opt.kind == "RMS":
             L.call("marl_clip_rmsprop_step", fl.data.data_ptr(), fl.grad.data_ptr(), opt.square_avg.data_ptr(), fl.numel,
                    fl.tail.data_ptr(), float(a.grad_norm_clip), float(self.lr), 0.99, 1e-8, self._partials.data_ptr(),
-                   self._loss_out.data_ptr(), sp)
+                   self._loss_host.data_ptr(), sp)
         else:
             L.call("marl_clip_adam_step", fl.data.data_ptr(), fl.grad.data_ptr(), opt.exp_avg.data_ptr(),
                    opt.exp_avg_sq.data_ptr(), fl.numel, fl.tail.data_ptr(), float(a.grad_norm_clip), float(self.lr),
                    0.9, 0.999, 1e-8, 0, opt.step_counter.data_ptr(), self._partials.data_ptr(),
-                   self._loss_out.data_ptr(), sp)
+                   self._loss_host.data_ptr(), sp)
         return 1 if fl.numel <= (1 << 18) else 2      # one cluster launch up to 2^18 parameters (csrc/optim.cu)
 
     def _device_step(self, bt, ws, B, Lq):
@@ -715,12 +746,11 @@ class QLearner:
         self._run(bt, ws, B, Lq)
         if train_step > 0 and train_step % self.args.target_update_cycle == 0:
             self._update_targets()
-        if self._loss_out is not self._loss_host:
-            self._loss_host.copy_(self._loss_out, non_blocking=True)
         th.cuda.current_stream().synchronize()
-        # hidden states as the reference leaves them ([B*N, H], q_learner.py:96-110)  (an nn.Module attribute store costs ~1.5 us:
-        # skipped while the controller already holds this working set's tensors)
-        he, ht = ws["h_last"][2 if self.args.double_q else 0], ws["h_last"][1]
+        # hidden states as the reference leaves them ([B*N, H], q_learner.py:96-110): those of each net's last unroll  (an nn.Module
+        # attribute store costs ~1.5 us: skipped while the controller already holds this working set's tensors)
+        last = {u.target: h for u, h in zip(self._agent_plan(B, Lq)[0], ws["h_last"])}
+        he, ht = last[False], last[True]
         if self.eval_net.hidden_states is not he:
             self.eval_net.hidden_states = he
         if self.target_net.hidden_states is not ht:
@@ -799,8 +829,6 @@ class QLearner:
         self._launch_optimizer()
         if train_step > 0 and train_step % a.target_update_cycle == 0:
             self._update_targets()
-        if self._loss_out is not self._loss_host:
-            self._loss_host.copy_(self._loss_out, non_blocking=True)
         th.cuda.current_stream().synchronize()
         self.max_episode_len = Lq
         self.last = dict(B=B, L=Lq, q_evals=q_evals.detach(), q_tot=q_tot.detach(), a_star=a_star,

@@ -16,7 +16,6 @@ raises here.
 """
 from __future__ import annotations
 
-import copy
 import ctypes as C
 import os
 
@@ -24,9 +23,8 @@ import torch as th
 
 from .. import _lib as L
 from ..network.mixer import QMixMixer
-from ..network.q_network import agent_param_struct, AGENT_FLAT_ORDER
 from ..network.qtran import QtranQBase, QtranV, net_struct, net_workspace, net_ws_struct
-from .q_learner import QLearner
+from .q_learner import QLearner, _EVAL_O, _TARGET_O_NEXT
 
 H = 64
 
@@ -64,45 +62,34 @@ class QTRANLearner(QLearner):
                       dnq=net_workspace(M, N, D, qh, dev), dnv=net_workspace(M, N, H, qh, dev))
         return ws
 
-    def _net_addrs(self, flat, prefix, module, source=None):
-        return [flat.ptr(prefix + n, source) for n, _ in module.named_parameters()]
+    def _agent_plan(self, B, Lq):
+        return (_EVAL_O, _TARGET_O_NEXT), False            # no double-Q unroll (qtran_learner.py:95-101), no early exit
 
-    def _launch_forward_backward(self, bt, ws, B, Lq):
-        a = self.args
-        d = self._dims(B, Lq)
-        sp = L.stream_ptr()
-        fl, tfl = self._flat, self._tflat
-        fl.grad_full.zero_()
+    def _mixer_prologue(self, bt, ws, d):
         ws["parts"].zero_()
-        pe = agent_param_struct({n: fl.ptr("agent." + n) for n in AGENT_FLAT_ORDER})
-        pt = agent_param_struct({n: tfl.ptr("agent." + n) for n in AGENT_FLAT_ORDER})
-        arr = (L.UnrollStream * 2)()
-        for i, (obs, shift, params, gates) in enumerate(((bt["o"], 1, pe, ws["gates"].data_ptr()), (bt["o_next"], 0, pt, None))):
-            s = arr[i]
-            s.obs, s.onehot, s.shift_onehot, s.full_input = obs.data_ptr(), bt["u_onehot"].data_ptr(), shift, 0
-            s.h0_from, s.h0, s.params = -1, None, params
-            s.q, s.hidden, s.h_last = ws["q"][i].data_ptr(), ws["hidden"][i].data_ptr(), ws["h_last"][i].data_ptr()
-            s.x, s.gi, s.gates = ws["x"][i].data_ptr(), ws["gi"][i].data_ptr(), gates
-            s.w_ih_t = ws["w_ih_t"].data_ptr() if gates else None       # W_ih^T for the backward's data gradient (same step)
-        L.call("marl_agent_unroll_fwd", C.byref(d), arr, 2, sp)
+        return 1
+
+    def _mixer_stage(self, bt, ws, d, fused):
+        a, sp = self.args, L.stream_ptr()
+        fl, tfl = self._flat, self._tflat
         L.call("marl_qtran_select", C.byref(d), ws["q"][0].data_ptr(), ws["q"][1].data_ptr(), bt["avail_u"].data_ptr(),
                bt["avail_u_next"].data_ptr(), bt["u"].data_ptr(), ws["oh_e"].data_ptr(), ws["oh_t"].data_ptr(),
                ws["opt_e"].data_ptr(), ws["q_max"].data_ptr(), ws["q_taken"].data_ptr(), sp)
-        M, N, S, A, qh = B * Lq, a.n_agents, a.state_shape, a.n_actions, a.qtran_hidden_dim
-        pq = net_struct(self._net_addrs(fl, "mixer.", self.mixer))
-        pqt = net_struct(self._net_addrs(tfl, "mixer.", self.target_mixer))
-        pv = net_struct(self._net_addrs(fl, "v.", self.v))
-        gq = net_struct(self._net_addrs(fl, "mixer.", self.mixer, fl.grad), L.QtranNetGrads)
-        gv = net_struct(self._net_addrs(fl, "v.", self.v, fl.grad), L.QtranNetGrads)
+        n = 1
+        M, N, S, A, qh = d.B * d.L, a.n_agents, a.state_shape, a.n_actions, a.qtran_hidden_dim
+        # net_struct takes the addresses in parameter order, the order the flat buffers list them in
+        pq = net_struct(fl.addrs("mixer.").values())
+        pqt = net_struct(tfl.addrs("mixer.").values())
+        pv = net_struct(fl.addrs("v.").values())
+        gq = net_struct(fl.addrs("mixer.", fl.grad).values(), L.QtranNetGrads)
+        gv = net_struct(fl.addrs("v.", fl.grad).values(), L.QtranNetGrads)
         hid_e, hid_t = ws["hidden"][0].data_ptr(), ws["hidden"][1].data_ptr()
         wq, wqt, wqh, wv = (net_ws_struct(ws[k]) for k in ("nq", "nqt", "nqh", "nv"))
         dwq, dwv = net_ws_struct(ws["dnq"]), net_ws_struct(ws["dnv"])
         # get_qtran (qtran_learner.py:165-200): the four network evaluations (joint Q at the taken actions, target joint Q, joint Q at
         # the greedy actions, V) only share their inputs -- chains of small, latency-bound products: three of them run on side
         # streams beside the first
-        cur = th.cuda.current_stream()
-        if getattr(self, "_net_streams", None) is None:
-            self._net_streams = [th.cuda.Stream() for _ in range(3)]
+        cur, sides = th.cuda.current_stream(), self._side_streams(3)
         calls = (
             (pq, bt["s"].data_ptr(), hid_e, bt["u_onehot"].data_ptr(), wq, ws["jq"], A),
             (pqt, bt["s_next"].data_ptr(), hid_t, ws["oh_t"].data_ptr(), wqt, ws["jq_t"], A),
@@ -113,42 +100,26 @@ class QTRANLearner(QLearner):
             if k == 0:
                 L.call("marl_qtran_net_fwd", M, N, S, a_enc, qh, C.byref(pp), st_, hid, act, C.byref(w_), out.data_ptr(), sp)
                 continue
-            side = self._net_streams[k - 1]
+            side = sides[k - 1]
             side.wait_stream(cur)
             with th.cuda.stream(side):
                 L.call("marl_qtran_net_fwd", M, N, S, a_enc, qh, C.byref(pp), st_, hid, act, C.byref(w_), out.data_ptr(), L.stream_ptr())
-        for side in self._net_streams:
+        for side in sides:
             cur.wait_stream(side)
+        n += 6 * len(calls)
         L.call("marl_qtran_losses_fwd_bwd", C.byref(d), ws["jq"].data_ptr(), ws["jq_t"].data_ptr(), ws["jq_hat"].data_ptr(),
                ws["vv"].data_ptr(), ws["q_max"].data_ptr(), ws["q_taken"].data_ptr(), ws["opt_e"].data_ptr(),
                bt["u"].data_ptr(), bt["avail_u"].data_ptr(), bt["r"].data_ptr(), bt["terminated"].data_ptr(),
                bt["padded"].data_ptr(), float(self.gamma), float(a.lambda_opt), float(a.lambda_nopt), ws["d_jq"].data_ptr(),
                ws["d_v"].data_ptr(), ws["dq"].data_ptr(), fl.tail.data_ptr(), ws["parts"].data_ptr(), sp)
+        n += 1
         # (measured and dropped: V's backward on a side stream into its own dL/dhidden buffer, folded afterwards -- 2851 .. 2951 us
         # per step against 2883: the two chains' products already share the machine through the weight-gradient lane)
         L.call("marl_qtran_net_bwd", M, N, S, A, qh, C.byref(pq), bt["s"].data_ptr(), hid_e, bt["u_onehot"].data_ptr(),
                C.byref(wq), ws["d_jq"].data_ptr(), C.byref(dwq), ws["dhid"].data_ptr(), 0, C.byref(gq), sp)
         L.call("marl_qtran_net_bwd", M, N, S, 0, qh, C.byref(pv), bt["s"].data_ptr(), hid_e, None, C.byref(wv),
                ws["d_v"].data_ptr(), C.byref(dwv), ws["dhid"].data_ptr(), 1, C.byref(gv), sp)
-        bw = L.UnrollBwd()
-        bw.obs, bw.onehot, bw.shift_onehot, bw.full_input = bt["o"].data_ptr(), bt["u_onehot"].data_ptr(), 1, 0
-        bw.params = pe
-        bw.hidden, bw.x, bw.gates = ws["hidden"][0].data_ptr(), ws["x"][0].data_ptr(), ws["gates"].data_ptr()
-        bw.h0, bw.dq, bw.dhidden = None, ws["dq"].data_ptr(), ws["dhid"].data_ptr()
-        bw.dhext, bw.dgi, bw.dgh, bw.dx = (ws[k].data_ptr() for k in ("dhext", "dgi", "dgh", "dx"))
-        bw.dh0 = None
-        bw.w_ih_t = ws["w_ih_t"].data_ptr()
-        bw.grads = agent_param_struct({n: fl.ptr("agent." + n, fl.grad) for n in AGENT_FLAT_ORDER}, L.AgentGrads)
-        L.call("marl_agent_unroll_bwd", C.byref(d), C.byref(bw), sp)
-        return 2 + 7 + 1 + 4 * 6 + 1 + 2 * 11 + 7
-
-    def train(self, batch, train_step, episode_num=None):
-        loss = super().train(batch, train_step, episode_num)
-        ws = self.last["ws"]
-        # hidden states as the reference leaves them (no double-Q unroll here)
-        self.eval_net.hidden_states = ws["h_last"][0]
-        self.target_net.hidden_states = ws["h_last"][1]
-        return loss
+        return n + 2 * 11, dict(dhidden=ws["dhid"].data_ptr())
 
     def save_models(self, train_step):
         num = str(train_step // self.args.save_cycle)

@@ -29,6 +29,7 @@ class FlatBuffer:
         self.params = [p for _, p in named_params]
         device = device if device is not None else (self.params[0].device if self.params else torch.device("cpu"))
         self.offsets, off = {}, 0
+        self._addrs = {}
         for n, p, tight in entries:
             if not tight:
                 off = _round_up(off)
@@ -59,6 +60,16 @@ class FlatBuffer:
     def ptr(self, name, source=None):
         src = self.data if source is None else source
         return src.data_ptr() + 4 * self.offsets[name]
+
+    def addrs(self, prefix, source=None):
+        """name -> device address of every entry under `prefix` (the prefix stripped), in packing order: the address map
+        of one module's flat_named_parameters() as packed with ``prefixed(prefix, ...)``.  Kept per (prefix, base address),
+        so the returned dict is shared: do not modify it."""
+        base = (self.data if source is None else source).data_ptr()
+        m = self._addrs.get((prefix, base))
+        if m is None:
+            m = self._addrs[prefix, base] = {n[len(prefix):]: base + 4 * o for n, o in self.offsets.items() if n.startswith(prefix)}
+        return m
 
     def adopt_grad_storage(self, grad_full):
         """Move the gradient buffer (numel + tail floats) into caller-provided device memory."""
