@@ -134,6 +134,15 @@ typedef struct marl_unroll_stream {
                                 episodes keep the index order, here and in the backward.) */
     int* row_order_bwd;      /* out [B*N] ints or NULL (needs an ep_len on some stream of the call): the same deal for the plan
                                 of marl_agent_unroll_bwd; hand it to marl_unroll_bwd.row_order of the SAME step */
+    int agent_stride;        /* 0: one parameter set shared by all agents (everything above).  Otherwise one network per agent
+                                (SeparatedMAC, share_params.py:389-610): `params` points at agent 0's set and agent n+1's set
+                                sits agent_stride floats behind agent n's (a multiple of 4).  Every stream of a call carries the
+                                same stride.  The input row of (b, t, n) is then
+                                [obs | onehot[b,t-shift,n] if last_action | eye(N)[n] if agent_id] (share_params.py:467-506),
+                                so fc1_w is [H, O + A*last_action + N*agent_id].  MARL_EINVAL together with full_input, w_ih_t,
+                                ep_len, padded, row_order or row_order_bwd */
+    int last_action;         /* separated only (ignored when agent_stride == 0): the input carries the last action */
+    int agent_id;            /* separated only: the input carries the agent's one-hot id */
 } marl_unroll_stream;
 
 /* ep_len[b] = 1 + the last step with padded[b, t] == 0 (at least 1): every step at or beyond it has mask = 0 in the loss
@@ -164,6 +173,11 @@ typedef struct marl_unroll_bwd {
                                 computes there: every upstream gradient is masked to zero) */
     const int* row_order;    /* [B*N] = marl_unroll_stream.row_order_bwd of this step's forward call, or NULL (index order); only
                                 read together with ep_len */
+    int agent_stride;        /* as marl_unroll_stream.agent_stride: 0 shared, else one network per agent with `params` and
+                                `grads` at agent 0's set and agent n+1's agent_stride floats behind agent n's.  MARL_EINVAL
+                                together with full_input, w_ih_t, ep_len or row_order */
+    int last_action;         /* separated only: as marl_unroll_stream.last_action */
+    int agent_id;            /* separated only: as marl_unroll_stream.agent_id */
 } marl_unroll_bwd;
 
 int marl_agent_unroll_bwd(const marl_dims* d, const marl_unroll_bwd* a, void* stream);

@@ -49,14 +49,16 @@ class UnrollStream(C.Structure):
                 ("h0_from", C.c_int), ("h0", c_ptr),
                 ("params", AgentParams), ("q", c_ptr), ("hidden", c_ptr), ("h_last", c_ptr), ("x", c_ptr),
                 ("gi", c_ptr), ("gates", c_ptr), ("w_ih_t", c_ptr), ("ep_len", c_ptr), ("padded", c_ptr),
-                ("row_order", c_ptr), ("row_order_bwd", c_ptr)]
+                ("row_order", c_ptr), ("row_order_bwd", c_ptr), ("agent_stride", C.c_int), ("last_action", C.c_int),
+                ("agent_id", C.c_int)]
 
 
 class UnrollBwd(C.Structure):
     _fields_ = [("obs", c_ptr), ("onehot", c_ptr), ("shift_onehot", C.c_int), ("full_input", C.c_int),
                 ("params", AgentParams), ("hidden", c_ptr), ("x", c_ptr), ("gates", c_ptr), ("h0", c_ptr), ("dq", c_ptr),
                 ("dhidden", c_ptr), ("dhext", c_ptr), ("dgi", c_ptr), ("dgh", c_ptr), ("dx", c_ptr), ("dh0", c_ptr),
-                ("grads", AgentGrads), ("dhext_ready", C.c_int), ("w_ih_t", c_ptr), ("ep_len", c_ptr), ("row_order", c_ptr)]
+                ("grads", AgentGrads), ("dhext_ready", C.c_int), ("w_ih_t", c_ptr), ("ep_len", c_ptr), ("row_order", c_ptr),
+                ("agent_stride", C.c_int), ("last_action", C.c_int), ("agent_id", C.c_int)]
 
 
 class PeerGroup(C.Structure):

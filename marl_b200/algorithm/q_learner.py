@@ -159,6 +159,7 @@ class QLearner:
         self._graph_key = None
         self._inplace_cache = {}
         self._ring_structs = {}
+        self._agent_sets = {}        # id(flat) -> agent stride (separated_stride), for the two flat buffers packed here
         # (loss, gradient norm) of a step: the optimiser kernel stores them straight into the page-locked host buffer (the host
         # pointer is the device pointer), so the read-back the reference's loss.item() implies is two posted PCIe writes at the end
         # of the step's last kernel instead of a copy queued behind it (317 -> 308 us per step, profiles/r2c_ab_loss_zerocopy.txt)
@@ -233,6 +234,7 @@ class QLearner:
             q_tot=f(B, Lq, 1), q_tot_t=f(B, Lq, 1), dq=f(B, Lq, N, A),
             dhext=f(rows, H), dgi=f(rows, 3 * H), dgh=f(rows, 3 * H), dx=f(rows, H),
         )
+        ws["h_last_sep"] = [h.view(B, N, H) for h in ws["h_last"]]
         if a.alg == "qmix":
             Ccols = N * 32 + 96
             ws.update(hy=f(M, Ccols), hy_t=f(M, Ccols), dhy=f(M, Ccols))
@@ -438,14 +440,26 @@ class QLearner:
         cut.  Measured on ragged batches (lengths U{T/2..T}, tools/early_exit_bench.py, profiles/r2c_early_exit.txt): the QMIX
         step is 7 % / 5.5 % / 6 % shorter at B = 128 / 256 / 1024 (640 / 1280 / 5120 rows); at config 2 (160 rows, one or two
         per CTA) the kernels still end with the CTA that holds the longest episode and the shorter chains of the others (-4 us
-        forward, -4 us BPTT in isolation) do not show in the step: 317.6 us either way"""
+        forward, -4 us BPTT in isolation) do not show in the step: 317.6 us either way.
+
+        With one network per agent (SeparatedMAC) the recurrences always run to L, whatever args.early_exit says: the rows of
+        a pass must belong to one agent, whose W_hh the pass holds in registers, and the length-sorted deal mixes agents."""
         a = self.args
         ee = getattr(a, "early_exit", None)
         early = (B * a.n_agents >= 640 and Lq >= 16) if ee is None else bool(ee)
-        return ((_EVAL_O, _TARGET_O_NEXT, _EVAL_O_NEXT) if a.double_q else (_EVAL_O, _TARGET_O_NEXT)), early
+        plan = (_EVAL_O, _TARGET_O_NEXT, _EVAL_O_NEXT) if a.double_q else (_EVAL_O, _TARGET_O_NEXT)
+        return plan, early and not self._separated
 
     def _agent_structs(self, flat, grad=False):
-        return agent_param_struct(flat.addrs("agent.", flat.grad if grad else None), L.AgentGrads if grad else L.AgentParams)
+        """(parameter or gradient struct, agent stride) of the agent in `flat`: the shared network with stride 0, or -- one
+        network per agent -- agent 0's set and the distance in floats from agent n's set to agent n+1's."""
+        cls, src = (L.AgentGrads, flat.grad) if grad else (L.AgentParams, None)
+        if not self._separated:
+            return agent_param_struct(flat.addrs("agent.", src), cls), 0
+        stride = self._agent_sets.get(id(flat))
+        if stride is None:
+            stride = self._agent_sets[id(flat)] = separated_stride(flat, self.args.n_agents)
+        return agent_param_struct(flat.addrs("agent.0.", src), cls), stride
 
     def _side_streams(self, n):
         self._side += [th.cuda.Stream() for _ in range(n - len(self._side))]
@@ -454,12 +468,15 @@ class QLearner:
     def _fusion(self):
         """What the VDN / QMIX mixing kernel takes over: the greedy selection (it gathers / arg-maxes its own sample, the [N, A]
         slabs of a warp's sample staged in shared memory), the agents' heads q = fc2(h) (no head GEMMs after the unroll) and,
-        dq having one non-zero per agent row, dq . fc2_w (no dgrad launch in the BPTT)."""
+        dq having one non-zero per agent row, dq . fc2_w (no dgrad launch in the BPTT).  With one network per agent only the
+        selection: the kernel stages one fc2, not one per agent."""
         a = self.args
-        fc2_w, fc2_wt = self._flat.ptr("agent.fc2.weight"), self._tflat.ptr("agent.fc2.weight")
         fuse = a.alg in ("vdn", "qmix") and bool(getattr(a, "fused_mixer_kernel", True))   # False: one kernel per stage
         fits = lambda heads: bool(L.load().marl_select_fits(int(a.alg == "qmix"), a.n_agents, a.n_actions, heads))
         select = fuse and fits(0)
+        if self._separated:
+            return _Fusion(select, False, False)
+        fc2_w, fc2_wt = self._flat.ptr("agent.fc2.weight"), self._tflat.ptr("agent.fc2.weight")
         return _Fusion(select, select and fits(1) and fc2_w % 16 == 0 and fc2_wt % 16 == 0, fuse and fc2_w % 8 == 0)
 
     def _launch_forward_backward(self, bt, ws, B, Lq):
@@ -476,7 +493,10 @@ class QLearner:
 
     def _agent_forward(self, bt, ws, d, plan, early, heads):
         """Every unroll of `plan` in one launch; `heads`: they also evaluate q = fc2(h) into ws["q"]."""
-        pe, pt = self._agent_structs(self._flat), self._agent_structs(self._tflat)
+        (pe, stride), (pt, t_stride) = self._agent_structs(self._flat), self._agent_structs(self._tflat)
+        if t_stride != stride:          # one stride per call: _pack lays both buffers' agents out alike
+            raise ValueError(f"target agent stride {t_stride} differs from the eval stride {stride}")
+        sep, last_action, agent_id = self._separated, int(self.args.last_action), int(self.args.reuse_network)
         continued = {u.h0_from for u in plan}
         arr = (L.UnrollStream * len(plan))()
         for i, u in enumerate(plan):
@@ -494,7 +514,8 @@ class QLearner:
             s.hidden, s.h_last = ws["hidden"][i].data_ptr(), ws["h_last"][i].data_ptr()
             s.x, s.gi = ws["x"][i].data_ptr(), ws["gi"][i].data_ptr()
             s.gates = ws["gates"].data_ptr() if u.keep else None
-            s.w_ih_t = ws["w_ih_t"].data_ptr() if u.keep else None       # W_ih^T for the backward's data gradient (same step)
+            s.w_ih_t = ws["w_ih_t"].data_ptr() if u.keep and not sep else None    # W_ih^T for the backward's data gradient
+            s.agent_stride, s.last_action, s.agent_id = stride, last_action, agent_id
         L.call("marl_agent_unroll_fwd", C.byref(d), arr, len(plan), L.stream_ptr())
         # + episode lengths and row orders, launched by marl_agent_unroll_fwd beside the input layers
         return (3 if heads else 2) * len(plan) + 1 + (2 if early else 0)
@@ -504,16 +525,17 @@ class QLearner:
         dq . fc2_w into ws["dhext"].  `join`: a side stream with work beside the BPTT, waited for after it."""
         bw = L.UnrollBwd()
         bw.obs, bw.onehot, bw.shift_onehot, bw.full_input = bt["o"].data_ptr(), bt["u_onehot"].data_ptr(), 1, 0
-        bw.params = self._agent_structs(self._flat)
+        bw.params, bw.agent_stride = self._agent_structs(self._flat)
+        bw.last_action, bw.agent_id = int(self.args.last_action), int(self.args.reuse_network)
         bw.hidden, bw.x, bw.gates = ws["hidden"][0].data_ptr(), ws["x"][0].data_ptr(), ws["gates"].data_ptr()
         bw.h0, bw.dq, bw.dhidden = None, ws["dq"].data_ptr(), dhidden
         bw.dhext, bw.dgi, bw.dgh, bw.dx = (ws[k].data_ptr() for k in ("dhext", "dgi", "dgh", "dx"))
         bw.dh0 = None
         bw.dhext_ready = int(dhext_ready)
-        bw.w_ih_t = ws["w_ih_t"].data_ptr()
+        bw.w_ih_t = None if self._separated else ws["w_ih_t"].data_ptr()
         bw.ep_len = ws["ep_len"].data_ptr() if early else None
         bw.row_order = ws["row_order"][3].data_ptr() if early else None
-        bw.grads = self._agent_structs(self._flat, grad=True)
+        bw.grads = self._agent_structs(self._flat, grad=True)[0]
         L.call("marl_agent_unroll_bwd", C.byref(d), C.byref(bw), L.stream_ptr())
         if join is not None:
             th.cuda.current_stream().wait_stream(join)
@@ -552,7 +574,7 @@ class QLearner:
         a, double_q = self.args, bool(self.args.double_q)
         qplex = a.alg == "qplex"
         n, sel = 0, None
-        fc2_w = self._flat.ptr("agent.fc2.weight")
+        fc2_w = self._flat.ptr("agent.fc2.weight") if (fused.heads or fused.dhext) else None
         if fused.select:
             sel = L.SelectFused()
             sel.q_evals, sel.q_targets = ws["q"][0].data_ptr(), ws["q"][1].data_ptr()
@@ -730,7 +752,7 @@ class QLearner:
         drives the target sync exactly like the reference's ``train_step``."""
         if self._dev.type != "cuda":
             raise L.MarlLibraryError("QLearner.train needs a CUDA device: marl_b200 has no CPU path")
-        if self._separated or getattr(self.args, "train_through_modules", False):
+        if getattr(self.args, "train_through_modules", False):
             return self._train_modules(batch, train_step)
         self._graph_key = None
         if isinstance(batch, DeviceEpisodeBatch):
@@ -747,9 +769,10 @@ class QLearner:
         if train_step > 0 and train_step % self.args.target_update_cycle == 0:
             self._update_targets()
         th.cuda.current_stream().synchronize()
-        # hidden states as the reference leaves them ([B*N, H], q_learner.py:96-110): those of each net's last unroll  (an nn.Module
-        # attribute store costs ~1.5 us: skipped while the controller already holds this working set's tensors)
-        last = {u.target: h for u, h in zip(self._agent_plan(B, Lq)[0], ws["h_last"])}
+        # hidden states as the reference leaves them ([B*N, H], q_learner.py:96-110; [B, N, H] for SeparatedMAC): those of each
+        # net's last unroll  (an nn.Module attribute store costs ~1.5 us: skipped while the controller already holds this working
+        # set's tensors)
+        last = {u.target: h for u, h in zip(self._agent_plan(B, Lq)[0], ws["h_last_sep" if self._separated else "h_last"])}
         he, ht = last[False], last[True]
         if self.eval_net.hidden_states is not he:
             self.eval_net.hidden_states = he
@@ -764,9 +787,8 @@ class QLearner:
     def _train_modules(self, batch, train_step):
         """q_learner.py:68-179 written against the controller / mixer modules: every unroll and every mixer call is a
         libmarl_b200 kernel sequence behind a torch.autograd.Function, the gather / mask / TD arithmetic between them is
-        torch on the GPU, clip + RMSprop/Adam is the flat optimiser kernel.  This is what SeparatedMAC trains with (its
-        per-agent weights do not fit the shared-weight fused kernels), and an independent second implementation of the
-        fused step for the tests."""
+        torch on the GPU, clip + RMSprop/Adam is the flat optimiser kernel.  ``args.train_through_modules`` selects it: an
+        independent second implementation of the fused step for the tests."""
         a, dev = self.args, self._dev
         if isinstance(batch, DeviceEpisodeBatch):
             Lq = batch.max_episode_len
@@ -884,6 +906,26 @@ class QLearner:
                     else:
                         q_tot_table[i, j] = self.mixer(chosen, one['s']).item()
             return q_tot_table, q_table_i, q_table_j
+
+
+def separated_stride(flat, n_agents):
+    """Distance in floats from agent n's parameter set to agent n+1's in a flat buffer packed agent after agent as
+    ``agent.{n}.*`` (QLearner._pack).  ValueError unless it is the same positive multiple of 4 for every agent and every
+    parameter: the library addresses agent n's set as agent 0's plus n strides."""
+    off = flat.offsets
+    names = [n[len("agent.0."):] for n in flat.names if n.startswith("agent.0.")]
+    if n_agents > 1:
+        stride = off["agent.1." + names[0]] - off["agent.0." + names[0]]
+    else:
+        end = max(off["agent.0." + k] + flat.view("agent.0." + k).numel() for k in names)
+        stride = (end - off["agent.0." + names[0]] + 3) // 4 * 4
+    for i in range(n_agents):
+        for k in names:
+            if off.get(f"agent.{i}.{k}") != off["agent.0." + k] + i * stride:
+                raise ValueError(f"agent parameter sets are not evenly spaced in the flat buffer (agent.{i}.{k})")
+    if stride <= 0 or stride % 4:
+        raise ValueError(f"agent parameter stride {stride} is not a positive multiple of 4 floats")
+    return stride
 
 
 def _to_numpy(x):

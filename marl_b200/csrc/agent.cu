@@ -77,6 +77,7 @@ struct GruFwdArgs {
     unsigned short rows_of[kMaxStreams][kNumSMs];   // rows of chain c advanced by CTA i (balanced on the host, see plan_rows)
     const int* row_order[kMaxStreams];              // per chain: logical position -> row (b*N + n), or null = identity (row_order_kernel)
     long long* trace;                                // debug (marl_tgemm_trace): clock64 phase stamps of steps 8..15, CTA 0 / CTA 100
+    int agent_stride;                                // separated networks (SEP instantiation): floats from agent n's parameters to n+1's
 };
 #ifdef MARL_GRU_TRACE      // tools/gru_trace.py with an A/B build (tools/ab_build.py trace -DMARL_GRU_TRACE)
 // (stamps of steps 8..15 stay in registers -- a store per stamp costs ~75 cycles and distorts the step -- and are written after the loop)
@@ -93,7 +94,17 @@ struct GruFwdArgs {
 // 128-thread named barrier: the CTA hosts one such group per chain, each advancing its own rows
 __device__ __forceinline__ void group_sync(int id) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(kGruThreads) : "memory"); }
 
-template <int R>
+// Separated networks (one parameter set per agent, SEP): logical positions are dealt agent-major, position p = n*B + b is row
+// b*N + n, and a pass never straddles two agents (gru_pass_rows), so the W_hh slice in registers is the pass's agent's.
+template <bool SEP>
+__device__ __forceinline__ int gru_position_row(int p, int B, int N) { return SEP ? (p % B) * N + p / B : p; }
+template <bool SEP>
+__device__ __forceinline__ int gru_pass_rows(int pos, int left, int B) {
+    const int n = min(kGruMaxRows, left);
+    return SEP ? min(n, B - pos % B) : n;
+}
+
+template <int R, bool SEP>
 __device__ __forceinline__ void gru_chain_fwd(const GruFwdArgs& a, int chain, int row0, int nrows, float* smem, int bar_id) {
     float (*hs)[R][MARL_H] = reinterpret_cast<float (*)[R][MARL_H]>(smem);                          // [2][R][H]
     float (*ring)[R][MARL_G] = reinterpret_cast<float (*)[R][MARL_G]>(smem + 2 * R * MARL_H);       // [D][R][3H]
@@ -103,7 +114,10 @@ __device__ __forceinline__ void gru_chain_fwd(const GruFwdArgs& a, int chain, in
     // (resolved once per pass into shared memory: the previous pass ended with a group barrier)
     __shared__ int srow_all[kGruGroups][kGruMaxRows];
     int* srow = srow_all[bar_id - 1];
-    if (tid < R) { const int* order = a.row_order[chain]; srow[tid] = (order && tid < nrows) ? __ldg(order + row0 + tid) : row0 + tid; }
+    if (tid < R) {
+        const int* order = a.row_order[chain];
+        srow[tid] = (order && tid < nrows) ? __ldg(order + row0 + tid) : gru_position_row<SEP>(row0 + tid, a.B, N);
+    }
     group_sync(bar_id);
     auto row_at = [&](int rr) { return srow[rr]; };
     constexpr int OWN = (R + 1) / 2;                  // rows whose gate math this lane owns: rr = ks + 2q
@@ -138,15 +152,18 @@ __device__ __forceinline__ void gru_chain_fwd(const GruFwdArgs& a, int chain, in
     int cur = 0;
     for (int sg = a.chain_start[chain]; sg < a.chain_start[chain] + a.chain_len[chain]; ++sg) {
         const GruSegment S = a.seg[sg];
+        const long long poff = SEP ? (long long)(row0 / a.B) * a.agent_stride : 0;      // this pass's agent
+        const float* w_hh = S.w_hh + poff;
+        const float* b_hh = S.b_hh + poff;
         f32x2 w[3][16];                                  // (w[k], w[k+1]) pairs of this lane's slice of rows g*H + j
 #pragma unroll
         for (int g = 0; g < 3; ++g)
 #pragma unroll
             for (int i = 0; i < 8; ++i) {
-                const float4 v = __ldg(reinterpret_cast<const float4*>(S.w_hh + (long long)(g * MARL_H + j) * MARL_H + 4 * (2 * i + ks)));
+                const float4 v = __ldg(reinterpret_cast<const float4*>(w_hh + (long long)(g * MARL_H + j) * MARL_H + 4 * (2 * i + ks)));
                 w[g][2 * i] = pack2(v.x, v.y); w[g][2 * i + 1] = pack2(v.z, v.w);
             }
-        const float bh_r = __ldg(S.b_hh + j), bh_z = __ldg(S.b_hh + MARL_H + j), bh_n = __ldg(S.b_hh + 2 * MARL_H + j);
+        const float bh_r = __ldg(b_hh + j), bh_z = __ldg(b_hh + MARL_H + j), bh_n = __ldg(b_hh + 2 * MARL_H + j);
         // per-step output pointers of the rows this lane owns: advanced by one time step (N rows) per iteration
         float* hp[OWN]; float* gp_out[OWN];
 #pragma unroll
@@ -272,12 +289,25 @@ __device__ __forceinline__ void cta_rows(int rows, int chain, int& begin, int& c
     begin = pos * base + (pos < rem ? pos : rem);
 }
 
+// Separated networks (agent-major positions): one contiguous group of CTAs per agent, each agent's B rows dealt evenly over its
+// group, so that no CTA holds rows of two agents; with more agents than CTAs the plain deal (passes split by gru_pass_rows)
+__device__ __forceinline__ void cta_rows_by_agent(int B, int N, int& begin, int& count) {
+    const int per = (int)gridDim.x / N;
+    if (per == 0) { cta_rows(B * N, 0, begin, count); return; }
+    const int n = (int)blockIdx.x / per, i = (int)blockIdx.x % per;
+    if (n >= N) { begin = 0; count = 0; return; }
+    const int base = B / per, rem = B % per;
+    count = base + (i < rem ? 1 : 0);
+    begin = n * B + i * base + (i < rem ? i : rem);
+}
+
 #ifndef MARL_GRU_SPARE_SMS
 #define MARL_GRU_SPARE_SMS 16
 #endif
 constexpr int kGruFwdSpareSMs = MARL_GRU_SPARE_SMS;
 constexpr size_t gru_fwd_smem(int R) { return (size_t)(2 * R * MARL_H + kGiDepth * R * MARL_G) * sizeof(float); }
 
+template <bool SEP>
 __global__ void __launch_bounds__(kGruThreads * kGruGroups) gru_unroll_fwd_kernel(GruFwdArgs a) {
     pdl_enter();
     extern __shared__ __align__(16) float gru_smem[];
@@ -288,12 +318,12 @@ __global__ void __launch_bounds__(kGruThreads * kGruGroups) gru_unroll_fwd_kerne
     int begin = 0;
     for (int i = 0; i < (int)blockIdx.x; ++i) begin += a.rows_of[chain][i];
     const int count = a.rows_of[chain][blockIdx.x];
-    for (int off = 0; off < count; off += kGruMaxRows) {
-        const int n = min(kGruMaxRows, count - off);
-        if (n == 1) gru_chain_fwd<1>(a, chain, begin + off, n, smem, 1 + grp);
-        else if (n == 2) gru_chain_fwd<2>(a, chain, begin + off, n, smem, 1 + grp);
-        else if (n <= 4) gru_chain_fwd<4>(a, chain, begin + off, n, smem, 1 + grp);
-        else gru_chain_fwd<8>(a, chain, begin + off, n, smem, 1 + grp);
+    for (int off = 0, n = 0; off < count; off += SEP ? n : kGruMaxRows) {
+        n = gru_pass_rows<SEP>(begin + off, count - off, a.B);
+        if (n == 1) gru_chain_fwd<1, SEP>(a, chain, begin + off, n, smem, 1 + grp);
+        else if (n == 2) gru_chain_fwd<2, SEP>(a, chain, begin + off, n, smem, 1 + grp);
+        else if (n <= 4) gru_chain_fwd<4, SEP>(a, chain, begin + off, n, smem, 1 + grp);
+        else gru_chain_fwd<8, SEP>(a, chain, begin + off, n, smem, 1 + grp);
         group_sync(1 + grp);
     }
 }
@@ -311,13 +341,14 @@ struct GruBwdArgs {
     int B, L, N;
     const int* ep_len;     // [B] or null: a row's chain starts at its episode's last real step
     const int* row_order;  // [B*N] or null: logical position -> row (row_order_kernel)
+    int agent_stride;      // separated networks (SEP instantiation): floats from agent n's W_hh to n+1's
 };
 
 constexpr int kBwdSlot = 7 * MARL_H;     // r, z, n, gh_n (4H) | h_prev | dh_ext | dh_ext2   per row and time step
 constexpr int bwd_depth(int R) { return R >= 8 ? 3 : MARL_BWD_DEPTH; }
 constexpr size_t gru_bwd_smem(int R) { return (size_t)(2 * R * MARL_G + bwd_depth(R) * R * kBwdSlot) * sizeof(float); }
 
-template <int R>
+template <int R, bool SEP>
 __device__ __forceinline__ void gru_rows_bwd(const GruBwdArgs& a, int row0, int nrows, float* gru_smem) {
     constexpr int D = bwd_depth(R);
     float (*sg)[R][MARL_G] = reinterpret_cast<float (*)[R][MARL_G]>(gru_smem);                       // [2][R][3H]
@@ -325,7 +356,7 @@ __device__ __forceinline__ void gru_rows_bwd(const GruBwdArgs& a, int row0, int 
     const int tid = threadIdx.x, ks = tid & 1, j = tid >> 1;
     const int L = a.L, N = a.N;
     __shared__ int srow[kGruMaxRows];         // (the previous pass ended with a block barrier)
-    if (tid < R) srow[tid] = (a.row_order && tid < nrows) ? __ldg(a.row_order + row0 + tid) : row0 + tid;
+    if (tid < R) srow[tid] = (a.row_order && tid < nrows) ? __ldg(a.row_order + row0 + tid) : gru_position_row<SEP>(row0 + tid, a.B, N);
     __syncthreads();
     auto row_at = [&](int rr) { return srow[rr]; };
     constexpr int OWN = (R + 1) / 2;
@@ -338,13 +369,14 @@ __device__ __forceinline__ void gru_rows_bwd(const GruBwdArgs& a, int row0, int 
         dh_carry[q] = 0.0f;
     }
     // column j of W_hh, rows m = 4*(2i+ks)+c, i = 0..23:  dh_prev[j] = dh z + sum_m dgh[m] W_hh[m, j]
+    const float* w_hh = a.w_hh + (SEP ? (long long)(row0 / a.B) * a.agent_stride : 0);      // this pass's agent
     f32x2 wt[48];                                          // (rows m, m+1) pairs
 #pragma unroll
     for (int i = 0; i < 24; ++i)
 #pragma unroll
         for (int c = 0; c < 2; ++c)
-            wt[2 * i + c] = pack2(__ldg(a.w_hh + (long long)(4 * (2 * i + ks) + 2 * c) * MARL_H + j),
-                                  __ldg(a.w_hh + (long long)(4 * (2 * i + ks) + 2 * c + 1) * MARL_H + j));
+            wt[2 * i + c] = pack2(__ldg(w_hh + (long long)(4 * (2 * i + ks) + 2 * c) * MARL_H + j),
+                                  __ldg(w_hh + (long long)(4 * (2 * i + ks) + 2 * c + 1) * MARL_H + j));
     // cp.async work list: per row 112 chunks of 16 B (64 gates, 16 h_prev, 16 dh_ext, 16 dh_ext2); the
     // per-chunk source pointer at t = 0 and its per-step stride are fixed, so they are computed once.
     constexpr int NCH = (R * 112 + kGruThreads - 1) / kGruThreads;
@@ -485,17 +517,19 @@ constexpr int kGruBwdCtasPerSm = MARL_GRU_BWD_CTAS;      // 254 registers x 128 
 static int gru_bwd_ctas(int rows) { return rows <= kGruBwdCtasPerSm * kNumSMs ? rows : kNumSMs; }
 constexpr size_t gru_bwd_smem_max() { return gru_bwd_smem(8) > gru_bwd_smem(4) ? gru_bwd_smem(8) : gru_bwd_smem(4); }
 
+template <bool SEP>
 __global__ void __launch_bounds__(kGruThreads) gru_unroll_bwd_kernel(GruBwdArgs a) {
     pdl_enter();
     extern __shared__ __align__(16) float gru_smem[];
     int begin, count;
-    cta_rows(a.B * a.N, 0, begin, count);
-    for (int off = 0; off < count; off += kGruMaxRows) {
-        const int n = min(kGruMaxRows, count - off);
-        if (n == 1) gru_rows_bwd<1>(a, begin + off, n, gru_smem);
-        else if (n == 2) gru_rows_bwd<2>(a, begin + off, n, gru_smem);
-        else if (n <= 4) gru_rows_bwd<4>(a, begin + off, n, gru_smem);
-        else gru_rows_bwd<8>(a, begin + off, n, gru_smem);
+    if (SEP) cta_rows_by_agent(a.B, a.N, begin, count);
+    else cta_rows(a.B * a.N, 0, begin, count);
+    for (int off = 0, n = 0; off < count; off += SEP ? n : kGruMaxRows) {
+        n = gru_pass_rows<SEP>(begin + off, count - off, a.B);
+        if (n == 1) gru_rows_bwd<1, SEP>(a, begin + off, n, gru_smem);
+        else if (n == 2) gru_rows_bwd<2, SEP>(a, begin + off, n, gru_smem);
+        else if (n <= 4) gru_rows_bwd<4, SEP>(a, begin + off, n, gru_smem);
+        else gru_rows_bwd<8, SEP>(a, begin + off, n, gru_smem);
     }
 }
 
@@ -503,35 +537,46 @@ __global__ void __launch_bounds__(kGruThreads) gru_unroll_bwd_kernel(GruBwdArgs 
 // (steps of the chain) x (rows it advances), so rows are dealt by water-filling on that weighted load: the first
 // chain evenly, every further chain onto the CTAs that carry the least so far.  At cfg 2 (160 rows, 148 CTAs) the 12
 // CTAs with two rows of the 240-step eval chain get no row of the 120-step target chain.
-static void plan_rows(GruFwdArgs& ga, int rows, int n_ctas) {
+// Separated networks (`agents` > 1): the CTAs form one contiguous group per agent (n_ctas / agents each, the rest idle) and
+// each agent's B rows are water-filled onto its own group, so that no CTA's range -- and no pass -- holds rows of two agents.
+// (With more agents than CTAs the plain deal is kept and the kernel splits a pass at an agent boundary, gru_pass_rows.)
+static void water_fill(const double* load, int c0, int c1, int rows, double w, int* cnt) {
+    // water level by bisection: CTA i takes floor((level - load_i) / w) rows
+    double lo = 0.0, hi = 0.0;
+    for (int i = c0; i < c1; ++i) hi = load[i] > hi ? load[i] : hi;
+    hi += w * (rows / (c1 - c0) + 2);
+    for (int it = 0; it < 60; ++it) {
+        const double mid = 0.5 * (lo + hi);
+        long long tot = 0;
+        for (int i = c0; i < c1; ++i) tot += mid > load[i] ? (long long)((mid - load[i]) / w) : 0;
+        if (tot >= rows) hi = mid; else lo = mid;
+    }
+    int tot = 0;
+    for (int i = c0; i < c1; ++i) { cnt[i] = lo > load[i] ? (int)((lo - load[i]) / w) : 0; tot += cnt[i]; }
+    while (tot < rows) {                       // the remainder goes, one row each, to the least loaded CTAs
+        int best = c0;
+        for (int i = c0 + 1; i < c1; ++i)
+            if (load[i] + w * cnt[i] < load[best] + w * cnt[best]) best = i;
+        ++cnt[best]; ++tot;
+    }
+    while (tot > rows) {                       // (bisection overshoot: take back from the most loaded)
+        int worst = -1;
+        for (int i = c0; i < c1; ++i)
+            if (cnt[i] > 0 && (worst < 0 || load[i] + w * cnt[i] > load[worst] + w * cnt[worst])) worst = i;
+        --cnt[worst]; --tot;
+    }
+}
+
+static void plan_rows(GruFwdArgs& ga, int rows, int n_ctas, int agents) {
     double load[kNumSMs] = {};
+    const int per = agents > 1 ? n_ctas / agents : 0;      // CTAs per agent group (0: one group of all CTAs)
     for (int c = 0; c < ga.n_chains; ++c) {
         const double w = (double)ga.chain_len[c];
         int cnt[kNumSMs] = {};
-        // water level by bisection: CTA i takes floor((level - load_i) / w) rows
-        double lo = 0.0, hi = 0.0;
-        for (int i = 0; i < n_ctas; ++i) hi = load[i] > hi ? load[i] : hi;
-        hi += w * (rows / n_ctas + 2);
-        for (int it = 0; it < 60; ++it) {
-            const double mid = 0.5 * (lo + hi);
-            long long tot = 0;
-            for (int i = 0; i < n_ctas; ++i) tot += mid > load[i] ? (long long)((mid - load[i]) / w) : 0;
-            if (tot >= rows) hi = mid; else lo = mid;
-        }
-        int tot = 0;
-        for (int i = 0; i < n_ctas; ++i) { cnt[i] = lo > load[i] ? (int)((lo - load[i]) / w) : 0; tot += cnt[i]; }
-        while (tot < rows) {                       // the remainder goes, one row each, to the least loaded CTAs
-            int best = 0;
-            for (int i = 1; i < n_ctas; ++i)
-                if (load[i] + w * cnt[i] < load[best] + w * cnt[best]) best = i;
-            ++cnt[best]; ++tot;
-        }
-        while (tot > rows) {                       // (bisection overshoot: take back from the most loaded)
-            int worst = -1;
-            for (int i = 0; i < n_ctas; ++i)
-                if (cnt[i] > 0 && (worst < 0 || load[i] + w * cnt[i] > load[worst] + w * cnt[worst])) worst = i;
-            --cnt[worst]; --tot;
-        }
+        if (per > 0)
+            for (int g = 0; g < agents; ++g) water_fill(load, g * per, (g + 1) * per, rows / agents, w, cnt);
+        else
+            water_fill(load, 0, n_ctas, rows, w, cnt);
         for (int i = 0; i < n_ctas; ++i) { ga.rows_of[c][i] = (unsigned short)cnt[i]; load[i] += w * cnt[i]; }
     }
 }
@@ -653,6 +698,33 @@ static int check_dims(const marl_dims* d) {
     return MARL_OK;
 }
 
+// Separated networks: the rows of agent z = blockIdx.z of a launch batched over the agents, row m = b*L + t of problem z being
+// row (b, t, z): [obs | last action (one step back within the episode when shifted) if last_action | eye(N)[z] if agent_id]
+static LinOperand separated_input(const marl_dims* d, const float* obs, const float* onehot, int shift, int last_action, int agent_id) {
+    LinOperand in = plain_operand(obs, d->N * d->O, d->O, d->O);
+    if (last_action) {
+        in.x2 = onehot; in.ldx2 = d->N * d->A; in.K2 = d->A; in.x2_bs = d->A;
+        in.x2_shift = shift ? 1 : 0; in.x2_period = d->L;
+    }
+    if (agent_id) { in.onehot_mod = d->N; in.onehot_z = 1; }
+    return in;
+}
+
+// the input width of the network: O + A + N shared; O + A*last_action + N*agent_id separated
+static int agent_input_width(const marl_dims* d, int stride, int last_action, int agent_id) {
+    return stride ? d->O + (last_action ? d->A : 0) + (agent_id ? d->N : 0) : d->O + d->A + d->N;
+}
+
+// A layer of the agent: one problem over all rows (shared), or one launch batched over the agents (separated: problem z is
+// agent z's B*L rows, N rows apart, with agent z's weights `stride` floats behind agent 0's)
+static LinearFwd agent_layer(const marl_dims* d, const LinOperand& in, const float* w, int ldw, const float* b, float* y, int width, int stride) {
+    LinearFwd f{};
+    f.in = in; f.w = w; f.ldw = ldw; f.bias = b; f.y = y; f.N = width;
+    if (stride) { f.M = d->B * d->L; f.batch = d->N; f.w_bs = stride; f.b_bs = stride; f.ldy = d->N * width; f.y_bs = width; }
+    else { f.M = d->B * d->L * d->N; f.batch = 1; f.ldy = width; }
+    return f;
+}
+
 static LinOperand agent_input(const marl_dims* d, const float* obs, const float* onehot, int shift, int full) {
     if (full) return plain_operand(obs, d->O + d->A + d->N, d->O + d->A + d->N);
     LinOperand in{};
@@ -681,16 +753,25 @@ extern "C" int marl_agent_unroll_fwd(const marl_dims* d, const marl_unroll_strea
     cudaStream_t st = (cudaStream_t)stream;
     pdl_scope((long long)d->B * d->L * d->N);
     const int rows_total = d->B * d->L * d->N;
-    const int I = d->O + d->A + d->N;
+    // separated networks: one stride for the call, no full input, no W_ih^T (batch 1 only), no early exit
+    const int stride = s[0].agent_stride;
+    const bool sep = stride != 0;
     for (int i = 0; i < n_streams; ++i) {
-        if (!s[i].obs || (!s[i].onehot && !s[i].full_input) || !s[i].hidden || !s[i].x || !s[i].gi) return MARL_EINVAL;
+        const marl_unroll_stream& u = s[i];
+        if (u.agent_stride != stride || stride < 0 || (stride & 3)) return MARL_EINVAL;
+        if (sep && (u.full_input || u.w_ih_t || u.ep_len || u.padded || u.row_order || u.row_order_bwd)) return MARL_EINVAL;
+        const bool need_onehot = sep ? u.last_action != 0 : !u.full_input;
+        if (!s[i].obs || (need_onehot && !s[i].onehot) || !s[i].hidden || !s[i].x || !s[i].gi) return MARL_EINVAL;
         if (!s[i].full_input && d->O <= 0) return MARL_EINVAL;
         if (s[i].h0_from >= i) return MARL_EINVAL;
         if (s[i].h0_from >= 0 && s[s[i].h0_from].ep_len) return MARL_EINVAL;     // a continued stream must run to L (header)
     }
     // phase B: build chains (a stream whose h0_from == j continues chain of j; j must be a chain tail)
+    const int I = agent_input_width(d, stride, s[0].last_action, s[0].agent_id);
+    for (int i = 0; i < n_streams; ++i)
+        if (agent_input_width(d, stride, s[i].last_action, s[i].agent_id) != I) return MARL_EINVAL;
     GruFwdArgs ga{};
-    ga.B = d->B; ga.L = d->L; ga.N = d->N;
+    ga.B = d->B; ga.L = d->L; ga.N = d->N; ga.agent_stride = stride;
     int order[kMaxStreams], n_ordered = 0;
     bool used[kMaxStreams] = {};
     for (int i = 0; i < n_streams; ++i) {
@@ -716,12 +797,15 @@ extern "C" int marl_agent_unroll_fwd(const marl_dims* d, const marl_unroll_strea
     // A recurrence CTA takes an SM's whole register file, so nothing else runs beside it.  When leaving a few SMs out does not
     // add a row to the fullest CTA, they go to the kernels sibling streams have queued (the target hyper-network forward of
     // QMIX otherwise waits for this kernel to END, in front of the mixing kernel).
+    // Separated networks deal each agent's B rows onto its own group of n_ctas / N CTAs (plan_rows), so the fullest CTA takes
+    // ceil(B / (n_ctas / N)) rows -- at cfg 4 (N = 27, B = 32) 7 where the plain deal would give 6 but split passes at agent
+    // boundaries -- and both choices below are made on that count.
     const int rows = d->B * d->N;
+    auto fullest = [&](int n) { return (sep && n / d->N > 0) ? (d->B + n / d->N - 1) / (n / d->N) : (rows + n - 1) / n; };
     int n_ctas = rows < kNumSMs ? rows : kNumSMs;
-    if (rows > kNumSMs && (rows + kNumSMs - kGruFwdSpareSMs - 1) / (kNumSMs - kGruFwdSpareSMs) == (rows + kNumSMs - 1) / kNumSMs)
-        n_ctas = kNumSMs - kGruFwdSpareSMs;
-    if ((rows + n_ctas - 1) / n_ctas + 2 > 65535) return MARL_EINVAL;
-    plan_rows(ga, rows, n_ctas);
+    if (rows > kNumSMs && fullest(kNumSMs - kGruFwdSpareSMs) == fullest(kNumSMs)) n_ctas = kNumSMs - kGruFwdSpareSMs;
+    if (fullest(n_ctas) + 2 > 65535) return MARL_EINVAL;      // rows_of is unsigned short
+    plan_rows(ga, rows, n_ctas, sep ? d->N : 1);
     std::unique_ptr<ForkJoin> order_lane;
     {
         // length-sorted deal of the rows (row_order_kernel): a chain whose streams carry an episode-length array and a scratch
@@ -772,21 +856,18 @@ extern "C" int marl_agent_unroll_fwd(const marl_dims* d, const marl_unroll_strea
     }
     // phase A: x = relu(fc1(input)), gi = W_ih x + b_ih for every stream
     auto fc1_of = [&](int i) {
-        LinearFwd f{};
-        f.in = agent_input(d, s[i].obs, s[i].onehot, s[i].shift_onehot, s[i].full_input);
-        f.w = s[i].params.fc1_w; f.ldw = I; f.bias = s[i].params.fc1_b;
-        f.y = s[i].x; f.ldy = MARL_H; f.M = rows_total; f.N = MARL_H; f.relu = 1; f.batch = 1;
+        const LinOperand in = sep ? separated_input(d, s[i].obs, s[i].onehot, s[i].shift_onehot, s[i].last_action, s[i].agent_id)
+                                  : agent_input(d, s[i].obs, s[i].onehot, s[i].shift_onehot, s[i].full_input);
+        LinearFwd f = agent_layer(d, in, s[i].params.fc1_w, I, s[i].params.fc1_b, s[i].x, MARL_H, stride);
+        f.relu = 1;
         return f;
     };
     auto ih_of = [&](int i) {
-        LinearFwd g{};
-        g.in = plain_operand(s[i].x, MARL_H, MARL_H);
-        g.w = s[i].params.w_ih; g.ldw = MARL_H; g.bias = s[i].params.b_ih;
-        g.y = s[i].gi; g.ldy = MARL_G; g.M = rows_total; g.N = MARL_G; g.batch = 1;
-        return g;
+        const LinOperand in = sep ? plain_operand(s[i].x, d->N * MARL_H, MARL_H, MARL_H) : plain_operand(s[i].x, MARL_H, MARL_H);
+        return agent_layer(d, in, s[i].params.w_ih, MARL_H, s[i].params.b_ih, s[i].gi, MARL_G, stride);
     };
     bool grouped = false;
-    {
+    if (!sep) {      // (the fused input-layer kernel stages one shared weight set: separated streams take the unfused path)
         // fused path (csrc/front.cu): both layers of every stream in ONE persistent launch, x handed from the first GEMM to the
         // second through tensor memory
         FrontArgs fa{};
@@ -812,7 +893,7 @@ extern "C" int marl_agent_unroll_fwd(const marl_dims* d, const marl_unroll_strea
                 if (rc) return rc;
             }
     }
-    if (!grouped && tgemm_enabled()) {
+    if (!grouped && !sep && tgemm_enabled()) {
         // TMA path: the streams of one layer are ONE grouped launch of persistent CTAs (csrc/tgemm.cu): 2 launches
         // instead of 2 x n_streams on forked streams
         TGBuilder b1, b2;
@@ -847,11 +928,16 @@ extern "C" int marl_agent_unroll_fwd(const marl_dims* d, const marl_unroll_strea
         ProfScope ps_("gru_unroll_fwd_kernel", st);
         const size_t sm = kGruGroups * gru_fwd_smem(kGruMaxRows);
         static bool attr_set = false;
-        if (!attr_set) { cudaFuncSetAttribute(gru_unroll_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm); attr_set = true; }
+        if (!attr_set) {
+            cudaFuncSetAttribute(gru_unroll_fwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+            cudaFuncSetAttribute(gru_unroll_fwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+            attr_set = true;
+        }
         ga.trace = trace_buffer();
         if (order_lane) order_lane->join();
         dim3 grid(n_ctas, (ga.n_chains + kGruGroups - 1) / kGruGroups);
-        launch_pdl_prio(kGruPrio, gru_unroll_fwd_kernel, grid, dim3(kGruThreads * kGruGroups), sm, st, ga);
+        launch_pdl_prio(kGruPrio, sep ? gru_unroll_fwd_kernel<true> : gru_unroll_fwd_kernel<false>, grid,
+                        dim3(kGruThreads * kGruGroups), sm, st, ga);
     }
     MARL_LAUNCH_CHECK();
     // phase C.  (The fork / join pair stays even when a fused mixer evaluates the heads and nothing is launched here: it takes the
@@ -861,11 +947,8 @@ extern "C" int marl_agent_unroll_fwd(const marl_dims* d, const marl_unroll_strea
     for (int i = 0; i < n_streams; ++i) {
         if (!s[i].q) continue;
         cudaStream_t st = fc.lane(i);
-        LinearFwd f{};
-        f.in = plain_operand(s[i].hidden, MARL_H, MARL_H);
-        f.w = s[i].params.fc2_w; f.ldw = MARL_H; f.bias = s[i].params.fc2_b;
-        f.y = s[i].q; f.ldy = d->A; f.M = rows_total; f.N = d->A; f.batch = 1;
-        int rc = linear_fwd(f, st);
+        const LinOperand in = sep ? plain_operand(s[i].hidden, d->N * MARL_H, MARL_H, MARL_H) : plain_operand(s[i].hidden, MARL_H, MARL_H);
+        int rc = linear_fwd(agent_layer(d, in, s[i].params.fc2_w, MARL_H, s[i].params.fc2_b, s[i].q, d->A, stride), st);
         if (rc) return rc;
     }
     fc.join();
@@ -876,25 +959,37 @@ extern "C" int marl_agent_unroll_bwd(const marl_dims* d, const marl_unroll_bwd* 
     if (check_dims(d) || !a || !a->hidden || !a->x || !a->gates || !a->dgi || !a->dgh || !a->dx) return MARL_EINVAL;
     if (a->dq && !a->dhext) return MARL_EINVAL;
     if (!a->full_input && d->O <= 0) return MARL_EINVAL;
+    const int stride = a->agent_stride;
+    const bool sep = stride != 0;
+    if (stride < 0 || (stride & 3)) return MARL_EINVAL;
+    if (sep && (a->full_input || a->w_ih_t || a->ep_len || a->row_order || (a->last_action && !a->onehot))) return MARL_EINVAL;
     cudaStream_t st = (cudaStream_t)stream;
     pdl_scope((long long)d->B * d->L * d->N);
     const int rows_total = d->B * d->L * d->N;
-    const int I = d->O + d->A + d->N;
+    const int I = agent_input_width(d, stride, a->last_action, a->agent_id);
+    // separated networks: every layer is one launch batched over the agents -- problem z holds agent z's B*L rows, which sit
+    // N rows apart (row pitch x N, column offset z x width), and its weights / gradients `stride` floats behind agent 0's
+    const int nb = sep ? d->N : 1, M = sep ? d->B * d->L : rows_total, rp = sep ? d->N : 1;
+    auto zs = [&](int width) -> long long { return sep ? width : 0; };
     int rc;
     if (a->dq && !a->dhext_ready) {
         // q = W2 h + b2:  dh_ext = dq . W2 ;  dW2 += dq^T h ; db2 += colsum(dq)
         LinearDgrad g{};
-        g.dy = a->dq; g.lddy = d->A; g.w = a->params.fc2_w; g.ldw = MARL_H; g.w_col0 = 0;
-        g.dx = a->dhext; g.lddx = MARL_H; g.M = rows_total; g.N = d->A; g.K = MARL_H; g.batch = 1;
+        g.dy = a->dq; g.lddy = rp * d->A; g.dy_bs = zs(d->A); g.w = a->params.fc2_w; g.ldw = MARL_H; g.w_bs = stride; g.w_col0 = 0;
+        g.dx = a->dhext; g.lddx = rp * MARL_H; g.dx_bs = zs(MARL_H); g.M = M; g.N = d->A; g.K = MARL_H; g.batch = nb;
         if ((rc = linear_dgrad(g, st))) return rc;
     }
     GruBwdArgs ga{a->gates, a->hidden, a->dq ? a->dhext : nullptr, a->dhidden, a->params.w_hh, a->h0, a->dgi, a->dgh, a->dh0,
-                  d->B, d->L, d->N, a->ep_len, (a->ep_len && d->B <= kMaxOrderEpisodes) ? a->row_order : nullptr};
+                  d->B, d->L, d->N, a->ep_len, (a->ep_len && d->B <= kMaxOrderEpisodes) ? a->row_order : nullptr, stride};
     const int rows = d->B * d->N;
     {
         ProfScope ps_("gru_unroll_bwd_kernel", st);
         static bool attr_set = false;
-        if (!attr_set) { cudaFuncSetAttribute(gru_unroll_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gru_bwd_smem_max()); attr_set = true; }
+        if (!attr_set) {
+            cudaFuncSetAttribute(gru_unroll_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gru_bwd_smem_max());
+            cudaFuncSetAttribute(gru_unroll_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gru_bwd_smem_max());
+            attr_set = true;
+        }
         const bool keep_ = pdl_small_problem();
         // measured: launched programmatically the 148 recurrence CTAs come up while the producer still runs and the
         // step gets 10-27 us slower on every config; a plain launch here, PDL for its consumers
@@ -902,41 +997,56 @@ extern "C" int marl_agent_unroll_bwd(const marl_dims* d, const marl_unroll_bwd* 
         // up to two rows per SM: one CTA per row -- two co-resident one-row CTAs overlap each other's latency, where one CTA with two
         // rows serialises 2 x 96 packed FMAs per thread on the dependent chain (the 12 two-row CTAs of config 2 ended the kernel)
         const int n_ctas = gru_bwd_ctas(rows);
-        launch_pdl_prio(kGruPrio, gru_unroll_bwd_kernel, dim3(n_ctas), dim3(kGruThreads), gru_bwd_smem_max(), st, ga);
+        launch_pdl_prio(kGruPrio, sep ? gru_unroll_bwd_kernel<true> : gru_unroll_bwd_kernel<false>, dim3(n_ctas), dim3(kGruThreads),
+                        gru_bwd_smem_max(), st, ga);
         pdl_small_problem() = keep_;
     }
     MARL_LAUNCH_CHECK();
     LinearWgrad w_fc2{}, w_hh{}, w_ih{}, w_fc1{}, w_h0{};
     LinearDgrad g_dx{};
     // dW2 += dq^T h ; db2 += colsum(dq)
-    w_fc2.dy = a->dq; w_fc2.lddy = d->A; w_fc2.in = plain_operand(a->hidden, MARL_H, MARL_H);
-    w_fc2.dw = a->grads.fc2_w; w_fc2.ldw = MARL_H; w_fc2.db = a->grads.fc2_b; w_fc2.M = rows_total; w_fc2.N = d->A; w_fc2.batch = 1;
+    w_fc2.dy = a->dq; w_fc2.lddy = rp * d->A; w_fc2.dy_bs = zs(d->A); w_fc2.in = plain_operand(a->hidden, rp * MARL_H, MARL_H, zs(MARL_H));
+    w_fc2.dw = a->grads.fc2_w; w_fc2.ldw = MARL_H; w_fc2.db = a->grads.fc2_b; w_fc2.M = M; w_fc2.N = d->A; w_fc2.batch = nb;
+    w_fc2.dw_bs = stride; w_fc2.db_bs = stride;
     // dW_hh += dgh^T . h_{t-1} (hidden shifted by one step, zeros at t = 0) ; db_hh
-    w_hh.dy = a->dgh; w_hh.lddy = MARL_G;
+    w_hh.dy = a->dgh; w_hh.lddy = rp * MARL_G; w_hh.dy_bs = zs(MARL_G);
     {
         LinOperand in{};
-        in.x = nullptr; in.K1 = 0; in.x2 = a->hidden; in.ldx2 = MARL_H; in.K2 = MARL_H;
-        in.x2_shift = d->N; in.x2_period = d->L * d->N; in.onehot_mod = 0;
+        in.x = nullptr; in.K1 = 0; in.x2 = a->hidden; in.ldx2 = rp * MARL_H; in.K2 = MARL_H; in.x2_bs = zs(MARL_H);
+        in.x2_shift = sep ? 1 : d->N; in.x2_period = sep ? d->L : d->L * d->N; in.onehot_mod = 0;
         w_hh.in = in;
     }
-    w_hh.dw = a->grads.w_hh; w_hh.ldw = MARL_H; w_hh.db = a->grads.b_hh; w_hh.M = rows_total; w_hh.N = MARL_G; w_hh.batch = 1;
-    // the t = 0 rows see h0 instead of zeros: one [N x H] problem per episode
-    w_h0.dy = a->dgh; w_h0.lddy = MARL_G; w_h0.dy_bs = (long long)d->L * d->N * MARL_G;
-    w_h0.in = plain_operand(a->h0, MARL_H, MARL_H, (long long)d->N * MARL_H);
-    w_h0.dw = a->grads.w_hh; w_h0.ldw = MARL_H; w_h0.db = nullptr; w_h0.M = d->N; w_h0.N = MARL_G; w_h0.batch = d->B;
+    w_hh.dw = a->grads.w_hh; w_hh.ldw = MARL_H; w_hh.db = a->grads.b_hh; w_hh.M = M; w_hh.N = MARL_G; w_hh.batch = nb;
+    w_hh.dw_bs = stride; w_hh.db_bs = stride;
+    // the t = 0 rows see h0 instead of zeros: one [N x H] problem per episode (separated: one [B x H] problem per agent)
+    w_h0.dw = a->grads.w_hh; w_h0.ldw = MARL_H; w_h0.db = nullptr; w_h0.N = MARL_G;
+    if (sep) {
+        w_h0.dy = a->dgh; w_h0.lddy = d->L * d->N * MARL_G; w_h0.dy_bs = MARL_G;
+        w_h0.in = plain_operand(a->h0, d->N * MARL_H, MARL_H, MARL_H);
+        w_h0.M = d->B; w_h0.batch = d->N; w_h0.dw_bs = stride;
+    } else {
+        w_h0.dy = a->dgh; w_h0.lddy = MARL_G; w_h0.dy_bs = (long long)d->L * d->N * MARL_G;
+        w_h0.in = plain_operand(a->h0, MARL_H, MARL_H, (long long)d->N * MARL_H);
+        w_h0.M = d->N; w_h0.batch = d->B;
+    }
     // dW_ih += dgi^T . x ; db_ih
-    w_ih.dy = a->dgi; w_ih.lddy = MARL_G; w_ih.in = plain_operand(a->x, MARL_H, MARL_H);
-    w_ih.dw = a->grads.w_ih; w_ih.ldw = MARL_H; w_ih.db = a->grads.b_ih; w_ih.M = rows_total; w_ih.N = MARL_G; w_ih.batch = 1;
+    w_ih.dy = a->dgi; w_ih.lddy = rp * MARL_G; w_ih.dy_bs = zs(MARL_G); w_ih.in = plain_operand(a->x, rp * MARL_H, MARL_H, zs(MARL_H));
+    w_ih.dw = a->grads.w_ih; w_ih.ldw = MARL_H; w_ih.db = a->grads.b_ih; w_ih.M = M; w_ih.N = MARL_G; w_ih.batch = nb;
+    w_ih.dw_bs = stride; w_ih.db_bs = stride;
     // dx = (dgi . W_ih) * (x > 0)
-    g_dx.dy = a->dgi; g_dx.lddy = MARL_G; g_dx.w = a->params.w_ih; g_dx.ldw = MARL_H; g_dx.w_col0 = 0;
-    g_dx.dx = a->dx; g_dx.lddx = MARL_H; g_dx.relu_src = a->x; g_dx.ldrs = MARL_H;
-    g_dx.M = rows_total; g_dx.N = MARL_G; g_dx.K = MARL_H; g_dx.batch = 1;
+    g_dx.dy = a->dgi; g_dx.lddy = rp * MARL_G; g_dx.dy_bs = zs(MARL_G); g_dx.w = a->params.w_ih; g_dx.ldw = MARL_H; g_dx.w_bs = stride;
+    g_dx.w_col0 = 0;
+    g_dx.dx = a->dx; g_dx.lddx = rp * MARL_H; g_dx.dx_bs = zs(MARL_H); g_dx.relu_src = a->x; g_dx.ldrs = rp * MARL_H; g_dx.rs_bs = zs(MARL_H);
+    g_dx.M = M; g_dx.N = MARL_G; g_dx.K = MARL_H; g_dx.batch = nb;
     g_dx.wt = a->w_ih_t; g_dx.ldwt = MARL_G;      // W_ih transposed by this step's forward pass (both operands then stage with 128-bit stores)
     // dW1 += dx^T . [obs | last_action | agent_id] ; db1
-    w_fc1.dy = a->dx; w_fc1.lddy = MARL_H; w_fc1.in = agent_input(d, a->obs, a->onehot, a->shift_onehot, a->full_input);
-    w_fc1.dw = a->grads.fc1_w; w_fc1.ldw = I; w_fc1.db = a->grads.fc1_b; w_fc1.M = rows_total; w_fc1.N = MARL_H; w_fc1.batch = 1;
+    w_fc1.dy = a->dx; w_fc1.lddy = rp * MARL_H; w_fc1.dy_bs = zs(MARL_H);
+    w_fc1.in = sep ? separated_input(d, a->obs, a->onehot, a->shift_onehot, a->last_action, a->agent_id)
+                   : agent_input(d, a->obs, a->onehot, a->shift_onehot, a->full_input);
+    w_fc1.dw = a->grads.fc1_w; w_fc1.ldw = I; w_fc1.db = a->grads.fc1_b; w_fc1.M = M; w_fc1.N = MARL_H; w_fc1.batch = nb;
+    w_fc1.dw_bs = stride; w_fc1.db_bs = stride;
 
-    if (tgemm_enabled()) {
+    if (!sep && tgemm_enabled()) {
         // TMA path (csrc/tgemm.cu): the data gradient and the three weight gradients that only need the BPTT's outputs are
         // ONE grouped launch, the fc1 weight gradient (needs dx) a second, and one deterministic reduce folds every
         // split partial into the flat gradient

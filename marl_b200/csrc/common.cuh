@@ -98,7 +98,9 @@ __device__ __forceinline__ float sigmoidf_acc(float x) { return 1.0f / (1.0f + e
 //       one-hot(m % onehot_mod) (onehot_mod cols) ]
 // which is how the agent input [obs | last_action | agent_id] (share_params.py:84-112) and the
 // QTRAN [hidden | action] / [state | encoding] concatenations are consumed without ever being
-// materialised.
+// materialised.  With onehot_z the one-hot column is the batched problem's index z instead: a
+// launch over z = agent whose problem z holds the rows of agent z only (SeparatedMAC's input,
+// share_params.py:467-495).
 // ------------------------------------------------------------------------------------------
 struct LinOperand {
     const float* x;   int ldx;  int K1;
@@ -107,6 +109,7 @@ struct LinOperand {
     int x2_period;
     int onehot_mod;   // 0 = none
     long long x_bs, x2_bs;   // blockIdx.z strides (batched problems)
+    int onehot_z;     // 1: the hot column is z (k == z) rather than m % onehot_mod
 };
 
 __device__ __forceinline__ float lin_load(const LinOperand& a, int z, int m, int k) {
@@ -121,7 +124,7 @@ __device__ __forceinline__ float lin_load(const LinOperand& a, int z, int m, int
         return __ldg(a.x2 + (long long)z * a.x2_bs + (long long)mm * a.ldx2 + k);
     }
     k -= a.K2;
-    return (m % a.onehot_mod) == k ? 1.0f : 0.0f;
+    return (a.onehot_z ? z : m % a.onehot_mod) == k ? 1.0f : 0.0f;
 }
 
 __host__ __device__ __forceinline__ int lin_width(const LinOperand& a) { return a.K1 + a.K2 + a.onehot_mod; }

@@ -56,7 +56,7 @@ int linear_wgrad(const LinearWgrad& a, cudaStream_t st);
 inline LinOperand plain_operand(const float* x, int ldx, int K, long long bs = 0) {
     LinOperand o{};
     o.x = x; o.ldx = ldx; o.K1 = K; o.x_bs = bs;
-    o.x2 = nullptr; o.ldx2 = 0; o.K2 = 0; o.x2_shift = 0; o.x2_period = 1; o.onehot_mod = 0; o.x2_bs = 0;
+    o.x2 = nullptr; o.ldx2 = 0; o.K2 = 0; o.x2_shift = 0; o.x2_period = 1; o.onehot_mod = 0; o.x2_bs = 0; o.onehot_z = 0;
     return o;
 }
 

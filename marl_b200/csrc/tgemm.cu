@@ -662,7 +662,7 @@ bool TGBuilder::add_fwd(const LinearFwd& a) {
     if (!tgemm_enabled() || g_.n >= TG_MAXP || a.batch != 1 || a.M <= 0 || a.N <= 0) return false;
     const LinOperand& in = a.in;
     const bool plain = in.K2 == 0 && in.onehot_mod == 0;
-    const bool agent = in.K1 > 0 && in.K2 > 0 && in.onehot_mod > 0 && in.x_bs == 0 && in.x2_bs == 0 && in.ldx2 == in.K2;
+    const bool agent = in.K1 > 0 && in.K2 > 0 && in.onehot_mod > 0 && !in.onehot_z && in.x_bs == 0 && in.x2_bs == 0 && in.ldx2 == in.K2;
     if (!plain && !agent) return false;
     const int K = lin_width(in);
     if (K > 768 || !al16(a.w) || (a.ldw & 3)) return false;
@@ -741,7 +741,7 @@ bool TGBuilder::add_wgrad(const LinearWgrad& a) {
     const LinOperand& in = a.in;
     const bool plain = in.K1 > 0 && in.K2 == 0 && in.onehot_mod == 0;
     const bool shifted = in.K1 == 0 && in.K2 > 0 && in.onehot_mod == 0 && in.x2_bs == 0;               // h_{t-1}
-    const bool agent = in.K1 > 0 && in.K2 > 0 && in.onehot_mod > 0 && in.x_bs == 0 && in.x2_bs == 0 && in.ldx2 == in.K2;
+    const bool agent = in.K1 > 0 && in.K2 > 0 && in.onehot_mod > 0 && !in.onehot_z && in.x_bs == 0 && in.x2_bs == 0 && in.ldx2 == in.K2;
     if (!plain && !shifted && !agent) return false;
     const int K_in = lin_width(in);
     const int Md = K_in + (a.db ? 1 : 0);

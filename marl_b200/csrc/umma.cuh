@@ -19,7 +19,7 @@ struct OpLin {
         if (o.x) rw.xr = o.x + (long long)z * o.x_bs + (long long)i * o.ldx;
         if (o.K2 > 0 && !(o.x2_shift && (i % o.x2_period) < o.x2_shift))
             rw.x2r = o.x2 + (long long)z * o.x2_bs + (long long)(i - o.x2_shift) * o.ldx2 - o.K1;
-        if (o.onehot_mod) rw.hot = o.K1 + o.K2 + (i % o.onehot_mod);
+        if (o.onehot_mod) rw.hot = o.K1 + o.K2 + (o.onehot_z ? z : i % o.onehot_mod);
         return rw;
     }
     __device__ __forceinline__ float4 quad_at(const Row& rw, int r) const {   // elements (row, r..r+3)
@@ -55,7 +55,7 @@ struct OpLin {
         const float* xr = o.x ? o.x + (long long)z * o.x_bs + (long long)i * o.ldx : nullptr;
         const bool x2_live = o.K2 > 0 && !(o.x2_shift && (i % o.x2_period) < o.x2_shift);
         const float* x2r = x2_live ? o.x2 + (long long)z * o.x2_bs + (long long)(i - o.x2_shift) * o.ldx2 - o.K1 : nullptr;
-        const int hot = o.onehot_mod ? o.K1 + o.K2 + (i % o.onehot_mod) : -1;
+        const int hot = o.onehot_mod ? o.K1 + o.K2 + (o.onehot_z ? z : i % o.onehot_mod) : -1;
         float e[4];
 #pragma unroll
         for (int c = 0; c < 4; ++c) {
