@@ -83,7 +83,7 @@ int marl_replay_gather_f32(const marl_episode_f32* ring, int T_ring, const long 
 
 /* ---- agent: network/q_network.py:6-21 unrolled by controller/share_params.py:125-168 ---- */
 typedef struct marl_agent_params {
-    const float* fc1_w;  /* [H, O+A+N] */  const float* fc1_b;  /* [H] */
+    const float* fc1_w;  /* [H, O+A+N], or as the input blocks select */  const float* fc1_b;  /* [H] */
     const float* w_ih;   /* [3H, H]   */  const float* w_hh;   /* [3H, H] */
     const float* b_ih;   /* [3H]      */  const float* b_hh;   /* [3H] */
     const float* fc2_w;  /* [A, H]    */  const float* fc2_b;  /* [A] */
@@ -141,8 +141,14 @@ typedef struct marl_unroll_stream {
                                 [obs | onehot[b,t-shift,n] if last_action | eye(N)[n] if agent_id] (share_params.py:467-506),
                                 so fc1_w is [H, O + A*last_action + N*agent_id].  MARL_EINVAL together with full_input, w_ih_t,
                                 ep_len, padded, row_order or row_order_bwd */
-    int last_action;         /* separated only (ignored when agent_stride == 0): the input carries the last action */
-    int agent_id;            /* separated only: the input carries the agent's one-hot id */
+    int last_action;         /* separated, or shared with input_flags = 1 (ignored otherwise): the input carries the last action */
+    int agent_id;            /* separated, or shared with input_flags = 1: the input carries the agent's one-hot id */
+    int input_flags;         /* agent_stride == 0 only.  1: last_action / agent_id select the input blocks as for separated
+                                networks, [obs | onehot[b,t-shift,n] if last_action | eye(N)[n] if agent_id], so fc1_w is
+                                [H, O + A*last_action + N*agent_id] (share_params.py:84-123 with args.last_action /
+                                args.reuse_network); onehot may be NULL when last_action is 0.  0: the default
+                                [obs | last action | agent id] whatever last_action / agent_id hold.  MARL_EINVAL together
+                                with full_input; every stream of a call has the same input width */
 } marl_unroll_stream;
 
 /* ep_len[b] = 1 + the last step with padded[b, t] == 0 (at least 1): every step at or beyond it has mask = 0 in the loss
@@ -176,8 +182,9 @@ typedef struct marl_unroll_bwd {
     int agent_stride;        /* as marl_unroll_stream.agent_stride: 0 shared, else one network per agent with `params` and
                                 `grads` at agent 0's set and agent n+1's agent_stride floats behind agent n's.  MARL_EINVAL
                                 together with full_input, w_ih_t, ep_len or row_order */
-    int last_action;         /* separated only: as marl_unroll_stream.last_action */
-    int agent_id;            /* separated only: as marl_unroll_stream.agent_id */
+    int last_action;         /* as marl_unroll_stream.last_action */
+    int agent_id;            /* as marl_unroll_stream.agent_id */
+    int input_flags;         /* agent_stride == 0 only: as marl_unroll_stream.input_flags (the forward's value) */
 } marl_unroll_bwd;
 
 int marl_agent_unroll_bwd(const marl_dims* d, const marl_unroll_bwd* a, void* stream);
@@ -218,6 +225,19 @@ int marl_agent_act(int n_envs, int N, int A, int O, const marl_agent_params* p, 
                    const unsigned char* explore, const long long* random_action, const double* explore_u,
                    const double* choice_u, double eps, const int* gate, long long* action, float* onehot, float* q,
                    void* stream);
+
+/* marl_agent_act with the input blocks chosen by last_action / agent_id (share_params.py:84-123 with args.last_action /
+ * args.reuse_network):
+ *   in = [obs[r] (O) | last_onehot[r] (A, only if last_action) | eye(N)[n] (N, only if agent_id)]
+ * so p->fc1_w is [64, O + A*last_action + N*agent_id].  Every other argument, the row layout, the exploration forms, gate
+ * and the outputs are those of marl_agent_act, which is this call with last_action = agent_id = 1; last_onehot may be NULL
+ * when last_action is 0.  MARL_EINVAL when last_action is set and last_onehot is NULL, and in every case marl_agent_act
+ * returns it. */
+int marl_agent_act_input(int n_envs, int N, int A, int O, int last_action, int agent_id, const marl_agent_params* p,
+                         const float* obs, const float* last_onehot, const float* avail, const float* h_in, float* h_out,
+                         const unsigned char* explore, const long long* random_action, const double* explore_u,
+                         const double* choice_u, double eps, const int* gate, long long* action, float* onehot, float* q,
+                         void* stream);
 
 /* marl_agent_act with one network per agent (SeparatedMAC, share_params.py:389-610): row r = e*N + n uses p[n], an
  * array of N parameter sets, and its input is

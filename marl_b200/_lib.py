@@ -50,7 +50,7 @@ class UnrollStream(C.Structure):
                 ("params", AgentParams), ("q", c_ptr), ("hidden", c_ptr), ("h_last", c_ptr), ("x", c_ptr),
                 ("gi", c_ptr), ("gates", c_ptr), ("w_ih_t", c_ptr), ("ep_len", c_ptr), ("padded", c_ptr),
                 ("row_order", c_ptr), ("row_order_bwd", c_ptr), ("agent_stride", C.c_int), ("last_action", C.c_int),
-                ("agent_id", C.c_int)]
+                ("agent_id", C.c_int), ("input_flags", C.c_int)]
 
 
 class UnrollBwd(C.Structure):
@@ -58,7 +58,7 @@ class UnrollBwd(C.Structure):
                 ("params", AgentParams), ("hidden", c_ptr), ("x", c_ptr), ("gates", c_ptr), ("h0", c_ptr), ("dq", c_ptr),
                 ("dhidden", c_ptr), ("dhext", c_ptr), ("dgi", c_ptr), ("dgh", c_ptr), ("dx", c_ptr), ("dh0", c_ptr),
                 ("grads", AgentGrads), ("dhext_ready", C.c_int), ("w_ih_t", c_ptr), ("ep_len", c_ptr), ("row_order", c_ptr),
-                ("agent_stride", C.c_int), ("last_action", C.c_int), ("agent_id", C.c_int)]
+                ("agent_stride", C.c_int), ("last_action", C.c_int), ("agent_id", C.c_int), ("input_flags", C.c_int)]
 
 
 class PeerGroup(C.Structure):
@@ -169,6 +169,7 @@ _SIGNATURES = {
     "marl_qtran_losses_fwd_bwd": ([_P(Dims)] + [c_ptr] * 12 + [C.c_float] * 3 + [c_ptr] * 5 + [c_ptr], C.c_int),
     "marl_epsgreedy_select": ([C.c_int, C.c_int] + [c_ptr] * 6 + [c_ptr], C.c_int),
     "marl_agent_act": ([C.c_int] * 4 + [_P(AgentParams)] + [c_ptr] * 9 + [C.c_double] + [c_ptr] * 5, C.c_int),
+    "marl_agent_act_input": ([C.c_int] * 6 + [_P(AgentParams)] + [c_ptr] * 9 + [C.c_double] + [c_ptr] * 5, C.c_int),
     "marl_agent_act_separated": ([C.c_int] * 6 + [_P(AgentParams)] + [c_ptr] * 9 + [C.c_double] + [c_ptr] * 5, C.c_int),
     "marl_rollout_record": ([_P(Dims), C.c_int, _P(EpisodeF32)] + [c_ptr] * 12 + [c_ptr], C.c_int),
     "marl_select_fits": ([C.c_int] * 4, C.c_int),

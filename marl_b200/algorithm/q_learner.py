@@ -515,7 +515,7 @@ class QLearner:
             s.x, s.gi = ws["x"][i].data_ptr(), ws["gi"][i].data_ptr()
             s.gates = ws["gates"].data_ptr() if u.keep else None
             s.w_ih_t = ws["w_ih_t"].data_ptr() if u.keep and not sep else None    # W_ih^T for the backward's data gradient
-            s.agent_stride, s.last_action, s.agent_id = stride, last_action, agent_id
+            s.agent_stride, s.last_action, s.agent_id, s.input_flags = stride, last_action, agent_id, int(not sep)
         L.call("marl_agent_unroll_fwd", C.byref(d), arr, len(plan), L.stream_ptr())
         # + episode lengths and row orders, launched by marl_agent_unroll_fwd beside the input layers
         return (3 if heads else 2) * len(plan) + 1 + (2 if early else 0)
@@ -527,6 +527,7 @@ class QLearner:
         bw.obs, bw.onehot, bw.shift_onehot, bw.full_input = bt["o"].data_ptr(), bt["u_onehot"].data_ptr(), 1, 0
         bw.params, bw.agent_stride = self._agent_structs(self._flat)
         bw.last_action, bw.agent_id = int(self.args.last_action), int(self.args.reuse_network)
+        bw.input_flags = int(not self._separated)          # the shared network's input follows the same two switches
         bw.hidden, bw.x, bw.gates = ws["hidden"][0].data_ptr(), ws["x"][0].data_ptr(), ws["gates"].data_ptr()
         bw.h0, bw.dq, bw.dhidden = None, ws["dq"].data_ptr(), dhidden
         bw.dhext, bw.dgi, bw.dgh, bw.dx = (ws[k].data_ptr() for k in ("dhext", "dgi", "dgh", "dx"))

@@ -5,7 +5,8 @@ Same surface as the reference's ``SharedMAC`` (``init_hidden``, ``get_current_q_
 ``load_models``, ``cuda``) and the same stateful ``hidden_states`` semantics -- the hidden
 state is carried between successive ``get_*_q_values`` calls until ``init_hidden`` -- but each
 T-step unroll is ONE call into libmarl_b200 instead of a Python loop over timesteps, and the
-input rows [obs | last_action | agent_id] (share_params.py:84-112) are never materialised.
+input rows [obs | last_action | agent_id] (share_params.py:84-112; the last two blocks as args.last_action /
+args.reuse_network select them) are never materialised.
 """
 from __future__ import annotations
 
@@ -24,6 +25,24 @@ def _as_f32_cuda(x, device):
     if not th.is_tensor(x):
         x = th.as_tensor(x)
     return x.to(device=device, dtype=th.float32, non_blocking=True).contiguous()
+
+
+def _input_shape(args):
+    """Width of the agent's input [obs | last action if args.last_action | agent id if args.reuse_network]
+    (share_params.py:114-123 and :497-506)."""
+    return args.obs_shape + (args.n_actions if args.last_action else 0) + (args.n_agents if args.reuse_network else 0)
+
+
+def _agent_row(args, obs, last_action, agent_num):
+    """The reference's host-side input row of one agent for choose_action (share_params.py:40-48 and :421-429)."""
+    inputs = np.asarray(obs, dtype=np.float64).copy()
+    agent_id = np.zeros(args.n_agents)
+    agent_id[agent_num] = 1.
+    if args.last_action:
+        inputs = np.hstack((inputs, last_action))
+    if args.reuse_network:
+        inputs = np.hstack((inputs, agent_id))
+    return inputs
 
 
 def _choose_actions(mac, obs, last_action, avail_actions, epsilon, evaluate, draws):
@@ -70,14 +89,15 @@ class SharedMAC:
         self.state_shape = args.state_shape
         self.obs_shape = args.obs_shape
         self.args = args
-        if not (args.last_action and args.reuse_network):
-            raise NotImplementedError("libmarl_b200 implements the default last_action=True, reuse_network=True input")
         self._build_agents(self._get_input_shape())
         self.hidden_states = None   # (n_episodes, n_agents, hidden_dim)
 
     # ---- construction -----------------------------------------------------------------------------
-    def _get_input_shape(self):
-        return self.obs_shape + self.n_actions + self.n_agents    # share_params.py:114-123
+    def _get_input_shape(self):                   # share_params.py:114-123
+        return _input_shape(self.args)
+
+    def _blocks(self):
+        return dict(last_action=bool(self.args.last_action), agent_id=bool(self.args.reuse_network))
 
     def _build_agents(self, input_shape):
         self.agent = RNNQNet(input_shape, self.args)
@@ -111,20 +131,20 @@ class SharedMAC:
         if dev.type != "cuda":
             raise L.MarlLibraryError("SharedMAC needs a CUDA device: marl_b200 has no CPU path")
         obs = _as_f32_cuda(obs, dev)[:, :max_episode_len].contiguous()
-        onehot = _as_f32_cuda(onehot, dev)[:, :max_episode_len].contiguous()
+        onehot = _as_f32_cuda(onehot, dev)[:, :max_episode_len].contiguous() if self.args.last_action else None
         h0 = self.hidden_states.reshape(-1, self.args.rnn_hidden_dim).to(dev).contiguous()
-        q, hidden, h_last = self.agent.unroll(obs, onehot, h0, shift)
+        q, hidden, h_last = self.agent.unroll(obs, onehot, h0, shift, **self._blocks())
         self.hidden_states = h_last            # [B*N, H], as left behind by the reference's loop
         return q, hidden
 
     def get_current_q_values(self, batch, max_episode_len):
         """Q-values of every transition's current observation (share_params.py:125-146):
-        step t consumes [o_t | u_onehot_{t-1} (zeros at t=0) | agent id]."""
+        step t consumes [o_t | u_onehot_{t-1} (zeros at t=0) if last_action | agent id if reuse_network]."""
         return self._unroll(batch["o"], batch["u_onehot"], max_episode_len, shift=1)
 
     def get_next_q_values(self, batch, max_episode_len):
         """Q-values of every transition's next observation (share_params.py:148-168):
-        step t consumes [o_next_t | u_onehot_t | agent id]."""
+        step t consumes [o_next_t | u_onehot_t if last_action | agent id if reuse_network]."""
         return self._unroll(batch["o_next"], batch["u_onehot"], max_episode_len, shift=0)
 
     def forward(self, ep_batch, t):
@@ -138,9 +158,9 @@ class SharedMAC:
         # step t needs u_onehot[t-1]: feed it unshifted alongside o_t
         dev = self.device
         obs = _as_f32_cuda(ep_batch["o"], dev)[:, t:t + 1].contiguous()
-        oh = _as_f32_cuda(ep_batch["u_onehot"], dev)[:, t - 1:t].contiguous()
+        oh = _as_f32_cuda(ep_batch["u_onehot"], dev)[:, t - 1:t].contiguous() if self.args.last_action else None
         h0 = self.hidden_states.reshape(-1, self.args.rnn_hidden_dim).to(dev).contiguous()
-        q, _, h_last = self.agent.unroll(obs, oh, h0, 0)
+        q, _, h_last = self.agent.unroll(obs, oh, h0, 0, **self._blocks())
         self.hidden_states = h_last
         return q[:, 0]
 
@@ -148,11 +168,8 @@ class SharedMAC:
     def choose_action(self, obs, last_action, agent_num, avail_actions, epsilon, evaluate=False):
         """Epsilon-greedy action of ONE agent (share_params.py:37-72); RNG order: one
         np.random.uniform(), then np.random.choice only when exploring."""
-        inputs = np.asarray(obs, dtype=np.float64).copy()
+        inputs = _agent_row(self.args, obs, last_action, agent_num)
         avail_actions_ind = np.nonzero(avail_actions)[0]
-        agent_id = np.zeros(self.n_agents)
-        agent_id[agent_num] = 1.
-        inputs = np.hstack((inputs, last_action, agent_id))
         dev = self.device
         hidden_state = self.hidden_states[:, agent_num, :]
         inputs = th.tensor(inputs, dtype=th.float32).unsqueeze(0).to(dev)
@@ -168,10 +185,11 @@ class SharedMAC:
         return action
 
     def choose_actions(self, obs, last_action, avail_actions, epsilon, evaluate=False, draws=None):
-        """Epsilon-greedy actions of every agent of every instance in ONE ``marl_agent_act`` launch: the batched
+        """Epsilon-greedy actions of every agent of every instance in ONE ``marl_agent_act_input`` launch: the batched
         counterpart of ``choose_action``.
 
-        obs [n, N, O], last_action [n, N, A], avail_actions [n, N, A] or None (all available); numpy arrays or tensors.
+        obs [n, N, O], last_action [n, N, A] (may be None when ``args.last_action`` is False), avail_actions [n, N, A] or
+        None (all available); numpy arrays or tensors.
         Agent a of instance e explores iff explore_u[e, a] < epsilon and then takes the
         min(floor(choice_u[e, a] * cnt), cnt - 1)-th of its cnt available actions (action 0 when it has none);
         ``draws=(explore_u, choice_u)`` ([n, N] uniforms in [0, 1)) supplies them, None draws them on the device from
@@ -181,13 +199,14 @@ class SharedMAC:
 
     def act(self, n, obs, last, avail, hidden, explore=None, random_action=None, explore_u=None, choice_u=None, eps=0.0,
             gate=None, actions=None, onehot=None, q=None):
-        """One ``marl_agent_act`` launch over n instances: contiguous device tensors, ``hidden`` [n * N, H] advanced in
-        place (include/marl_b200.h documents every argument).  Returns ``actions`` [n, N] int64."""
+        """One ``marl_agent_act_input`` launch over n instances: contiguous device tensors, ``hidden`` [n * N, H] advanced
+        in place, ``last`` may be None without a last-action input (include/marl_b200.h documents every argument).
+        Returns ``actions`` [n, N] int64."""
         if actions is None:
             actions = th.empty(n, self.n_agents, dtype=th.int64, device=self.device)
         p = agent_param_struct(self.agent.param_addresses())
-        L.call("marl_agent_act", n, self.n_agents, self.n_actions, self.obs_shape, C.byref(p), obs.data_ptr(),
-               last.data_ptr(), L.ptr(avail), hidden.data_ptr(), hidden.data_ptr(), L.ptr(explore), L.ptr(random_action),
+        L.call("marl_agent_act_input", n, self.n_agents, self.n_actions, self.obs_shape, int(self.args.last_action),
+               int(self.args.reuse_network), C.byref(p), obs.data_ptr(), L.ptr(last), L.ptr(avail), hidden.data_ptr(), hidden.data_ptr(), L.ptr(explore), L.ptr(random_action),
                L.ptr(explore_u), L.ptr(choice_u), float(eps), L.ptr(gate), actions.data_ptr(), L.ptr(onehot), L.ptr(q),
                L.stream_ptr())
         return actions
@@ -220,12 +239,7 @@ class SeparatedMAC:
         self.hidden_states = None
 
     def _get_input_shape(self):                   # share_params.py:497-506
-        input_shape = self.obs_shape
-        if self.args.last_action:
-            input_shape += self.n_actions
-        if self.args.reuse_network:
-            input_shape += self.n_agents
-        return input_shape
+        return _input_shape(self.args)
 
     def _build_agents(self, input_shape):
         self.agent = [RNNQNet(input_shape, self.args) for _ in range(self.n_agents)]
@@ -300,14 +314,8 @@ class SeparatedMAC:
 
     def choose_action(self, obs, last_action, agent_num, avail_actions, epsilon, evaluate=False):
         """share_params.py:419-453 with the agent's own network; same RNG order as SharedMAC.choose_action."""
-        inputs = np.asarray(obs, dtype=np.float64).copy()
+        inputs = _agent_row(self.args, obs, last_action, agent_num)
         avail_actions_ind = np.nonzero(avail_actions)[0]
-        agent_id = np.zeros(self.n_agents)
-        agent_id[agent_num] = 1.
-        if self.args.last_action:
-            inputs = np.hstack((inputs, last_action))
-        if self.args.reuse_network:
-            inputs = np.hstack((inputs, agent_id))
         dev = self.device
         hidden_state = self.hidden_states[:, agent_num, :]
         inputs = th.tensor(inputs, dtype=th.float32).unsqueeze(0).to(dev)

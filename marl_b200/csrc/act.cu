@@ -41,7 +41,7 @@ inline ActLayout act_layout(int I, int A) {
 
 struct ActArgs {
     int rows, n_envs, N, A, O;
-    int last_action, agent_id;                              // input blocks present (the shared agent has both)
+    int last_action, agent_id;                              // input blocks present (marl_agent_act: both)
     const float* obs; const float* last; const float* avail;
     const float* h_in; float* h_out;                       // may alias
     const unsigned char* explore; const long long* random_action;
@@ -349,20 +349,31 @@ static bool params_complete(const marl_agent_params& p) {
     return p.fc1_w && p.fc1_b && p.w_ih && p.w_hh && p.b_ih && p.b_hh && p.fc2_w && p.fc2_b;
 }
 
-extern "C" int marl_agent_act(int n_envs, int N, int A, int O, const marl_agent_params* p, const float* obs,
-                              const float* last_onehot, const float* avail, const float* h_in, float* h_out,
-                              const unsigned char* explore, const long long* random_action, const double* explore_u,
-                              const double* choice_u, double eps, const int* gate, long long* action, float* onehot,
-                              float* q, void* stream) {
-    if (n_envs < 0 || N <= 0 || A <= 0 || O < 0 || !p || !obs || !last_onehot || !h_in || !h_out || !action) return MARL_EINVAL;
+extern "C" int marl_agent_act_input(int n_envs, int N, int A, int O, int last_action, int agent_id,
+                                    const marl_agent_params* p, const float* obs, const float* last_onehot,
+                                    const float* avail, const float* h_in, float* h_out, const unsigned char* explore,
+                                    const long long* random_action, const double* explore_u, const double* choice_u,
+                                    double eps, const int* gate, long long* action, float* onehot, float* q, void* stream) {
+    if (n_envs < 0 || N <= 0 || A <= 0 || O < 0 || !p || !obs || !h_in || !h_out || !action) return MARL_EINVAL;
+    if (last_action && !last_onehot) return MARL_EINVAL;
     if (!params_complete(*p)) return MARL_EINVAL;
     if (!explore != !random_action || !explore_u != !choice_u || (explore && explore_u)) return MARL_EINVAL;
     const long long rows = (long long)n_envs * N;
     if (rows > 0x7fffffffLL) return MARL_EINVAL;
     const ActParams<1> ps{{*p}};
-    const ActArgs a{(int)rows, n_envs, N, A, O, 1, 1, obs, last_onehot, avail, h_in, h_out, explore, random_action, explore_u,
-                    choice_u, eps, gate, action, onehot, q};
-    return act_launch("agent_act_kernel", ps, a, O + A + N, (rows + kActRows - 1) / kActRows, stream);
+    const ActArgs a{(int)rows, n_envs, N, A, O, last_action ? 1 : 0, agent_id ? 1 : 0, obs, last_onehot, avail, h_in, h_out,
+                    explore, random_action, explore_u, choice_u, eps, gate, action, onehot, q};
+    const int I = O + (last_action ? A : 0) + (agent_id ? N : 0);
+    return act_launch("agent_act_kernel", ps, a, I, (rows + kActRows - 1) / kActRows, stream);
+}
+
+extern "C" int marl_agent_act(int n_envs, int N, int A, int O, const marl_agent_params* p, const float* obs,
+                              const float* last_onehot, const float* avail, const float* h_in, float* h_out,
+                              const unsigned char* explore, const long long* random_action, const double* explore_u,
+                              const double* choice_u, double eps, const int* gate, long long* action, float* onehot,
+                              float* q, void* stream) {
+    return marl_agent_act_input(n_envs, N, A, O, 1, 1, p, obs, last_onehot, avail, h_in, h_out, explore, random_action,
+                                explore_u, choice_u, eps, gate, action, onehot, q, stream);
 }
 
 extern "C" int marl_agent_act_separated(int n_envs, int N, int A, int O, int last_action, int agent_id,

@@ -710,9 +710,17 @@ static LinOperand separated_input(const marl_dims* d, const float* obs, const fl
     return in;
 }
 
-// the input width of the network: O + A + N shared; O + A*last_action + N*agent_id separated
-static int agent_input_width(const marl_dims* d, int stride, int last_action, int agent_id) {
-    return stride ? d->O + (last_action ? d->A : 0) + (agent_id ? d->N : 0) : d->O + d->A + d->N;
+// The input blocks a stream reads: separated networks and shared streams that opt in (input_flags) select them with
+// last_action / agent_id; any other shared stream reads all three, whatever those fields hold
+struct InputBlocks { int last_action, agent_id; };
+static InputBlocks input_blocks(int stride, int input_flags, int last_action, int agent_id) {
+    if (stride || input_flags) return InputBlocks{last_action ? 1 : 0, agent_id ? 1 : 0};
+    return InputBlocks{1, 1};
+}
+
+// the input width of the network: O + A*last_action + N*agent_id (a full input row is as wide as the composed one)
+static int agent_input_width(const marl_dims* d, InputBlocks f) {
+    return d->O + (f.last_action ? d->A : 0) + (f.agent_id ? d->N : 0);
 }
 
 // A layer of the agent: one problem over all rows (shared), or one launch batched over the agents (separated: problem z is
@@ -725,14 +733,17 @@ static LinearFwd agent_layer(const marl_dims* d, const LinOperand& in, const flo
     return f;
 }
 
-static LinOperand agent_input(const marl_dims* d, const float* obs, const float* onehot, int shift, int full) {
+// Shared network: row m = (b*L + t)*N + n is [obs | last action (N rows back when shifted) if present | eye(N)[n] if present]
+static LinOperand agent_input(const marl_dims* d, const float* obs, const float* onehot, int shift, int full, InputBlocks f) {
     if (full) return plain_operand(obs, d->O + d->A + d->N, d->O + d->A + d->N);
     LinOperand in{};
     in.x = obs; in.ldx = d->O; in.K1 = d->O; in.x_bs = 0;
-    in.x2 = onehot; in.ldx2 = d->A; in.K2 = d->A; in.x2_bs = 0;
-    in.x2_shift = shift ? d->N : 0;
-    in.x2_period = d->L * d->N;
-    in.onehot_mod = d->N;
+    if (f.last_action) {
+        in.x2 = onehot; in.ldx2 = d->A; in.K2 = d->A; in.x2_bs = 0;
+        in.x2_shift = shift ? d->N : 0;
+        in.x2_period = d->L * d->N;
+    }
+    in.onehot_mod = f.agent_id ? d->N : 0;
     return in;
 }
 
@@ -756,20 +767,22 @@ extern "C" int marl_agent_unroll_fwd(const marl_dims* d, const marl_unroll_strea
     // separated networks: one stride for the call, no full input, no W_ih^T (batch 1 only), no early exit
     const int stride = s[0].agent_stride;
     const bool sep = stride != 0;
+    auto blocks = [&](int i) { return input_blocks(stride, s[i].input_flags, s[i].last_action, s[i].agent_id); };
     for (int i = 0; i < n_streams; ++i) {
         const marl_unroll_stream& u = s[i];
         if (u.agent_stride != stride || stride < 0 || (stride & 3)) return MARL_EINVAL;
         if (sep && (u.full_input || u.w_ih_t || u.ep_len || u.padded || u.row_order || u.row_order_bwd)) return MARL_EINVAL;
-        const bool need_onehot = sep ? u.last_action != 0 : !u.full_input;
+        if (!sep && u.input_flags && u.full_input) return MARL_EINVAL;
+        const bool need_onehot = !u.full_input && blocks(i).last_action;
         if (!s[i].obs || (need_onehot && !s[i].onehot) || !s[i].hidden || !s[i].x || !s[i].gi) return MARL_EINVAL;
         if (!s[i].full_input && d->O <= 0) return MARL_EINVAL;
         if (s[i].h0_from >= i) return MARL_EINVAL;
         if (s[i].h0_from >= 0 && s[s[i].h0_from].ep_len) return MARL_EINVAL;     // a continued stream must run to L (header)
     }
     // phase B: build chains (a stream whose h0_from == j continues chain of j; j must be a chain tail)
-    const int I = agent_input_width(d, stride, s[0].last_action, s[0].agent_id);
+    const int I = agent_input_width(d, blocks(0));
     for (int i = 0; i < n_streams; ++i)
-        if (agent_input_width(d, stride, s[i].last_action, s[i].agent_id) != I) return MARL_EINVAL;
+        if (agent_input_width(d, blocks(i)) != I) return MARL_EINVAL;
     GruFwdArgs ga{};
     ga.B = d->B; ga.L = d->L; ga.N = d->N; ga.agent_stride = stride;
     int order[kMaxStreams], n_ordered = 0;
@@ -857,7 +870,7 @@ extern "C" int marl_agent_unroll_fwd(const marl_dims* d, const marl_unroll_strea
     // phase A: x = relu(fc1(input)), gi = W_ih x + b_ih for every stream
     auto fc1_of = [&](int i) {
         const LinOperand in = sep ? separated_input(d, s[i].obs, s[i].onehot, s[i].shift_onehot, s[i].last_action, s[i].agent_id)
-                                  : agent_input(d, s[i].obs, s[i].onehot, s[i].shift_onehot, s[i].full_input);
+                                  : agent_input(d, s[i].obs, s[i].onehot, s[i].shift_onehot, s[i].full_input, blocks(i));
         LinearFwd f = agent_layer(d, in, s[i].params.fc1_w, I, s[i].params.fc1_b, s[i].x, MARL_H, stride);
         f.relu = 1;
         return f;
@@ -873,7 +886,7 @@ extern "C" int marl_agent_unroll_fwd(const marl_dims* d, const marl_unroll_strea
         FrontArgs fa{};
         fa.rows = rows_total; fa.I = I;
         for (int i = 0; i < n_streams; ++i) {
-            fa.s[i].in = agent_input(d, s[i].obs, s[i].onehot, s[i].shift_onehot, s[i].full_input);
+            fa.s[i].in = agent_input(d, s[i].obs, s[i].onehot, s[i].shift_onehot, s[i].full_input, blocks(i));
             fa.s[i].x = s[i].x; fa.s[i].gi = s[i].gi;
             fa.s[i].store_x = s[i].gates != nullptr;
             fa.set[i].w1 = s[i].params.fc1_w; fa.set[i].b1 = s[i].params.fc1_b;
@@ -962,11 +975,14 @@ extern "C" int marl_agent_unroll_bwd(const marl_dims* d, const marl_unroll_bwd* 
     const int stride = a->agent_stride;
     const bool sep = stride != 0;
     if (stride < 0 || (stride & 3)) return MARL_EINVAL;
-    if (sep && (a->full_input || a->w_ih_t || a->ep_len || a->row_order || (a->last_action && !a->onehot))) return MARL_EINVAL;
+    if (sep && (a->full_input || a->w_ih_t || a->ep_len || a->row_order)) return MARL_EINVAL;
+    if (!sep && a->input_flags && a->full_input) return MARL_EINVAL;
+    const InputBlocks blk = input_blocks(stride, a->input_flags, a->last_action, a->agent_id);
+    if (!a->full_input && blk.last_action && !a->onehot) return MARL_EINVAL;
     cudaStream_t st = (cudaStream_t)stream;
     pdl_scope((long long)d->B * d->L * d->N);
     const int rows_total = d->B * d->L * d->N;
-    const int I = agent_input_width(d, stride, a->last_action, a->agent_id);
+    const int I = agent_input_width(d, blk);
     // separated networks: every layer is one launch batched over the agents -- problem z holds agent z's B*L rows, which sit
     // N rows apart (row pitch x N, column offset z x width), and its weights / gradients `stride` floats behind agent 0's
     const int nb = sep ? d->N : 1, M = sep ? d->B * d->L : rows_total, rp = sep ? d->N : 1;
@@ -1042,7 +1058,7 @@ extern "C" int marl_agent_unroll_bwd(const marl_dims* d, const marl_unroll_bwd* 
     // dW1 += dx^T . [obs | last_action | agent_id] ; db1
     w_fc1.dy = a->dx; w_fc1.lddy = rp * MARL_H; w_fc1.dy_bs = zs(MARL_H);
     w_fc1.in = sep ? separated_input(d, a->obs, a->onehot, a->shift_onehot, a->last_action, a->agent_id)
-                   : agent_input(d, a->obs, a->onehot, a->shift_onehot, a->full_input);
+                   : agent_input(d, a->obs, a->onehot, a->shift_onehot, a->full_input, blk);
     w_fc1.dw = a->grads.fc1_w; w_fc1.ldw = I; w_fc1.db = a->grads.fc1_b; w_fc1.M = M; w_fc1.N = MARL_H; w_fc1.batch = nb;
     w_fc1.dw_bs = stride; w_fc1.db_bs = stride;
 

@@ -32,10 +32,11 @@ def agent_param_struct(named, cls=L.AgentParams):
 
 class _UnrollFn(torch.autograd.Function):
     """Differentiable T-step unroll (used by the drop-in module surface; the fused learner
-    calls the same C entry points directly and bypasses autograd)."""
+    calls the same C entry points directly and bypasses autograd).  `blocks`: None for the default [obs | last action |
+    agent id] input (or a full input), else the (last_action, agent_id) input blocks (marl_unroll_stream.input_flags)."""
 
     @staticmethod
-    def forward(ctx, obs, onehot, h0, shift, full_input, dims, *params):
+    def forward(ctx, obs, onehot, h0, shift, full_input, dims, blocks, *params):
         B, Lq, N, A, O = dims
         dev = obs.device
         rows = B * Lq * N
@@ -56,16 +57,18 @@ class _UnrollFn(torch.autograd.Function):
         st.q, st.hidden, st.h_last = q.data_ptr(), hidden.data_ptr(), h_last.data_ptr()
         st.x, st.gi, st.gates = x.data_ptr(), gi.data_ptr(), gates.data_ptr()
         st.w_ih_t = w_ih_t.data_ptr()
+        if blocks is not None:
+            st.input_flags, st.last_action, st.agent_id = 1, int(blocks[0]), int(blocks[1])
         L.call("marl_agent_unroll_fwd", C.byref(d), C.byref(st), 1, L.stream_ptr())
         ctx.save_for_backward(obs, onehot if onehot is not None else obs, h0 if h0 is not None else obs,
                               hidden, x, gates, w_ih_t, *params)
-        ctx.meta = (dims, int(shift), int(full_input), onehot is None, h0 is not None)
+        ctx.meta = (dims, int(shift), int(full_input), onehot is None, h0 is not None, blocks)
         ctx.mark_non_differentiable(h_last)
         return q, hidden, h_last
 
     @staticmethod
     def backward(ctx, dq, dhidden, _dh_last):
-        dims, shift, full_input, no_onehot, had_h0 = ctx.meta
+        dims, shift, full_input, no_onehot, had_h0, blocks = ctx.meta
         obs, onehot, h0, hidden, x, gates, w_ih_t, *params = ctx.saved_tensors
         B, Lq, N, A, O = dims
         dev = obs.device
@@ -78,6 +81,8 @@ class _UnrollFn(torch.autograd.Function):
         a.params = agent_param_struct({n: p.data_ptr() for n, p in zip(AGENT_FLAT_ORDER, params)})
         a.hidden, a.x, a.gates = hidden.data_ptr(), x.data_ptr(), gates.data_ptr()
         a.w_ih_t = w_ih_t.data_ptr()
+        if blocks is not None:
+            a.input_flags, a.last_action, a.agent_id = 1, int(blocks[0]), int(blocks[1])
         dq = None if dq is None else dq.contiguous()
         dhidden = None if dhidden is None else dhidden.contiguous()
         a.dq, a.dhidden = L.ptr(dq), L.ptr(dhidden)
@@ -88,7 +93,7 @@ class _UnrollFn(torch.autograd.Function):
         a.grads = agent_param_struct({n: g.data_ptr() for n, g in zip(AGENT_FLAT_ORDER, gflat)}, L.AgentGrads)
         d = L.Dims(B, Lq, N, A, O, 0)
         L.call("marl_agent_unroll_bwd", C.byref(d), C.byref(a), L.stream_ptr())
-        return (None, None, dh0, None, None, None, *gflat)
+        return (None, None, dh0, None, None, None, None, *gflat)
 
 
 class RNNQNet(FlatPackedMixin, nn.Module):
@@ -134,7 +139,7 @@ class RNNQNet(FlatPackedMixin, nn.Module):
         A = self.args.n_actions
         dims = (R, 1, 1, A, self.input_shape - A - 1)
         params = [p for _, p in self.flat_named_parameters()]
-        q, hidden, _ = _UnrollFn.apply(obs, None, h_in, 0, 1, dims, *params)
+        q, hidden, _ = _UnrollFn.apply(obs, None, h_in, 0, 1, dims, None, *params)
         return q.view(R, A), hidden.view(R, H)
 
     def unroll_full(self, x, h0):
@@ -143,11 +148,12 @@ class RNNQNet(FlatPackedMixin, nn.Module):
         A = self.args.n_actions
         dims = (B, T, 1, A, I - A - 1)                 # only O + A + N = input_shape matters for a full input
         params = [p for _, p in self.flat_named_parameters()]
-        return _UnrollFn.apply(x, None, h0, 0, 1, dims, *params)
+        return _UnrollFn.apply(x, None, h0, 0, 1, dims, None, *params)
 
-    def unroll(self, obs, onehot, h0, shift):
-        """[B,T,N,O], [B,T,N,A] -> q [B,T,N,A], hidden [B,T,N,H], h_last [B*N,H]."""
+    def unroll(self, obs, onehot, h0, shift, last_action=True, agent_id=True):
+        """[B,T,N,O], [B,T,N,A] -> q [B,T,N,A], hidden [B,T,N,H], h_last [B*N,H].  The input row is
+        [obs | onehot (if last_action) | eye(N)[n] (if agent_id)]; onehot may be None without last_action."""
         B, T, N, O = obs.shape
         dims = (B, T, N, self.args.n_actions, O)
         params = [p for _, p in self.flat_named_parameters()]
-        return _UnrollFn.apply(obs, onehot, h0, int(shift), 0, dims, *params)
+        return _UnrollFn.apply(obs, onehot, h0, int(shift), 0, dims, (bool(last_action), bool(agent_id)), *params)

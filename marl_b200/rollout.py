@@ -93,7 +93,7 @@ class BatchedRolloutWorker:
             rand_d = th.randint(0, A, (n, N), device=dev, dtype=th.int64)
         # the worker's view of the game at the only step: obs = get_obs() (zeros), no last action, fresh hidden state
         obs = th.zeros(n, N, self.obs_shape, device=dev)
-        last = th.zeros(n, N, A, device=dev)
+        last = th.zeros(n, N, A, device=dev) if self.args.last_action else None
         hidden = th.zeros(n * N, self.args.rnn_hidden_dim, device=dev)
         actions = self.mac.act(n, obs, last, None, hidden, explore=explore_d, random_action=rand_d)
         self.mac.hidden_states = hidden                                                 # [n*N, H], as an unroll leaves it
