@@ -253,6 +253,41 @@ int marl_agent_act_separated(int n_envs, int N, int A, int O, int last_action, i
                              const double* explore_u, const double* choice_u, double eps, const int* gate,
                              long long* action, float* onehot, float* q, void* stream);
 
+/* Philox exploration form: every row draws its own pair from a counter-based generator inside the act launch, so the
+ * draws are a pure function of (seed, episode, step, agent) -- the same whichever call or device plays the episode -- and
+ * no draw buffer exists.  Philox4x64-10 (Random123's constants and rounds, numpy's np.random.Philox) under key
+ * (seed, 0); row r = e*N + n at step `step` uses counter (episode_base + e, step, n, 0) (word 0 wraps modulo 2^64).
+ * explore_u = (word0 >> 11) * 2^-53 and choice_u = (word1 >> 11) * 2^-53 (numpy's Generator.random() conversion), then
+ * the uniform form's rule: explore iff explore_u < eps (float64), where eps is eps_table[min(e, eps_len - 1)] when
+ * eps_table (device float64) is set and the call's eps otherwise. */
+typedef struct {
+    unsigned long long seed;          /* Philox key word 0 (word 1 = 0) */
+    unsigned long long episode_base;  /* counter word 0 of row e*N + n is episode_base + e */
+    int step;                         /* counter word 1 (>= 0) */
+    const double* eps_table;          /* nullable: instance e explores with eps_table[min(e, eps_len - 1)]; else eps */
+    int eps_len;
+} marl_act_philox;
+
+/* marl_agent_act_input with the exploration drawn as marl_act_philox describes (no flag or uniform arrays).  MARL_EINVAL
+ * when philox is NULL, philox->step < 0, eps_table is set with eps_len < 1, and in every case marl_agent_act_input
+ * returns it. */
+int marl_agent_act_philox(int n_envs, int N, int A, int O, int last_action, int agent_id, const marl_agent_params* p,
+                          const float* obs, const float* last_onehot, const float* avail, const float* h_in, float* h_out,
+                          const marl_act_philox* philox, double eps, const int* gate, long long* action, float* onehot,
+                          float* q, void* stream);
+
+/* marl_agent_act_separated with the exploration drawn as marl_act_philox describes; MARL_EINVAL as
+ * marl_agent_act_philox and marl_agent_act_separated return it. */
+int marl_agent_act_separated_philox(int n_envs, int N, int A, int O, int last_action, int agent_id,
+                                    const marl_agent_params* p, const float* obs, const float* last_onehot,
+                                    const float* avail, const float* h_in, float* h_out, const marl_act_philox* philox,
+                                    double eps, const int* gate, long long* action, float* onehot, float* q, void* stream);
+
+/* The pairs marl_agent_act_philox draws, for testing the generator bit for bit: out[r] = (explore_u, choice_u) of row
+ * r = e*N + n, [n_envs * N, 2] float64 on the device. */
+int marl_philox_uniforms(unsigned long long seed, unsigned long long episode_base, int step, int n_envs, int N,
+                         double* out, void* stream);
+
 /* Bookkeeping of the batched multi-step rollout (rollout.py:52-149), one launch per environment step.
  * d: B = n instances, L = T (episode_limit), N, A, O, S; ep: the [n, T, ...] episode buffers (padding pre-filled by the
  * caller: zeros, padded = terminated = 1).  Phase t (1 <= t <= T), for every instance e that was active in step t-1:

@@ -61,6 +61,11 @@ class UnrollBwd(C.Structure):
                 ("agent_stride", C.c_int), ("last_action", C.c_int), ("agent_id", C.c_int), ("input_flags", C.c_int)]
 
 
+class ActPhilox(C.Structure):      # include/marl_b200.h: marl_act_philox
+    _fields_ = [("seed", C.c_ulonglong), ("episode_base", C.c_ulonglong), ("step", C.c_int), ("eps_table", c_ptr),
+                ("eps_len", C.c_int)]
+
+
 class PeerGroup(C.Structure):
     _fields_ = [("world", C.c_int), ("rank", C.c_int), ("grads", c_ptr * 8), ("flags", c_ptr * 8), ("epoch", c_ptr),
                 ("error", c_ptr)]
@@ -171,6 +176,11 @@ _SIGNATURES = {
     "marl_agent_act": ([C.c_int] * 4 + [_P(AgentParams)] + [c_ptr] * 9 + [C.c_double] + [c_ptr] * 5, C.c_int),
     "marl_agent_act_input": ([C.c_int] * 6 + [_P(AgentParams)] + [c_ptr] * 9 + [C.c_double] + [c_ptr] * 5, C.c_int),
     "marl_agent_act_separated": ([C.c_int] * 6 + [_P(AgentParams)] + [c_ptr] * 9 + [C.c_double] + [c_ptr] * 5, C.c_int),
+    "marl_agent_act_philox": ([C.c_int] * 6 + [_P(AgentParams)] + [c_ptr] * 5 + [_P(ActPhilox), C.c_double] + [c_ptr] * 5,
+                              C.c_int),
+    "marl_agent_act_separated_philox": ([C.c_int] * 6 + [_P(AgentParams)] + [c_ptr] * 5 + [_P(ActPhilox), C.c_double]
+                                        + [c_ptr] * 5, C.c_int),
+    "marl_philox_uniforms": ([C.c_ulonglong, C.c_ulonglong, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr], C.c_int),
     "marl_rollout_record": ([_P(Dims), C.c_int, _P(EpisodeF32)] + [c_ptr] * 12 + [c_ptr], C.c_int),
     "marl_select_fits": ([C.c_int] * 4, C.c_int),
     "marl_episode_lengths": ([c_ptr, C.c_int, C.c_int, c_ptr, c_ptr], C.c_int),

@@ -11,6 +11,7 @@ args.reuse_network select them) are never materialised.
 from __future__ import annotations
 
 import ctypes as C
+from typing import NamedTuple
 
 import numpy as np
 import torch as th
@@ -25,6 +26,44 @@ def _as_f32_cuda(x, device):
     if not th.is_tensor(x):
         x = th.as_tensor(x)
     return x.to(device=device, dtype=th.float32, non_blocking=True).contiguous()
+
+
+class PhiloxDraws(NamedTuple):
+    """Exploration drawn inside the act launch from Philox4x64-10 (include/marl_b200.h, marl_act_philox): agent n of
+    instance e draws from key (seed, 0) and counter (episode_base + e, step, n, 0), so the draws depend on nothing but
+    these numbers -- not on torch's or numpy's generator, nor on how the instances are split between calls or devices."""
+    seed: int
+    episode_base: int = 0
+    step: int = 0
+
+
+def _philox_struct(philox, eps_table):
+    """The marl_act_philox descriptor of a PhiloxDraws and an optional device float64 epsilon table."""
+    seed, base, step = (int(x) for x in philox)
+    if not (0 <= seed < 1 << 64 and 0 <= base < 1 << 64 and 0 <= step < 1 << 31):
+        raise ValueError(f"PhiloxDraws out of range: {philox}")
+    if eps_table is not None and (eps_table.dtype != th.float64 or not eps_table.is_contiguous() or eps_table.dim() != 1):
+        raise ValueError("eps_table must be a contiguous 1-D float64 device tensor")
+    return L.ActPhilox(seed, base, step, L.ptr(eps_table), 0 if eps_table is None else eps_table.numel())
+
+
+def _act(mac, fn, fn_philox, p, n, obs, last, avail, hidden, explore, random_action, explore_u, choice_u, eps, gate,
+         actions, onehot, q, philox, eps_table):
+    """The library call behind SharedMAC.act / SeparatedMAC.act: fn, or fn_philox when philox is given."""
+    if actions is None:
+        actions = th.empty(n, mac.n_agents, dtype=th.int64, device=mac.device)
+    head = (n, mac.n_agents, mac.n_actions, mac.obs_shape, int(mac.args.last_action), int(mac.args.reuse_network), p,
+            obs.data_ptr(), L.ptr(last), L.ptr(avail), hidden.data_ptr(), hidden.data_ptr())
+    tail = (float(eps), L.ptr(gate), actions.data_ptr(), L.ptr(onehot), L.ptr(q), L.stream_ptr())
+    if philox is None:
+        if eps_table is not None:
+            raise ValueError("eps_table belongs to the Philox form: pass philox= as well")
+        L.call(fn, *head, L.ptr(explore), L.ptr(random_action), L.ptr(explore_u), L.ptr(choice_u), *tail)
+    else:
+        if any(x is not None for x in (explore, random_action, explore_u, choice_u)):
+            raise ValueError("philox= replaces explore / random_action / explore_u / choice_u")
+        L.call(fn_philox, *head, C.byref(_philox_struct(philox, eps_table)), *tail)
+    return actions
 
 
 def _input_shape(args):
@@ -66,15 +105,17 @@ def _choose_actions(mac, obs, last_action, avail_actions, epsilon, evaluate, dra
     if h is None or h.numel() != n * N * H:
         raise ValueError(f"hidden_states must hold {n} x {N} rows: call init_hidden({n}) first")
     work = h if (h.is_cuda and h.dtype == th.float32 and h.is_contiguous()) else h.to(dev, th.float32).contiguous()
-    explore_u = choice_u = None
+    explore_u = choice_u = philox = None
     if not evaluate:
-        if draws is None:
+        if isinstance(draws, PhiloxDraws):
+            philox = draws
+        elif draws is None:
             explore_u = th.rand(n, N, dtype=th.float64, device=dev)
             choice_u = th.rand(n, N, dtype=th.float64, device=dev)
         else:
             explore_u, choice_u = (th.as_tensor(d, dtype=th.float64).to(dev).reshape(n, N).contiguous() for d in draws)
     with th.no_grad():
-        actions = mac.act(n, obs, last, avail, work, explore_u=explore_u, choice_u=choice_u, eps=float(epsilon))
+        actions = mac.act(n, obs, last, avail, work, explore_u=explore_u, choice_u=choice_u, eps=float(epsilon), philox=philox)
         if work is not h:
             h.copy_(work.view_as(h))
     return actions
@@ -193,23 +234,21 @@ class SharedMAC:
         Agent a of instance e explores iff explore_u[e, a] < epsilon and then takes the
         min(floor(choice_u[e, a] * cnt), cnt - 1)-th of its cnt available actions (action 0 when it has none);
         ``draws=(explore_u, choice_u)`` ([n, N] uniforms in [0, 1)) supplies them, None draws them on the device from
-        torch's generator.  ``evaluate=True`` is greedy.  Advances ``self.hidden_states`` (n * N rows, e.g. after
+        torch's generator, and ``draws=PhiloxDraws(seed, episode_base, step)`` has the act launch draw them itself from
+        Philox (instance e is episode episode_base + e; no draw buffer).  ``evaluate=True`` is greedy.  Advances ``self.hidden_states`` (n * N rows, e.g. after
         ``init_hidden(n)``) in place and keeps its shape.  Returns the int64 CUDA actions [n, N]; nothing waits for the GPU."""
         return _choose_actions(self, obs, last_action, avail_actions, epsilon, evaluate, draws)
 
     def act(self, n, obs, last, avail, hidden, explore=None, random_action=None, explore_u=None, choice_u=None, eps=0.0,
-            gate=None, actions=None, onehot=None, q=None):
+            gate=None, actions=None, onehot=None, q=None, philox=None, eps_table=None):
         """One ``marl_agent_act_input`` launch over n instances: contiguous device tensors, ``hidden`` [n * N, H] advanced
         in place, ``last`` may be None without a last-action input (include/marl_b200.h documents every argument).
-        Returns ``actions`` [n, N] int64."""
-        if actions is None:
-            actions = th.empty(n, self.n_agents, dtype=th.int64, device=self.device)
-        p = agent_param_struct(self.agent.param_addresses())
-        L.call("marl_agent_act_input", n, self.n_agents, self.n_actions, self.obs_shape, int(self.args.last_action),
-               int(self.args.reuse_network), C.byref(p), obs.data_ptr(), L.ptr(last), L.ptr(avail), hidden.data_ptr(), hidden.data_ptr(), L.ptr(explore), L.ptr(random_action),
-               L.ptr(explore_u), L.ptr(choice_u), float(eps), L.ptr(gate), actions.data_ptr(), L.ptr(onehot), L.ptr(q),
-               L.stream_ptr())
-        return actions
+        ``philox=PhiloxDraws(...)`` selects the Philox exploration form (``marl_agent_act_philox``) in place of the four
+        exploration arrays, with ``eps_table`` (optional contiguous float64 device tensor) giving instance e the
+        epsilon ``eps_table[min(e, len - 1)]`` instead of ``eps``.  Returns ``actions`` [n, N] int64."""
+        p = C.byref(agent_param_struct(self.agent.param_addresses()))
+        return _act(self, "marl_agent_act_input", "marl_agent_act_philox", p, n, obs, last, avail, hidden, explore,
+                    random_action, explore_u, choice_u, eps, gate, actions, onehot, q, philox, eps_table)
 
 
 class SeparatedMAC:
@@ -337,16 +376,11 @@ class SeparatedMAC:
         return _choose_actions(self, obs, last_action, avail_actions, epsilon, evaluate, draws)
 
     def act(self, n, obs, last, avail, hidden, explore=None, random_action=None, explore_u=None, choice_u=None, eps=0.0,
-            gate=None, actions=None, onehot=None, q=None):
-        """``SharedMAC.act`` with each agent's own network: one ``marl_agent_act_separated`` launch over n instances,
-        ``hidden`` [n * N, H] advanced in place, ``last`` may be None without a last-action input.  Returns ``actions``
-        [n, N] int64."""
-        if actions is None:
-            actions = th.empty(n, self.n_agents, dtype=th.int64, device=self.device)
+            gate=None, actions=None, onehot=None, q=None, philox=None, eps_table=None):
+        """``SharedMAC.act`` with each agent's own network: one ``marl_agent_act_separated`` launch over n instances
+        (``marl_agent_act_separated_philox`` with ``philox=``), ``hidden`` [n * N, H] advanced in place, ``last`` may be
+        None without a last-action input.  Returns ``actions`` [n, N] int64."""
         # rebuilt on every call: a learner's flat buffer or .cuda() re-packs the agents and moves their addresses
         p = (L.AgentParams * self.n_agents)(*(agent_param_struct(net.param_addresses()) for net in self.agent))
-        L.call("marl_agent_act_separated", n, self.n_agents, self.n_actions, self.obs_shape, int(self.args.last_action),
-               int(self.args.reuse_network), p, obs.data_ptr(), L.ptr(last), L.ptr(avail), hidden.data_ptr(),
-               hidden.data_ptr(), L.ptr(explore), L.ptr(random_action), L.ptr(explore_u), L.ptr(choice_u), float(eps),
-               L.ptr(gate), actions.data_ptr(), L.ptr(onehot), L.ptr(q), L.stream_ptr())
-        return actions
+        return _act(self, "marl_agent_act_separated", "marl_agent_act_separated_philox", p, n, obs, last, avail, hidden,
+                    explore, random_action, explore_u, choice_u, eps, gate, actions, onehot, q, philox, eps_table)

@@ -5,6 +5,7 @@
 
 #include "common.cuh"
 #include "../../include/marl_b200.h"
+#include "philox.cuh"
 #include "profile.h"
 
 namespace marl {
@@ -50,6 +51,30 @@ struct ActArgs {
     long long* action; float* onehot; float* q;
 };
 
+// Philox exploration form (marl_act_philox): the selection thread of row e*N + n draws its own pair.
+struct ActPhilox {
+    unsigned long long seed, episode_base;
+    int step;
+    const double* eps_table; int eps_len;
+};
+
+// The uniform form's random action: the min(floor(u * cnt), cnt - 1)-th of the cnt available actions, 0 when cnt == 0.
+// The Philox form calls it; the uniform form keeps its own copy inline in agent_act_kernel, so that its code is what it
+// was before the Philox form existed.
+__device__ __forceinline__ int kth_available(const float* av, int A, int cnt, double u) {
+    int best = 0;
+    if (cnt > 0) {
+        const double c = (double)cnt;
+        const int kth = (int)fmin(floor(u * c), c - 1.0);
+        for (int k = 0, seen = 0; k < A; ++k)
+            if (!av || av[k] != 0.0f) {
+                if (seen == kth) { best = k; break; }
+                ++seen;
+            }
+    }
+    return best;
+}
+
 constexpr int kActMaxAgents = 128;  // parameter sets one separated launch carries (8 KB of kernel parameters)
 
 template <int kSets>
@@ -58,9 +83,10 @@ struct ActParams { marl_agent_params p[kSets]; };
 // kSets == 1: the shared agent; a tile is 32 consecutive rows, tiles dealt round-robin.
 // kSets > 1: agent n's own weights; a tile is up to 32 instances of ONE agent (rows e*N + n), tiles are agent-major and
 // every CTA takes a contiguous range of them, so it restages weights only when its agent changes.
-template <int kSets>
+// kPhilox: exploration from ph (a's four exploration pointers are NULL); otherwise ph is not read.
+template <int kSets, bool kPhilox>
 __global__ void __launch_bounds__(kActThreads) agent_act_kernel(const __grid_constant__ ActParams<kSets> ps, ActArgs a,
-                                                                ActLayout l) {
+                                                                ActLayout l, ActPhilox ph) {
     constexpr bool kSep = kSets > 1;
     if (a.gate && *(volatile const int*)a.gate == 0) return;
     extern __shared__ float sm[];
@@ -213,7 +239,13 @@ __global__ void __launch_bounds__(kActThreads) agent_act_kernel(const __grid_con
                 if (v > bv) { bv = v; best = k; }          // strict: first maximum; all masked -> 0 like th.argmax
                 cnt_av += ok;
             }
-            if (a.explore) {
+            if constexpr (kPhilox) {
+                const int e = (int)(row / a.N), n = (int)(row - (long long)e * a.N);
+                const double eps = ph.eps_table ? ph.eps_table[min(e, ph.eps_len - 1)] : a.eps;
+                double eu, cu;
+                philox_act_uniforms(ph.seed, ph.episode_base + (unsigned long long)e, ph.step, n, eu, cu);
+                if (eu < eps) best = kth_available(av, A, cnt_av, cu);
+            } else if (a.explore) {
                 if (a.explore[row]) best = (int)a.random_action[row];
             } else if (a.explore_u && a.explore_u[row] < a.eps) {
                 best = 0;                                   // no available action: action 0
@@ -312,9 +344,10 @@ __global__ void __launch_bounds__(kRecWarps * 32) rollout_record_kernel(RecArgs 
 
 using namespace marl;
 
-// Validates the on-chip footprint of one parameter set of input width I and launches agent_act_kernel<kSets>.
-template <int kSets>
-static int act_launch(const char* name, const ActParams<kSets>& ps, const ActArgs& a, int I, long long tiles, void* stream) {
+// Validates the on-chip footprint of one parameter set of input width I and launches agent_act_kernel<kSets, kPhilox>.
+template <int kSets, bool kPhilox>
+static int act_launch(const char* name, const ActParams<kSets>& ps, const ActArgs& a, const ActPhilox& ph, int I,
+                      long long tiles, void* stream) {
     const ActLayout l = act_layout(I, a.A);
     const size_t smem = (size_t)l.total * sizeof(float);
     int dev = 0, sms = 0, optin = 0;
@@ -328,19 +361,20 @@ static int act_launch(const char* name, const ActParams<kSets>& ps, const ActArg
     static int blocks_per_sm[64] = {};
     static size_t blocks_for[64] = {};
     const int slot = dev & 63;
+    auto kernel = agent_act_kernel<kSets, kPhilox>;
     if (smem_set[slot] < smem) {
-        e = cudaFuncSetAttribute(agent_act_kernel<kSets>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return (int)e;
         smem_set[slot] = smem;
     }
     if (blocks_for[slot] != smem) {
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm[slot], agent_act_kernel<kSets>, kActThreads, smem);
+        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm[slot], kernel, kActThreads, smem);
         if (e != cudaSuccess) return (int)e;
         blocks_for[slot] = smem;
     }
     const long long cap = (long long)sms * (blocks_per_sm[slot] > 0 ? blocks_per_sm[slot] : 1);
     { ProfScope ps_(name, (cudaStream_t)stream);
-      agent_act_kernel<kSets><<<(int)(tiles < cap ? tiles : cap), kActThreads, smem, (cudaStream_t)stream>>>(ps, a, l); }
+      kernel<<<(int)(tiles < cap ? tiles : cap), kActThreads, smem, (cudaStream_t)stream>>>(ps, a, l, ph); }
     MARL_LAUNCH_CHECK();
     return MARL_OK;
 }
@@ -349,22 +383,49 @@ static bool params_complete(const marl_agent_params& p) {
     return p.fc1_w && p.fc1_b && p.w_ih && p.w_hh && p.b_ih && p.b_hh && p.fc2_w && p.fc2_b;
 }
 
+// The checks every marl_agent_act* call makes, then the launch: the shared agent (kSep false, p -> one parameter set)
+// or one network per agent (p -> N sets).
+template <bool kSep, bool kPhilox>
+static int act_call(int n_envs, int N, int A, int O, int last_action, int agent_id, const marl_agent_params* p,
+                    const float* obs, const float* last_onehot, const float* avail, const float* h_in, float* h_out,
+                    const unsigned char* explore, const long long* random_action, const double* explore_u,
+                    const double* choice_u, double eps, const int* gate, long long* action, float* onehot, float* q,
+                    const ActPhilox& ph, void* stream) {
+    if (n_envs < 0 || N <= 0 || (kSep && N > kActMaxAgents) || A <= 0 || O < 0 || !p || !obs || !h_in || !h_out || !action)
+        return MARL_EINVAL;
+    if (last_action && !last_onehot) return MARL_EINVAL;
+    for (int n = 0; n < (kSep ? N : 1); ++n)
+        if (!params_complete(p[n])) return MARL_EINVAL;
+    if (!explore != !random_action || !explore_u != !choice_u || (explore && explore_u)) return MARL_EINVAL;
+    const long long rows = (long long)n_envs * N;
+    if (rows > 0x7fffffffLL) return MARL_EINVAL;
+    const ActArgs a{(int)rows, n_envs, N, A, O, last_action ? 1 : 0, agent_id ? 1 : 0, obs, last_onehot, avail, h_in, h_out,
+                    explore, random_action, explore_u, choice_u, eps, gate, action, onehot, q};
+    const int I = O + (last_action ? A : 0) + (agent_id ? N : 0);
+    if constexpr (kSep) {
+        ActParams<kActMaxAgents> ps{};
+        for (int n = 0; n < N; ++n) ps.p[n] = p[n];
+        return act_launch<kActMaxAgents, kPhilox>("agent_act_separated_kernel", ps, a, ph, I,
+                                                  (long long)N * ((n_envs + kActRows - 1) / kActRows), stream);
+    } else {
+        const ActParams<1> ps{{*p}};
+        return act_launch<1, kPhilox>("agent_act_kernel", ps, a, ph, I, (rows + kActRows - 1) / kActRows, stream);
+    }
+}
+
+static bool philox_ok(const marl_act_philox* d, ActPhilox& ph) {
+    if (!d || d->step < 0 || (d->eps_table && d->eps_len < 1)) return false;
+    ph = ActPhilox{d->seed, d->episode_base, d->step, d->eps_table, d->eps_len};
+    return true;
+}
+
 extern "C" int marl_agent_act_input(int n_envs, int N, int A, int O, int last_action, int agent_id,
                                     const marl_agent_params* p, const float* obs, const float* last_onehot,
                                     const float* avail, const float* h_in, float* h_out, const unsigned char* explore,
                                     const long long* random_action, const double* explore_u, const double* choice_u,
                                     double eps, const int* gate, long long* action, float* onehot, float* q, void* stream) {
-    if (n_envs < 0 || N <= 0 || A <= 0 || O < 0 || !p || !obs || !h_in || !h_out || !action) return MARL_EINVAL;
-    if (last_action && !last_onehot) return MARL_EINVAL;
-    if (!params_complete(*p)) return MARL_EINVAL;
-    if (!explore != !random_action || !explore_u != !choice_u || (explore && explore_u)) return MARL_EINVAL;
-    const long long rows = (long long)n_envs * N;
-    if (rows > 0x7fffffffLL) return MARL_EINVAL;
-    const ActParams<1> ps{{*p}};
-    const ActArgs a{(int)rows, n_envs, N, A, O, last_action ? 1 : 0, agent_id ? 1 : 0, obs, last_onehot, avail, h_in, h_out,
-                    explore, random_action, explore_u, choice_u, eps, gate, action, onehot, q};
-    const int I = O + (last_action ? A : 0) + (agent_id ? N : 0);
-    return act_launch("agent_act_kernel", ps, a, I, (rows + kActRows - 1) / kActRows, stream);
+    return act_call<false, false>(n_envs, N, A, O, last_action, agent_id, p, obs, last_onehot, avail, h_in, h_out, explore,
+                                  random_action, explore_u, choice_u, eps, gate, action, onehot, q, ActPhilox{}, stream);
 }
 
 extern "C" int marl_agent_act(int n_envs, int N, int A, int O, const marl_agent_params* p, const float* obs,
@@ -382,21 +443,52 @@ extern "C" int marl_agent_act_separated(int n_envs, int N, int A, int O, int las
                                         const long long* random_action, const double* explore_u, const double* choice_u,
                                         double eps, const int* gate, long long* action, float* onehot, float* q,
                                         void* stream) {
-    if (n_envs < 0 || N <= 0 || N > kActMaxAgents || A <= 0 || O < 0 || !p || !obs || !h_in || !h_out || !action)
-        return MARL_EINVAL;
-    if (last_action && !last_onehot) return MARL_EINVAL;
-    ActParams<kActMaxAgents> ps{};
-    for (int n = 0; n < N; ++n) {
-        if (!params_complete(p[n])) return MARL_EINVAL;
-        ps.p[n] = p[n];
-    }
-    if (!explore != !random_action || !explore_u != !choice_u || (explore && explore_u)) return MARL_EINVAL;
+    return act_call<true, false>(n_envs, N, A, O, last_action, agent_id, p, obs, last_onehot, avail, h_in, h_out, explore,
+                                 random_action, explore_u, choice_u, eps, gate, action, onehot, q, ActPhilox{}, stream);
+}
+
+extern "C" int marl_agent_act_philox(int n_envs, int N, int A, int O, int last_action, int agent_id,
+                                     const marl_agent_params* p, const float* obs, const float* last_onehot,
+                                     const float* avail, const float* h_in, float* h_out, const marl_act_philox* philox,
+                                     double eps, const int* gate, long long* action, float* onehot, float* q,
+                                     void* stream) {
+    ActPhilox ph;
+    if (!philox_ok(philox, ph)) return MARL_EINVAL;
+    return act_call<false, true>(n_envs, N, A, O, last_action, agent_id, p, obs, last_onehot, avail, h_in, h_out, nullptr,
+                                 nullptr, nullptr, nullptr, eps, gate, action, onehot, q, ph, stream);
+}
+
+extern "C" int marl_agent_act_separated_philox(int n_envs, int N, int A, int O, int last_action, int agent_id,
+                                               const marl_agent_params* p, const float* obs, const float* last_onehot,
+                                               const float* avail, const float* h_in, float* h_out,
+                                               const marl_act_philox* philox, double eps, const int* gate,
+                                               long long* action, float* onehot, float* q, void* stream) {
+    ActPhilox ph;
+    if (!philox_ok(philox, ph)) return MARL_EINVAL;
+    return act_call<true, true>(n_envs, N, A, O, last_action, agent_id, p, obs, last_onehot, avail, h_in, h_out, nullptr,
+                                nullptr, nullptr, nullptr, eps, gate, action, onehot, q, ph, stream);
+}
+
+namespace marl {
+__global__ void philox_uniforms_kernel(unsigned long long seed, unsigned long long episode_base, int step, int n_envs,
+                                       int N, double* out) {
+    const long long row = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (row >= (long long)n_envs * N) return;
+    const int e = (int)(row / N), n = (int)(row - (long long)e * N);
+    philox_act_uniforms(seed, episode_base + (unsigned long long)e, step, n, out[2 * row], out[2 * row + 1]);
+}
+}  // namespace marl
+
+extern "C" int marl_philox_uniforms(unsigned long long seed, unsigned long long episode_base, int step, int n_envs, int N,
+                                    double* out, void* stream) {
+    if (n_envs < 0 || N <= 0 || step < 0 || !out || (long long)n_envs * N > 0x7fffffffLL) return MARL_EINVAL;
     const long long rows = (long long)n_envs * N;
-    if (rows > 0x7fffffffLL) return MARL_EINVAL;
-    const ActArgs a{(int)rows, n_envs, N, A, O, last_action ? 1 : 0, agent_id ? 1 : 0, obs, last_onehot, avail, h_in, h_out,
-                    explore, random_action, explore_u, choice_u, eps, gate, action, onehot, q};
-    const int I = O + (last_action ? A : 0) + (agent_id ? N : 0);
-    return act_launch("agent_act_separated_kernel", ps, a, I, (long long)N * ((n_envs + kActRows - 1) / kActRows), stream);
+    if (rows == 0) return MARL_OK;
+    { ProfScope ps_("philox_uniforms_kernel", (cudaStream_t)stream);
+      philox_uniforms_kernel<<<(int)((rows + 255) / 256), 256, 0, (cudaStream_t)stream>>>(seed, episode_base, step, n_envs,
+                                                                                         N, out); }
+    MARL_LAUNCH_CHECK();
+    return MARL_OK;
 }
 
 extern "C" int marl_rollout_record(const marl_dims* d, int t, const marl_episode_f32* ep, const float* obs, const float* state,
