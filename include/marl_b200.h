@@ -11,8 +11,8 @@
  *   - tensors are dense, row-major fp32 in the reference's episode-major layout
  *     (common/replaybuffer.py:19-30), rows of the folded agent batch are (b, n) with n minor
  *     (controller/share_params.py:110); action ids are int64.
- *   - H = rnn_hidden_dim = 64 and E = qmix_hidden_dim = 32 are compile-time constants
- *     (common/arguments.py:88-89); everything else is a run-time size.
+ *   - H = rnn_hidden_dim = 64 is a compile-time constant (common/arguments.py:88); E = qmix_hidden_dim
+ *     (:89, 1..128) travels in the QMIX parameter structs; everything else is a run-time size.
  */
 #ifndef MARL_B200_H
 #define MARL_B200_H
@@ -25,7 +25,8 @@ extern "C" {
 
 #define MARL_B200_VERSION 100
 #define MARL_HIDDEN 64
-#define MARL_QMIX_EMBED 32
+#define MARL_QMIX_EMBED 32          /* default qmix_hidden_dim (marl_qmix_params.embed = 0) */
+#define MARL_QMIX_MAX_EMBED 128
 
 int marl_version(void);
 /* Runtime probe: fills sm count / compute capability of the current device. */
@@ -339,9 +340,14 @@ int marl_vdn_td_fwd_bwd(const marl_dims* d, float* q_chosen, float* q_targets_ch
 /* ---- QMIX: network/mixer.py:57-80 ----
  * Hyper-network weights are passed concatenated (the host lays the parameters out that way):
  *   wcat [C, S], bcat [C] with C = N*E + 3E rows in the order
- *   hyper_w1 (N*E) | hyper_b1 (E) | hyper_w2 (E) | hyper_b2.0 (E);  wb2 [E], bb2 [1] = hyper_b2.2. */
-typedef struct marl_qmix_params { const float* wcat; const float* bcat; const float* wb2; const float* bb2; } marl_qmix_params;
-typedef struct marl_qmix_grads { float* wcat; float* bcat; float* wb2; float* bb2; } marl_qmix_grads;
+ *   hyper_w1 (N*E) | hyper_b1 (E) | hyper_w2 (E) | hyper_b2.0 (E);  wb2 [E], bb2 [1] = hyper_b2.2.
+ * embed = E = qmix_hidden_dim, 1..128; 0 means 32 (zero-initialised structs keep the default width).  Every marl_qmix_*
+ * entry point takes E from its parameter struct (marl_qmix_hyper_wgrad: from its gradient struct) and returns MARL_EINVAL
+ * when E is out of range or when the structs of one call (eval / target / gradient) carry different widths.
+ * The workspaces hy / hy_target / dhy are [M, C] with row pitch C = N*E + 3E in the order
+ *   w1 (N*E, hyper_w1 before the abs) | b1 (E) | w2 (E, before the abs) | b2.0 (E, before the ReLU). */
+typedef struct marl_qmix_params { const float* wcat; const float* bcat; const float* wb2; const float* bb2; int embed; } marl_qmix_params;
+typedef struct marl_qmix_grads { float* wcat; float* bcat; float* wb2; float* bb2; int embed; } marl_qmix_grads;
 
 /* q_tot[M] = QMixMixer(q[M,N], s[M,S]);  hy [M,C] workspace keeps the hyper-network outputs for the backward. */
 int marl_qmix_fwd(int M, int N, int S, const marl_qmix_params* p, const float* q, const float* s,
@@ -378,6 +384,8 @@ int marl_qmix_hyper_wgrad(int M, int N, int S, const float* s, const float* dhy,
 typedef struct marl_qmix_hyper2 {
     const float* w_in; const float* b_in; const float* w1_out; const float* b1_out; const float* w2_out; const float* b2_out;
     const float* w_b1; const float* b_b1; const float* w_b20; const float* b_b20; int hh;
+    int embed;               /* E as in marl_qmix_params (0 means 32); the hy it fills / reads has pitch C = N*E + 3E and must
+                                meet mixing calls whose marl_qmix_params carry the same E */
 } marl_qmix_hyper2;
 typedef struct marl_qmix_hyper2_grads {
     float* w_in; float* b_in; float* w1_out; float* b1_out; float* w2_out; float* b2_out;

@@ -77,19 +77,19 @@ class SelectFused(C.Structure):
                                      "fc2_b_target")]
 
 
-class QmixParams(C.Structure):
-    _fields_ = [(k, c_ptr) for k in ("wcat", "bcat", "wb2", "bb2")]
+class QmixParams(C.Structure):       # embed = qmix_hidden_dim (0 means 32)
+    _fields_ = [(k, c_ptr) for k in ("wcat", "bcat", "wb2", "bb2")] + [("embed", C.c_int)]
 
 
 class QmixGrads(C.Structure):
-    _fields_ = [(k, c_ptr) for k in ("wcat", "bcat", "wb2", "bb2")]
+    _fields_ = [(k, c_ptr) for k in ("wcat", "bcat", "wb2", "bb2")] + [("embed", C.c_int)]
 
 
 QMIX_HYPER2_FIELDS = ("w_in", "b_in", "w1_out", "b1_out", "w2_out", "b2_out", "w_b1", "b_b1", "w_b20", "b_b20")
 
 
 class QmixHyper2(C.Structure):       # two_hyper_layers=True parameters (include/marl_b200.h: marl_qmix_hyper2)
-    _fields_ = [(k, c_ptr) for k in QMIX_HYPER2_FIELDS] + [("hh", C.c_int)]
+    _fields_ = [(k, c_ptr) for k in QMIX_HYPER2_FIELDS] + [("hh", C.c_int), ("embed", C.c_int)]
 
 
 class QmixHyper2Grads(C.Structure):

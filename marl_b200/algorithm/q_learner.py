@@ -31,7 +31,7 @@ from .. import _lib as L
 from ..flat import FlatBuffer, prefixed
 from ..parallel import shard_bounds, allreduce_flat, PeerGradients
 from ..common.replaybuffer import DeviceEpisodeBatch
-from ..network.mixer import VDNMixer, QMixMixer, qmix_struct, qmix2_struct, qmix_tail_struct
+from ..network.mixer import VDNMixer, QMixMixer, hy_cols, qmix_struct, qmix2_struct, qmix_tail_struct
 from ..network.q_network import agent_param_struct
 
 H = 64
@@ -236,7 +236,7 @@ class QLearner:
         )
         ws["h_last_sep"] = [h.view(B, N, H) for h in ws["h_last"]]
         if a.alg == "qmix":
-            Ccols = N * 32 + 96
+            Ccols = hy_cols(N, a.qmix_hidden_dim)
             ws.update(hy=f(M, Ccols), hy_t=f(M, Ccols), dhy=f(M, Ccols))
             if getattr(a, "two_hyper_layers", False):
                 hh2 = 2 * a.hyper_hidden_dim
@@ -606,12 +606,12 @@ class QLearner:
 
     def _qmix_structs(self, flat, grad=False):
         """(mixing kernel, two-layer hyper-networks or None) structs of the QMIX mixer in `flat` or its gradient."""
-        addr = flat.addrs("mixer.", flat.grad if grad else None)
+        addr, E = flat.addrs("mixer.", flat.grad if grad else None), self.args.qmix_hidden_dim
         if not getattr(self.args, "two_hyper_layers", False):
-            return qmix_struct(addr, L.QmixGrads if grad else L.QmixParams), None
+            return qmix_struct(addr, E, L.QmixGrads if grad else L.QmixParams), None
         if grad:
-            return qmix_tail_struct(addr, L.QmixGrads), qmix2_struct(addr, None, L.QmixHyper2Grads)
-        return qmix_tail_struct(addr), qmix2_struct(addr, self.args.hyper_hidden_dim)
+            return qmix_tail_struct(addr, E, L.QmixGrads), qmix2_struct(addr, E, None, L.QmixHyper2Grads)
+        return qmix_tail_struct(addr, E), qmix2_struct(addr, E, self.args.hyper_hidden_dim)
 
     def _qmix_stage(self, bt, ws, d, fused):
         a, M, sp = self.args, d.B * d.L, L.stream_ptr()

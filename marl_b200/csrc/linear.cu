@@ -606,9 +606,9 @@ static bool vec_ok_mat(const float* p, int ld, long long bs, int col0 = 0) {
         else launch_pdl_prio(linear_prio(), KERNEL<false, false>, GRID, dim3(UTH), kUmmaSmem, ST, __VA_ARGS__);                      \
     } while (0)
 
-int linear_fwd(const LinearFwd& a, cudaStream_t st) {
+int linear_fwd(const LinearFwd& a, cudaStream_t st, bool tma) {
     if (a.M <= 0 || a.N <= 0 || a.batch <= 0) return MARL_OK;
-    { TGBuilder tg; if (tg.add_fwd(a)) return tg.launch(st); }       // TMA-addressable operands: tgemm.cu
+    if (tma) { TGBuilder tg; if (tg.add_fwd(a)) return tg.launch(st); }       // TMA-addressable operands: tgemm.cu
     dim3 grid(cdiv(a.M, UM), cdiv(a.N, UN), a.batch);
     const bool va = vec_ok_lin(a.in), vb = vec_ok_mat(a.w, a.ldw, a.w_bs);
     { if (prof_enabled()) prof_note(a.M, a.N, lin_width(a.in)); ProfScope ps_("linear_fwd_kernel", st); MARL_DISPATCH2(linear_fwd_kernel, va, vb, grid, st, a); }
@@ -640,10 +640,10 @@ int transpose_weights(const float* w, int ldw, int col0, int N, int K, float* wt
     return MARL_OK;
 }
 
-int linear_dgrad(const LinearDgrad& a, cudaStream_t st) {
+int linear_dgrad(const LinearDgrad& a, cudaStream_t st, bool tma) {
     if (a.M <= 0 || a.K <= 0 || a.batch <= 0) return MARL_OK;
     if (a.wt && a.batch != 1) return MARL_EINVAL;
-    if (!a.wt) { TGBuilder tg; if (tg.add_dgrad(a)) return tg.launch(st); }
+    if (!a.wt && tma) { TGBuilder tg; if (tg.add_dgrad(a)) return tg.launch(st); }
     dim3 grid(cdiv(a.M, UM), cdiv(a.K, UN), a.batch);
     const bool va = vec_ok_mat(a.dy, a.lddy, a.dy_bs), vb = vec_ok_mat(a.w, a.ldw, a.w_bs, a.w_col0);
     if (a.wt) {
@@ -665,9 +665,9 @@ int linear_dgrad(const LinearDgrad& a, cudaStream_t st) {
     return MARL_OK;
 }
 
-int linear_wgrad(const LinearWgrad& a, cudaStream_t st) {
+int linear_wgrad(const LinearWgrad& a, cudaStream_t st, bool tma) {
     if (a.M <= 0 || a.N <= 0 || a.batch <= 0) return MARL_OK;
-    {
+    if (tma) {
         TGBuilder tg;
         if (tg.add_wgrad(a)) { const int rc = tg.launch(st); return rc ? rc : tg.launch_reduce(st); }
     }

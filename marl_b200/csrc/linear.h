@@ -49,9 +49,10 @@ void set_deterministic_wgrad(int on);
 // wt[k, n] = w[n, col0 + k] for n < N, k < K (one small launch); wt pitch = N rounded up to 4 floats
 int transpose_weights(const float* w, int ldw, int col0, int N, int K, float* wt, cudaStream_t st);
 inline int transposed_pitch(int N) { return (N + 3) & ~3; }
-int linear_fwd(const LinearFwd& a, cudaStream_t st);
-int linear_dgrad(const LinearDgrad& a, cudaStream_t st);
-int linear_wgrad(const LinearWgrad& a, cudaStream_t st);
+// tma = false: the register-staged kernels of this file even when the TMA back end (tgemm.cu) is on and would take the operands
+int linear_fwd(const LinearFwd& a, cudaStream_t st, bool tma = true);
+int linear_dgrad(const LinearDgrad& a, cudaStream_t st, bool tma = true);
+int linear_wgrad(const LinearWgrad& a, cudaStream_t st, bool tma = true);
 
 inline LinOperand plain_operand(const float* x, int ldx, int K, long long bs = 0) {
     LinOperand o{};

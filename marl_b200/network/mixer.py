@@ -14,7 +14,12 @@ import torch.nn as nn
 from .. import _lib as L
 from ..flat import FlatBuffer, FlatPackedMixin
 
-E = 32
+MAX_EMBED = 128        # qmix_hidden_dim served by the mixing kernel (include/marl_b200.h: MARL_QMIX_MAX_EMBED)
+
+
+def hy_cols(N, E):
+    """Row pitch of the hyper-network outputs hy [M, C]: w1 (N E) | b1 | w2 | b2.0 (E each)."""
+    return N * E + 3 * E
 
 
 class VDNMixer(nn.Module):
@@ -35,13 +40,17 @@ class VDNMixer(nn.Module):
 QMIX_FLAT_ORDER = ("hyper_w1.weight", "hyper_b1.weight", "hyper_w2.weight", "hyper_b2.0.weight",
                    "hyper_w1.bias", "hyper_b1.bias", "hyper_w2.bias", "hyper_b2.0.bias",
                    "hyper_b2.2.weight", "hyper_b2.2.bias")
+# ... packed tight behind hyper_w1: wcat [N*E + 3E, S] and bcat [N*E + 3E] stay one matrix / vector whatever E is
+QMIX_TIGHT = frozenset(("hyper_b1.weight", "hyper_w2.weight", "hyper_b2.0.weight", "hyper_b1.bias", "hyper_w2.bias",
+                        "hyper_b2.0.bias"))
 
 
-def qmix_struct(addr, cls=L.QmixParams):
-    """addr: name -> device address for QMIX_FLAT_ORDER names (contiguity is guaranteed by FlatBuffer)."""
+def qmix_struct(addr, embed, cls=L.QmixParams):
+    """addr: name -> device address for QMIX_FLAT_ORDER names (contiguity is guaranteed by FlatBuffer); embed: E."""
     s = cls()
     s.wcat, s.bcat = addr["hyper_w1.weight"], addr["hyper_w1.bias"]
     s.wb2, s.bb2 = addr["hyper_b2.2.weight"], addr["hyper_b2.2.bias"]
+    s.embed = embed
     return s
 
 
@@ -52,8 +61,8 @@ QMIX2_FLAT_ORDER = ("hyper_w1.0.weight", "hyper_w2.0.weight", "hyper_w1.0.bias",
                     "hyper_b2.2.weight", "hyper_b2.2.bias")
 
 
-def qmix2_struct(addr, hh=None, cls=L.QmixHyper2):
-    """addr: name -> device address for QMIX2_FLAT_ORDER names."""
+def qmix2_struct(addr, embed, hh=None, cls=L.QmixHyper2):
+    """addr: name -> device address for QMIX2_FLAT_ORDER names; embed: E (kept by the parameter struct only)."""
     s = cls()
     s.w_in, s.b_in = addr["hyper_w1.0.weight"], addr["hyper_w1.0.bias"]
     s.w1_out, s.b1_out = addr["hyper_w1.2.weight"], addr["hyper_w1.2.bias"]
@@ -61,14 +70,15 @@ def qmix2_struct(addr, hh=None, cls=L.QmixHyper2):
     s.w_b1, s.b_b1 = addr["hyper_b1.weight"], addr["hyper_b1.bias"]
     s.w_b20, s.b_b20 = addr["hyper_b2.0.weight"], addr["hyper_b2.0.bias"]
     if hh is not None:
-        s.hh = hh
+        s.hh, s.embed = hh, embed
     return s
 
 
-def qmix_tail_struct(addr, cls=L.QmixParams):
+def qmix_tail_struct(addr, embed, cls=L.QmixParams):
     """Only the last layer of hyper_b2 (what the mixing kernel itself reads); wcat / bcat stay null."""
     s = cls()
     s.wb2, s.bb2 = addr["hyper_b2.2.weight"], addr["hyper_b2.2.bias"]
+    s.embed = embed
     return s
 
 
@@ -76,22 +86,22 @@ class _Qmix2Fn(torch.autograd.Function):
     """QMixMixer with two_hyper_layers=True: hyper2 GEMMs -> mixing kernel, and the reverse."""
 
     @staticmethod
-    def forward(ctx, q, s, N, S, hh, *params):
+    def forward(ctx, q, s, N, S, E, hh, *params):
         M, dev = q.shape[0], q.device
         h = torch.empty(M, 2 * hh, dtype=torch.float32, device=dev)
-        hy = torch.empty(M, N * E + 3 * E, dtype=torch.float32, device=dev)
+        hy = torch.empty(M, hy_cols(N, E), dtype=torch.float32, device=dev)
         q_tot = torch.empty(M, dtype=torch.float32, device=dev)
         addr = {n: t.data_ptr() for n, t in zip(QMIX2_FLAT_ORDER, params)}
-        p2, pt = qmix2_struct(addr, hh), qmix_tail_struct(addr)
+        p2, pt = qmix2_struct(addr, E, hh), qmix_tail_struct(addr, E)
         L.call("marl_qmix_hyper2_fwd", M, N, S, C.byref(p2), s.data_ptr(), h.data_ptr(), hy.data_ptr(), L.stream_ptr())
         L.call("marl_qmix_mix_fwd", M, N, C.byref(pt), q.data_ptr(), hy.data_ptr(), q_tot.data_ptr(), L.stream_ptr())
         ctx.save_for_backward(q, s, h, hy, *params)
-        ctx.meta = (N, S, hh)
+        ctx.meta = (N, S, E, hh)
         return q_tot
 
     @staticmethod
     def backward(ctx, dq_tot):
-        N, S, hh = ctx.meta
+        N, S, E, hh = ctx.meta
         q, s, h, hy, *params = ctx.saved_tensors
         M, dev = q.shape[0], q.device
         sizes = [p.numel() for p in params]
@@ -102,8 +112,8 @@ class _Qmix2Fn(torch.autograd.Function):
             off += n
         addr = {n: t.data_ptr() for n, t in zip(QMIX2_FLAT_ORDER, params)}
         gaddr = {n: v.data_ptr() for n, v in zip(QMIX2_FLAT_ORDER, views)}
-        p2, pt = qmix2_struct(addr, hh), qmix_tail_struct(addr)
-        g2, gt = qmix2_struct(gaddr, None, L.QmixHyper2Grads), qmix_tail_struct(gaddr, L.QmixGrads)
+        p2, pt = qmix2_struct(addr, E, hh), qmix_tail_struct(addr, E)
+        g2, gt = qmix2_struct(gaddr, E, None, L.QmixHyper2Grads), qmix_tail_struct(gaddr, E, L.QmixGrads)
         dhy = torch.empty_like(hy)
         dh = torch.empty_like(h)
         dq = torch.empty(M, N, dtype=torch.float32, device=dev)
@@ -111,26 +121,26 @@ class _Qmix2Fn(torch.autograd.Function):
                dhy.data_ptr(), dq.data_ptr(), C.byref(gt), L.stream_ptr())
         L.call("marl_qmix_hyper2_bwd", M, N, S, C.byref(p2), s.data_ptr(), h.data_ptr(), dhy.data_ptr(), dh.data_ptr(),
                C.byref(g2), L.stream_ptr())
-        return (dq, None, None, None, None, *views)
+        return (dq, None, None, None, None, None, *views)
 
 
 class _QmixFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, q, s, N, S, flat_params, *params):
+    def forward(ctx, q, s, N, S, E, *params):
         M = q.shape[0]
         dev = q.device
-        hy = torch.empty(M, N * E + 3 * E, dtype=torch.float32, device=dev)
+        hy = torch.empty(M, hy_cols(N, E), dtype=torch.float32, device=dev)
         q_tot = torch.empty(M, dtype=torch.float32, device=dev)
-        p = qmix_struct({n: t.data_ptr() for n, t in zip(QMIX_FLAT_ORDER, params)})
+        p = qmix_struct({n: t.data_ptr() for n, t in zip(QMIX_FLAT_ORDER, params)}, E)
         L.call("marl_qmix_fwd", M, N, S, C.byref(p), q.data_ptr(), s.data_ptr(), hy.data_ptr(), q_tot.data_ptr(),
                L.stream_ptr())
         ctx.save_for_backward(q, s, hy, *params)
-        ctx.meta = (N, S)
+        ctx.meta = (N, S, E)
         return q_tot
 
     @staticmethod
     def backward(ctx, dq_tot):
-        N, S = ctx.meta
+        N, S, E = ctx.meta
         q, s, hy, *params = ctx.saved_tensors
         M = q.shape[0]
         dev = q.device
@@ -142,8 +152,8 @@ class _QmixFn(torch.autograd.Function):
             views.append(gbuf[off:off + n].view(p.shape))
             off += n
         addr = {n: v.data_ptr() for n, v in zip(QMIX_FLAT_ORDER, views)}
-        g = qmix_struct(addr, L.QmixGrads)
-        pst = qmix_struct({n: t.data_ptr() for n, t in zip(QMIX_FLAT_ORDER, params)})
+        g = qmix_struct(addr, E, L.QmixGrads)
+        pst = qmix_struct({n: t.data_ptr() for n, t in zip(QMIX_FLAT_ORDER, params)}, E)
         dhy = torch.empty_like(hy)
         dq = torch.empty(M, N, dtype=torch.float32, device=dev)
         L.call("marl_qmix_bwd", M, N, S, C.byref(pst), q.data_ptr(), s.data_ptr(), hy.data_ptr(),
@@ -157,8 +167,9 @@ class QMixMixer(FlatPackedMixin, nn.Module):
     def __init__(self, args):
         super().__init__()
         self.args = args
-        if args.qmix_hidden_dim != E:
-            raise ValueError("libmarl_b200 is specialised for qmix_hidden_dim = 32")
+        E = args.qmix_hidden_dim
+        if not 1 <= E <= MAX_EMBED:
+            raise ValueError(f"qmix_hidden_dim must be an integer in 1..{MAX_EMBED}, got {E!r}")
         S, N = args.state_shape, args.n_agents
         self.two_hyper_layers = bool(getattr(args, "two_hyper_layers", False))
         if self.two_hyper_layers:                     # mixer.py:36-43
@@ -177,7 +188,9 @@ class QMixMixer(FlatPackedMixin, nn.Module):
 
     def flat_named_parameters(self):
         table = dict(self.named_parameters())
-        return [(n, table[n]) for n in (QMIX2_FLAT_ORDER if self.two_hyper_layers else QMIX_FLAT_ORDER)]
+        if self.two_hyper_layers:
+            return [(n, table[n]) for n in QMIX2_FLAT_ORDER]
+        return [(n, table[n], "tight") if n in QMIX_TIGHT else (n, table[n]) for n in QMIX_FLAT_ORDER]
 
     def _pack(self, device):
         self._flat = FlatBuffer(self.flat_named_parameters(), device=device, with_grad=False)
@@ -191,20 +204,20 @@ class QMixMixer(FlatPackedMixin, nn.Module):
         return out
 
     def param_addresses(self):
-        return {n: p.data_ptr() for n, p in self.flat_named_parameters()}
+        return {e[0]: e[1].data_ptr() for e in self.flat_named_parameters()}
 
     def forward(self, q_values, states):
         # states (episode_num, max_episode_len, state_shape); q_values (episode_num, max_episode_len, n_agents)
         episode_num = q_values.size(0)
         self.ensure_packed()      # the kernels read the four heads as ONE matrix: a copied module is re-packed first
-        N, S = self.args.n_agents, self.args.state_shape
+        N, S, E = self.args.n_agents, self.args.state_shape, self.args.qmix_hidden_dim
         q = L.require_cuda(q_values, "q_values").reshape(-1, N).to(torch.float32).contiguous()
         s = L.require_cuda(states, "states").reshape(-1, S).to(torch.float32).contiguous()
-        params = [p for _, p in self.flat_named_parameters()]
+        params = [e[1] for e in self.flat_named_parameters()]
         if self.two_hyper_layers:
-            q_tot = _Qmix2Fn.apply(q, s, N, S, self.args.hyper_hidden_dim, *params)
+            q_tot = _Qmix2Fn.apply(q, s, N, S, E, self.args.hyper_hidden_dim, *params)
         else:
-            q_tot = _QmixFn.apply(q, s, N, S, None, *params)
+            q_tot = _QmixFn.apply(q, s, N, S, E, *params)
         return q_tot.view(episode_num, -1, 1)
 
 
