@@ -11,8 +11,9 @@
  *   - tensors are dense, row-major fp32 in the reference's episode-major layout
  *     (common/replaybuffer.py:19-30), rows of the folded agent batch are (b, n) with n minor
  *     (controller/share_params.py:110); action ids are int64.
- *   - H = rnn_hidden_dim = 64 is a compile-time constant (common/arguments.py:88); E = qmix_hidden_dim
- *     (:89, 1..128) travels in the QMIX parameter structs; everything else is a run-time size.
+ *   - H = rnn_hidden_dim (common/arguments.py:88, one of 32, 64, 128) travels in marl_agent_params.hidden and
+ *     marl_qtran_net_params.hidden; E = qmix_hidden_dim (:89, 1..128) travels in the QMIX parameter structs;
+ *     everything else is a run-time size.
  */
 #ifndef MARL_B200_H
 #define MARL_B200_H
@@ -24,7 +25,7 @@ extern "C" {
 #endif
 
 #define MARL_B200_VERSION 100
-#define MARL_HIDDEN 64
+#define MARL_HIDDEN 64              /* default rnn_hidden_dim (marl_agent_params.hidden = 0) */
 #define MARL_QMIX_EMBED 32          /* default qmix_hidden_dim (marl_qmix_params.embed = 0) */
 #define MARL_QMIX_MAX_EMBED 128
 
@@ -88,6 +89,9 @@ typedef struct marl_agent_params {
     const float* w_ih;   /* [3H, H]   */  const float* w_hh;   /* [3H, H] */
     const float* b_ih;   /* [3H]      */  const float* b_hh;   /* [3H] */
     const float* fc2_w;  /* [A, H]    */  const float* fc2_b;  /* [A] */
+    int hidden;          /* H: 32, 64 or 128; 0 means 64 (MARL_HIDDEN).  Any other width: MARL_EINVAL from every entry point
+                            that receives the struct, as are streams of one marl_agent_unroll_fwd call, or the N sets of a
+                            separated act call, that carry different widths */
 } marl_agent_params;
 
 typedef struct marl_agent_grads {
@@ -230,7 +234,7 @@ int marl_agent_act(int n_envs, int N, int A, int O, const marl_agent_params* p, 
 /* marl_agent_act with the input blocks chosen by last_action / agent_id (share_params.py:84-123 with args.last_action /
  * args.reuse_network):
  *   in = [obs[r] (O) | last_onehot[r] (A, only if last_action) | eye(N)[n] (N, only if agent_id)]
- * so p->fc1_w is [64, O + A*last_action + N*agent_id].  Every other argument, the row layout, the exploration forms, gate
+ * so p->fc1_w is [H, O + A*last_action + N*agent_id].  Every other argument, the row layout, the exploration forms, gate
  * and the outputs are those of marl_agent_act, which is this call with last_action = agent_id = 1; last_onehot may be NULL
  * when last_action is 0.  MARL_EINVAL when last_action is set and last_onehot is NULL, and in every case marl_agent_act
  * returns it. */
@@ -243,7 +247,7 @@ int marl_agent_act_input(int n_envs, int N, int A, int O, int last_action, int a
 /* marl_agent_act with one network per agent (SeparatedMAC, share_params.py:389-610): row r = e*N + n uses p[n], an
  * array of N parameter sets, and its input is
  *   in = [obs[r] (O) | last_onehot[r] (A, only if last_action) | eye(N)[n] (N, only if agent_id)]  (share_params.py:467-506)
- * so p[n].fc1_w is [64, O + A*last_action + N*agent_id].  Every other argument, the row layout, the exploration forms,
+ * so p[n].fc1_w is [H, O + A*last_action + N*agent_id].  Every other argument, the row layout, the exploration forms,
  * gate and the outputs are those of marl_agent_act; last_onehot may be NULL when last_action is 0.  A tile holds up to
  * 32 instances of one agent, so the launch stages each agent's weights in shared memory once per CTA that serves it.
  * MARL_EINVAL when N > 128, when any of the N parameter sets has a NULL pointer, when last_action is set and last_onehot
@@ -319,7 +323,8 @@ int marl_td_loss(int M, const float* q_tot, const float* q_tot_target, const flo
  * dq [B,L,N,A] receives dL/dq_evals (dense: dq_tot at the chosen action, 0 elsewhere).
  * Learner fusions (all nullable; the same as marl_qmix_td_fwd_bwd's):
  *   fc2_w [A,H] + dhext [B,L,N,H]: also emit dhext = dq . fc2_w (one scaled row of fc2_w per agent, dq has one non-zero
- *     per row); pass it on with marl_unroll_bwd.dhext_ready = 1;
+ *     per row); pass it on with marl_unroll_bwd.dhext_ready = 1.  Caller contract: H = 64 only (the kernel reads fc2_w
+ *     and dhext with 64-float rows and receives no width to check); leave both NULL at any other width;
  *   sel: also do marl_q_select's work (q_learner.py:100-117: gather, in-place mask of q_targets, double-Q arg-max);
  *     q_chosen / q_targets_chosen are then OUTPUTS (MARL_EINVAL when 64 N A bytes of staging exceed 160 KB). */
 typedef struct marl_select_fused {   /* inputs of marl_q_select, for the fused forms of the mixers below */
@@ -328,7 +333,8 @@ typedef struct marl_select_fused {   /* inputs of marl_q_select, for the fused f
     /* hidden_evals != NULL: the agents' heads are evaluated here as well (q = fc2_w h + fc2_b, network/q_network.py:21-22):
      * q_evals / q_evals_next / q_targets [B,L,N,A] are then OUTPUTS (q_targets masked as the reference leaves it), computed
      * from the hidden states [B,L,N,H] of the eval net on o, the target net on o_next and (double-Q) the eval net on
-     * o_next -- run marl_agent_unroll_fwd with q = NULL.  All seven pointers 16-byte aligned. */
+     * o_next -- run marl_agent_unroll_fwd with q = NULL.  All seven pointers 16-byte aligned.  Caller contract: H = 64 only
+ * (the heads read 64-float hidden rows and fc2_w [A, 64]); at any other width leave hidden_evals NULL. */
     const float* hidden_evals; const float* hidden_targets; const float* hidden_evals_next;
     const float* fc2_w; const float* fc2_b; const float* fc2_w_target; const float* fc2_b_target;
 } marl_select_fused;
@@ -358,7 +364,8 @@ int marl_qmix_bwd(int M, int N, int S, const marl_qmix_params* p, const float* q
 /* Learner fusion (q_learner.py:161-168 + backward): eval mixer on (q_chosen, s), target mixer on
  * (q_targets_chosen, s_next), TD loss, gradient to the eval mixer parameters and dense dq [B,L,N,A].
  * With fc2_w / dhext the kernel also emits dhext = dq . fc2_w (dq has one non-zero per row, so this is one scaled row
- * of fc2_w per agent): pass it on with marl_unroll_bwd.dhext_ready = 1.
+ * of fc2_w per agent): pass it on with marl_unroll_bwd.dhext_ready = 1.  Caller contract, as for marl_vdn_td_fwd_bwd:
+ * fc2_w / dhext and the heads of sel (hidden_evals) at H = 64 only.
  * With sel the kernel also does marl_q_select's work (q_learner.py:100-117: gather, in-place mask of q_targets, double-Q
  * arg-max) for its own sample: q_chosen / q_targets_chosen are then OUTPUTS and no marl_q_select call is needed
  * (MARL_EINVAL when 64 N A bytes of staging exceed 160 KB: call marl_q_select yourself then). */
@@ -441,7 +448,10 @@ int marl_scatter_dq(const marl_dims* d, const float* dq_small, const long long* 
  *   QtranQBase: we1/we2 = hidden_action_encoding.{0,2}, w0/w2/w4 = q.{0,2,4}
  *   QtranV    : we1/we2 = hidden_encoding.{0,2},        w0/w2/w4 = v.{0,2,4}
  * Workspaces (kept for the backward): e1 [M*N, D], es [M, D], enc [M, D], a1 [M, qh], a2 [M, qh]. */
-typedef struct marl_qtran_net_params { const float *we1, *be1, *we2, *be2, *w0, *b0, *w2, *b2, *w4, *b4; } marl_qtran_net_params;
+typedef struct marl_qtran_net_params {
+    const float *we1, *be1, *we2, *be2, *w0, *b0, *w2, *b2, *w4, *b4;
+    int hidden;          /* H of the agents' hidden states: 32, 64 or 128; 0 means 64.  Any other width: MARL_EINVAL */
+} marl_qtran_net_params;
 typedef struct marl_qtran_net_grads { float *we1, *be1, *we2, *be2, *w0, *b0, *w2, *b2, *w4, *b4; } marl_qtran_net_grads;
 typedef struct marl_qtran_net_ws { float *e1, *es, *enc, *a1, *a2; } marl_qtran_net_ws;
 

@@ -36,8 +36,8 @@ class EpisodeF64(C.Structure):
 AGENT_KEYS = ("fc1_w", "fc1_b", "w_ih", "w_hh", "b_ih", "b_hh", "fc2_w", "fc2_b")
 
 
-class AgentParams(C.Structure):
-    _fields_ = [(k, c_ptr) for k in AGENT_KEYS]
+class AgentParams(C.Structure):       # hidden = rnn_hidden_dim (0 means 64)
+    _fields_ = [(k, c_ptr) for k in AGENT_KEYS] + [("hidden", C.c_int)]
 
 
 class AgentGrads(C.Structure):
@@ -118,8 +118,8 @@ class QplexWs(C.Structure):
 QTRAN_FIELDS = ("we1", "be1", "we2", "be2", "w0", "b0", "w2", "b2", "w4", "b4")
 
 
-class QtranNetParams(C.Structure):
-    _fields_ = [(k, c_ptr) for k in QTRAN_FIELDS]
+class QtranNetParams(C.Structure):    # hidden = rnn_hidden_dim (0 means 64)
+    _fields_ = [(k, c_ptr) for k in QTRAN_FIELDS] + [("hidden", C.c_int)]
 
 
 class QtranNetGrads(C.Structure):

@@ -34,7 +34,6 @@ from ..common.replaybuffer import DeviceEpisodeBatch
 from ..network.mixer import VDNMixer, QMixMixer, hy_cols, qmix_struct, qmix2_struct, qmix_tail_struct
 from ..network.q_network import agent_param_struct
 
-H = 64
 BATCH_KEYS = ("o", "u", "s", "r", "o_next", "s_next", "avail_u", "avail_u_next", "u_onehot", "padded", "terminated")
 
 
@@ -214,7 +213,7 @@ class QLearner:
         if ws is not None:
             return ws
         a, dev = self.args, self._dev
-        N, A, O, S = a.n_agents, a.n_actions, a.obs_shape, a.state_shape
+        N, A, O, S, H = a.n_agents, a.n_actions, a.obs_shape, a.state_shape, a.rnn_hidden_dim
         rows, M = B * Lq * N, B * Lq
         f = lambda *shape: th.empty(*shape, dtype=th.float32, device=dev)
         ws = dict(
@@ -454,12 +453,13 @@ class QLearner:
         """(parameter or gradient struct, agent stride) of the agent in `flat`: the shared network with stride 0, or -- one
         network per agent -- agent 0's set and the distance in floats from agent n's set to agent n+1's."""
         cls, src = (L.AgentGrads, flat.grad) if grad else (L.AgentParams, None)
+        H = self.args.rnn_hidden_dim
         if not self._separated:
-            return agent_param_struct(flat.addrs("agent.", src), cls), 0
+            return agent_param_struct(flat.addrs("agent.", src), cls, H), 0
         stride = self._agent_sets.get(id(flat))
         if stride is None:
             stride = self._agent_sets[id(flat)] = separated_stride(flat, self.args.n_agents)
-        return agent_param_struct(flat.addrs("agent.0.", src), cls), stride
+        return agent_param_struct(flat.addrs("agent.0.", src), cls, H), stride
 
     def _side_streams(self, n):
         self._side += [th.cuda.Stream() for _ in range(n - len(self._side))]
@@ -469,12 +469,13 @@ class QLearner:
         """What the VDN / QMIX mixing kernel takes over: the greedy selection (it gathers / arg-maxes its own sample, the [N, A]
         slabs of a warp's sample staged in shared memory), the agents' heads q = fc2(h) (no head GEMMs after the unroll) and,
         dq having one non-zero per agent row, dq . fc2_w (no dgrad launch in the BPTT).  With one network per agent only the
-        selection: the kernel stages one fc2, not one per agent."""
+        selection: the kernel stages one fc2, not one per agent.  The heads and dq . fc2_w read 64-wide hidden rows and fc2
+        rows: at any other rnn_hidden_dim only the selection."""
         a = self.args
         fuse = a.alg in ("vdn", "qmix") and bool(getattr(a, "fused_mixer_kernel", True))   # False: one kernel per stage
         fits = lambda heads: bool(L.load().marl_select_fits(int(a.alg == "qmix"), a.n_agents, a.n_actions, heads))
         select = fuse and fits(0)
-        if self._separated:
+        if self._separated or a.rnn_hidden_dim != 64:
             return _Fusion(select, False, False)
         fc2_w, fc2_wt = self._flat.ptr("agent.fc2.weight"), self._tflat.ptr("agent.fc2.weight")
         return _Fusion(select, select and fits(1) and fc2_w % 16 == 0 and fc2_wt % 16 == 0, fuse and fc2_w % 8 == 0)

@@ -26,7 +26,6 @@ from ..network.mixer import QMixMixer
 from ..network.qtran import QtranQBase, QtranV, net_struct, net_workspace, net_ws_struct
 from .q_learner import QLearner, _EVAL_O, _TARGET_O_NEXT
 
-H = 64
 
 
 class QTRANLearner(QLearner):
@@ -51,7 +50,7 @@ class QTRANLearner(QLearner):
         ws = super()._workspace(B, Lq)
         if fresh:
             a, dev = self.args, self._dev
-            N, A, M = a.n_agents, a.n_actions, B * Lq
+            N, A, M, H = a.n_agents, a.n_actions, B * Lq, a.rnn_hidden_dim
             f = lambda *shape: th.empty(*shape, dtype=th.float32, device=dev)
             D, qh = H + A, a.qtran_hidden_dim
             ws.update(oh_e=f(B, Lq, N, A), oh_t=f(B, Lq, N, A), opt_e=th.empty(B, Lq, N, dtype=th.int64, device=dev),
@@ -78,9 +77,10 @@ class QTRANLearner(QLearner):
         n = 1
         M, N, S, A, qh = d.B * d.L, a.n_agents, a.state_shape, a.n_actions, a.qtran_hidden_dim
         # net_struct takes the addresses in parameter order, the order the flat buffers list them in
-        pq = net_struct(fl.addrs("mixer.").values())
-        pqt = net_struct(tfl.addrs("mixer.").values())
-        pv = net_struct(fl.addrs("v.").values())
+        H = a.rnn_hidden_dim
+        pq = net_struct(fl.addrs("mixer.").values(), hidden=H)
+        pqt = net_struct(tfl.addrs("mixer.").values(), hidden=H)
+        pv = net_struct(fl.addrs("v.").values(), hidden=H)
         gq = net_struct(fl.addrs("mixer.", fl.grad).values(), L.QtranNetGrads)
         gv = net_struct(fl.addrs("v.", fl.grad).values(), L.QtranNetGrads)
         hid_e, hid_t = ws["hidden"][0].data_ptr(), ws["hidden"][1].data_ptr()

@@ -17,7 +17,7 @@ import numpy as np
 import torch as th
 
 from .. import _lib as L
-from ..network.q_network import RNNQNet, agent_param_struct
+from ..network.q_network import RNNQNet
 
 
 def _as_f32_cuda(x, device):
@@ -246,7 +246,7 @@ class SharedMAC:
         ``philox=PhiloxDraws(...)`` selects the Philox exploration form (``marl_agent_act_philox``) in place of the four
         exploration arrays, with ``eps_table`` (optional contiguous float64 device tensor) giving instance e the
         epsilon ``eps_table[min(e, len - 1)]`` instead of ``eps``.  Returns ``actions`` [n, N] int64."""
-        p = C.byref(agent_param_struct(self.agent.param_addresses()))
+        p = C.byref(self.agent.param_struct())
         return _act(self, "marl_agent_act_input", "marl_agent_act_philox", p, n, obs, last, avail, hidden, explore,
                     random_action, explore_u, choice_u, eps, gate, actions, onehot, q, philox, eps_table)
 
@@ -381,6 +381,6 @@ class SeparatedMAC:
         (``marl_agent_act_separated_philox`` with ``philox=``), ``hidden`` [n * N, H] advanced in place, ``last`` may be
         None without a last-action input.  Returns ``actions`` [n, N] int64."""
         # rebuilt on every call: a learner's flat buffer or .cuda() re-packs the agents and moves their addresses
-        p = (L.AgentParams * self.n_agents)(*(agent_param_struct(net.param_addresses()) for net in self.agent))
+        p = (L.AgentParams * self.n_agents)(*(net.param_struct() for net in self.agent))
         return _act(self, "marl_agent_act_separated", "marl_agent_act_separated_philox", p, n, obs, last, avail, hidden,
                     explore, random_action, explore_u, choice_u, eps, gate, actions, onehot, q, philox, eps_table)

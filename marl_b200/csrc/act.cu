@@ -272,6 +272,226 @@ __global__ void __launch_bounds__(kActThreads) agent_act_kernel(const __grid_con
     }
 }
 
+// ---- acting at rnn_hidden_dim H = 32 and 128 ---------------------------------------------------------------------------------
+// The H = 64 kernel above stages the whole network in shared memory; at H = 128 the two GRU matrices alone (2 x 384 x 129
+// floats) pass the 227 KB a block may hold.  This kernel keeps only the biases and fc2 resident and streams fc1, W_ih and
+// W_hh through shared memory in chunks of kActWC reduction columns: every chunk serves the 32 rows of a tile, and a parameter
+// set (at most 0.4 MB) stays in L2 across tiles.  Same tiles, same thread grid (thread (jg, rg) owns rows {rg, rg + 16} x
+// columns {jg + 16 c}, c < H / 16), same selection rules as agent_act_kernel; the H = 64 kernel keeps its own source.
+constexpr int kActWC = 16;         // reduction columns per staged weight chunk
+
+struct ActLayoutW {
+    int I, A, qw, hp;              // hp: odd row stride of the H-wide operands
+    int wc, b1, bih, bhh, w2, b2, in, xq, h, total;
+};
+
+inline ActLayoutW act_layout_w(int H, int I, int A) {
+    ActLayoutW l;
+    l.I = I; l.A = A; l.hp = H + 1; l.qw = A > l.hp ? A : l.hp;
+    int o = 0;
+    l.wc = o;  o += 2 * 3 * H * (kActWC + 1);     // W_ih | W_hh chunk [3H, WC] each (fc1 chunk [H, WC] in the first part)
+    l.b1 = o;  o += H;
+    l.bih = o; o += 3 * H;
+    l.bhh = o; o += 3 * H;
+    l.w2 = o;  o += A * l.hp;
+    l.b2 = o;  o += A;
+    l.in = o;  o += kActRows * (kActWC + 1);
+    l.xq = o;  o += kActRows * l.qw;
+    l.h = o;   o += kActRows * l.hp;
+    l.total = o;
+    return l;
+}
+
+// (min blocks: two CTAs an SM at H = 128 (128 registers), four at H = 32 (64 registers; the default plan spilled 4 bytes there))
+template <int H, int kSets, bool kPhilox>
+__global__ void __launch_bounds__(kActThreads, H >= 128 ? 2 : 4) agent_act_kernel_w(const __grid_constant__ ActParams<kSets> ps, ActArgs a,
+                                                                  ActLayoutW l, ActPhilox ph) {
+    constexpr bool kSep = kSets > 1;
+    constexpr int C = H / 16, HP = H + 1, WP = kActWC + 1;
+    if (a.gate && *(volatile const int*)a.gate == 0) return;
+    extern __shared__ float sm[];
+    __shared__ int act_s[kActRows];
+    float *wc = sm + l.wc, *b1 = sm + l.b1, *bih = sm + l.bih, *bhh = sm + l.bhh, *w2 = sm + l.w2, *b2 = sm + l.b2;
+    float *ins = sm + l.in, *xq = sm + l.xq, *hs = sm + l.h;
+    const int tid = threadIdx.x, A = a.A, O = a.O, I = l.I;
+
+    auto stage = [&](const marl_agent_params& p) {         // the resident part of a parameter set
+        for (int i = tid; i < A * H; i += kActThreads) w2[(i / H) * HP + (i % H)] = __ldg(p.fc2_w + i);
+        for (int i = tid; i < H; i += kActThreads) b1[i] = __ldg(p.fc1_b + i);
+        for (int i = tid; i < 3 * H; i += kActThreads) { bih[i] = __ldg(p.b_ih + i); bhh[i] = __ldg(p.b_hh + i); }
+        for (int i = tid; i < A; i += kActThreads) b2[i] = __ldg(p.fc2_b + i);
+    };
+
+    const int jg = tid & 15, rg = tid >> 4;
+    const int K = O + (a.last_action ? A : 0);
+    const int per_agent = (a.n_envs + kActRows - 1) / kActRows;
+    const int ntiles = kSep ? per_agent * a.N : (a.rows + kActRows - 1) / kActRows;
+    const int t_begin = kSep ? (int)((long long)ntiles * blockIdx.x / gridDim.x) : blockIdx.x;
+    const int t_end = kSep ? (int)((long long)ntiles * (blockIdx.x + 1) / gridDim.x) : ntiles;
+    const int t_step = kSep ? 1 : gridDim.x;
+    int staged = -1;
+    if (!kSep) stage(ps.p[0]);
+    for (int tile = t_begin; tile < t_end; tile += t_step) {
+        int n_tile = 0, stride = 1, cnt;
+        long long base;
+        if (kSep) {
+            n_tile = tile / per_agent;
+            const int e0 = (tile - n_tile * per_agent) * kActRows;
+            base = (long long)e0 * a.N + n_tile; stride = a.N; cnt = min(kActRows, a.n_envs - e0);
+            if (n_tile != staged) {
+                __syncthreads();
+                stage(ps.p[n_tile]);
+                staged = n_tile;
+            }
+        } else {
+            base = (long long)tile * kActRows; cnt = min(kActRows, a.rows - (int)base);
+        }
+        const marl_agent_params& p = ps.p[kSep ? n_tile : 0];
+        __syncthreads();
+        for (int i = tid; i < kActRows * H; i += kActThreads) {
+            const int r = i / H, k = i % H;
+            hs[r * HP + k] = r < cnt ? a.h_in[(base + (long long)r * stride) * H + k] : 0.f;
+        }
+        // ---- x = relu(fc1 [obs | last | eye(N)[n]] + b1), fc1 streamed in [H, WC] chunks
+        float acc[2][C];
+#pragma unroll
+        for (int c = 0; c < C; ++c) acc[0][c] = acc[1][c] = b1[jg + 16 * c];
+        for (int k0 = 0; k0 < K; k0 += kActWC) {
+            const int kc = min(kActWC, K - k0);
+            __syncthreads();
+            for (int i = tid; i < kActRows * kActWC; i += kActThreads) {
+                const int r = i / kActWC, kk = i % kActWC, k = k0 + kk;
+                const long long row = base + (long long)r * stride;
+                float v = 0.f;
+                if (r < cnt && kk < kc)
+                    v = k < O ? __ldg(a.obs + row * O + k) : __ldg(a.last + row * A + (k - O));
+                ins[r * WP + kk] = v;
+            }
+            for (int i = tid; i < H * kActWC; i += kActThreads) {
+                const int j = i / kActWC, kk = i % kActWC;
+                wc[j * WP + kk] = kk < kc ? __ldg(p.fc1_w + (long long)j * I + k0 + kk) : 0.f;
+            }
+            __syncthreads();
+            for (int kk = 0; kk < kc; ++kk) {
+                const float v0 = ins[rg * WP + kk], v1 = ins[(rg + 16) * WP + kk];
+#pragma unroll
+                for (int c = 0; c < C; ++c) {
+                    const float w = wc[(jg + 16 * c) * WP + kk];
+                    acc[0][c] = fmaf(w, v0, acc[0][c]);
+                    acc[1][c] = fmaf(w, v1, acc[1][c]);
+                }
+            }
+        }
+#pragma unroll
+        for (int rr = 0; rr < 2; ++rr) {
+            const int r = rg + 16 * rr, n = kSep ? n_tile : ((int)base + r) % a.N;
+#pragma unroll
+            for (int c = 0; c < C; ++c) {
+                const int j = jg + 16 * c;
+                xq[r * HP + j] = fmaxf(a.agent_id ? acc[rr][c] + __ldg(p.fc1_w + (long long)j * I + K + n) : acc[rr][c], 0.f);
+            }
+        }
+        // ---- GRUCell, gate order r, z, n (torch); W_ih and W_hh streamed in [3H, WC] chunks
+        float gi[2][3][C], gh[2][3][C];
+#pragma unroll
+        for (int g = 0; g < 3; ++g)
+#pragma unroll
+            for (int c = 0; c < C; ++c) {
+                gi[0][g][c] = gi[1][g][c] = bih[g * H + jg + 16 * c];
+                gh[0][g][c] = gh[1][g][c] = bhh[g * H + jg + 16 * c];
+            }
+        float* wih = wc;
+        float* whh = wc + 3 * H * WP;
+        for (int k0 = 0; k0 < H; k0 += kActWC) {
+            __syncthreads();              // x written / the previous chunk consumed
+            for (int i = tid; i < 3 * H * kActWC; i += kActThreads) {
+                const int m = i / kActWC, kk = i % kActWC;
+                wih[m * WP + kk] = __ldg(p.w_ih + (long long)m * H + k0 + kk);
+                whh[m * WP + kk] = __ldg(p.w_hh + (long long)m * H + k0 + kk);
+            }
+            __syncthreads();
+#pragma unroll 4
+            for (int kk = 0; kk < kActWC; ++kk) {
+                const int k = k0 + kk;
+                const float x0 = xq[rg * HP + k], x1 = xq[(rg + 16) * HP + k];
+                const float h0 = hs[rg * HP + k], h1 = hs[(rg + 16) * HP + k];
+#pragma unroll
+                for (int g = 0; g < 3; ++g)
+#pragma unroll
+                    for (int c = 0; c < C; ++c) {
+                        const int o = (g * H + jg + 16 * c) * WP + kk;
+                        const float wi = wih[o], wh = whh[o];
+                        gi[0][g][c] = fmaf(wi, x0, gi[0][g][c]); gi[1][g][c] = fmaf(wi, x1, gi[1][g][c]);
+                        gh[0][g][c] = fmaf(wh, h0, gh[0][g][c]); gh[1][g][c] = fmaf(wh, h1, gh[1][g][c]);
+                    }
+            }
+        }
+        float hn[2][C];
+#pragma unroll
+        for (int rr = 0; rr < 2; ++rr)
+#pragma unroll
+            for (int c = 0; c < C; ++c) {
+                const float r = sigmoidf_acc(gi[rr][0][c] + gh[rr][0][c]);
+                const float z = sigmoidf_acc(gi[rr][1][c] + gh[rr][1][c]);
+                const float nn = tanhf(gi[rr][2][c] + r * gh[rr][2][c]);
+                hn[rr][c] = (1.f - z) * nn + z * hs[(rg + 16 * rr) * HP + jg + 16 * c];
+            }
+        __syncthreads();                  // every read of x and h done
+#pragma unroll
+        for (int rr = 0; rr < 2; ++rr)
+#pragma unroll
+            for (int c = 0; c < C; ++c) hs[(rg + 16 * rr) * HP + jg + 16 * c] = hn[rr][c];
+        __syncthreads();
+        for (int i = tid; i < kActRows * H; i += kActThreads) {
+            const int r = i / H, k = i % H;
+            if (r < cnt) a.h_out[(base + (long long)r * stride) * H + k] = hs[r * HP + k];
+        }
+        // ---- q = fc2 h' + b2 (the q tile reuses the x tile)
+        for (int i = tid; i < kActRows * A; i += kActThreads) {
+            const int r = i / A, act = i - r * A;
+            float s = b2[act];
+#pragma unroll 8
+            for (int k = 0; k < H; ++k) s = fmaf(w2[act * HP + k], hs[r * HP + k], s);
+            xq[r * A + act] = s;
+            if (a.q && r < cnt) a.q[(base + (long long)r * stride) * A + act] = s;
+        }
+        __syncthreads();
+        // ---- masked first maximum, then the exploration forms (those of agent_act_kernel)
+        if (tid < cnt) {
+            const long long row = base + (long long)tid * stride;
+            const float* av = a.avail ? a.avail + row * A : nullptr;
+            int best = 0, cnt_av = 0;
+            float bv = -INFINITY;
+            for (int k = 0; k < A; ++k) {
+                const bool ok = !av || av[k] != 0.0f;
+                const float v = ok ? xq[tid * A + k] : -INFINITY;
+                if (v > bv) { bv = v; best = k; }
+                cnt_av += ok;
+            }
+            if constexpr (kPhilox) {
+                const int e = (int)(row / a.N), n = (int)(row - (long long)e * a.N);
+                const double eps = ph.eps_table ? ph.eps_table[min(e, ph.eps_len - 1)] : a.eps;
+                double eu, cu;
+                philox_act_uniforms(ph.seed, ph.episode_base + (unsigned long long)e, ph.step, n, eu, cu);
+                if (eu < eps) best = kth_available(av, A, cnt_av, cu);
+            } else if (a.explore) {
+                if (a.explore[row]) best = (int)a.random_action[row];
+            } else if (a.explore_u && a.explore_u[row] < a.eps) {
+                best = kth_available(av, A, cnt_av, a.choice_u[row]);
+            }
+            act_s[tid] = best;
+            a.action[row] = best;
+        }
+        if (a.onehot) {
+            __syncthreads();
+            for (int i = tid; i < kActRows * A; i += kActThreads) {
+                const int r = i / A, act = i - r * A;
+                if (r < cnt) a.onehot[(base + (long long)r * stride) * A + act] = act == act_s[r] ? 1.0f : 0.0f;
+            }
+        }
+    }
+}
+
 // One warp per instance.  Phase t (1 <= t <= T) closes step t-1 for the instances that acted in it (what env.step
 // returned, the one-hot of their action, and the observation / state / availability read after it) and opens step t
 // for the instances still active (the getters' values are the step's o / s / avail_u).
@@ -344,12 +564,16 @@ __global__ void __launch_bounds__(kRecWarps * 32) rollout_record_kernel(RecArgs 
 
 using namespace marl;
 
-// Validates the on-chip footprint of one parameter set of input width I and launches agent_act_kernel<kSets, kPhilox>.
-template <int kSets, bool kPhilox>
+// Validates the on-chip footprint of one parameter set of input width I and launches agent_act_kernel<kSets, kPhilox>
+// (H = 64) or agent_act_kernel_w<H, kSets, kPhilox>.
+template <int H, int kSets, bool kPhilox>
 static int act_launch(const char* name, const ActParams<kSets>& ps, const ActArgs& a, const ActPhilox& ph, int I,
                       long long tiles, void* stream) {
-    const ActLayout l = act_layout(I, a.A);
-    const size_t smem = (size_t)l.total * sizeof(float);
+    ActLayout l{};
+    ActLayoutW lw{};
+    size_t smem;
+    if constexpr (H == MARL_H) { l = act_layout(I, a.A); smem = (size_t)l.total * sizeof(float); }
+    else { lw = act_layout_w(H, I, a.A); smem = (size_t)lw.total * sizeof(float); }
     int dev = 0, sms = 0, optin = 0;
     cudaError_t e = cudaGetDevice(&dev);
     if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
@@ -361,7 +585,9 @@ static int act_launch(const char* name, const ActParams<kSets>& ps, const ActArg
     static int blocks_per_sm[64] = {};
     static size_t blocks_for[64] = {};
     const int slot = dev & 63;
-    auto kernel = agent_act_kernel<kSets, kPhilox>;
+    const void* kernel;
+    if constexpr (H == MARL_H) kernel = (const void*)agent_act_kernel<kSets, kPhilox>;
+    else kernel = (const void*)agent_act_kernel_w<H, kSets, kPhilox>;
     if (smem_set[slot] < smem) {
         e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return (int)e;
@@ -373,10 +599,21 @@ static int act_launch(const char* name, const ActParams<kSets>& ps, const ActArg
         blocks_for[slot] = smem;
     }
     const long long cap = (long long)sms * (blocks_per_sm[slot] > 0 ? blocks_per_sm[slot] : 1);
+    const int grid = (int)(tiles < cap ? tiles : cap);
     { ProfScope ps_(name, (cudaStream_t)stream);
-      kernel<<<(int)(tiles < cap ? tiles : cap), kActThreads, smem, (cudaStream_t)stream>>>(ps, a, l, ph); }
+      if constexpr (H == MARL_H) agent_act_kernel<kSets, kPhilox><<<grid, kActThreads, smem, (cudaStream_t)stream>>>(ps, a, l, ph);
+      else agent_act_kernel_w<H, kSets, kPhilox><<<grid, kActThreads, smem, (cudaStream_t)stream>>>(ps, a, lw, ph); }
     MARL_LAUNCH_CHECK();
     return MARL_OK;
+}
+
+// act_launch at the parameter sets' width
+template <int kSets, bool kPhilox>
+static int act_launch_h(int H, const char* name, const ActParams<kSets>& ps, const ActArgs& a, const ActPhilox& ph, int I,
+                        long long tiles, void* stream) {
+    if (H == 32) return act_launch<32, kSets, kPhilox>(name, ps, a, ph, I, tiles, stream);
+    if (H == 128) return act_launch<128, kSets, kPhilox>(name, ps, a, ph, I, tiles, stream);
+    return act_launch<MARL_H, kSets, kPhilox>(name, ps, a, ph, I, tiles, stream);
 }
 
 static bool params_complete(const marl_agent_params& p) {
@@ -394,8 +631,10 @@ static int act_call(int n_envs, int N, int A, int O, int last_action, int agent_
     if (n_envs < 0 || N <= 0 || (kSep && N > kActMaxAgents) || A <= 0 || O < 0 || !p || !obs || !h_in || !h_out || !action)
         return MARL_EINVAL;
     if (last_action && !last_onehot) return MARL_EINVAL;
+    const int H = hidden_width(p->hidden);
     for (int n = 0; n < (kSep ? N : 1); ++n)
-        if (!params_complete(p[n])) return MARL_EINVAL;
+        if (!params_complete(p[n]) || hidden_width(p[n].hidden) != H) return MARL_EINVAL;
+    if (H < 0) return MARL_EINVAL;
     if (!explore != !random_action || !explore_u != !choice_u || (explore && explore_u)) return MARL_EINVAL;
     const long long rows = (long long)n_envs * N;
     if (rows > 0x7fffffffLL) return MARL_EINVAL;
@@ -405,11 +644,11 @@ static int act_call(int n_envs, int N, int A, int O, int last_action, int agent_
     if constexpr (kSep) {
         ActParams<kActMaxAgents> ps{};
         for (int n = 0; n < N; ++n) ps.p[n] = p[n];
-        return act_launch<kActMaxAgents, kPhilox>("agent_act_separated_kernel", ps, a, ph, I,
-                                                  (long long)N * ((n_envs + kActRows - 1) / kActRows), stream);
+        return act_launch_h<kActMaxAgents, kPhilox>(H, "agent_act_separated_kernel", ps, a, ph, I,
+                                                    (long long)N * ((n_envs + kActRows - 1) / kActRows), stream);
     } else {
         const ActParams<1> ps{{*p}};
-        return act_launch<1, kPhilox>("agent_act_kernel", ps, a, ph, I, (rows + kActRows - 1) / kActRows, stream);
+        return act_launch_h<1, kPhilox>(H, "agent_act_kernel", ps, a, ph, I, (rows + kActRows - 1) / kActRows, stream);
     }
 }
 

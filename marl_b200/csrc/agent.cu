@@ -533,6 +533,396 @@ __global__ void __launch_bounds__(kGruThreads) gru_unroll_bwd_kernel(GruBwdArgs 
     }
 }
 
+// ---- the recurrence at rnn_hidden_dim H = 32 and 128 ------------------------------------------------------------------------
+// The scheme of the H = 64 kernels above, with the reduction split KS = H / 32 ways: thread (j, ks) = (tid / KS, tid % KS)
+// owns hidden unit j and reduction indices 4 (KS i + ks) + c, so every thread keeps 96 W_hh weights in registers at every
+// width and the KS lanes of a unit sit side by side in one warp.  A group is H x KS threads (32 at H = 32, 512 at H = 128).
+// The H = 64 kernels keep their own source: routing them through this template would change their instruction schedule,
+// so a fix to one belongs in both.
+template <int H>
+struct GruWidth {
+    static constexpr int KS = H / 32;                 // lanes per hidden unit
+    static constexpr int T = H * KS;                  // threads of one group
+    static constexpr int G = 3 * H;
+    static constexpr int kGroups = T >= 512 ? 1 : 2;  // forward: chains side by side in one CTA (512 threads fill the register file)
+    static constexpr int kMaxRows = H >= 128 ? 2 : 4; // rows per pass: what fits the registers without spills (at most 128 a
+                                                      // thread in a 512-thread group; at H = 32 every lane owns every row)
+    static_assert(KS >= 1 && (KS & (KS - 1)) == 0 && KS <= 32, "KS must be a power of two inside a warp");
+};
+
+template <int H>
+__device__ __forceinline__ void group_sync_w(int id) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(GruWidth<H>::T) : "memory"); }
+
+// the KS partial sums of one hidden unit, summed over its lanes (butterfly: every lane ends with the total)
+template <int KS>
+__device__ __forceinline__ float lanes_sum(float v) {
+#pragma unroll
+    for (int o = 1; o < KS; o <<= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    return v;
+}
+
+// v[q * KS + ks] with a register index fixed at compile time (rows past R read v[q * KS])
+template <int KS, int R>
+__device__ __forceinline__ float lane_pick(const float (&v)[R], int q, int ks) {
+    float r = v[q * KS];
+#pragma unroll
+    for (int c = 1; c < KS; ++c)
+        if (q * KS + c < R && ks == c) r = v[q * KS + c];
+    return r;
+}
+
+template <int H, bool SEP>
+__device__ __forceinline__ int gru_pass_rows_w(int pos, int left, int B) {
+    const int n = min(GruWidth<H>::kMaxRows, left);
+    return SEP ? min(n, B - pos % B) : n;
+}
+
+template <int H>
+constexpr size_t gru_fwd_smem_w(int R) { return (size_t)(2 * R * H + kGiDepth * R * 3 * H) * sizeof(float); }
+
+template <int H, int R, bool SEP>
+__device__ __forceinline__ void gru_chain_fwd_w(const GruFwdArgs& a, int chain, int row0, int nrows, float* smem, int bar_id) {
+    using W = GruWidth<H>;
+    constexpr int KS = W::KS, T = W::T, G = W::G, CPR = G / 4;       // CPR: 16-byte chunks of gi per row and step
+    float (*hs)[R][H] = reinterpret_cast<float (*)[R][H]>(smem);                              // [2][R][H]
+    float (*ring)[R][G] = reinterpret_cast<float (*)[R][G]>(smem + 2 * R * H);                // [D][R][3H]
+    const int tid = threadIdx.x % T, ks = tid % KS, j = tid / KS;
+    const int L = a.L, N = a.N;
+    __shared__ int srow_all[W::kGroups][W::kMaxRows];
+    int* srow = srow_all[bar_id - 1];
+    if (tid < R) {
+        const int* order = a.row_order[chain];
+        srow[tid] = (order && tid < nrows) ? __ldg(order + row0 + tid) : gru_position_row<SEP>(row0 + tid, a.B, N);
+    }
+    group_sync_w<H>(bar_id);
+    constexpr int OWN = (R + KS - 1) / KS;            // rows whose gate math this lane owns: rr = ks + KS q
+    bool own[OWN]; long long base[OWN];
+#pragma unroll
+    for (int q = 0; q < OWN; ++q) {
+        const int rr = ks + KS * q;
+        own[q] = rr < nrows;
+        const int row = own[q] ? srow[rr] : 0;
+        base[q] = own[q] ? ((long long)(row / N) * L * N + (row % N)) : 0;
+    }
+    const float* h0 = a.h0[chain];
+    for (int idx = tid; idx < R * H; idx += T) {
+        const int rr = idx / H, jj = idx % H;
+        hs[0][rr][jj] = (h0 && rr < nrows) ? h0[(long long)srow[rr] * H + jj] : 0.0f;
+    }
+    int cur = 0;
+    for (int sg = a.chain_start[chain]; sg < a.chain_start[chain] + a.chain_len[chain]; ++sg) {
+        const GruSegment S = a.seg[sg];
+        const long long poff = SEP ? (long long)(row0 / a.B) * a.agent_stride : 0;
+        const float* w_hh = S.w_hh + poff;
+        const float* b_hh = S.b_hh + poff;
+        f32x2 w[3][16];
+#pragma unroll
+        for (int g = 0; g < 3; ++g)
+#pragma unroll
+            for (int i = 0; i < 8; ++i) {
+                const float4 v = __ldg(reinterpret_cast<const float4*>(w_hh + (long long)(g * H + j) * H + 4 * (KS * i + ks)));
+                w[g][2 * i] = pack2(v.x, v.y); w[g][2 * i + 1] = pack2(v.z, v.w);
+            }
+        const float bh_r = __ldg(b_hh + j), bh_z = __ldg(b_hh + H + j), bh_n = __ldg(b_hh + 2 * H + j);
+        long long idx[OWN];                          // (b, t, n) index of the owned rows at step t: one register pair per row
+#pragma unroll
+        for (int q = 0; q < OWN; ++q) idx[q] = base[q];
+        int Lp = L;
+        if (S.ep_len) {
+            Lp = 1;
+            for (int rr = 0; rr < nrows; ++rr) Lp = max(Lp, min(L, __ldg(S.ep_len + srow[rr] / N)));
+        }
+        // (the chunk sources are recomputed per step: a list of them would not fit the register budget)
+        auto issue = [&](int t) {
+            if (t < Lp) {
+                for (int c = tid; c < nrows * CPR; c += T) {
+                    const int rr = c / CPR, ch = c % CPR, row = srow[rr];
+                    cp_async16(&ring[t % kGiDepth][rr][ch * 4], S.gi + (((long long)(row / N) * L + t) * N + (row % N)) * G + ch * 4);
+                }
+            }
+            cp_async_commit();
+        };
+#pragma unroll
+        for (int t = 0; t < kGiDepth - 1; ++t) issue(t);
+        for (int t = 0; t < Lp; ++t) {
+            cp_async_wait<kGiDepth - 2>();
+            group_sync_w<H>(bar_id);
+            issue(t + kGiDepth - 1);
+            float acc[3][R];
+            f32x2 pacc[3][R];
+#pragma unroll
+            for (int g = 0; g < 3; ++g)
+#pragma unroll
+                for (int rr = 0; rr < R; ++rr) pacc[g][rr] = 0ull;
+#pragma unroll
+            for (int i = 0; i < 8; ++i)
+#pragma unroll
+                for (int rr = 0; rr < R; ++rr) {
+                    const ulonglong2 hv = *reinterpret_cast<const ulonglong2*>(&hs[cur][rr][4 * (KS * i + ks)]);
+#pragma unroll
+                    for (int g = 0; g < 3; ++g) {
+                        pacc[g][rr] = ffma2(w[g][2 * i], hv.x, pacc[g][rr]);
+                        pacc[g][rr] = ffma2(w[g][2 * i + 1], hv.y, pacc[g][rr]);
+                    }
+                }
+#pragma unroll
+            for (int g = 0; g < 3; ++g)
+#pragma unroll
+                for (int rr = 0; rr < R; ++rr) {
+                    float ev, od;
+                    unpack2(pacc[g][rr], ev, od);
+                    acc[g][rr] = lanes_sum<KS>(ev + od);
+                }
+            const float* gring = &ring[t % kGiDepth][0][0];
+#pragma unroll
+            for (int q = 0; q < OWN; ++q) {
+                const float ar = lane_pick<KS>(acc[0], q, ks), az = lane_pick<KS>(acc[1], q, ks), an = lane_pick<KS>(acc[2], q, ks);
+                if (own[q]) {
+                    const int rr = ks + KS * q;
+                    const float* gp = gring + rr * G;
+                    const float gh_n = an + bh_n;
+                    const float r = gate_sigmoid((ar + bh_r) + gp[j]);
+                    const float z = gate_sigmoid((az + bh_z) + gp[H + j]);
+                    const float n = gate_tanh(fmaf(r, gh_n, gp[2 * H + j]));
+                    const float hold = hs[cur][rr][j];
+                    const float hnew = fmaf(hold - n, z, n);
+                    hs[cur ^ 1][rr][j] = hnew;
+                    S.hidden[idx[q] * H + j] = hnew;
+                    if (S.gates) {
+                        float* go = S.gates + idx[q] * (4 * H) + j;
+                        go[0] = r; go[H] = z; go[2 * H] = n; go[3 * H] = gh_n;
+                    }
+                }
+                idx[q] += N;
+            }
+            cur ^= 1;
+        }
+        cp_async_wait<0>();
+        group_sync_w<H>(bar_id);
+        if (S.h_last) {
+#pragma unroll
+            for (int q = 0; q < OWN; ++q)
+                if (own[q]) S.h_last[(long long)srow[ks + KS * q] * H + j] = hs[cur][ks + KS * q][j];
+        }
+    }
+}
+
+template <int H, bool SEP>
+__global__ void __launch_bounds__(GruWidth<H>::T * GruWidth<H>::kGroups) gru_unroll_fwd_kernel_w(GruFwdArgs a) {
+    using W = GruWidth<H>;
+    pdl_enter();
+    extern __shared__ __align__(16) float gru_smem[];
+    const int grp = threadIdx.x / W::T;
+    const int chain = blockIdx.y * W::kGroups + grp;
+    if (chain >= a.n_chains) return;
+    float* smem = gru_smem + grp * (gru_fwd_smem_w<H>(W::kMaxRows) / sizeof(float));
+    int begin = 0;
+    for (int i = 0; i < (int)blockIdx.x; ++i) begin += a.rows_of[chain][i];
+    const int count = a.rows_of[chain][blockIdx.x];
+    for (int off = 0, n = 0; off < count; off += SEP ? n : W::kMaxRows) {
+        n = gru_pass_rows_w<H, SEP>(begin + off, count - off, a.B);
+        if (n == 1) gru_chain_fwd_w<H, 1, SEP>(a, chain, begin + off, n, smem, 1 + grp);
+        else if (n == 2 || W::kMaxRows == 2) gru_chain_fwd_w<H, 2, SEP>(a, chain, begin + off, n, smem, 1 + grp);
+        else if (n <= 4) gru_chain_fwd_w<H, (W::kMaxRows < 4 ? 2 : 4), SEP>(a, chain, begin + off, n, smem, 1 + grp);
+        else gru_chain_fwd_w<H, W::kMaxRows, SEP>(a, chain, begin + off, n, smem, 1 + grp);
+        group_sync_w<H>(1 + grp);
+    }
+}
+
+template <int H>
+constexpr size_t gru_bwd_smem_w(int R) { return (size_t)(2 * R * 3 * H + bwd_depth(R) * R * 7 * H) * sizeof(float); }
+
+template <int H, int R, bool SEP>
+__device__ __forceinline__ void gru_rows_bwd_w(const GruBwdArgs& a, int row0, int nrows, float* gru_smem) {
+    using W = GruWidth<H>;
+    constexpr int KS = W::KS, T = W::T, G = W::G, SLOT = 7 * H, CPR = SLOT / 4;
+    constexpr int D = bwd_depth(R);
+    float (*sg)[R][G] = reinterpret_cast<float (*)[R][G]>(gru_smem);                          // [2][R][3H]
+    float (*ring)[R][SLOT] = reinterpret_cast<float (*)[R][SLOT]>(gru_smem + 2 * R * G);     // [D][R][7H]
+    const int tid = threadIdx.x, ks = tid % KS, j = tid / KS;
+    const int L = a.L, N = a.N;
+    __shared__ int srow[W::kMaxRows];
+    if (tid < R) srow[tid] = (a.row_order && tid < nrows) ? __ldg(a.row_order + row0 + tid) : gru_position_row<SEP>(row0 + tid, a.B, N);
+    __syncthreads();
+    constexpr int OWN = (R + KS - 1) / KS;
+    bool own[OWN]; long long base[OWN]; float dh_carry[OWN];
+#pragma unroll
+    for (int q = 0; q < OWN; ++q) {
+        const int rr = ks + KS * q;
+        own[q] = rr < nrows;
+        const int row = own[q] ? srow[rr] : 0;
+        base[q] = own[q] ? ((long long)(row / N) * L * N + (row % N)) : 0;
+        dh_carry[q] = 0.0f;
+    }
+    // column j of W_hh, rows m = 4 (KS i + ks) + c, i = 0..23
+    const float* w_hh = a.w_hh + (SEP ? (long long)(row0 / a.B) * a.agent_stride : 0);
+    f32x2 wt[48];
+#pragma unroll
+    for (int i = 0; i < 24; ++i)
+#pragma unroll
+        for (int c = 0; c < 2; ++c)
+            wt[2 * i + c] = pack2(__ldg(w_hh + (long long)(4 * (KS * i + ks) + 2 * c) * H + j),
+                                  __ldg(w_hh + (long long)(4 * (KS * i + ks) + 2 * c + 1) * H + j));
+    // cp.async work list, per row and step 7H/4 chunks of 16 B: gates (H chunks), h_prev, dh_ext, dh_ext2 (H/4 each).  The
+    // chunk's source is recomputed per step from (row, kind, column): a list of pointers would not fit 128 registers at H = 128.
+    auto issue = [&](int t) {
+        if (t >= 0) {
+            float* slot = &ring[t % D][0][0];
+            for (int c = tid; c < nrows * CPR; c += T) {
+                const int rr = c / CPR, ch = c % CPR, row = srow[rr];
+                const long long idx = ((long long)(row / N) * L + t) * N + (row % N);
+                const float* src = nullptr;
+                if (ch < H) src = a.gates + idx * (4 * H) + ch * 4;
+                else if (ch < H + H / 4) {
+                    if (t > 0) src = a.hidden + (idx - N) * H + (ch - H) * 4;
+                    else if (a.h0) src = a.h0 + (long long)row * H + (ch - H) * 4;     // (zeros without h0: the consumer)
+                } else if (ch < H + H / 2) { if (a.dh_ext) src = a.dh_ext + idx * H + (ch - H - H / 4) * 4; }
+                else if (a.dh_ext2) src = a.dh_ext2 + idx * H + (ch - H - H / 2) * 4;
+                if (src) cp_async16(slot + rr * SLOT + ch * 4, src);
+            }
+        }
+        cp_async_commit();
+    };
+    for (int idx = tid; idx < 2 * R * G; idx += T) (&sg[0][0][0])[idx] = 0.0f;
+    float* pi_[OWN]; float* ph_[OWN];
+#pragma unroll
+    for (int q = 0; q < OWN; ++q) {
+        pi_[q] = a.dgi + (base[q] + (long long)(L - 1) * N) * G + j;
+        ph_[q] = a.dgh + (base[q] + (long long)(L - 1) * N) * G + j;
+    }
+    const long long ostep = (long long)N * G;
+    int Lp = L;
+    if (a.ep_len) {
+        Lp = 1;
+        for (int rr = 0; rr < nrows; ++rr) Lp = max(Lp, min(L, __ldg(a.ep_len + srow[rr] / N)));
+        const int tail = L - Lp;
+        for (int idx = tid; idx < tail * nrows * (G / 4); idx += T) {
+            const int c4 = idx % (G / 4), rr = (idx / (G / 4)) % nrows, t = Lp + idx / ((G / 4) * nrows);
+            const int row = srow[rr];
+            const long long off = (((long long)(row / N) * L + t) * N + (row % N)) * G + 4 * c4;
+            *reinterpret_cast<float4*>(a.dgi + off) = make_float4(0.f, 0.f, 0.f, 0.f);
+            *reinterpret_cast<float4*>(a.dgh + off) = make_float4(0.f, 0.f, 0.f, 0.f);
+        }
+#pragma unroll
+        for (int q = 0; q < OWN; ++q) { pi_[q] -= (long long)tail * ostep; ph_[q] -= (long long)tail * ostep; }
+    }
+#pragma unroll
+    for (int d = 0; d < D - 1; ++d) issue(Lp - 1 - d);
+    cp_async_wait<D - 2>();
+    __syncthreads();
+    int cur = 0;
+    for (int t = Lp - 1; t >= 0; --t) {
+        float dh_dir[OWN];
+#pragma unroll
+        for (int q = 0; q < OWN; ++q) {
+            dh_dir[q] = 0.0f;
+            if (own[q]) {
+                const int rr = ks + KS * q;
+                const float* sl = &ring[t % D][rr][0];
+                const float g_r = sl[j], g_z = sl[H + j], g_n = sl[2 * H + j], g_hn = sl[3 * H + j];
+                const float hprev = (t > 0 || a.h0) ? sl[4 * H + j] : 0.0f;
+                float dh = dh_carry[q];
+                if (a.dh_ext) dh += sl[5 * H + j];
+                if (a.dh_ext2) dh += sl[6 * H + j];
+                const float dn_pre = dh * (1.0f - g_z) * (1.0f - g_n * g_n);
+                const float dz_pre = dh * (hprev - g_n) * g_z * (1.0f - g_z);
+                const float dr_pre = dn_pre * g_hn * g_r * (1.0f - g_r);
+                const float dghn = dn_pre * g_r;
+                dh_dir[q] = dh * g_z;
+                float* pi = pi_[q];
+                float* ph = ph_[q];
+                pi[0] = dr_pre; pi[H] = dz_pre; pi[2 * H] = dn_pre;
+                ph[0] = dr_pre; ph[H] = dz_pre; ph[2 * H] = dghn;
+                sg[cur][rr][j] = dr_pre; sg[cur][rr][H + j] = dz_pre; sg[cur][rr][2 * H + j] = dghn;
+            }
+            pi_[q] -= ostep; ph_[q] -= ostep;
+        }
+        issue(t - (D - 1));
+        cp_async_wait<D - 2>();
+        __syncthreads();                 // dgh of step t visible; ring[t-1] visible
+        float part[R];
+        f32x2 pab[R], pcd[R];
+#pragma unroll
+        for (int rr = 0; rr < R; ++rr) { pab[rr] = 0ull; pcd[rr] = 0ull; }
+#pragma unroll
+        for (int i = 0; i < 24; ++i)
+#pragma unroll
+            for (int rr = 0; rr < R; ++rr) {
+                const ulonglong2 v = *reinterpret_cast<const ulonglong2*>(&sg[cur][rr][4 * (KS * i + ks)]);
+                pab[rr] = ffma2(wt[2 * i], v.x, pab[rr]);
+                pcd[rr] = ffma2(wt[2 * i + 1], v.y, pcd[rr]);
+            }
+#pragma unroll
+        for (int rr = 0; rr < R; ++rr) {
+            float pa, pb, pc, pd;
+            unpack2(pab[rr], pa, pb); unpack2(pcd[rr], pc, pd);
+            part[rr] = lanes_sum<KS>((pa + pb) + (pc + pd));
+        }
+#pragma unroll
+        for (int q = 0; q < OWN; ++q) dh_carry[q] = dh_dir[q] + lane_pick<KS>(part, q, ks);
+        cur ^= 1;
+    }
+    cp_async_wait<0>();
+    if (a.dh0) {
+#pragma unroll
+        for (int q = 0; q < OWN; ++q)
+            if (own[q]) a.dh0[(long long)srow[ks + KS * q] * H + j] = dh_carry[q];
+    }
+    __syncthreads();
+}
+
+template <int H>
+constexpr size_t gru_bwd_smem_max_w() {
+    return gru_bwd_smem_w<H>(GruWidth<H>::kMaxRows) > gru_bwd_smem_w<H>(2) ? gru_bwd_smem_w<H>(GruWidth<H>::kMaxRows) : gru_bwd_smem_w<H>(2);
+}
+
+template <int H, bool SEP>
+__global__ void __launch_bounds__(GruWidth<H>::T) gru_unroll_bwd_kernel_w(GruBwdArgs a) {
+    using W = GruWidth<H>;
+    pdl_enter();
+    extern __shared__ __align__(16) float gru_smem[];
+    int begin, count;
+    if (SEP) cta_rows_by_agent(a.B, a.N, begin, count);
+    else cta_rows(a.B * a.N, 0, begin, count);
+    for (int off = 0, n = 0; off < count; off += SEP ? n : W::kMaxRows) {
+        n = gru_pass_rows_w<H, SEP>(begin + off, count - off, a.B);
+        if (n == 1) gru_rows_bwd_w<H, 1, SEP>(a, begin + off, n, gru_smem);
+        else if (n == 2 || W::kMaxRows == 2) gru_rows_bwd_w<H, 2, SEP>(a, begin + off, n, gru_smem);
+        else if (n <= 4) gru_rows_bwd_w<H, (W::kMaxRows < 4 ? 2 : 4), SEP>(a, begin + off, n, gru_smem);
+        else gru_rows_bwd_w<H, W::kMaxRows, SEP>(a, begin + off, n, gru_smem);
+    }
+}
+
+// Launches of the H = 32 / 128 recurrence.  Forward: the H = 64 grid (one CTA per SM and chain group), a group per chain.
+// Backward: the H = 64 CTA count, so that the row deal marl_agent_unroll_fwd plans for it (row_order_bwd) holds.
+template <int H>
+static void gru_fwd_launch_w(const GruFwdArgs& ga, int n_ctas, bool sep, cudaStream_t st) {
+    using W = GruWidth<H>;
+    const size_t sm = W::kGroups * gru_fwd_smem_w<H>(W::kMaxRows);
+    static bool attr_set = false;
+    if (!attr_set) {
+        cudaFuncSetAttribute(gru_unroll_fwd_kernel_w<H, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+        cudaFuncSetAttribute(gru_unroll_fwd_kernel_w<H, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+        attr_set = true;
+    }
+    const dim3 grid(n_ctas, (ga.n_chains + W::kGroups - 1) / W::kGroups);
+    launch_pdl_prio(kGruPrio, sep ? gru_unroll_fwd_kernel_w<H, true> : gru_unroll_fwd_kernel_w<H, false>, grid,
+                    dim3(W::T * W::kGroups), sm, st, ga);
+}
+
+template <int H>
+static void gru_bwd_launch_w(const GruBwdArgs& ga, int rows, bool sep, cudaStream_t st) {
+    const size_t sm = gru_bwd_smem_max_w<H>();
+    static bool attr_set = false;
+    if (!attr_set) {
+        cudaFuncSetAttribute(gru_unroll_bwd_kernel_w<H, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+        cudaFuncSetAttribute(gru_unroll_bwd_kernel_w<H, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+        attr_set = true;
+    }
+    launch_pdl_prio(kGruPrio, sep ? gru_unroll_bwd_kernel_w<H, true> : gru_unroll_bwd_kernel_w<H, false>, dim3(gru_bwd_ctas(rows)),
+                    dim3(GruWidth<H>::T), sm, st, ga);
+}
+
 // Rows of every chain per CTA.  The kernel ends when its slowest CTA does, and a CTA's time is roughly
 // (steps of the chain) x (rows it advances), so rows are dealt by water-filling on that weighted load: the first
 // chain evenly, every further chain onto the CTAs that carry the least so far.  At cfg 2 (160 rows, 148 CTAs) the 12
@@ -779,6 +1169,11 @@ extern "C" int marl_agent_unroll_fwd(const marl_dims* d, const marl_unroll_strea
         if (s[i].h0_from >= i) return MARL_EINVAL;
         if (s[i].h0_from >= 0 && s[s[i].h0_from].ep_len) return MARL_EINVAL;     // a continued stream must run to L (header)
     }
+    // rnn_hidden_dim: one width for every stream of the call
+    const int H = hidden_width(s[0].params.hidden), G = 3 * H;
+    if (H < 0) return MARL_EINVAL;
+    for (int i = 0; i < n_streams; ++i)
+        if (hidden_width(s[i].params.hidden) != H) return MARL_EINVAL;
     // phase B: build chains (a stream whose h0_from == j continues chain of j; j must be a chain tail)
     const int I = agent_input_width(d, blocks(0));
     for (int i = 0; i < n_streams; ++i)
@@ -843,7 +1238,7 @@ extern "C" int marl_agent_unroll_fwd(const marl_dims* d, const marl_unroll_strea
                 for (int k = 0; k < n_streams && !len; ++k) len = s[k].ep_len;
                 if (!len) return MARL_EINVAL;
                 unsigned short cnt[kMaxOrderCtas];
-                const int nb = gru_bwd_ctas(rows);
+                const int nb = gru_bwd_ctas(rows);      // (the same CTA count at every width)
                 for (int c = 0; c < nb; ++c) cnt[c] = (unsigned short)(rows / nb + (c < rows % nb ? 1 : 0));     // cta_rows()
                 order_plan_fill(oa.bwd, cnt, nb, len, s[i].row_order_bwd);
                 any = true;
@@ -871,20 +1266,20 @@ extern "C" int marl_agent_unroll_fwd(const marl_dims* d, const marl_unroll_strea
     auto fc1_of = [&](int i) {
         const LinOperand in = sep ? separated_input(d, s[i].obs, s[i].onehot, s[i].shift_onehot, s[i].last_action, s[i].agent_id)
                                   : agent_input(d, s[i].obs, s[i].onehot, s[i].shift_onehot, s[i].full_input, blocks(i));
-        LinearFwd f = agent_layer(d, in, s[i].params.fc1_w, I, s[i].params.fc1_b, s[i].x, MARL_H, stride);
+        LinearFwd f = agent_layer(d, in, s[i].params.fc1_w, I, s[i].params.fc1_b, s[i].x, H, stride);
         f.relu = 1;
         return f;
     };
     auto ih_of = [&](int i) {
-        const LinOperand in = sep ? plain_operand(s[i].x, d->N * MARL_H, MARL_H, MARL_H) : plain_operand(s[i].x, MARL_H, MARL_H);
-        return agent_layer(d, in, s[i].params.w_ih, MARL_H, s[i].params.b_ih, s[i].gi, MARL_G, stride);
+        const LinOperand in = sep ? plain_operand(s[i].x, d->N * H, H, H) : plain_operand(s[i].x, H, H);
+        return agent_layer(d, in, s[i].params.w_ih, H, s[i].params.b_ih, s[i].gi, G, stride);
     };
     bool grouped = false;
     if (!sep) {      // (the fused input-layer kernel stages one shared weight set: separated streams take the unfused path)
         // fused path (csrc/front.cu): both layers of every stream in ONE persistent launch, x handed from the first GEMM to the
         // second through tensor memory
         FrontArgs fa{};
-        fa.rows = rows_total; fa.I = I;
+        fa.rows = rows_total; fa.I = I; fa.hidden = H;
         for (int i = 0; i < n_streams; ++i) {
             fa.s[i].in = agent_input(d, s[i].obs, s[i].onehot, s[i].shift_onehot, s[i].full_input, blocks(i));
             fa.s[i].x = s[i].x; fa.s[i].gi = s[i].gi;
@@ -902,13 +1297,14 @@ extern "C" int marl_agent_unroll_fwd(const marl_dims* d, const marl_unroll_strea
     if (!grouped) {
         for (int i = 0; i < n_streams; ++i)
             if (s[i].w_ih_t) {
-                const int rc = transpose_weights(s[i].params.w_ih, MARL_H, 0, MARL_G, MARL_H, s[i].w_ih_t, st);
+                const int rc = transpose_weights(s[i].params.w_ih, H, 0, G, H, s[i].w_ih_t, st);
                 if (rc) return rc;
             }
     }
-    if (!grouped && !sep && tgemm_enabled()) {
+    if (!grouped && !sep && H == MARL_H && tgemm_enabled()) {
         // TMA path: the streams of one layer are ONE grouped launch of persistent CTAs (csrc/tgemm.cu): 2 launches
-        // instead of 2 x n_streams on forked streams
+        // instead of 2 x n_streams on forked streams.  (Other widths take the register-staged kernels of linear.cu: the
+        // TMA builders have only been checked on the 64-wide agent layers.)
         TGBuilder b1, b2;
         bool ok = true;
         for (int i = 0; i < n_streams && ok; ++i) ok = b1.add_fwd(fc1_of(i));
@@ -939,18 +1335,24 @@ extern "C" int marl_agent_unroll_fwd(const marl_dims* d, const marl_unroll_strea
     {
         // one CTA per SM; each CTA advances its share of every chain side by side (one 128-thread group per chain)
         ProfScope ps_("gru_unroll_fwd_kernel", st);
-        const size_t sm = kGruGroups * gru_fwd_smem(kGruMaxRows);
-        static bool attr_set = false;
-        if (!attr_set) {
-            cudaFuncSetAttribute(gru_unroll_fwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-            cudaFuncSetAttribute(gru_unroll_fwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-            attr_set = true;
-        }
         ga.trace = trace_buffer();
         if (order_lane) order_lane->join();
-        dim3 grid(n_ctas, (ga.n_chains + kGruGroups - 1) / kGruGroups);
-        launch_pdl_prio(kGruPrio, sep ? gru_unroll_fwd_kernel<true> : gru_unroll_fwd_kernel<false>, grid,
-                        dim3(kGruThreads * kGruGroups), sm, st, ga);
+        if (H == MARL_H) {
+            const size_t sm = kGruGroups * gru_fwd_smem(kGruMaxRows);
+            static bool attr_set = false;
+            if (!attr_set) {
+                cudaFuncSetAttribute(gru_unroll_fwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+                cudaFuncSetAttribute(gru_unroll_fwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+                attr_set = true;
+            }
+            dim3 grid(n_ctas, (ga.n_chains + kGruGroups - 1) / kGruGroups);
+            launch_pdl_prio(kGruPrio, sep ? gru_unroll_fwd_kernel<true> : gru_unroll_fwd_kernel<false>, grid,
+                            dim3(kGruThreads * kGruGroups), sm, st, ga);
+        } else if (H == 32) {
+            gru_fwd_launch_w<32>(ga, n_ctas, sep, st);
+        } else {
+            gru_fwd_launch_w<128>(ga, n_ctas, sep, st);
+        }
     }
     MARL_LAUNCH_CHECK();
     // phase C.  (The fork / join pair stays even when a fused mixer evaluates the heads and nothing is launched here: it takes the
@@ -960,8 +1362,8 @@ extern "C" int marl_agent_unroll_fwd(const marl_dims* d, const marl_unroll_strea
     for (int i = 0; i < n_streams; ++i) {
         if (!s[i].q) continue;
         cudaStream_t st = fc.lane(i);
-        const LinOperand in = sep ? plain_operand(s[i].hidden, d->N * MARL_H, MARL_H, MARL_H) : plain_operand(s[i].hidden, MARL_H, MARL_H);
-        int rc = linear_fwd(agent_layer(d, in, s[i].params.fc2_w, MARL_H, s[i].params.fc2_b, s[i].q, d->A, stride), st);
+        const LinOperand in = sep ? plain_operand(s[i].hidden, d->N * H, H, H) : plain_operand(s[i].hidden, H, H);
+        int rc = linear_fwd(agent_layer(d, in, s[i].params.fc2_w, H, s[i].params.fc2_b, s[i].q, d->A, stride), st);
         if (rc) return rc;
     }
     fc.join();
@@ -979,6 +1381,8 @@ extern "C" int marl_agent_unroll_bwd(const marl_dims* d, const marl_unroll_bwd* 
     if (!sep && a->input_flags && a->full_input) return MARL_EINVAL;
     const InputBlocks blk = input_blocks(stride, a->input_flags, a->last_action, a->agent_id);
     if (!a->full_input && blk.last_action && !a->onehot) return MARL_EINVAL;
+    const int H = hidden_width(a->params.hidden), G = 3 * H;
+    if (H < 0) return MARL_EINVAL;
     cudaStream_t st = (cudaStream_t)stream;
     pdl_scope((long long)d->B * d->L * d->N);
     const int rows_total = d->B * d->L * d->N;
@@ -991,8 +1395,8 @@ extern "C" int marl_agent_unroll_bwd(const marl_dims* d, const marl_unroll_bwd* 
     if (a->dq && !a->dhext_ready) {
         // q = W2 h + b2:  dh_ext = dq . W2 ;  dW2 += dq^T h ; db2 += colsum(dq)
         LinearDgrad g{};
-        g.dy = a->dq; g.lddy = rp * d->A; g.dy_bs = zs(d->A); g.w = a->params.fc2_w; g.ldw = MARL_H; g.w_bs = stride; g.w_col0 = 0;
-        g.dx = a->dhext; g.lddx = rp * MARL_H; g.dx_bs = zs(MARL_H); g.M = M; g.N = d->A; g.K = MARL_H; g.batch = nb;
+        g.dy = a->dq; g.lddy = rp * d->A; g.dy_bs = zs(d->A); g.w = a->params.fc2_w; g.ldw = H; g.w_bs = stride; g.w_col0 = 0;
+        g.dx = a->dhext; g.lddx = rp * H; g.dx_bs = zs(H); g.M = M; g.N = d->A; g.K = H; g.batch = nb;
         if ((rc = linear_dgrad(g, st))) return rc;
     }
     GruBwdArgs ga{a->gates, a->hidden, a->dq ? a->dhext : nullptr, a->dhidden, a->params.w_hh, a->h0, a->dgi, a->dgh, a->dh0,
@@ -1013,56 +1417,59 @@ extern "C" int marl_agent_unroll_bwd(const marl_dims* d, const marl_unroll_bwd* 
         // up to two rows per SM: one CTA per row -- two co-resident one-row CTAs overlap each other's latency, where one CTA with two
         // rows serialises 2 x 96 packed FMAs per thread on the dependent chain (the 12 two-row CTAs of config 2 ended the kernel)
         const int n_ctas = gru_bwd_ctas(rows);
-        launch_pdl_prio(kGruPrio, sep ? gru_unroll_bwd_kernel<true> : gru_unroll_bwd_kernel<false>, dim3(n_ctas), dim3(kGruThreads),
-                        gru_bwd_smem_max(), st, ga);
+        if (H == MARL_H)
+            launch_pdl_prio(kGruPrio, sep ? gru_unroll_bwd_kernel<true> : gru_unroll_bwd_kernel<false>, dim3(n_ctas),
+                            dim3(kGruThreads), gru_bwd_smem_max(), st, ga);
+        else if (H == 32) gru_bwd_launch_w<32>(ga, rows, sep, st);
+        else gru_bwd_launch_w<128>(ga, rows, sep, st);
         pdl_small_problem() = keep_;
     }
     MARL_LAUNCH_CHECK();
     LinearWgrad w_fc2{}, w_hh{}, w_ih{}, w_fc1{}, w_h0{};
     LinearDgrad g_dx{};
     // dW2 += dq^T h ; db2 += colsum(dq)
-    w_fc2.dy = a->dq; w_fc2.lddy = rp * d->A; w_fc2.dy_bs = zs(d->A); w_fc2.in = plain_operand(a->hidden, rp * MARL_H, MARL_H, zs(MARL_H));
-    w_fc2.dw = a->grads.fc2_w; w_fc2.ldw = MARL_H; w_fc2.db = a->grads.fc2_b; w_fc2.M = M; w_fc2.N = d->A; w_fc2.batch = nb;
+    w_fc2.dy = a->dq; w_fc2.lddy = rp * d->A; w_fc2.dy_bs = zs(d->A); w_fc2.in = plain_operand(a->hidden, rp * H, H, zs(H));
+    w_fc2.dw = a->grads.fc2_w; w_fc2.ldw = H; w_fc2.db = a->grads.fc2_b; w_fc2.M = M; w_fc2.N = d->A; w_fc2.batch = nb;
     w_fc2.dw_bs = stride; w_fc2.db_bs = stride;
     // dW_hh += dgh^T . h_{t-1} (hidden shifted by one step, zeros at t = 0) ; db_hh
-    w_hh.dy = a->dgh; w_hh.lddy = rp * MARL_G; w_hh.dy_bs = zs(MARL_G);
+    w_hh.dy = a->dgh; w_hh.lddy = rp * G; w_hh.dy_bs = zs(G);
     {
         LinOperand in{};
-        in.x = nullptr; in.K1 = 0; in.x2 = a->hidden; in.ldx2 = rp * MARL_H; in.K2 = MARL_H; in.x2_bs = zs(MARL_H);
+        in.x = nullptr; in.K1 = 0; in.x2 = a->hidden; in.ldx2 = rp * H; in.K2 = H; in.x2_bs = zs(H);
         in.x2_shift = sep ? 1 : d->N; in.x2_period = sep ? d->L : d->L * d->N; in.onehot_mod = 0;
         w_hh.in = in;
     }
-    w_hh.dw = a->grads.w_hh; w_hh.ldw = MARL_H; w_hh.db = a->grads.b_hh; w_hh.M = M; w_hh.N = MARL_G; w_hh.batch = nb;
+    w_hh.dw = a->grads.w_hh; w_hh.ldw = H; w_hh.db = a->grads.b_hh; w_hh.M = M; w_hh.N = G; w_hh.batch = nb;
     w_hh.dw_bs = stride; w_hh.db_bs = stride;
     // the t = 0 rows see h0 instead of zeros: one [N x H] problem per episode (separated: one [B x H] problem per agent)
-    w_h0.dw = a->grads.w_hh; w_h0.ldw = MARL_H; w_h0.db = nullptr; w_h0.N = MARL_G;
+    w_h0.dw = a->grads.w_hh; w_h0.ldw = H; w_h0.db = nullptr; w_h0.N = G;
     if (sep) {
-        w_h0.dy = a->dgh; w_h0.lddy = d->L * d->N * MARL_G; w_h0.dy_bs = MARL_G;
-        w_h0.in = plain_operand(a->h0, d->N * MARL_H, MARL_H, MARL_H);
+        w_h0.dy = a->dgh; w_h0.lddy = d->L * d->N * G; w_h0.dy_bs = G;
+        w_h0.in = plain_operand(a->h0, d->N * H, H, H);
         w_h0.M = d->B; w_h0.batch = d->N; w_h0.dw_bs = stride;
     } else {
-        w_h0.dy = a->dgh; w_h0.lddy = MARL_G; w_h0.dy_bs = (long long)d->L * d->N * MARL_G;
-        w_h0.in = plain_operand(a->h0, MARL_H, MARL_H, (long long)d->N * MARL_H);
+        w_h0.dy = a->dgh; w_h0.lddy = G; w_h0.dy_bs = (long long)d->L * d->N * G;
+        w_h0.in = plain_operand(a->h0, H, H, (long long)d->N * H);
         w_h0.M = d->N; w_h0.batch = d->B;
     }
     // dW_ih += dgi^T . x ; db_ih
-    w_ih.dy = a->dgi; w_ih.lddy = rp * MARL_G; w_ih.dy_bs = zs(MARL_G); w_ih.in = plain_operand(a->x, rp * MARL_H, MARL_H, zs(MARL_H));
-    w_ih.dw = a->grads.w_ih; w_ih.ldw = MARL_H; w_ih.db = a->grads.b_ih; w_ih.M = M; w_ih.N = MARL_G; w_ih.batch = nb;
+    w_ih.dy = a->dgi; w_ih.lddy = rp * G; w_ih.dy_bs = zs(G); w_ih.in = plain_operand(a->x, rp * H, H, zs(H));
+    w_ih.dw = a->grads.w_ih; w_ih.ldw = H; w_ih.db = a->grads.b_ih; w_ih.M = M; w_ih.N = G; w_ih.batch = nb;
     w_ih.dw_bs = stride; w_ih.db_bs = stride;
     // dx = (dgi . W_ih) * (x > 0)
-    g_dx.dy = a->dgi; g_dx.lddy = rp * MARL_G; g_dx.dy_bs = zs(MARL_G); g_dx.w = a->params.w_ih; g_dx.ldw = MARL_H; g_dx.w_bs = stride;
+    g_dx.dy = a->dgi; g_dx.lddy = rp * G; g_dx.dy_bs = zs(G); g_dx.w = a->params.w_ih; g_dx.ldw = H; g_dx.w_bs = stride;
     g_dx.w_col0 = 0;
-    g_dx.dx = a->dx; g_dx.lddx = rp * MARL_H; g_dx.dx_bs = zs(MARL_H); g_dx.relu_src = a->x; g_dx.ldrs = rp * MARL_H; g_dx.rs_bs = zs(MARL_H);
-    g_dx.M = M; g_dx.N = MARL_G; g_dx.K = MARL_H; g_dx.batch = nb;
-    g_dx.wt = a->w_ih_t; g_dx.ldwt = MARL_G;      // W_ih transposed by this step's forward pass (both operands then stage with 128-bit stores)
+    g_dx.dx = a->dx; g_dx.lddx = rp * H; g_dx.dx_bs = zs(H); g_dx.relu_src = a->x; g_dx.ldrs = rp * H; g_dx.rs_bs = zs(H);
+    g_dx.M = M; g_dx.N = G; g_dx.K = H; g_dx.batch = nb;
+    g_dx.wt = a->w_ih_t; g_dx.ldwt = G;      // W_ih transposed by this step's forward pass (both operands then stage with 128-bit stores)
     // dW1 += dx^T . [obs | last_action | agent_id] ; db1
-    w_fc1.dy = a->dx; w_fc1.lddy = rp * MARL_H; w_fc1.dy_bs = zs(MARL_H);
+    w_fc1.dy = a->dx; w_fc1.lddy = rp * H; w_fc1.dy_bs = zs(H);
     w_fc1.in = sep ? separated_input(d, a->obs, a->onehot, a->shift_onehot, a->last_action, a->agent_id)
                    : agent_input(d, a->obs, a->onehot, a->shift_onehot, a->full_input, blk);
-    w_fc1.dw = a->grads.fc1_w; w_fc1.ldw = I; w_fc1.db = a->grads.fc1_b; w_fc1.M = M; w_fc1.N = MARL_H; w_fc1.batch = nb;
+    w_fc1.dw = a->grads.fc1_w; w_fc1.ldw = I; w_fc1.db = a->grads.fc1_b; w_fc1.M = M; w_fc1.N = H; w_fc1.batch = nb;
     w_fc1.dw_bs = stride; w_fc1.db_bs = stride;
 
-    if (!sep && tgemm_enabled()) {
+    if (!sep && H == MARL_H && tgemm_enabled()) {
         // TMA path (csrc/tgemm.cu): the data gradient and the three weight gradients that only need the BPTT's outputs are
         // ONE grouped launch, the fc1 weight gradient (needs dx) a second, and one deterministic reduce folds every
         // split partial into the flat gradient

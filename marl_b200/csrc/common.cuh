@@ -22,6 +22,13 @@ namespace marl {
 
 constexpr int kNumSMs = 148;
 
+// rnn_hidden_dim as a parameter struct carries it (marl_agent_params.hidden, marl_qtran_net_params.hidden): 0 means 64;
+// -1 for a width the kernels do not serve (only 32, 64 and 128 are built)
+inline int hidden_width(int hidden) {
+    const int h = hidden ? hidden : MARL_H;
+    return (h == 32 || h == MARL_H || h == 128) ? h : -1;
+}
+
 // ---- programmatic dependent launch ------------------------------------------------------------------------
 // Kernels on the step's dependent chain start with pdl_enter(): wait until the grids they depend on have completed
 // and flushed (a no-op when launched normally), then let the NEXT kernel of the stream be scheduled early -- its CTAs

@@ -545,6 +545,7 @@ bool make_map(CUtensorMap* m, const float* base, int cols, long long rows, long 
 bool front_plan(FrontArgs& a, int n_streams) {
     if (!front_enabled() || !encoder() || n_streams < 1 || n_streams > kFrontMaxStreams || a.rows <= 0) return false;
     if (a.I <= 0 || a.I > 256) return false;            // GEMM 1 keeps one main accumulator: <= 32 accumulator updates
+    if (a.hidden != MARL_H) return false;               // x [rows, 64], gi [rows, 192] and the W_ih staging are 64-wide
     for (int i = 0; i < n_streams; ++i) {
         if (!aligned16(a.s[i].gi) || !a.s[i].x || !aligned16(a.s[i].x)) return false;
         if (!aligned16(a.set[i].w_ih)) return false;

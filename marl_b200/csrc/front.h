@@ -29,12 +29,13 @@ struct FrontArgs {
     int n_sets;
     int rows;               // rows per stream
     int I;                  // input width (<= 256)
+    int hidden;             // rnn_hidden_dim: the kernel is built for 64 and declines any other width
     int tiles_per_stream;
     long long* trace;       // debug phase trace of CTA 0 (marl_tgemm_trace), else null
 };
 
 bool front_enabled();
-// false: the shapes do not qualify (I > 256, misaligned outputs) -- the caller runs the layers one by one
+// false: the shapes do not qualify (I > 256, hidden != 64, misaligned outputs) -- the caller runs the layers one by one
 bool front_plan(FrontArgs& a, int n_streams);
 int front_launch(const FrontArgs& a, int n_streams, int prio, cudaStream_t st);
 

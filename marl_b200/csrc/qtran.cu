@@ -227,7 +227,9 @@ extern "C" int marl_qtran_net_fwd(int M, int N, int S, int A_enc, int qh, const 
     if (M < 0 || N < 1 || S < 1 || A_enc < 0 || qh < 1 || !net_ok(p, ws) || !s || !hidden || !out) return MARL_EINVAL;
     if (A_enc > 0 && !actions) return MARL_EINVAL;
     if (M == 0) return MARL_OK;
-    const JointLayout l{N, S, MARL_H, A_enc, MARL_H + A_enc, qh};
+    const int H = hidden_width(p->hidden);
+    if (H < 0) return MARL_EINVAL;
+    const JointLayout l{N, S, H, A_enc, H + A_enc, qh};
     return joint_fwd(M, l, p, s, hidden, actions, ws, out, (cudaStream_t)stream);
 }
 
@@ -240,7 +242,9 @@ extern "C" int marl_qtran_net_bwd(int M, int N, int S, int A_enc, int qh, const 
     if (!dws->e1 || !dws->es || !dws->enc || !dws->a1 || !dws->a2) return MARL_EINVAL;
     if (A_enc > 0 && !actions) return MARL_EINVAL;
     if (M == 0) return MARL_OK;
-    const JointLayout l{N, S, MARL_H, A_enc, MARL_H + A_enc, qh};
+    const int H = hidden_width(p->hidden);
+    if (H < 0) return MARL_EINVAL;
+    const JointLayout l{N, S, H, A_enc, H + A_enc, qh};
     return joint_bwd(M, l, p, s, hidden, actions, ws, dout, dws, dhidden, accumulate_dhidden, g, (cudaStream_t)stream);
 }
 

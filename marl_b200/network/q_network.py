@@ -16,17 +16,26 @@ import torch.nn as nn
 from .. import _lib as L
 from ..flat import FlatBuffer, FlatPackedMixin
 
-H = 64
+HIDDEN_WIDTHS = (32, 64, 128)     # rnn_hidden_dim values the recurrence and acting kernels are built for
 
 AGENT_FLAT_ORDER = ("fc1.weight", "fc1.bias", "rnn.weight_ih", "rnn.weight_hh", "rnn.bias_ih", "rnn.bias_hh",
                     "fc2.weight", "fc2.bias")
 
 
-def agent_param_struct(named, cls=L.AgentParams):
-    """named: dict name -> device address, in AGENT_FLAT_ORDER naming."""
+def check_hidden(hidden):
+    """rnn_hidden_dim as the kernels take it; ValueError for any width they are not built for."""
+    if hidden not in HIDDEN_WIDTHS:
+        raise ValueError(f"libmarl_b200 supports rnn_hidden_dim in {HIDDEN_WIDTHS}, got {hidden}")
+    return int(hidden)
+
+
+def agent_param_struct(named, cls=L.AgentParams, hidden=64):
+    """named: dict name -> device address, in AGENT_FLAT_ORDER naming; hidden = rnn_hidden_dim (parameter structs only)."""
     s = cls()
     for field, name in zip(L.AGENT_KEYS, AGENT_FLAT_ORDER):
         setattr(s, field, named[name])
+    if cls is L.AgentParams:
+        s.hidden = hidden
     return s
 
 
@@ -38,6 +47,7 @@ class _UnrollFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, obs, onehot, h0, shift, full_input, dims, blocks, *params):
         B, Lq, N, A, O = dims
+        H = params[0].shape[0]                       # fc1.weight [H, I]
         dev = obs.device
         rows = B * Lq * N
         d = L.Dims(B, Lq, N, A, O, 0)
@@ -53,7 +63,7 @@ class _UnrollFn(torch.autograd.Function):
         st.obs, st.onehot = obs.data_ptr(), (None if onehot is None else onehot.data_ptr())
         st.shift_onehot, st.full_input, st.h0_from = int(shift), int(full_input), -1
         st.h0 = None if h0 is None else h0.data_ptr()
-        st.params = agent_param_struct({n: p.data_ptr() for n, p in zip(AGENT_FLAT_ORDER, params)})
+        st.params = agent_param_struct({n: p.data_ptr() for n, p in zip(AGENT_FLAT_ORDER, params)}, hidden=H)
         st.q, st.hidden, st.h_last = q.data_ptr(), hidden.data_ptr(), h_last.data_ptr()
         st.x, st.gi, st.gates = x.data_ptr(), gi.data_ptr(), gates.data_ptr()
         st.w_ih_t = w_ih_t.data_ptr()
@@ -71,6 +81,7 @@ class _UnrollFn(torch.autograd.Function):
         dims, shift, full_input, no_onehot, had_h0, blocks = ctx.meta
         obs, onehot, h0, hidden, x, gates, w_ih_t, *params = ctx.saved_tensors
         B, Lq, N, A, O = dims
+        H = params[0].shape[0]
         dev = obs.device
         rows = B * Lq * N
         f32 = dict(dtype=torch.float32, device=dev)
@@ -78,7 +89,7 @@ class _UnrollFn(torch.autograd.Function):
         a = L.UnrollBwd()
         a.obs, a.onehot = obs.data_ptr(), (None if no_onehot else onehot.data_ptr())
         a.shift_onehot, a.full_input = shift, full_input
-        a.params = agent_param_struct({n: p.data_ptr() for n, p in zip(AGENT_FLAT_ORDER, params)})
+        a.params = agent_param_struct({n: p.data_ptr() for n, p in zip(AGENT_FLAT_ORDER, params)}, hidden=H)
         a.hidden, a.x, a.gates = hidden.data_ptr(), x.data_ptr(), gates.data_ptr()
         a.w_ih_t = w_ih_t.data_ptr()
         if blocks is not None:
@@ -101,8 +112,7 @@ class RNNQNet(FlatPackedMixin, nn.Module):
     def __init__(self, input_shape, args):
         super().__init__()
         self.args = args
-        if args.rnn_hidden_dim != H:
-            raise ValueError("libmarl_b200 is specialised for rnn_hidden_dim = 64")
+        H = self.hidden = check_hidden(args.rnn_hidden_dim)
         self.input_shape = input_shape
         self.fc1 = nn.Linear(input_shape, H)
         self.rnn = nn.GRUCell(H, H)
@@ -127,12 +137,17 @@ class RNNQNet(FlatPackedMixin, nn.Module):
         self._pack(self.fc1.weight.device)
         return out
 
+    def param_struct(self):
+        """marl_agent_params of this network's parameters."""
+        return agent_param_struct(self.param_addresses(), hidden=self.hidden)
+
     def param_addresses(self):
         return {n: p.data_ptr() for n, p in self.flat_named_parameters()}
 
     # ---- reference surface ----------------------------------------------------------------------
     def forward(self, obs, hidden_state):
-        """obs [R, input_shape] (already [obs | last_action | agent_id]); hidden_state [..., 64]."""
+        """obs [R, input_shape] (already [obs | last_action | agent_id]); hidden_state [..., H]."""
+        H = self.hidden
         obs = L.require_cuda(obs, "obs").to(torch.float32).contiguous()
         h_in = hidden_state.reshape(-1, H).to(torch.float32).contiguous()
         R = obs.shape[0]

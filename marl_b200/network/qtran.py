@@ -12,14 +12,17 @@ import torch.nn as nn
 from .. import _lib as L
 from ..flat import FlatBuffer, FlatPackedMixin
 
-H = 64
+from .q_network import check_hidden
 
 
-def net_struct(addrs, cls=L.QtranNetParams):
-    """addrs: the 10 device addresses in parameter order (we1, be1, we2, be2, w0, b0, w2, b2, w4, b4)."""
+def net_struct(addrs, cls=L.QtranNetParams, hidden=64):
+    """addrs: the 10 device addresses in parameter order (we1, be1, we2, be2, w0, b0, w2, b2, w4, b4); hidden =
+    rnn_hidden_dim (parameter structs only)."""
     s = cls()
     for f, a in zip(L.QTRAN_FIELDS, addrs):
         setattr(s, f, a)
+    if cls is L.QtranNetParams:
+        s.hidden = hidden
     return s
 
 
@@ -37,10 +40,10 @@ def net_ws_struct(ws):
 class _JointNetFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, s, hidden, actions, meta, *params):
-        M, N, S, A_enc, qh = meta
+        M, N, S, A_enc, qh, H = meta
         ws = net_workspace(M, N, H + A_enc, qh, s.device)
         out = torch.empty(M, 1, dtype=torch.float32, device=s.device)
-        p = net_struct([t.data_ptr() for t in params])
+        p = net_struct([t.data_ptr() for t in params], hidden=H)
         wss = net_ws_struct(ws)
         L.call("marl_qtran_net_fwd", M, N, S, A_enc, qh, C.byref(p), s.data_ptr(), hidden.data_ptr(), L.ptr(actions),
                C.byref(wss), out.data_ptr(), L.stream_ptr())
@@ -50,13 +53,13 @@ class _JointNetFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, dout):
-        M, N, S, A_enc, qh = ctx.meta
+        M, N, S, A_enc, qh, H = ctx.meta
         s, hidden, actions, *params = ctx.saved_tensors
         dev = s.device
         grads = [torch.zeros_like(t) for t in params]
         dws = net_workspace(M, N, H + A_enc, qh, dev)
         dhidden = torch.empty(M * N, H, dtype=torch.float32, device=dev)
-        p = net_struct([t.data_ptr() for t in params])
+        p = net_struct([t.data_ptr() for t in params], hidden=H)
         g = net_struct([t.data_ptr() for t in grads], L.QtranNetGrads)
         wss, dwss = net_ws_struct(ctx.ws), net_ws_struct(dws)
         L.call("marl_qtran_net_bwd", M, N, S, A_enc, qh, C.byref(p), s.data_ptr(), hidden.data_ptr(),
@@ -87,10 +90,11 @@ class _JointNet(FlatPackedMixin, nn.Module):
     def _run(self, state, hidden, actions):
         B, T, N, _ = hidden.shape
         a = self.args
+        H = a.rnn_hidden_dim
         s = L.require_cuda(state, "state").reshape(B * T, -1).to(torch.float32).contiguous()
         h = L.require_cuda(hidden, "hidden").reshape(B * T * N, H).to(torch.float32).contiguous()
         act = None if actions is None else actions.reshape(B * T * N, -1).to(torch.float32).contiguous()
-        meta = (B * T, N, a.state_shape, 0 if act is None else a.n_actions, a.qtran_hidden_dim)
+        meta = (B * T, N, a.state_shape, 0 if act is None else a.n_actions, a.qtran_hidden_dim, H)
         return _JointNetFn.apply(s, h, act, meta, *[p for _, p in self.named_parameters()])
 
 
@@ -100,6 +104,7 @@ class QtranQBase(_JointNet):
     def __init__(self, args):
         super().__init__()
         self.args = args
+        check_hidden(args.rnn_hidden_dim)
         ae_input = args.rnn_hidden_dim + args.n_actions
         qh = args.qtran_hidden_dim
         self.hidden_action_encoding = nn.Sequential(nn.Linear(ae_input, ae_input), nn.ReLU(), nn.Linear(ae_input, ae_input))
@@ -117,7 +122,7 @@ class QtranV(_JointNet):
     def __init__(self, args):
         super().__init__()
         self.args = args
-        hd, qh = args.rnn_hidden_dim, args.qtran_hidden_dim
+        hd, qh = check_hidden(args.rnn_hidden_dim), args.qtran_hidden_dim
         self.hidden_encoding = nn.Sequential(nn.Linear(hd, hd), nn.ReLU(), nn.Linear(hd, hd))
         self.v = nn.Sequential(nn.Linear(args.state_shape + hd, qh), nn.ReLU(), nn.Linear(qh, qh), nn.ReLU(), nn.Linear(qh, 1))
         self._finish()
