@@ -161,6 +161,15 @@ typedef struct marl_unroll_stream {
 int marl_episode_lengths(const float* padded, int B, int L, int* ep_len, void* stream);
 
 int marl_agent_unroll_fwd(const marl_dims* d, const marl_unroll_stream* streams, int n_streams, void* stream);
+/* Split forward of a latency-bound double-Q call: three streams of the shared network at H = 64, one continuing another through
+ * h0_from (the continued one with an h_last), none cut at its episode's end (no ep_len / padded / row_order / row_order_bwd) and
+ * B*N <= 170.  marl_agent_unroll_fwd then runs the input layers of the continued chain's head and of the other two streams
+ * as two launches side by side, the head's recurrence (level 0) and the lone chain's on disjoint SMs, and the continuation (level
+ * 1) from level 0's h_last: five launches instead of two, bit-identical results.  marl_agent_unroll_fwd_split returns 1 when a
+ * call with these arguments takes it, 0 otherwise (MARL_EINVAL for invalid dims).  marl_fwd_split_enable: the A/B switch
+ * (default on, MARL_B200_FWD_SPLIT=0 turns it off); returns the previous setting.  No reference counterpart. */
+int marl_agent_unroll_fwd_split(const marl_dims* d, const marl_unroll_stream* streams, int n_streams);
+int marl_fwd_split_enable(int on);
 
 /* BPTT of one unroll (autograd of share_params.py:125-146 as triggered by
  * loss.backward(), q_learner.py:171).  dq [B,L,N,A] and dhidden [B,L,N,H] (either may be NULL) are

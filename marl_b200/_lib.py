@@ -141,6 +141,8 @@ _SIGNATURES = {
     "marl_replay_gather_f32": ([_P(EpisodeF32), C.c_int, c_ptr, _P(Dims), _P(EpisodeF32), c_ptr], C.c_int),
     "marl_fma_probe": ([c_ptr, C.c_int, C.c_int, _P(C.c_double), c_ptr], C.c_int),
     "marl_agent_unroll_fwd": ([_P(Dims), _P(UnrollStream), C.c_int, c_ptr], C.c_int),
+    "marl_agent_unroll_fwd_split": ([_P(Dims), _P(UnrollStream), C.c_int], C.c_int),
+    "marl_fwd_split_enable": ([C.c_int], C.c_int),
     "marl_agent_unroll_bwd": ([_P(Dims), _P(UnrollBwd), c_ptr], C.c_int),
     "marl_q_select": ([_P(Dims)] + [c_ptr] * 12 + [c_ptr], C.c_int),
     "marl_td_loss": ([C.c_int] + [c_ptr] * 5 + [C.c_float, c_ptr, c_ptr, c_ptr], C.c_int),

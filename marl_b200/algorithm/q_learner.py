@@ -518,8 +518,10 @@ class QLearner:
             s.w_ih_t = ws["w_ih_t"].data_ptr() if u.keep and not sep else None    # W_ih^T for the backward's data gradient
             s.agent_stride, s.last_action, s.agent_id, s.input_flags = stride, last_action, agent_id, int(not sep)
         L.call("marl_agent_unroll_fwd", C.byref(d), arr, len(plan), L.stream_ptr())
-        # + episode lengths and row orders, launched by marl_agent_unroll_fwd beside the input layers
-        return (3 if heads else 2) * len(plan) + 1 + (2 if early else 0)
+        # + episode lengths and row orders, launched by marl_agent_unroll_fwd beside the input layers; the split forward
+        # (include/marl_b200.h) launches the input layers twice and the recurrence three times
+        split = L.load().marl_agent_unroll_fwd_split(C.byref(d), arr, len(plan)) == 1
+        return (3 if heads else 2) * len(plan) + 1 + (2 if early else 0) + (3 if split else 0)
 
     def _agent_backward(self, bt, ws, d, early, dhidden=None, dhext_ready=False, join=None):
         """BPTT through stream 0 (which kept its gates) from ws["dq"] and `dhidden`.  `dhext_ready`: the mixing kernel wrote

@@ -1137,9 +1137,186 @@ static LinOperand agent_input(const marl_dims* d, const float* obs, const float*
     return in;
 }
 
+// Fused input layers (csrc/front.cu) of the streams idx[0 .. n) of a shared-network call, as stream k of the launch
+static FrontArgs front_args(const marl_dims* d, const marl_unroll_stream* s, const int* idx, int n, int I, int H) {
+    FrontArgs fa{};
+    fa.rows = d->B * d->L * d->N; fa.I = I; fa.hidden = H;
+    for (int k = 0; k < n; ++k) {
+        const marl_unroll_stream& u = s[idx[k]];
+        fa.s[k].in = agent_input(d, u.obs, u.onehot, u.shift_onehot, u.full_input, input_blocks(0, u.input_flags, u.last_action, u.agent_id));
+        fa.s[k].x = u.x; fa.s[k].gi = u.gi;
+        fa.s[k].store_x = u.gates != nullptr;
+        fa.set[k].w1 = u.params.fc1_w; fa.set[k].b1 = u.params.fc1_b;
+        fa.set[k].w_ih = u.params.w_ih; fa.set[k].b_ih = u.params.b_ih;
+        fa.set[k].w_ih_t = u.w_ih_t;
+    }
+    return fa;
+}
+
+// ---- split forward -----------------------------------------------------------------------------------------------------------
+// A double-Q step (eval on o, target on o_next, eval on o_next continued from the first) at a few hundred agent rows is one
+// latency-bound chain: input layers of all three streams -> the 240-step eval chain.  Only the eval/o stream feeds the first 120
+// steps, so the forward is split into two levels on disjoint SMs:
+//   main lane:    A = input layers of eval/o (~half the SMs, at most two tiles each) -> level 0 = eval/o chain (two rows per CTA)
+//                 -> [waits for B] -> level 1 = eval/o_next chain from level 0's h_last
+//   forked lane:  B = input layers of the two o_next streams (the other SMs) -> D = target chain (on the SMs B frees)
+// A front CTA fills an SM's shared memory, and every recurrence CTA of the split reserves all of it (kernel shared memory size
+// below), so no two of these kernels -- nor a GEMM CTA of another stream -- ever share an SM.  Every row is computed by the same
+// code on the same inputs as in the one-launch plan: results are bit-identical.
+#ifndef MARL_FWD_SPLIT_MAX_ROWS
+#define MARL_FWD_SPLIT_MAX_ROWS 170
+#endif
+// B*N: the SMs a level launch leaves (148 - B*N/2) carry the input layers of the two o_next streams, which must end before level
+// 0 does, then the target chain at two rows per thread group (which holds up to 196 rows).  Measured on a B200 at T = 120
+// (tools/fwd_split_bench.py, profiles/r10_bench_parent_vs_pr.txt): QMIX step -6.8 % at 160 rows, -0.4 % at 180, +2.5 % at 195
+constexpr int kFwdSplitMaxRows = MARL_FWD_SPLIT_MAX_ROWS;
+static int g_split_on = -1;
+static bool fwd_split_enabled() {
+    if (g_split_on < 0) { const char* e = getenv("MARL_B200_FWD_SPLIT"); g_split_on = (e && e[0] == '0') ? 0 : 1; }
+    return g_split_on == 1;
+}
+
+struct SplitPlan {
+    int head, cont, other;       // streams: the continued chain's head (eval/o), its continuation (eval/o_next), the lone chain (target)
+    int n_level, n_target;       // recurrence CTAs of each level and of the target chain
+    FrontArgs fa, fb;            // input layers of `head` / of `other` and `cont`
+};
+
+// The split applies to a shared-network (H = 64) call of exactly three streams, one continuing another, none cut at its episode's
+// end, with B*N <= kFwdSplitMaxRows and the fused input-layer kernel available; every other call keeps the one-launch plan.
+static bool split_plan(const marl_dims* d, const marl_unroll_stream* s, int n_streams, SplitPlan& p) {
+    if (!fwd_split_enabled() || n_streams != 3) return false;
+    const int rows = d->B * d->N;
+    if (rows > kFwdSplitMaxRows) return false;
+    p.cont = -1;
+    for (int i = 0; i < n_streams; ++i) {
+        const marl_unroll_stream& u = s[i];
+        if (u.agent_stride || hidden_width(u.params.hidden) != MARL_H || u.full_input) return false;
+        if (u.ep_len || u.padded || u.row_order || u.row_order_bwd) return false;
+        if (u.h0_from >= 0) { if (p.cont >= 0) return false; p.cont = i; }
+    }
+    if (p.cont < 0) return false;
+    p.head = s[p.cont].h0_from;
+    p.other = 3 - p.head - p.cont;
+    if (s[p.head].h0_from >= 0 || !s[p.head].h_last) return false;     // level 1 starts from level 0's h_last
+    const InputBlocks b0 = input_blocks(0, s[0].input_flags, s[0].last_action, s[0].agent_id);
+    const int I = agent_input_width(d, b0);
+    for (int i = 1; i < n_streams; ++i)
+        if (agent_input_width(d, input_blocks(0, s[i].input_flags, s[i].last_action, s[i].agent_id)) != I) return false;
+    p.n_level = (rows + 1) / 2;
+    const int spare = kNumSMs - p.n_level;          // SMs beside a level launch: B's front, then the target chain
+    if (spare < 2) return false;
+    const int idx_b[2] = {p.other, p.cont};
+    p.fb = front_args(d, s, idx_b, 2, I, MARL_H);
+    if (!front_plan(p.fb, 2, spare)) return false;
+    int grid_b = 0;
+    for (int k = 0; k < p.fb.n_sets; ++k) grid_b += p.fb.set[k].n_ctas;
+    p.fa = front_args(d, s, &p.head, 1, I, MARL_H);
+    if (!front_plan(p.fa, 1, kNumSMs - grid_b)) return false;
+    // the target chain: two thread groups per CTA with at most two rows each, on the fewest CTAs that allow it
+    const int per = (rows + 2 * spare - 1) / (2 * spare);
+    if (per > 2) return false;
+    p.n_target = (rows + 2 * per - 1) / (2 * per);
+    return true;
+}
+
+// The rows of one stream (continued from h0) as `parts` chains, one per thread group of a CTA (two at most): chain c takes the
+// episodes [B c / parts, B (c + 1) / parts), addressed through offset pointers, its rows dealt over n_ctas CTAs by water-filling
+// on the rows a CTA already carries
+static GruFwdArgs single_chain(const marl_dims* d, const marl_unroll_stream& u, const float* h0, int n_ctas, int parts) {
+    GruFwdArgs g{};
+    g.B = d->B; g.L = d->L; g.N = d->N;
+    g.n_chains = parts;
+    double load[kNumSMs] = {};
+    for (int c = 0; c < parts; ++c) {
+        const int b0 = d->B * c / parts, b1 = d->B * (c + 1) / parts;
+        const long long step = (long long)b0 * d->L * d->N, row = (long long)b0 * d->N;      // first (b, t, n) / (b, n) of the slice
+        g.chain_start[c] = c; g.chain_len[c] = 1;
+        g.h0[c] = h0 ? h0 + row * MARL_H : nullptr;
+        g.seg[c] = GruSegment{u.gi + step * MARL_G, u.params.w_hh, u.params.b_hh, u.hidden + step * MARL_H,
+                              u.gates ? u.gates + step * 4 * MARL_H : nullptr, u.h_last ? u.h_last + row * MARL_H : nullptr, u.ep_len};
+        int cnt[kNumSMs] = {};
+        water_fill(load, 0, n_ctas, (b1 - b0) * d->N, 1.0, cnt);
+        for (int i = 0; i < n_ctas; ++i) { g.rows_of[c][i] = (unsigned short)cnt[i]; load[i] += cnt[i]; }
+    }
+    g.trace = trace_buffer();
+    return g;
+}
+
+// the dynamic shared memory the H = 64 forward kernel may be launched with: raised to the largest size asked for so far
+static void gru_fwd_smem_attr(size_t bytes) {
+    static size_t cur = 0;
+    if (bytes <= cur) return;
+    cudaFuncSetAttribute(gru_unroll_fwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    cudaFuncSetAttribute(gru_unroll_fwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    cur = bytes;
+}
+
+// A recurrence launch of the split forward: it reserves the whole of the SM's shared memory, so that nothing runs beside it
+static void gru_fwd_launch_solo(const GruFwdArgs& ga, int n_ctas, bool pdl, cudaStream_t st) {
+    static size_t solo = 0;
+    if (!solo) {
+        int dev = 0, optin = 0;
+        cudaGetDevice(&dev);
+        cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+        cudaFuncAttributes fa{};
+        cudaFuncGetAttributes(&fa, gru_unroll_fwd_kernel<false>);
+        solo = (size_t)optin - fa.sharedSizeBytes;
+    }
+    gru_fwd_smem_attr(solo);
+    ProfScope ps_("gru_unroll_fwd_kernel", st);
+    const bool keep_ = pdl_small_problem();
+    pdl_small_problem() = keep_ && pdl;
+    launch_pdl_prio(kGruPrio, gru_unroll_fwd_kernel<false>, dim3(n_ctas, (ga.n_chains + kGruGroups - 1) / kGruGroups),
+                    dim3(kGruThreads * kGruGroups), solo, st, ga);
+    pdl_small_problem() = keep_;
+}
+
+static int split_forward(const marl_dims* d, const marl_unroll_stream* s, const SplitPlan& p, cudaStream_t st) {
+    static cudaEvent_t ev_b[8];
+    static int ring = -1;
+    if (ring < 0) { for (auto& e : ev_b) cudaEventCreateWithFlags(&e, cudaEventDisableTiming); ring = 0; }
+    ring = (ring + 1) & 7;
+    ForkJoin fj(st, 2);
+    cudaStream_t side = fj.lane(1);
+    int rc = front_launch(p.fa, 1, kGruPrio, st);                  // A
+    if (rc) return rc;
+    if ((rc = front_launch(p.fb, 2, kGruPrio, side))) return rc;    // B
+    cudaEventRecord(ev_b[ring], side);
+    // level 0 behind A (programmatic: its CTAs take A's SMs as A's CTAs leave)
+    gru_fwd_launch_solo(single_chain(d, s[p.head], s[p.head].h0, p.n_level, 1), p.n_level, true, st);
+    MARL_LAUNCH_CHECK();
+    // the target chain behind B, on the SMs B frees: its rows in two slices, one per thread group, at most two rows per group
+    // (a single group with three rows, the four-row pass, takes twice as long per step as one with two)
+    gru_fwd_launch_solo(single_chain(d, s[p.other], s[p.other].h0, p.n_target, 2), p.n_target, true, side);
+    MARL_LAUNCH_CHECK();
+    // level 1 from level 0's final hidden state.  A plain launch: launched programmatically its CTAs would become resident beside
+    // level 0 as soon as B ends and take the SMs the target chain is about to use
+    cudaStreamWaitEvent(st, ev_b[ring], 0);
+    gru_fwd_launch_solo(single_chain(d, s[p.cont], s[p.head].h_last, p.n_level, 1), p.n_level, false, st);
+    MARL_LAUNCH_CHECK();
+    fj.join();
+    return MARL_OK;
+}
+
 }  // namespace marl
 
 using namespace marl;
+
+// A/B switch of the split forward (MARL_B200_FWD_SPLIT, default on); returns the previous setting
+extern "C" int marl_fwd_split_enable(int on) {
+    const int prev = fwd_split_enabled() ? 1 : 0;
+    g_split_on = on ? 1 : 0;
+    return prev;
+}
+
+// 1 when marl_agent_unroll_fwd would run these streams as the split forward (five launches for the input layers and the
+// recurrence instead of two), 0 otherwise
+extern "C" int marl_agent_unroll_fwd_split(const marl_dims* d, const marl_unroll_stream* s, int n_streams) {
+    if (check_dims(d) || !s || n_streams < 1 || n_streams > kMaxStreams) return MARL_EINVAL;
+    SplitPlan p;
+    return split_plan(d, s, n_streams, p) ? 1 : 0;
+}
 
 extern "C" int marl_episode_lengths(const float* padded, int B, int L, int* ep_len, void* stream) {
     if (!padded || !ep_len || B <= 0 || L <= 0) return MARL_EINVAL;
@@ -1275,19 +1452,17 @@ extern "C" int marl_agent_unroll_fwd(const marl_dims* d, const marl_unroll_strea
         return agent_layer(d, in, s[i].params.w_ih, H, s[i].params.b_ih, s[i].gi, G, stride);
     };
     bool grouped = false;
-    if (!sep) {      // (the fused input-layer kernel stages one shared weight set: separated streams take the unfused path)
+    SplitPlan split;
+    const bool split_on = split_plan(d, s, n_streams, split);
+    if (split_on) {
+        const int rc = split_forward(d, s, split, st);
+        if (rc) return rc;
+        grouped = true;
+    } else if (!sep) {      // (the fused input-layer kernel stages one shared weight set: separated streams take the unfused path)
         // fused path (csrc/front.cu): both layers of every stream in ONE persistent launch, x handed from the first GEMM to the
         // second through tensor memory
-        FrontArgs fa{};
-        fa.rows = rows_total; fa.I = I; fa.hidden = H;
-        for (int i = 0; i < n_streams; ++i) {
-            fa.s[i].in = agent_input(d, s[i].obs, s[i].onehot, s[i].shift_onehot, s[i].full_input, blocks(i));
-            fa.s[i].x = s[i].x; fa.s[i].gi = s[i].gi;
-            fa.s[i].store_x = s[i].gates != nullptr;
-            fa.set[i].w1 = s[i].params.fc1_w; fa.set[i].b1 = s[i].params.fc1_b;
-            fa.set[i].w_ih = s[i].params.w_ih; fa.set[i].b_ih = s[i].params.b_ih;
-            fa.set[i].w_ih_t = s[i].w_ih_t;
-        }
+        const int idx[kMaxStreams] = {0, 1, 2, 3};
+        FrontArgs fa = front_args(d, s, idx, n_streams, I, H);
         if (front_plan(fa, n_streams)) {
             const int rc = front_launch(fa, n_streams, kGruPrio, st);
             if (rc) return rc;
@@ -1332,19 +1507,14 @@ extern "C" int marl_agent_unroll_fwd(const marl_dims* d, const marl_unroll_strea
         }
         fa.join();
     }
-    {
+    if (!split_on) {
         // one CTA per SM; each CTA advances its share of every chain side by side (one 128-thread group per chain)
         ProfScope ps_("gru_unroll_fwd_kernel", st);
         ga.trace = trace_buffer();
         if (order_lane) order_lane->join();
         if (H == MARL_H) {
             const size_t sm = kGruGroups * gru_fwd_smem(kGruMaxRows);
-            static bool attr_set = false;
-            if (!attr_set) {
-                cudaFuncSetAttribute(gru_unroll_fwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-                cudaFuncSetAttribute(gru_unroll_fwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-                attr_set = true;
-            }
+            gru_fwd_smem_attr(sm);
             dim3 grid(n_ctas, (ga.n_chains + kGruGroups - 1) / kGruGroups);
             launch_pdl_prio(kGruPrio, sep ? gru_unroll_fwd_kernel<true> : gru_unroll_fwd_kernel<false>, grid,
                             dim3(kGruThreads * kGruGroups), sm, st, ga);

@@ -542,7 +542,9 @@ bool make_map(CUtensorMap* m, const float* base, int cols, long long rows, long 
 // Groups the streams into parameter sets and deals the CTAs of the grid to the sets in proportion to their tiles.
 // a.s[0 .. n_streams), a.rows, a.I are filled by the caller, together with one FrontSet per stream in a.set[i]
 // (w1 / b1 / w_ih / b_ih of stream i); this merges equal sets.
-bool front_plan(FrontArgs& a, int n_streams) {
+// budget > 0: at most that many CTAs, and every set keeps only as many as its fullest CTA's tile count needs -- a launch that
+// shares the machine with another one (marl_agent_unroll_fwd's split forward) leaves the SMs it could not use to the other.
+bool front_plan(FrontArgs& a, int n_streams, int budget) {
     if (!front_enabled() || !encoder() || n_streams < 1 || n_streams > kFrontMaxStreams || a.rows <= 0) return false;
     if (a.I <= 0 || a.I > 256) return false;            // GEMM 1 keeps one main accumulator: <= 32 accumulator updates
     if (a.hidden != MARL_H) return false;               // x [rows, 64], gi [rows, 192] and the W_ih staging are 64-wide
@@ -568,7 +570,9 @@ bool front_plan(FrontArgs& a, int n_streams) {
     }
     a.tiles_per_stream = (a.rows + FM - 1) / FM;
     const long long total = (long long)n_streams * a.tiles_per_stream;
-    const int grid = (int)(total < kNumSMs ? total : kNumSMs);
+    const int cap = budget > 0 && budget < kNumSMs ? budget : kNumSMs;
+    if (cap < ns) return false;
+    const int grid = (int)(total < cap ? total : cap);
     int ctas[kFrontMaxStreams];
     for (int k = 0; k < ns; ++k) ctas[k] = 1;
     for (int left = grid - ns; left > 0; --left) {       // the next CTA goes to the set with the most tiles per CTA
@@ -577,6 +581,11 @@ bool front_plan(FrontArgs& a, int n_streams) {
             if ((double)sets[k].n_streams / ctas[k] > (double)sets[best].n_streams / ctas[best]) best = k;
         ++ctas[best];
     }
+    if (budget > 0)
+        for (int k = 0; k < ns; ++k) {                   // fewest CTAs at the same tiles per CTA (150 tiles on 80 CTAs: 75 x 2)
+            const int t = sets[k].n_streams * a.tiles_per_stream, per = (t + ctas[k] - 1) / ctas[k];
+            ctas[k] = (t + per - 1) / per;
+        }
     int c0 = 0;
     for (int k = 0; k < ns; ++k) { sets[k].cta0 = c0; sets[k].n_ctas = ctas[k]; c0 += ctas[k]; a.set[k] = sets[k]; }
     a.n_sets = ns;

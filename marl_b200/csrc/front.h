@@ -35,8 +35,9 @@ struct FrontArgs {
 };
 
 bool front_enabled();
-// false: the shapes do not qualify (I > 256, hidden != 64, misaligned outputs) -- the caller runs the layers one by one
-bool front_plan(FrontArgs& a, int n_streams);
+// false: the shapes do not qualify (I > 256, hidden != 64, misaligned outputs) -- the caller runs the layers one by one.
+// budget: 0 = up to one CTA per SM; > 0 = at most that many CTAs, trimmed to the fewest that keep the tiles per CTA
+bool front_plan(FrontArgs& a, int n_streams, int budget = 0);
 int front_launch(const FrontArgs& a, int n_streams, int prio, cudaStream_t st);
 
 }  // namespace marl
