@@ -11,31 +11,44 @@
 namespace marl {
 
 constexpr int kActThreads = 256;
-constexpr int kActRows = 32;       // rows per tile: thread (jg, rg) owns rows {rg, rg + 16} x columns {jg + 16 c}
-constexpr int kActKC = 32;         // input columns staged per chunk
-constexpr int kHP = MARL_H + 1;    // odd row stride of the 64-wide operands: 16 column groups read 16 distinct banks
+constexpr int kActRows = 32;       // rows per tile: thread (jg, rg) owns rows {rg, rg + 16} x columns {jg + 16 c}, c < H / 16
+constexpr int kActKC = 32;         // input columns staged per chunk (resident weights)
+constexpr int kActWC = 16;         // reduction columns per staged weight chunk (streamed weights)
+
+// Where fc1, W_ih and W_hh are read from.  Resident (H = 64): the whole parameter set is staged once per set, rows at an odd
+// pitch; the input width is capped by what fits on chip (MARL_EINVAL past it).  Streamed (H = 32, 128): only the biases and fc2
+// stay resident and the three matrices pass through shared memory in kActWC-column chunks per tile (at H = 128 the two GRU
+// matrices alone, 2 x 384 x 129 floats, pass the 227 KB a block may hold); any input width runs, which is why H = 32 streams too.
+constexpr bool act_resident(int H) { return H == MARL_H; }
 
 // Shared-memory carve-up (in floats).  Every weight stays in its global [out, in] layout; rows are padded to an odd stride.
+// Streamed: w1 / wih point into one chunk region (W_ih | W_hh chunks [3H, WC] each, the fc1 chunk [H, WC] in the first part).
 struct ActLayout {
     int I, Ip, A, qw;
     int w1, b1, wih, whh, bih, bhh, w2, b2, in, xq, h, total;
 };
 
-inline ActLayout act_layout(int I, int A) {
+inline ActLayout act_layout(int H, int I, int A) {
     ActLayout l;
-    l.I = I; l.Ip = I | 1; l.A = A; l.qw = A > kHP ? A : kHP;
+    const int hp = H + 1, wp = kActWC + 1;
+    l.I = I; l.Ip = I | 1; l.A = A; l.qw = A > hp ? A : hp;
     int o = 0;
-    l.w1 = o;  o += MARL_H * l.Ip;
-    l.b1 = o;  o += MARL_H;
-    l.wih = o; o += MARL_G * kHP;
-    l.whh = o; o += MARL_G * kHP;
-    l.bih = o; o += MARL_G;
-    l.bhh = o; o += MARL_G;
-    l.w2 = o;  o += A * kHP;
+    if (act_resident(H)) {
+        l.w1 = o;  o += H * l.Ip;
+        l.b1 = o;  o += H;
+        l.wih = o; o += 3 * H * hp;
+        l.whh = o; o += 3 * H * hp;
+    } else {
+        l.w1 = l.wih = o; l.whh = o + 3 * H * wp; o += 2 * 3 * H * wp;
+        l.b1 = o;  o += H;
+    }
+    l.bih = o; o += 3 * H;
+    l.bhh = o; o += 3 * H;
+    l.w2 = o;  o += A * hp;
     l.b2 = o;  o += A;
-    l.in = o;  o += kActRows * (kActKC + 1);
+    l.in = o;  o += kActRows * ((act_resident(H) ? kActKC : kActWC) + 1);
     l.xq = o;  o += kActRows * l.qw;      // relu(fc1) tile, then the q tile
-    l.h = o;   o += kActRows * kHP;
+    l.h = o;   o += kActRows * hp;
     l.total = o;
     return l;
 }
@@ -58,14 +71,13 @@ struct ActPhilox {
     const double* eps_table; int eps_len;
 };
 
-// The uniform form's random action: the min(floor(u * cnt), cnt - 1)-th of the cnt available actions, 0 when cnt == 0.
-// The Philox form calls it; the uniform form keeps its own copy inline in agent_act_kernel, so that its code is what it
-// was before the Philox form existed.
-__device__ __forceinline__ int kth_available(const float* av, int A, int cnt, double u) {
+// The random action of the exploration forms: the min(floor(u * cnt), cnt - 1)-th of the cnt available actions, 0 when cnt == 0.
+// (u is read only when cnt > 0: the uniform form loads its choice_u entry only then)
+__device__ __forceinline__ int kth_available(const float* av, int A, int cnt, const double* u) {
     int best = 0;
     if (cnt > 0) {
         const double c = (double)cnt;
-        const int kth = (int)fmin(floor(u * c), c - 1.0);
+        const int kth = (int)fmin(floor(*u * c), c - 1.0);
         for (int k = 0, seen = 0; k < A; ++k)
             if (!av || av[k] != 0.0f) {
                 if (seen == kth) { best = k; break; }
@@ -84,27 +96,38 @@ struct ActParams { marl_agent_params p[kSets]; };
 // kSets > 1: agent n's own weights; a tile is up to 32 instances of ONE agent (rows e*N + n), tiles are agent-major and
 // every CTA takes a contiguous range of them, so it restages weights only when its agent changes.
 // kPhilox: exploration from ph (a's four exploration pointers are NULL); otherwise ph is not read.
-template <int kSets, bool kPhilox>
-__global__ void __launch_bounds__(kActThreads) agent_act_kernel(const __grid_constant__ ActParams<kSets> ps, ActArgs a,
-                                                                ActLayout l, ActPhilox ph) {
-    constexpr bool kSep = kSets > 1;
+// min blocks per SM: none asked at H = 64 (0: the compiler's own register plan); two at H = 128 (128 registers), four at H = 32
+// (64 registers; the default plan spilled 4 bytes there)
+template <int H>
+constexpr int act_min_blocks() { return act_resident(H) ? 0 : H >= 128 ? 2 : 4; }
+
+template <int H, int kSets, bool kPhilox>
+__global__ void __launch_bounds__(kActThreads, act_min_blocks<H>()) agent_act_kernel(const __grid_constant__ ActParams<kSets> ps,
+                                                                                     ActArgs a, ActLayout l, ActPhilox ph) {
+    constexpr bool kSep = kSets > 1, kRes = act_resident(H);
+    constexpr int C = H / 16, HP = H + 1;
+    constexpr int KC = kRes ? kActKC : kActWC, KP = KC + 1;     // input columns per chunk and the pitch of their tiles
+    constexpr int KW = kRes ? H : kActWC, WP = kRes ? HP : KP;  // W_ih / W_hh columns per pass and their row pitch
     if (a.gate && *(volatile const int*)a.gate == 0) return;
     extern __shared__ float sm[];
     __shared__ int act_s[kActRows];
     float *w1 = sm + l.w1, *b1 = sm + l.b1, *wih = sm + l.wih, *whh = sm + l.whh, *bih = sm + l.bih, *bhh = sm + l.bhh;
     float *w2 = sm + l.w2, *b2 = sm + l.b2, *ins = sm + l.in, *xq = sm + l.xq, *hs = sm + l.h;
+    if constexpr (!kRes) { w1 = wih = sm + l.wih; whh = wih + 3 * H * WP; }      // (the chunk region at compile-time offsets)
     const int tid = threadIdx.x, A = a.A, O = a.O, I = l.I, Ip = l.Ip;
 
-    auto stage = [&](const marl_agent_params& p) {
-        for (int i = tid; i < MARL_H * I; i += kActThreads) { const int j = i / I; w1[j * Ip + (i - j * I)] = __ldg(p.fc1_w + i); }
-        for (int i = tid; i < MARL_G * MARL_H; i += kActThreads) {
-            const int g = i >> 6, k = i & 63;
-            wih[g * kHP + k] = __ldg(p.w_ih + i);
-            whh[g * kHP + k] = __ldg(p.w_hh + i);
+    auto stage = [&](const marl_agent_params& p) {         // the resident part of a parameter set
+        if constexpr (kRes) {
+            for (int i = tid; i < H * I; i += kActThreads) { const int j = i / I; w1[j * Ip + (i - j * I)] = __ldg(p.fc1_w + i); }
+            for (int i = tid; i < 3 * H * H; i += kActThreads) {
+                const int g = i / H, k = i % H;
+                wih[g * HP + k] = __ldg(p.w_ih + i);
+                whh[g * HP + k] = __ldg(p.w_hh + i);
+            }
         }
-        for (int i = tid; i < A * MARL_H; i += kActThreads) w2[(i >> 6) * kHP + (i & 63)] = __ldg(p.fc2_w + i);
-        for (int i = tid; i < MARL_H; i += kActThreads) b1[i] = __ldg(p.fc1_b + i);
-        for (int i = tid; i < MARL_G; i += kActThreads) { bih[i] = __ldg(p.b_ih + i); bhh[i] = __ldg(p.b_hh + i); }
+        for (int i = tid; i < A * H; i += kActThreads) w2[(i / H) * HP + (i % H)] = __ldg(p.fc2_w + i);
+        for (int i = tid; i < H; i += kActThreads) b1[i] = __ldg(p.fc1_b + i);
+        for (int i = tid; i < 3 * H; i += kActThreads) { bih[i] = __ldg(p.b_ih + i); bhh[i] = __ldg(p.b_hh + i); }
         for (int i = tid; i < A; i += kActThreads) b2[i] = __ldg(p.fc2_b + i);
     };
 
@@ -133,250 +156,38 @@ __global__ void __launch_bounds__(kActThreads) agent_act_kernel(const __grid_con
         } else {
             base = (long long)tile * kActRows; cnt = min(kActRows, a.rows - (int)base);
         }
+        const marl_agent_params& p = ps.p[kSep ? n_tile : 0];     // (streamed: the matrices are read from here per tile)
         __syncthreads();                  // weights staged / the previous tile's q tile consumed
-        for (int i = tid; i < kActRows * MARL_H; i += kActThreads) {
-            const int r = i >> 6, k = i & 63;
-            hs[r * kHP + k] = r < cnt ? a.h_in[(base + (long long)r * stride) * MARL_H + k] : 0.f;
-        }
-        // ---- x = relu(fc1 [obs | last | eye(N)[n]] + b1)
-        float acc[2][4];
-#pragma unroll
-        for (int c = 0; c < 4; ++c) acc[0][c] = acc[1][c] = b1[jg + 16 * c];
-        for (int k0 = 0; k0 < K; k0 += kActKC) {
-            const int kc = min(kActKC, K - k0);
-            __syncthreads();
-            for (int i = tid; i < kActRows * kActKC; i += kActThreads) {
-                const int r = i / kActKC, kk = i % kActKC, k = k0 + kk;
-                const long long row = base + (long long)r * stride;
-                float v = 0.f;
-                if (r < cnt && kk < kc)
-                    v = k < O ? __ldg(a.obs + row * O + k) : __ldg(a.last + row * A + (k - O));
-                ins[r * (kActKC + 1) + kk] = v;
-            }
-            __syncthreads();
-            for (int kk = 0; kk < kc; ++kk) {
-                const float v0 = ins[rg * (kActKC + 1) + kk], v1 = ins[(rg + 16) * (kActKC + 1) + kk];
-#pragma unroll
-                for (int c = 0; c < 4; ++c) {
-                    const float w = w1[(jg + 16 * c) * Ip + k0 + kk];
-                    acc[0][c] = fmaf(w, v0, acc[0][c]);
-                    acc[1][c] = fmaf(w, v1, acc[1][c]);
-                }
-            }
-        }
-#pragma unroll
-        for (int rr = 0; rr < 2; ++rr) {
-            const int r = rg + 16 * rr, n = kSep ? n_tile : ((int)base + r) % a.N;
-#pragma unroll
-            for (int c = 0; c < 4; ++c) {
-                const int j = jg + 16 * c;
-                xq[r * kHP + j] = fmaxf(a.agent_id ? acc[rr][c] + w1[j * Ip + K + n] : acc[rr][c], 0.f);
-            }
-        }
-        __syncthreads();
-        // ---- GRUCell, gate order r, z, n (torch)
-        float gi[2][3][4], gh[2][3][4];
-#pragma unroll
-        for (int g = 0; g < 3; ++g)
-#pragma unroll
-            for (int c = 0; c < 4; ++c) {
-                gi[0][g][c] = gi[1][g][c] = bih[g * MARL_H + jg + 16 * c];
-                gh[0][g][c] = gh[1][g][c] = bhh[g * MARL_H + jg + 16 * c];
-            }
-#pragma unroll 4
-        for (int k = 0; k < MARL_H; ++k) {
-            const float x0 = xq[rg * kHP + k], x1 = xq[(rg + 16) * kHP + k];
-            const float h0 = hs[rg * kHP + k], h1 = hs[(rg + 16) * kHP + k];
-#pragma unroll
-            for (int g = 0; g < 3; ++g)
-#pragma unroll
-                for (int c = 0; c < 4; ++c) {
-                    const int o = (g * MARL_H + jg + 16 * c) * kHP + k;
-                    const float wi = wih[o], wh = whh[o];
-                    gi[0][g][c] = fmaf(wi, x0, gi[0][g][c]); gi[1][g][c] = fmaf(wi, x1, gi[1][g][c]);
-                    gh[0][g][c] = fmaf(wh, h0, gh[0][g][c]); gh[1][g][c] = fmaf(wh, h1, gh[1][g][c]);
-                }
-        }
-        float hn[2][4];
-#pragma unroll
-        for (int rr = 0; rr < 2; ++rr)
-#pragma unroll
-            for (int c = 0; c < 4; ++c) {
-                const float r = sigmoidf_acc(gi[rr][0][c] + gh[rr][0][c]);
-                const float z = sigmoidf_acc(gi[rr][1][c] + gh[rr][1][c]);
-                const float nn = tanhf(gi[rr][2][c] + r * gh[rr][2][c]);
-                hn[rr][c] = (1.f - z) * nn + z * hs[(rg + 16 * rr) * kHP + jg + 16 * c];
-            }
-        __syncthreads();                  // every read of x and h done
-#pragma unroll
-        for (int rr = 0; rr < 2; ++rr)
-#pragma unroll
-            for (int c = 0; c < 4; ++c) hs[(rg + 16 * rr) * kHP + jg + 16 * c] = hn[rr][c];
-        __syncthreads();
-        for (int i = tid; i < kActRows * MARL_H; i += kActThreads) {
-            const int r = i >> 6, k = i & 63;
-            if (r < cnt) a.h_out[(base + (long long)r * stride) * MARL_H + k] = hs[r * kHP + k];
-        }
-        // ---- q = fc2 h' + b2 (the q tile reuses the x tile)
-        for (int i = tid; i < kActRows * A; i += kActThreads) {
-            const int r = i / A, act = i - r * A;
-            float s = b2[act];
-#pragma unroll 8
-            for (int k = 0; k < MARL_H; ++k) s = fmaf(w2[act * kHP + k], hs[r * kHP + k], s);
-            xq[r * A + act] = s;
-            if (a.q && r < cnt) a.q[(base + (long long)r * stride) * A + act] = s;
-        }
-        __syncthreads();
-        // ---- masked first maximum, then the exploration forms
-        if (tid < cnt) {
-            const long long row = base + (long long)tid * stride;
-            const float* av = a.avail ? a.avail + row * A : nullptr;
-            int best = 0, cnt_av = 0;
-            float bv = -INFINITY;
-            for (int k = 0; k < A; ++k) {
-                const bool ok = !av || av[k] != 0.0f;
-                const float v = ok ? xq[tid * A + k] : -INFINITY;
-                if (v > bv) { bv = v; best = k; }          // strict: first maximum; all masked -> 0 like th.argmax
-                cnt_av += ok;
-            }
-            if constexpr (kPhilox) {
-                const int e = (int)(row / a.N), n = (int)(row - (long long)e * a.N);
-                const double eps = ph.eps_table ? ph.eps_table[min(e, ph.eps_len - 1)] : a.eps;
-                double eu, cu;
-                philox_act_uniforms(ph.seed, ph.episode_base + (unsigned long long)e, ph.step, n, eu, cu);
-                if (eu < eps) best = kth_available(av, A, cnt_av, cu);
-            } else if (a.explore) {
-                if (a.explore[row]) best = (int)a.random_action[row];
-            } else if (a.explore_u && a.explore_u[row] < a.eps) {
-                best = 0;                                   // no available action: action 0
-                if (cnt_av > 0) {
-                    const double c = (double)cnt_av;
-                    const int kth = (int)fmin(floor(a.choice_u[row] * c), c - 1.0);
-                    for (int k = 0, seen = 0; k < A; ++k)
-                        if (!av || av[k] != 0.0f) {
-                            if (seen == kth) { best = k; break; }
-                            ++seen;
-                        }
-                }
-            }
-            act_s[tid] = best;
-            a.action[row] = best;
-        }
-        if (a.onehot) {
-            __syncthreads();
-            for (int i = tid; i < kActRows * A; i += kActThreads) {
-                const int r = i / A, act = i - r * A;
-                if (r < cnt) a.onehot[(base + (long long)r * stride) * A + act] = act == act_s[r] ? 1.0f : 0.0f;
-            }
-        }
-    }
-}
-
-// ---- acting at rnn_hidden_dim H = 32 and 128 ---------------------------------------------------------------------------------
-// The H = 64 kernel above stages the whole network in shared memory; at H = 128 the two GRU matrices alone (2 x 384 x 129
-// floats) pass the 227 KB a block may hold.  This kernel keeps only the biases and fc2 resident and streams fc1, W_ih and
-// W_hh through shared memory in chunks of kActWC reduction columns: every chunk serves the 32 rows of a tile, and a parameter
-// set (at most 0.4 MB) stays in L2 across tiles.  Same tiles, same thread grid (thread (jg, rg) owns rows {rg, rg + 16} x
-// columns {jg + 16 c}, c < H / 16), same selection rules as agent_act_kernel; the H = 64 kernel keeps its own source.
-constexpr int kActWC = 16;         // reduction columns per staged weight chunk
-
-struct ActLayoutW {
-    int I, A, qw, hp;              // hp: odd row stride of the H-wide operands
-    int wc, b1, bih, bhh, w2, b2, in, xq, h, total;
-};
-
-inline ActLayoutW act_layout_w(int H, int I, int A) {
-    ActLayoutW l;
-    l.I = I; l.A = A; l.hp = H + 1; l.qw = A > l.hp ? A : l.hp;
-    int o = 0;
-    l.wc = o;  o += 2 * 3 * H * (kActWC + 1);     // W_ih | W_hh chunk [3H, WC] each (fc1 chunk [H, WC] in the first part)
-    l.b1 = o;  o += H;
-    l.bih = o; o += 3 * H;
-    l.bhh = o; o += 3 * H;
-    l.w2 = o;  o += A * l.hp;
-    l.b2 = o;  o += A;
-    l.in = o;  o += kActRows * (kActWC + 1);
-    l.xq = o;  o += kActRows * l.qw;
-    l.h = o;   o += kActRows * l.hp;
-    l.total = o;
-    return l;
-}
-
-// (min blocks: two CTAs an SM at H = 128 (128 registers), four at H = 32 (64 registers; the default plan spilled 4 bytes there))
-template <int H, int kSets, bool kPhilox>
-__global__ void __launch_bounds__(kActThreads, H >= 128 ? 2 : 4) agent_act_kernel_w(const __grid_constant__ ActParams<kSets> ps, ActArgs a,
-                                                                  ActLayoutW l, ActPhilox ph) {
-    constexpr bool kSep = kSets > 1;
-    constexpr int C = H / 16, HP = H + 1, WP = kActWC + 1;
-    if (a.gate && *(volatile const int*)a.gate == 0) return;
-    extern __shared__ float sm[];
-    __shared__ int act_s[kActRows];
-    float *wc = sm + l.wc, *b1 = sm + l.b1, *bih = sm + l.bih, *bhh = sm + l.bhh, *w2 = sm + l.w2, *b2 = sm + l.b2;
-    float *ins = sm + l.in, *xq = sm + l.xq, *hs = sm + l.h;
-    const int tid = threadIdx.x, A = a.A, O = a.O, I = l.I;
-
-    auto stage = [&](const marl_agent_params& p) {         // the resident part of a parameter set
-        for (int i = tid; i < A * H; i += kActThreads) w2[(i / H) * HP + (i % H)] = __ldg(p.fc2_w + i);
-        for (int i = tid; i < H; i += kActThreads) b1[i] = __ldg(p.fc1_b + i);
-        for (int i = tid; i < 3 * H; i += kActThreads) { bih[i] = __ldg(p.b_ih + i); bhh[i] = __ldg(p.b_hh + i); }
-        for (int i = tid; i < A; i += kActThreads) b2[i] = __ldg(p.fc2_b + i);
-    };
-
-    const int jg = tid & 15, rg = tid >> 4;
-    const int K = O + (a.last_action ? A : 0);
-    const int per_agent = (a.n_envs + kActRows - 1) / kActRows;
-    const int ntiles = kSep ? per_agent * a.N : (a.rows + kActRows - 1) / kActRows;
-    const int t_begin = kSep ? (int)((long long)ntiles * blockIdx.x / gridDim.x) : blockIdx.x;
-    const int t_end = kSep ? (int)((long long)ntiles * (blockIdx.x + 1) / gridDim.x) : ntiles;
-    const int t_step = kSep ? 1 : gridDim.x;
-    int staged = -1;
-    if (!kSep) stage(ps.p[0]);
-    for (int tile = t_begin; tile < t_end; tile += t_step) {
-        int n_tile = 0, stride = 1, cnt;
-        long long base;
-        if (kSep) {
-            n_tile = tile / per_agent;
-            const int e0 = (tile - n_tile * per_agent) * kActRows;
-            base = (long long)e0 * a.N + n_tile; stride = a.N; cnt = min(kActRows, a.n_envs - e0);
-            if (n_tile != staged) {
-                __syncthreads();
-                stage(ps.p[n_tile]);
-                staged = n_tile;
-            }
-        } else {
-            base = (long long)tile * kActRows; cnt = min(kActRows, a.rows - (int)base);
-        }
-        const marl_agent_params& p = ps.p[kSep ? n_tile : 0];
-        __syncthreads();
         for (int i = tid; i < kActRows * H; i += kActThreads) {
             const int r = i / H, k = i % H;
             hs[r * HP + k] = r < cnt ? a.h_in[(base + (long long)r * stride) * H + k] : 0.f;
         }
-        // ---- x = relu(fc1 [obs | last | eye(N)[n]] + b1), fc1 streamed in [H, WC] chunks
+        // ---- x = relu(fc1 [obs | last | eye(N)[n]] + b1)
         float acc[2][C];
 #pragma unroll
         for (int c = 0; c < C; ++c) acc[0][c] = acc[1][c] = b1[jg + 16 * c];
-        for (int k0 = 0; k0 < K; k0 += kActWC) {
-            const int kc = min(kActWC, K - k0);
+        for (int k0 = 0; k0 < K; k0 += KC) {
+            const int kc = min(KC, K - k0);
             __syncthreads();
-            for (int i = tid; i < kActRows * kActWC; i += kActThreads) {
-                const int r = i / kActWC, kk = i % kActWC, k = k0 + kk;
+            for (int i = tid; i < kActRows * KC; i += kActThreads) {
+                const int r = i / KC, kk = i % KC, k = k0 + kk;
                 const long long row = base + (long long)r * stride;
                 float v = 0.f;
                 if (r < cnt && kk < kc)
                     v = k < O ? __ldg(a.obs + row * O + k) : __ldg(a.last + row * A + (k - O));
-                ins[r * WP + kk] = v;
+                ins[r * KP + kk] = v;
             }
-            for (int i = tid; i < H * kActWC; i += kActThreads) {
-                const int j = i / kActWC, kk = i % kActWC;
-                wc[j * WP + kk] = kk < kc ? __ldg(p.fc1_w + (long long)j * I + k0 + kk) : 0.f;
-            }
+            if constexpr (!kRes)
+                for (int i = tid; i < H * KC; i += kActThreads) {
+                    const int j = i / KC, kk = i % KC;
+                    w1[j * KP + kk] = kk < kc ? __ldg(p.fc1_w + (long long)j * I + k0 + kk) : 0.f;
+                }
             __syncthreads();
             for (int kk = 0; kk < kc; ++kk) {
-                const float v0 = ins[rg * WP + kk], v1 = ins[(rg + 16) * WP + kk];
+                const float v0 = ins[rg * KP + kk], v1 = ins[(rg + 16) * KP + kk];
 #pragma unroll
                 for (int c = 0; c < C; ++c) {
-                    const float w = wc[(jg + 16 * c) * WP + kk];
+                    const float w = kRes ? w1[(jg + 16 * c) * Ip + k0 + kk] : w1[(jg + 16 * c) * KP + kk];
                     acc[0][c] = fmaf(w, v0, acc[0][c]);
                     acc[1][c] = fmaf(w, v1, acc[1][c]);
                 }
@@ -388,10 +199,12 @@ __global__ void __launch_bounds__(kActThreads, H >= 128 ? 2 : 4) agent_act_kerne
 #pragma unroll
             for (int c = 0; c < C; ++c) {
                 const int j = jg + 16 * c;
-                xq[r * HP + j] = fmaxf(a.agent_id ? acc[rr][c] + __ldg(p.fc1_w + (long long)j * I + K + n) : acc[rr][c], 0.f);
+                xq[r * HP + j] = fmaxf(a.agent_id ? acc[rr][c] + (kRes ? w1[j * Ip + K + n] : __ldg(p.fc1_w + (long long)j * I + K + n))
+                                                  : acc[rr][c], 0.f);
             }
         }
-        // ---- GRUCell, gate order r, z, n (torch); W_ih and W_hh streamed in [3H, WC] chunks
+        if constexpr (kRes) __syncthreads();
+        // ---- GRUCell, gate order r, z, n (torch); streamed: W_ih and W_hh staged in [3H, WC] chunks
         float gi[2][3][C], gh[2][3][C];
 #pragma unroll
         for (int g = 0; g < 3; ++g)
@@ -400,18 +213,18 @@ __global__ void __launch_bounds__(kActThreads, H >= 128 ? 2 : 4) agent_act_kerne
                 gi[0][g][c] = gi[1][g][c] = bih[g * H + jg + 16 * c];
                 gh[0][g][c] = gh[1][g][c] = bhh[g * H + jg + 16 * c];
             }
-        float* wih = wc;
-        float* whh = wc + 3 * H * WP;
-        for (int k0 = 0; k0 < H; k0 += kActWC) {
-            __syncthreads();              // x written / the previous chunk consumed
-            for (int i = tid; i < 3 * H * kActWC; i += kActThreads) {
-                const int m = i / kActWC, kk = i % kActWC;
-                wih[m * WP + kk] = __ldg(p.w_ih + (long long)m * H + k0 + kk);
-                whh[m * WP + kk] = __ldg(p.w_hh + (long long)m * H + k0 + kk);
+        for (int k0 = 0; k0 < H; k0 += KW) {
+            if constexpr (!kRes) {
+                __syncthreads();          // x written / the previous chunk consumed
+                for (int i = tid; i < 3 * H * KW; i += kActThreads) {
+                    const int m = i / KW, kk = i % KW;
+                    wih[m * WP + kk] = __ldg(p.w_ih + (long long)m * H + k0 + kk);
+                    whh[m * WP + kk] = __ldg(p.w_hh + (long long)m * H + k0 + kk);
+                }
+                __syncthreads();
             }
-            __syncthreads();
 #pragma unroll 4
-            for (int kk = 0; kk < kActWC; ++kk) {
+            for (int kk = 0; kk < KW; ++kk) {
                 const int k = k0 + kk;
                 const float x0 = xq[rg * HP + k], x1 = xq[(rg + 16) * HP + k];
                 const float h0 = hs[rg * HP + k], h1 = hs[(rg + 16) * HP + k];
@@ -419,7 +232,7 @@ __global__ void __launch_bounds__(kActThreads, H >= 128 ? 2 : 4) agent_act_kerne
                 for (int g = 0; g < 3; ++g)
 #pragma unroll
                     for (int c = 0; c < C; ++c) {
-                        const int o = (g * H + jg + 16 * c) * WP + kk;
+                        const int o = (g * H + jg + 16 * c) * WP + (kRes ? k : kk);
                         const float wi = wih[o], wh = whh[o];
                         gi[0][g][c] = fmaf(wi, x0, gi[0][g][c]); gi[1][g][c] = fmaf(wi, x1, gi[1][g][c]);
                         gh[0][g][c] = fmaf(wh, h0, gh[0][g][c]); gh[1][g][c] = fmaf(wh, h1, gh[1][g][c]);
@@ -456,7 +269,7 @@ __global__ void __launch_bounds__(kActThreads, H >= 128 ? 2 : 4) agent_act_kerne
             if (a.q && r < cnt) a.q[(base + (long long)r * stride) * A + act] = s;
         }
         __syncthreads();
-        // ---- masked first maximum, then the exploration forms (those of agent_act_kernel)
+        // ---- masked first maximum, then the exploration forms
         if (tid < cnt) {
             const long long row = base + (long long)tid * stride;
             const float* av = a.avail ? a.avail + row * A : nullptr;
@@ -465,7 +278,7 @@ __global__ void __launch_bounds__(kActThreads, H >= 128 ? 2 : 4) agent_act_kerne
             for (int k = 0; k < A; ++k) {
                 const bool ok = !av || av[k] != 0.0f;
                 const float v = ok ? xq[tid * A + k] : -INFINITY;
-                if (v > bv) { bv = v; best = k; }
+                if (v > bv) { bv = v; best = k; }          // strict: first maximum; all masked -> 0 like th.argmax
                 cnt_av += ok;
             }
             if constexpr (kPhilox) {
@@ -473,11 +286,11 @@ __global__ void __launch_bounds__(kActThreads, H >= 128 ? 2 : 4) agent_act_kerne
                 const double eps = ph.eps_table ? ph.eps_table[min(e, ph.eps_len - 1)] : a.eps;
                 double eu, cu;
                 philox_act_uniforms(ph.seed, ph.episode_base + (unsigned long long)e, ph.step, n, eu, cu);
-                if (eu < eps) best = kth_available(av, A, cnt_av, cu);
+                if (eu < eps) best = kth_available(av, A, cnt_av, &cu);
             } else if (a.explore) {
                 if (a.explore[row]) best = (int)a.random_action[row];
             } else if (a.explore_u && a.explore_u[row] < a.eps) {
-                best = kth_available(av, A, cnt_av, a.choice_u[row]);
+                best = kth_available(av, A, cnt_av, a.choice_u + row);
             }
             act_s[tid] = best;
             a.action[row] = best;
@@ -564,16 +377,12 @@ __global__ void __launch_bounds__(kRecWarps * 32) rollout_record_kernel(RecArgs 
 
 using namespace marl;
 
-// Validates the on-chip footprint of one parameter set of input width I and launches agent_act_kernel<kSets, kPhilox>
-// (H = 64) or agent_act_kernel_w<H, kSets, kPhilox>.
+// Validates the on-chip footprint of one parameter set of input width I and launches agent_act_kernel<H, kSets, kPhilox>.
 template <int H, int kSets, bool kPhilox>
 static int act_launch(const char* name, const ActParams<kSets>& ps, const ActArgs& a, const ActPhilox& ph, int I,
                       long long tiles, void* stream) {
-    ActLayout l{};
-    ActLayoutW lw{};
-    size_t smem;
-    if constexpr (H == MARL_H) { l = act_layout(I, a.A); smem = (size_t)l.total * sizeof(float); }
-    else { lw = act_layout_w(H, I, a.A); smem = (size_t)lw.total * sizeof(float); }
+    const ActLayout l = act_layout(H, I, a.A);
+    const size_t smem = (size_t)l.total * sizeof(float);
     int dev = 0, sms = 0, optin = 0;
     cudaError_t e = cudaGetDevice(&dev);
     if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
@@ -585,9 +394,7 @@ static int act_launch(const char* name, const ActParams<kSets>& ps, const ActArg
     static int blocks_per_sm[64] = {};
     static size_t blocks_for[64] = {};
     const int slot = dev & 63;
-    const void* kernel;
-    if constexpr (H == MARL_H) kernel = (const void*)agent_act_kernel<kSets, kPhilox>;
-    else kernel = (const void*)agent_act_kernel_w<H, kSets, kPhilox>;
+    const void* kernel = (const void*)agent_act_kernel<H, kSets, kPhilox>;
     if (smem_set[slot] < smem) {
         e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return (int)e;
@@ -601,8 +408,7 @@ static int act_launch(const char* name, const ActParams<kSets>& ps, const ActArg
     const long long cap = (long long)sms * (blocks_per_sm[slot] > 0 ? blocks_per_sm[slot] : 1);
     const int grid = (int)(tiles < cap ? tiles : cap);
     { ProfScope ps_(name, (cudaStream_t)stream);
-      if constexpr (H == MARL_H) agent_act_kernel<kSets, kPhilox><<<grid, kActThreads, smem, (cudaStream_t)stream>>>(ps, a, l, ph);
-      else agent_act_kernel_w<H, kSets, kPhilox><<<grid, kActThreads, smem, (cudaStream_t)stream>>>(ps, a, lw, ph); }
+      agent_act_kernel<H, kSets, kPhilox><<<grid, kActThreads, smem, (cudaStream_t)stream>>>(ps, a, l, ph); }
     MARL_LAUNCH_CHECK();
     return MARL_OK;
 }

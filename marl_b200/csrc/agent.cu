@@ -25,7 +25,6 @@ namespace marl {
 
 constexpr int kMaxStreams = 4;
 constexpr int kGruPrio = -1;        // launch priority of the recurrence kernels (see launch_pdl_prio)
-constexpr int kGruThreads = 128;   // 64 hidden units x 2-way split of the reduction, one warp per SM sub-partition
 #ifndef MARL_GI_DEPTH
 #define MARL_GI_DEPTH 4
 #endif
@@ -33,8 +32,6 @@ constexpr int kGruThreads = 128;   // 64 hidden units x 2-way split of the reduc
 #define MARL_BWD_DEPTH 6
 #endif
 constexpr int kGiDepth = MARL_GI_DEPTH;   // cp.async ring depth (time steps) of the forward's input gates
-constexpr int kGruGroups = 2;      // chains advanced side by side in one CTA (one 128-thread group each)
-constexpr int kGruMaxRows = 8;     // rows per group and pass
 
 // MUFU-based gate non-linearities: ex2.approx / rcp.approx are accurate to ~2 ulp, i.e. <= 2e-7 absolute on
 // the (0,1) / (-1,1) outputs -- the same order as the fp32 rounding of the reference's own libm path.
@@ -89,54 +86,101 @@ struct GruFwdArgs {
 #define GRU_STAMP(tag) do { } while (0)
 #endif
 
-// One CTA advances R rows (b,n) of one chain through all its segments.  Thread (j, ks): hidden unit j,
-// half ks of the 64-long reduction; its 3 x 32 W_hh weights stay in registers for the whole segment.
-// 128-thread named barrier: the CTA hosts one such group per chain, each advancing its own rows
-__device__ __forceinline__ void group_sync(int id) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(kGruThreads) : "memory"); }
+// One CTA advances R rows (b,n) of one chain through all its segments.  Thread (j, ks) = (tid / KS, tid % KS) of a group owns
+// hidden unit j and the reduction indices 4 (KS i + ks) + c, so every thread keeps its 3 x 32 W_hh weights in registers for the
+// whole segment at every width, and the KS lanes of a unit sit side by side in one warp.
+template <int H>
+struct GruWidth {
+    static_assert(H == 32 || H == 64 || H == 128, "rnn_hidden_dim is 32, 64 or 128");
+    static constexpr int KS = H / 32;                 // lanes per hidden unit
+    static constexpr int T = H * KS;                  // threads of one group (at H = 64 one warp per SM sub-partition)
+    static constexpr int G = 3 * H;
+    static constexpr int kGroups = T >= 512 ? 1 : 2;  // forward: chains side by side in one CTA (512 threads fill the register file)
+    // rows per pass: what fits the registers without spills (at most 128 a thread in a 512-thread group; at H = 32 every lane
+    // owns every row)
+    static constexpr int kMaxRows = H == 32 ? 4 : H == 64 ? 8 : 2;
+    static constexpr int rows(int r) { return r < kMaxRows ? r : kMaxRows; }      // a pass size of the ladder 1, 2, 4, 8, clamped
+    // row slots of a pass: lane ks reads slot ks + KS q for every q < ceil(R / KS), past the pass's rows when KS > R
+    static constexpr int kSlots = kMaxRows > KS ? kMaxRows : KS;
+};
+
+// named barrier of one thread group: the forward CTA hosts one group per chain, each advancing its own rows
+template <int H>
+__device__ __forceinline__ void group_sync(int id) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(GruWidth<H>::T) : "memory"); }
+
+// the KS partial sums of one hidden unit, summed over its lanes (butterfly: every lane ends with the total)
+template <int KS>
+__device__ __forceinline__ float lanes_sum(float v) {
+#pragma unroll
+    for (int o = 1; o < KS; o <<= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    return v;
+}
+
+// v[q * KS + ks] with register indices fixed at compile time (rows past R read v[q * KS])
+template <int KS, int R>
+__device__ __forceinline__ float lane_pick(const float (&v)[R], int q, int ks) {
+    if constexpr (KS == 2) {      // one select of two registers (the loop below schedules the H = 64 kernels differently)
+        const int e = 2 * q, o = (2 * q + 1 < R) ? 2 * q + 1 : 2 * q;
+        return ks ? v[o] : v[e];
+    } else {
+        float r = v[q * KS];
+#pragma unroll
+        for (int c = 1; c < KS; ++c)
+            if (q * KS + c < R && ks == c) r = v[q * KS + c];
+        return r;
+    }
+}
 
 // Separated networks (one parameter set per agent, SEP): logical positions are dealt agent-major, position p = n*B + b is row
 // b*N + n, and a pass never straddles two agents (gru_pass_rows), so the W_hh slice in registers is the pass's agent's.
 template <bool SEP>
 __device__ __forceinline__ int gru_position_row(int p, int B, int N) { return SEP ? (p % B) * N + p / B : p; }
-template <bool SEP>
+template <int H, bool SEP>
 __device__ __forceinline__ int gru_pass_rows(int pos, int left, int B) {
-    const int n = min(kGruMaxRows, left);
+    const int n = min(GruWidth<H>::kMaxRows, left);
     return SEP ? min(n, B - pos % B) : n;
 }
 
-template <int R, bool SEP>
+template <int H>
+constexpr size_t gru_fwd_smem(int R) { return (size_t)(2 * R * H + kGiDepth * R * 3 * H) * sizeof(float); }
+
+template <int H, int R, bool SEP>
 __device__ __forceinline__ void gru_chain_fwd(const GruFwdArgs& a, int chain, int row0, int nrows, float* smem, int bar_id) {
-    float (*hs)[R][MARL_H] = reinterpret_cast<float (*)[R][MARL_H]>(smem);                          // [2][R][H]
-    float (*ring)[R][MARL_G] = reinterpret_cast<float (*)[R][MARL_G]>(smem + 2 * R * MARL_H);       // [D][R][3H]
-    const int tid = threadIdx.x & (kGruThreads - 1), ks = tid & 1, j = tid >> 1;
+    using W = GruWidth<H>;
+    constexpr int KS = W::KS, T = W::T, G = W::G, CPR = G / 4;       // CPR: 16-byte chunks of gi per row and step
+    float (*hs)[R][H] = reinterpret_cast<float (*)[R][H]>(smem);                              // [2][R][H]
+    float (*ring)[R][G] = reinterpret_cast<float (*)[R][G]>(smem + 2 * R * H);                // [D][R][3H]
+    const int tid = threadIdx.x % T, ks = tid % KS, j = tid / KS;
     const int L = a.L, N = a.N;
     // logical position (what the CTAs are dealt) -> row b*N + n: identity, or the length-sorted deal of row_order_kernel
     // (resolved once per pass into shared memory: the previous pass ended with a group barrier)
-    __shared__ int srow_all[kGruGroups][kGruMaxRows];
+    __shared__ int srow_all[W::kGroups][W::kSlots];
     int* srow = srow_all[bar_id - 1];
     if (tid < R) {
         const int* order = a.row_order[chain];
         srow[tid] = (order && tid < nrows) ? __ldg(order + row0 + tid) : gru_position_row<SEP>(row0 + tid, a.B, N);
     }
-    group_sync(bar_id);
+    group_sync<H>(bar_id);
     auto row_at = [&](int rr) { return srow[rr]; };
-    constexpr int OWN = (R + 1) / 2;                  // rows whose gate math this lane owns: rr = ks + 2q
+    constexpr int OWN = (R + KS - 1) / KS;            // rows whose gate math this lane owns: rr = ks + KS q
     bool own[OWN]; long long base[OWN];
 #pragma unroll
     for (int q = 0; q < OWN; ++q) {
-        const int rr = ks + 2 * q, row = row_at(rr);
+        const int rr = ks + KS * q, row = row_at(rr);
         own[q] = rr < nrows;
         base[q] = own[q] ? ((long long)(row / N) * L * N + (row % N)) : 0;
     }
-    // cp.async work list: R rows x 48 chunks of 16 B per time step
-    constexpr int NCH = (R * 48 + kGruThreads - 1) / kGruThreads;
+    // cp.async work list: R rows x CPR chunks of 16 B per time step, their sources computed once -- except in a 512-thread group,
+    // whose 128 registers a thread do not hold the list: it recomputes each chunk's source per step
+    constexpr bool kChunkList = T < 512;
+    constexpr int NCH = (R * CPR + T - 1) / T;
     long long csrc[NCH]; int cdst[NCH];
 #pragma unroll
-    for (int l = 0; l < NCH; ++l) {
-        const int c = tid + l * kGruThreads, rr = c / 48, ch = c % 48, row = row_at(rr);
-        if (c < R * 48 && rr < nrows) {
-            csrc[l] = ((long long)(row / N) * L * N + (row % N)) * MARL_G + ch * 4;
-            cdst[l] = rr * MARL_G + ch * 4;
+    for (int l = 0; l < (kChunkList ? NCH : 0); ++l) {
+        const int c = tid + l * T, rr = c / CPR, ch = c % CPR, row = row_at(rr);
+        if (c < R * CPR && rr < nrows) {
+            csrc[l] = ((long long)(row / N) * L * N + (row % N)) * G + ch * 4;
+            cdst[l] = rr * G + ch * 4;
         } else { csrc[l] = -1; cdst[l] = 0; }
     }
 #ifdef MARL_GRU_TRACE
@@ -145,9 +189,9 @@ __device__ __forceinline__ void gru_chain_fwd(const GruFwdArgs& a, int chain, in
     if (trace) { trace[508] = R; trace[509] = nrows; }
 #endif
     const float* h0 = a.h0[chain];
-    for (int idx = tid; idx < R * MARL_H; idx += kGruThreads) {
-        const int rr = idx / MARL_H, jj = idx % MARL_H, row = row_at(rr);
-        hs[0][rr][jj] = (h0 && rr < nrows) ? h0[(long long)row * MARL_H + jj] : 0.0f;
+    for (int idx = tid; idx < R * H; idx += T) {
+        const int rr = idx / H, jj = idx % H, row = row_at(rr);
+        hs[0][rr][jj] = (h0 && rr < nrows) ? h0[(long long)row * H + jj] : 0.0f;
     }
     int cur = 0;
     for (int sg = a.chain_start[chain]; sg < a.chain_start[chain] + a.chain_len[chain]; ++sg) {
@@ -160,18 +204,21 @@ __device__ __forceinline__ void gru_chain_fwd(const GruFwdArgs& a, int chain, in
         for (int g = 0; g < 3; ++g)
 #pragma unroll
             for (int i = 0; i < 8; ++i) {
-                const float4 v = __ldg(reinterpret_cast<const float4*>(w_hh + (long long)(g * MARL_H + j) * MARL_H + 4 * (2 * i + ks)));
+                const float4 v = __ldg(reinterpret_cast<const float4*>(w_hh + (long long)(g * H + j) * H + 4 * (KS * i + ks)));
                 w[g][2 * i] = pack2(v.x, v.y); w[g][2 * i + 1] = pack2(v.z, v.w);
             }
-        const float bh_r = __ldg(b_hh + j), bh_z = __ldg(b_hh + MARL_H + j), bh_n = __ldg(b_hh + 2 * MARL_H + j);
-        // per-step output pointers of the rows this lane owns: advanced by one time step (N rows) per iteration
-        float* hp[OWN]; float* gp_out[OWN];
+        const float bh_r = __ldg(b_hh + j), bh_z = __ldg(b_hh + H + j), bh_n = __ldg(b_hh + 2 * H + j);
+        // per-step output pointers of the rows this lane owns, advanced by one time step (N rows) per iteration; a 512-thread group
+        // keeps the (b, t, n) index of each row instead (two registers a row where the pointers take four)
+        float* hp[OWN]; float* gp_out[OWN]; long long idx[OWN];
 #pragma unroll
         for (int q = 0; q < OWN; ++q) {
-            hp[q] = S.hidden + base[q] * MARL_H + j;
-            gp_out[q] = S.gates ? S.gates + base[q] * (4 * MARL_H) + j : nullptr;
+            if constexpr (kChunkList) {
+                hp[q] = S.hidden + base[q] * H + j;
+                gp_out[q] = S.gates ? S.gates + base[q] * (4 * H) + j : nullptr;
+            } else idx[q] = base[q];
         }
-        const long long hstep = (long long)N * MARL_H, gstep = (long long)N * 4 * MARL_H;
+        const long long hstep = (long long)N * H, gstep = (long long)N * 4 * H;
         // (measured and dropped: the time loop of the one- and two-row passes unrolled by the ring depth, ring slots and h-buffer side as
         // compile-time constants -- the loop-back went from 90 to 28 cycles and the refill from 60 to 40 in the clock64 trace, the
         // two-row CTAs from 720 to ~635 cycles per step, but the CTAs that run a target group beside their eval row stayed at ~730
@@ -184,9 +231,16 @@ __device__ __forceinline__ void gru_chain_fwd(const GruFwdArgs& a, int chain, in
         }
         auto issue = [&](int t) {
             if (t < Lp) {
+                if constexpr (kChunkList) {
 #pragma unroll
-                for (int l = 0; l < NCH; ++l)
-                    if (csrc[l] >= 0) cp_async16(&ring[t % kGiDepth][0][0] + cdst[l], S.gi + csrc[l] + (long long)t * N * MARL_G);
+                    for (int l = 0; l < NCH; ++l)
+                        if (csrc[l] >= 0) cp_async16(&ring[t % kGiDepth][0][0] + cdst[l], S.gi + csrc[l] + (long long)t * N * G);
+                } else {
+                    for (int c = tid; c < nrows * CPR; c += T) {
+                        const int rr = c / CPR, ch = c % CPR, row = row_at(rr);
+                        cp_async16(&ring[t % kGiDepth][rr][ch * 4], S.gi + (((long long)(row / N) * L + t) * N + (row % N)) * G + ch * 4);
+                    }
+                }
             }
             cp_async_commit();
         };
@@ -195,12 +249,13 @@ __device__ __forceinline__ void gru_chain_fwd(const GruFwdArgs& a, int chain, in
         for (int t = 0; t < Lp; ++t) {
             GRU_STAMP(0);
             cp_async_wait<kGiDepth - 2>();           // this thread's copies for step t have landed
-            group_sync(bar_id);                      // ... the whole group's; also orders the h double buffer
+            group_sync<H>(bar_id);                   // ... the whole group's; also orders the h double buffer
             GRU_STAMP(1);
             // Few rows per CTA = latency-bound chain: the refill's address math and LSU hand-off (~150 cycles when it sat
             // here, measured with clock64) go behind the FMAs, where they overlap the FMA drain.  Many rows per CTA =
-            // throughput-bound: keep the prefetch as early as possible.
-            constexpr bool kLateIssue = R <= 2;
+            // throughput-bound: keep the prefetch as early as possible.  (A 512-thread group issues early: the late refill's
+            // registers, live beside the accumulators, do not fit its 128 a thread.)
+            constexpr bool kLateIssue = R <= 2 && T < 512;
             if (!kLateIssue) issue(t + kGiDepth - 1);   // refill the slot consumed in step t-1
             float acc[3][R];
             f32x2 pacc[3][R];                     // (even k, odd k) partial sums of each dot product, packed
@@ -212,7 +267,7 @@ __device__ __forceinline__ void gru_chain_fwd(const GruFwdArgs& a, int chain, in
             for (int i = 0; i < 8; ++i)
 #pragma unroll
                 for (int rr = 0; rr < R; ++rr) {
-                    const ulonglong2 hv = *reinterpret_cast<const ulonglong2*>(&hs[cur][rr][4 * (2 * i + ks)]);
+                    const ulonglong2 hv = *reinterpret_cast<const ulonglong2*>(&hs[cur][rr][4 * (KS * i + ks)]);
 #pragma unroll
                     for (int g = 0; g < 3; ++g) {
                         pacc[g][rr] = ffma2(w[g][2 * i], hv.x, pacc[g][rr]);
@@ -228,36 +283,41 @@ __device__ __forceinline__ void gru_chain_fwd(const GruFwdArgs& a, int chain, in
                 for (int rr = 0; rr < R; ++rr) {
                     float ev, od;
                     unpack2(pacc[g][rr], ev, od);
-                    acc[g][rr] = ev + od;
-                    acc[g][rr] += __shfl_xor_sync(0xffffffffu, acc[g][rr], 1);
+                    acc[g][rr] = lanes_sum<KS>(ev + od);
                 }
             GRU_STAMP(4);
             const float* gring = &ring[t % kGiDepth][0][0];
 #pragma unroll
             for (int q = 0; q < OWN; ++q) {
-                const int e = 2 * q, o = (2 * q + 1 < R) ? 2 * q + 1 : 2 * q;      // static register indices
-                const float ar = ks ? acc[0][o] : acc[0][e];
-                const float az = ks ? acc[1][o] : acc[1][e];
-                const float an = ks ? acc[2][o] : acc[2][e];
+                float ar, az, an;
+                if constexpr (KS == 2) {      // (written out: through lane_pick the H = 64 kernel compiles to another schedule)
+                    const int e = 2 * q, o = (2 * q + 1 < R) ? 2 * q + 1 : 2 * q;      // static register indices
+                    ar = ks ? acc[0][o] : acc[0][e]; az = ks ? acc[1][o] : acc[1][e]; an = ks ? acc[2][o] : acc[2][e];
+                } else {
+                    ar = lane_pick<KS>(acc[0], q, ks); az = lane_pick<KS>(acc[1], q, ks); an = lane_pick<KS>(acc[2], q, ks);
+                }
                 if (own[q]) {
-                    const int rr = ks + 2 * q;
+                    const int rr = ks + KS * q;
                     // GRUCell (aten gru_cell): r,z = sigmoid(gi + gh); n = tanh(gi_n + r * gh_n); h' = (h - n) z + n
-                    const float* gp = gring + rr * MARL_G;
+                    const float* gp = gring + rr * G;
                     const float gh_n = an + bh_n;
                     const float r = gate_sigmoid((ar + bh_r) + gp[j]);
-                    const float z = gate_sigmoid((az + bh_z) + gp[MARL_H + j]);
-                    const float n = gate_tanh(fmaf(r, gh_n, gp[2 * MARL_H + j]));
+                    const float z = gate_sigmoid((az + bh_z) + gp[H + j]);
+                    const float n = gate_tanh(fmaf(r, gh_n, gp[2 * H + j]));
                     const float hold = hs[cur][rr][j];
                     const float hnew = fmaf(hold - n, z, n);
                     hs[cur ^ 1][rr][j] = hnew;
-                    *hp[q] = hnew;
-                    if (gp_out[q]) {
-                        float* go = gp_out[q];
-                        go[0] = r; go[MARL_H] = z; go[2 * MARL_H] = n; go[3 * MARL_H] = gh_n;
+                    if constexpr (kChunkList) *hp[q] = hnew;
+                    else S.hidden[idx[q] * H + j] = hnew;
+                    if (kChunkList ? gp_out[q] != nullptr : S.gates != nullptr) {
+                        float* go = kChunkList ? gp_out[q] : S.gates + idx[q] * (4 * H) + j;
+                        go[0] = r; go[H] = z; go[2 * H] = n; go[3 * H] = gh_n;
                     }
                 }
-                hp[q] += hstep;
-                if (gp_out[q]) gp_out[q] += gstep;
+                if constexpr (kChunkList) {
+                    hp[q] += hstep;
+                    if (gp_out[q]) gp_out[q] += gstep;
+                } else idx[q] += N;
             }
             cur ^= 1;
             GRU_STAMP(5);
@@ -270,11 +330,11 @@ __device__ __forceinline__ void gru_chain_fwd(const GruFwdArgs& a, int chain, in
         }
 #endif
         cp_async_wait<0>();
-        group_sync(bar_id);
+        group_sync<H>(bar_id);
         if (S.h_last) {
 #pragma unroll
             for (int q = 0; q < OWN; ++q)
-                if (own[q]) S.h_last[(long long)row_at(ks + 2 * q) * MARL_H + j] = hs[cur][ks + 2 * q][j];
+                if (own[q]) S.h_last[(long long)row_at(ks + KS * q) * H + j] = hs[cur][ks + KS * q][j];
         }
     }
 }
@@ -305,26 +365,26 @@ __device__ __forceinline__ void cta_rows_by_agent(int B, int N, int& begin, int&
 #define MARL_GRU_SPARE_SMS 16
 #endif
 constexpr int kGruFwdSpareSMs = MARL_GRU_SPARE_SMS;
-constexpr size_t gru_fwd_smem(int R) { return (size_t)(2 * R * MARL_H + kGiDepth * R * MARL_G) * sizeof(float); }
 
-template <bool SEP>
-__global__ void __launch_bounds__(kGruThreads * kGruGroups) gru_unroll_fwd_kernel(GruFwdArgs a) {
+template <int H, bool SEP>
+__global__ void __launch_bounds__(GruWidth<H>::T * GruWidth<H>::kGroups) gru_unroll_fwd_kernel(GruFwdArgs a) {
+    using W = GruWidth<H>;
     pdl_enter();
     extern __shared__ __align__(16) float gru_smem[];
-    const int grp = threadIdx.x >> 7;
-    const int chain = blockIdx.y * kGruGroups + grp;
+    const int grp = threadIdx.x / W::T;
+    const int chain = blockIdx.y * W::kGroups + grp;
     if (chain >= a.n_chains) return;
-    float* smem = gru_smem + grp * (gru_fwd_smem(kGruMaxRows) / sizeof(float));
+    float* smem = gru_smem + grp * (gru_fwd_smem<H>(W::kMaxRows) / sizeof(float));
     int begin = 0;
     for (int i = 0; i < (int)blockIdx.x; ++i) begin += a.rows_of[chain][i];
     const int count = a.rows_of[chain][blockIdx.x];
-    for (int off = 0, n = 0; off < count; off += SEP ? n : kGruMaxRows) {
-        n = gru_pass_rows<SEP>(begin + off, count - off, a.B);
-        if (n == 1) gru_chain_fwd<1, SEP>(a, chain, begin + off, n, smem, 1 + grp);
-        else if (n == 2) gru_chain_fwd<2, SEP>(a, chain, begin + off, n, smem, 1 + grp);
-        else if (n <= 4) gru_chain_fwd<4, SEP>(a, chain, begin + off, n, smem, 1 + grp);
-        else gru_chain_fwd<8, SEP>(a, chain, begin + off, n, smem, 1 + grp);
-        group_sync(1 + grp);
+    for (int off = 0, n = 0; off < count; off += SEP ? n : W::kMaxRows) {
+        n = gru_pass_rows<H, SEP>(begin + off, count - off, a.B);
+        if (n == 1) gru_chain_fwd<H, 1, SEP>(a, chain, begin + off, n, smem, 1 + grp);
+        else if (W::kMaxRows == 2 || n == 2) gru_chain_fwd<H, 2, SEP>(a, chain, begin + off, n, smem, 1 + grp);
+        else if (W::kMaxRows == 4 || n <= 4) gru_chain_fwd<H, W::rows(4), SEP>(a, chain, begin + off, n, smem, 1 + grp);
+        else gru_chain_fwd<H, W::rows(8), SEP>(a, chain, begin + off, n, smem, 1 + grp);
+        group_sync<H>(1 + grp);
     }
 }
 
@@ -344,446 +404,95 @@ struct GruBwdArgs {
     int agent_stride;      // separated networks (SEP instantiation): floats from agent n's W_hh to n+1's
 };
 
-constexpr int kBwdSlot = 7 * MARL_H;     // r, z, n, gh_n (4H) | h_prev | dh_ext | dh_ext2   per row and time step
 constexpr int bwd_depth(int R) { return R >= 8 ? 3 : MARL_BWD_DEPTH; }
-constexpr size_t gru_bwd_smem(int R) { return (size_t)(2 * R * MARL_G + bwd_depth(R) * R * kBwdSlot) * sizeof(float); }
+// ring slot per row and time step: r, z, n, gh_n (4H) | h_prev | dh_ext | dh_ext2
+template <int H>
+constexpr size_t gru_bwd_smem(int R) { return (size_t)(2 * R * 3 * H + bwd_depth(R) * R * 7 * H) * sizeof(float); }
 
-template <int R, bool SEP>
+template <int H, int R, bool SEP>
 __device__ __forceinline__ void gru_rows_bwd(const GruBwdArgs& a, int row0, int nrows, float* gru_smem) {
+    using W = GruWidth<H>;
+    constexpr int KS = W::KS, T = W::T, G = W::G, SLOT = 7 * H, CPR = SLOT / 4;   // CPR: 16-byte chunks of a slot
     constexpr int D = bwd_depth(R);
-    float (*sg)[R][MARL_G] = reinterpret_cast<float (*)[R][MARL_G]>(gru_smem);                       // [2][R][3H]
-    float (*ring)[R][kBwdSlot] = reinterpret_cast<float (*)[R][kBwdSlot]>(gru_smem + 2 * R * MARL_G); // [D][R][7H]
-    const int tid = threadIdx.x, ks = tid & 1, j = tid >> 1;
+    float (*sg)[R][G] = reinterpret_cast<float (*)[R][G]>(gru_smem);                          // [2][R][3H]
+    float (*ring)[R][SLOT] = reinterpret_cast<float (*)[R][SLOT]>(gru_smem + 2 * R * G);     // [D][R][7H]
+    const int tid = threadIdx.x, ks = tid % KS, j = tid / KS;
     const int L = a.L, N = a.N;
-    __shared__ int srow[kGruMaxRows];         // (the previous pass ended with a block barrier)
+    __shared__ int srow[W::kSlots];           // (the previous pass ended with a block barrier)
     if (tid < R) srow[tid] = (a.row_order && tid < nrows) ? __ldg(a.row_order + row0 + tid) : gru_position_row<SEP>(row0 + tid, a.B, N);
     __syncthreads();
     auto row_at = [&](int rr) { return srow[rr]; };
-    constexpr int OWN = (R + 1) / 2;
+    constexpr int OWN = (R + KS - 1) / KS;
     bool own[OWN]; long long base[OWN]; float dh_carry[OWN];
 #pragma unroll
     for (int q = 0; q < OWN; ++q) {
-        const int rr = ks + 2 * q, row = row_at(rr);
+        const int rr = ks + KS * q, row = row_at(rr);
         own[q] = rr < nrows;
         base[q] = own[q] ? ((long long)(row / N) * L * N + (row % N)) : 0;
         dh_carry[q] = 0.0f;
     }
-    // column j of W_hh, rows m = 4*(2i+ks)+c, i = 0..23:  dh_prev[j] = dh z + sum_m dgh[m] W_hh[m, j]
+    // column j of W_hh, rows m = 4 (KS i + ks) + c, i = 0..23:  dh_prev[j] = dh z + sum_m dgh[m] W_hh[m, j]
     const float* w_hh = a.w_hh + (SEP ? (long long)(row0 / a.B) * a.agent_stride : 0);      // this pass's agent
     f32x2 wt[48];                                          // (rows m, m+1) pairs
 #pragma unroll
     for (int i = 0; i < 24; ++i)
 #pragma unroll
         for (int c = 0; c < 2; ++c)
-            wt[2 * i + c] = pack2(__ldg(w_hh + (long long)(4 * (2 * i + ks) + 2 * c) * MARL_H + j),
-                                  __ldg(w_hh + (long long)(4 * (2 * i + ks) + 2 * c + 1) * MARL_H + j));
-    // cp.async work list: per row 112 chunks of 16 B (64 gates, 16 h_prev, 16 dh_ext, 16 dh_ext2); the
-    // per-chunk source pointer at t = 0 and its per-step stride are fixed, so they are computed once.
-    constexpr int NCH = (R * 112 + kGruThreads - 1) / kGruThreads;
-    const float* csrc[NCH]; int cstride[NCH], cdst[NCH], ckind[NCH];
-#pragma unroll
-    for (int l = 0; l < NCH; ++l) {
-        const int c = tid + l * kGruThreads, rr = c / 112, ch = c % 112, row = row_at(rr);
-        csrc[l] = nullptr; cstride[l] = 0; cdst[l] = rr * kBwdSlot + ch * 4; ckind[l] = 0;
-        if (c < R * 112 && rr < nrows) {
-            const long long idx0 = (long long)(row / N) * L * N + (row % N);
-            if (ch < 64) { csrc[l] = a.gates + idx0 * (4 * MARL_H) + ch * 4; cstride[l] = N * 4 * MARL_H; }
-            else if (ch < 80) { csrc[l] = a.hidden + (idx0 - N) * MARL_H + (ch - 64) * 4; cstride[l] = N * MARL_H; ckind[l] = 1;
-                                 if (a.h0) ckind[l] = 2; }
-            else if (ch < 96) { if (a.dh_ext) { csrc[l] = a.dh_ext + idx0 * MARL_H + (ch - 80) * 4; cstride[l] = N * MARL_H; } }
-            else { if (a.dh_ext2) { csrc[l] = a.dh_ext2 + idx0 * MARL_H + (ch - 96) * 4; cstride[l] = N * MARL_H; } }
-        }
-    }
-    auto issue = [&](int t) {
-        if (t >= 0) {
-            float* slot = &ring[t % D][0][0];
-#pragma unroll
-            for (int l = 0; l < NCH; ++l) {
-                if (!csrc[l]) continue;
-                if (ckind[l] != 0 && t == 0) {      // h_prev of the first step: h0 (or zeros, handled by the consumer)
-                    if (ckind[l] == 2) cp_async16(slot + cdst[l], a.h0 + (long long)row_at(cdst[l] / kBwdSlot) * MARL_H + (cdst[l] % kBwdSlot - 4 * MARL_H));
-                    continue;
-                }
-                cp_async16(slot + cdst[l], csrc[l] + (long long)t * cstride[l]);
-            }
-        }
-        cp_async_commit();
-    };
-    for (int idx = tid; idx < 2 * R * MARL_G; idx += kGruThreads) (&sg[0][0][0])[idx] = 0.0f;
-    // per-step output pointers of the rows this lane owns, walked backwards one time step (N rows) per iteration
-    float* pi_[OWN]; float* ph_[OWN];
-#pragma unroll
-    for (int q = 0; q < OWN; ++q) {
-        pi_[q] = a.dgi + (base[q] + (long long)(L - 1) * N) * MARL_G + j;
-        ph_[q] = a.dgh + (base[q] + (long long)(L - 1) * N) * MARL_G + j;
-    }
-    const long long ostep = (long long)N * MARL_G;
-    // early exit (SURVEY 8(f) N3): behind the longest episode of this pass every upstream gradient is masked to zero, so the
-    // chain would only produce zeros there -- they are written directly and the chain starts at that episode's last step
-    int Lp = L;
-    if (a.ep_len) {
-        Lp = 1;
-        for (int rr = 0; rr < nrows; ++rr) Lp = max(Lp, min(L, __ldg(a.ep_len + row_at(rr) / N)));
-        const int tail = L - Lp;
-        for (int idx = tid; idx < tail * nrows * (MARL_G / 4); idx += kGruThreads) {
-            const int c4 = idx % (MARL_G / 4), rr = (idx / (MARL_G / 4)) % nrows, t = Lp + idx / ((MARL_G / 4) * nrows);
-            const int row = row_at(rr);
-            const long long off = (((long long)(row / N) * L + t) * N + (row % N)) * MARL_G + 4 * c4;
-            *reinterpret_cast<float4*>(a.dgi + off) = make_float4(0.f, 0.f, 0.f, 0.f);
-            *reinterpret_cast<float4*>(a.dgh + off) = make_float4(0.f, 0.f, 0.f, 0.f);
-        }
-#pragma unroll
-        for (int q = 0; q < OWN; ++q) { pi_[q] -= (long long)tail * ostep; ph_[q] -= (long long)tail * ostep; }
-    }
-#pragma unroll
-    for (int d = 0; d < D - 1; ++d) issue(Lp - 1 - d);
-    cp_async_wait<D - 2>();
-    __syncthreads();
-    int cur = 0;
-    for (int t = Lp - 1; t >= 0; --t) {
-        float dh_dir[OWN];
-#pragma unroll
-        for (int q = 0; q < OWN; ++q) {
-            dh_dir[q] = 0.0f;
-            if (own[q]) {
-                const int rr = ks + 2 * q;
-                const float* sl = &ring[t % D][rr][0];
-                const float g_r = sl[j], g_z = sl[MARL_H + j], g_n = sl[2 * MARL_H + j], g_hn = sl[3 * MARL_H + j];
-                const float hprev = (t > 0 || a.h0) ? sl[4 * MARL_H + j] : 0.0f;
-                float dh = dh_carry[q];
-                if (a.dh_ext) dh += sl[5 * MARL_H + j];
-                if (a.dh_ext2) dh += sl[6 * MARL_H + j];
-                // h' = (h - n) z + n ; n = tanh(gi_n + r (W_hn h + b_hn)) ; r, z = sigmoid(gi + gh)
-                const float dn_pre = dh * (1.0f - g_z) * (1.0f - g_n * g_n);
-                const float dz_pre = dh * (hprev - g_n) * g_z * (1.0f - g_z);
-                const float dr_pre = dn_pre * g_hn * g_r * (1.0f - g_r);
-                const float dghn = dn_pre * g_r;
-                dh_dir[q] = dh * g_z;
-                float* pi = pi_[q];
-                float* ph = ph_[q];
-                pi[0] = dr_pre; pi[MARL_H] = dz_pre; pi[2 * MARL_H] = dn_pre;
-                ph[0] = dr_pre; ph[MARL_H] = dz_pre; ph[2 * MARL_H] = dghn;
-                sg[cur][rr][j] = dr_pre; sg[cur][rr][MARL_H + j] = dz_pre; sg[cur][rr][2 * MARL_H + j] = dghn;
-            }
-            pi_[q] -= ostep; ph_[q] -= ostep;
-        }
-        // the refill of the slot of step t+1 (consumed before the previous barrier): early when many rows keep the CTA
-        // throughput-bound, behind the FMAs (see the forward kernel) when the chain is latency-bound
-        constexpr bool kLateIssue = R <= 2;
-        if (!kLateIssue) { issue(t - (D - 1)); cp_async_wait<D - 2>(); }
-        else cp_async_wait<D - 3>();     // only D-2 groups are pending here: step t-1 has landed
-        __syncthreads();                 // dgh of step t visible; ring[t-1] visible
-        float part[R];
-        f32x2 pab[R], pcd[R];                   // four partial sums per row in two packed accumulators: short dependent chains
-#pragma unroll
-        for (int rr = 0; rr < R; ++rr) { pab[rr] = 0ull; pcd[rr] = 0ull; }
-#pragma unroll
-        for (int i = 0; i < 24; ++i)
-#pragma unroll
-            for (int rr = 0; rr < R; ++rr) {
-                const ulonglong2 v = *reinterpret_cast<const ulonglong2*>(&sg[cur][rr][4 * (2 * i + ks)]);
-                pab[rr] = ffma2(wt[2 * i], v.x, pab[rr]);
-                pcd[rr] = ffma2(wt[2 * i + 1], v.y, pcd[rr]);
-            }
-        if (kLateIssue) issue(t - (D - 1));
-#pragma unroll
-        for (int rr = 0; rr < R; ++rr) {
-            float pa, pb, pc, pd;
-            unpack2(pab[rr], pa, pb); unpack2(pcd[rr], pc, pd);
-            part[rr] = (pa + pb) + (pc + pd);
-            part[rr] += __shfl_xor_sync(0xffffffffu, part[rr], 1);
-        }
-#pragma unroll
-        for (int q = 0; q < OWN; ++q) {
-            const int e = 2 * q, o = (2 * q + 1 < R) ? 2 * q + 1 : 2 * q;
-            dh_carry[q] = dh_dir[q] + (ks ? part[o] : part[e]);
-        }
-        cur ^= 1;
-    }
-    cp_async_wait<0>();
-    if (a.dh0) {
-#pragma unroll
-        for (int q = 0; q < OWN; ++q)
-            if (own[q]) a.dh0[(long long)row_at(ks + 2 * q) * MARL_H + j] = dh_carry[q];
-    }
-    __syncthreads();
-}
-
-#ifndef MARL_GRU_BWD_CTAS
-#define MARL_GRU_BWD_CTAS 2
-#endif
-constexpr int kGruBwdCtasPerSm = MARL_GRU_BWD_CTAS;      // 254 registers x 128 threads and ~55 KB of shared memory: two CTAs fit an SM
-// up to two rows per SM: one CTA per row (see marl_agent_unroll_bwd)
-static int gru_bwd_ctas(int rows) { return rows <= kGruBwdCtasPerSm * kNumSMs ? rows : kNumSMs; }
-constexpr size_t gru_bwd_smem_max() { return gru_bwd_smem(8) > gru_bwd_smem(4) ? gru_bwd_smem(8) : gru_bwd_smem(4); }
-
-template <bool SEP>
-__global__ void __launch_bounds__(kGruThreads) gru_unroll_bwd_kernel(GruBwdArgs a) {
-    pdl_enter();
-    extern __shared__ __align__(16) float gru_smem[];
-    int begin, count;
-    if (SEP) cta_rows_by_agent(a.B, a.N, begin, count);
-    else cta_rows(a.B * a.N, 0, begin, count);
-    for (int off = 0, n = 0; off < count; off += SEP ? n : kGruMaxRows) {
-        n = gru_pass_rows<SEP>(begin + off, count - off, a.B);
-        if (n == 1) gru_rows_bwd<1, SEP>(a, begin + off, n, gru_smem);
-        else if (n == 2) gru_rows_bwd<2, SEP>(a, begin + off, n, gru_smem);
-        else if (n <= 4) gru_rows_bwd<4, SEP>(a, begin + off, n, gru_smem);
-        else gru_rows_bwd<8, SEP>(a, begin + off, n, gru_smem);
-    }
-}
-
-// ---- the recurrence at rnn_hidden_dim H = 32 and 128 ------------------------------------------------------------------------
-// The scheme of the H = 64 kernels above, with the reduction split KS = H / 32 ways: thread (j, ks) = (tid / KS, tid % KS)
-// owns hidden unit j and reduction indices 4 (KS i + ks) + c, so every thread keeps 96 W_hh weights in registers at every
-// width and the KS lanes of a unit sit side by side in one warp.  A group is H x KS threads (32 at H = 32, 512 at H = 128).
-// The H = 64 kernels keep their own source: routing them through this template would change their instruction schedule,
-// so a fix to one belongs in both.
-template <int H>
-struct GruWidth {
-    static constexpr int KS = H / 32;                 // lanes per hidden unit
-    static constexpr int T = H * KS;                  // threads of one group
-    static constexpr int G = 3 * H;
-    static constexpr int kGroups = T >= 512 ? 1 : 2;  // forward: chains side by side in one CTA (512 threads fill the register file)
-    static constexpr int kMaxRows = H >= 128 ? 2 : 4; // rows per pass: what fits the registers without spills (at most 128 a
-                                                      // thread in a 512-thread group; at H = 32 every lane owns every row)
-    static_assert(KS >= 1 && (KS & (KS - 1)) == 0 && KS <= 32, "KS must be a power of two inside a warp");
-};
-
-template <int H>
-__device__ __forceinline__ void group_sync_w(int id) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(GruWidth<H>::T) : "memory"); }
-
-// the KS partial sums of one hidden unit, summed over its lanes (butterfly: every lane ends with the total)
-template <int KS>
-__device__ __forceinline__ float lanes_sum(float v) {
-#pragma unroll
-    for (int o = 1; o < KS; o <<= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
-
-// v[q * KS + ks] with a register index fixed at compile time (rows past R read v[q * KS])
-template <int KS, int R>
-__device__ __forceinline__ float lane_pick(const float (&v)[R], int q, int ks) {
-    float r = v[q * KS];
-#pragma unroll
-    for (int c = 1; c < KS; ++c)
-        if (q * KS + c < R && ks == c) r = v[q * KS + c];
-    return r;
-}
-
-template <int H, bool SEP>
-__device__ __forceinline__ int gru_pass_rows_w(int pos, int left, int B) {
-    const int n = min(GruWidth<H>::kMaxRows, left);
-    return SEP ? min(n, B - pos % B) : n;
-}
-
-template <int H>
-constexpr size_t gru_fwd_smem_w(int R) { return (size_t)(2 * R * H + kGiDepth * R * 3 * H) * sizeof(float); }
-
-template <int H, int R, bool SEP>
-__device__ __forceinline__ void gru_chain_fwd_w(const GruFwdArgs& a, int chain, int row0, int nrows, float* smem, int bar_id) {
-    using W = GruWidth<H>;
-    constexpr int KS = W::KS, T = W::T, G = W::G, CPR = G / 4;       // CPR: 16-byte chunks of gi per row and step
-    float (*hs)[R][H] = reinterpret_cast<float (*)[R][H]>(smem);                              // [2][R][H]
-    float (*ring)[R][G] = reinterpret_cast<float (*)[R][G]>(smem + 2 * R * H);                // [D][R][3H]
-    const int tid = threadIdx.x % T, ks = tid % KS, j = tid / KS;
-    const int L = a.L, N = a.N;
-    __shared__ int srow_all[W::kGroups][W::kMaxRows];
-    int* srow = srow_all[bar_id - 1];
-    if (tid < R) {
-        const int* order = a.row_order[chain];
-        srow[tid] = (order && tid < nrows) ? __ldg(order + row0 + tid) : gru_position_row<SEP>(row0 + tid, a.B, N);
-    }
-    group_sync_w<H>(bar_id);
-    constexpr int OWN = (R + KS - 1) / KS;            // rows whose gate math this lane owns: rr = ks + KS q
-    bool own[OWN]; long long base[OWN];
-#pragma unroll
-    for (int q = 0; q < OWN; ++q) {
-        const int rr = ks + KS * q;
-        own[q] = rr < nrows;
-        const int row = own[q] ? srow[rr] : 0;
-        base[q] = own[q] ? ((long long)(row / N) * L * N + (row % N)) : 0;
-    }
-    const float* h0 = a.h0[chain];
-    for (int idx = tid; idx < R * H; idx += T) {
-        const int rr = idx / H, jj = idx % H;
-        hs[0][rr][jj] = (h0 && rr < nrows) ? h0[(long long)srow[rr] * H + jj] : 0.0f;
-    }
-    int cur = 0;
-    for (int sg = a.chain_start[chain]; sg < a.chain_start[chain] + a.chain_len[chain]; ++sg) {
-        const GruSegment S = a.seg[sg];
-        const long long poff = SEP ? (long long)(row0 / a.B) * a.agent_stride : 0;
-        const float* w_hh = S.w_hh + poff;
-        const float* b_hh = S.b_hh + poff;
-        f32x2 w[3][16];
-#pragma unroll
-        for (int g = 0; g < 3; ++g)
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-                const float4 v = __ldg(reinterpret_cast<const float4*>(w_hh + (long long)(g * H + j) * H + 4 * (KS * i + ks)));
-                w[g][2 * i] = pack2(v.x, v.y); w[g][2 * i + 1] = pack2(v.z, v.w);
-            }
-        const float bh_r = __ldg(b_hh + j), bh_z = __ldg(b_hh + H + j), bh_n = __ldg(b_hh + 2 * H + j);
-        long long idx[OWN];                          // (b, t, n) index of the owned rows at step t: one register pair per row
-#pragma unroll
-        for (int q = 0; q < OWN; ++q) idx[q] = base[q];
-        int Lp = L;
-        if (S.ep_len) {
-            Lp = 1;
-            for (int rr = 0; rr < nrows; ++rr) Lp = max(Lp, min(L, __ldg(S.ep_len + srow[rr] / N)));
-        }
-        // (the chunk sources are recomputed per step: a list of them would not fit the register budget)
-        auto issue = [&](int t) {
-            if (t < Lp) {
-                for (int c = tid; c < nrows * CPR; c += T) {
-                    const int rr = c / CPR, ch = c % CPR, row = srow[rr];
-                    cp_async16(&ring[t % kGiDepth][rr][ch * 4], S.gi + (((long long)(row / N) * L + t) * N + (row % N)) * G + ch * 4);
-                }
-            }
-            cp_async_commit();
-        };
-#pragma unroll
-        for (int t = 0; t < kGiDepth - 1; ++t) issue(t);
-        for (int t = 0; t < Lp; ++t) {
-            cp_async_wait<kGiDepth - 2>();
-            group_sync_w<H>(bar_id);
-            issue(t + kGiDepth - 1);
-            float acc[3][R];
-            f32x2 pacc[3][R];
-#pragma unroll
-            for (int g = 0; g < 3; ++g)
-#pragma unroll
-                for (int rr = 0; rr < R; ++rr) pacc[g][rr] = 0ull;
-#pragma unroll
-            for (int i = 0; i < 8; ++i)
-#pragma unroll
-                for (int rr = 0; rr < R; ++rr) {
-                    const ulonglong2 hv = *reinterpret_cast<const ulonglong2*>(&hs[cur][rr][4 * (KS * i + ks)]);
-#pragma unroll
-                    for (int g = 0; g < 3; ++g) {
-                        pacc[g][rr] = ffma2(w[g][2 * i], hv.x, pacc[g][rr]);
-                        pacc[g][rr] = ffma2(w[g][2 * i + 1], hv.y, pacc[g][rr]);
-                    }
-                }
-#pragma unroll
-            for (int g = 0; g < 3; ++g)
-#pragma unroll
-                for (int rr = 0; rr < R; ++rr) {
-                    float ev, od;
-                    unpack2(pacc[g][rr], ev, od);
-                    acc[g][rr] = lanes_sum<KS>(ev + od);
-                }
-            const float* gring = &ring[t % kGiDepth][0][0];
-#pragma unroll
-            for (int q = 0; q < OWN; ++q) {
-                const float ar = lane_pick<KS>(acc[0], q, ks), az = lane_pick<KS>(acc[1], q, ks), an = lane_pick<KS>(acc[2], q, ks);
-                if (own[q]) {
-                    const int rr = ks + KS * q;
-                    const float* gp = gring + rr * G;
-                    const float gh_n = an + bh_n;
-                    const float r = gate_sigmoid((ar + bh_r) + gp[j]);
-                    const float z = gate_sigmoid((az + bh_z) + gp[H + j]);
-                    const float n = gate_tanh(fmaf(r, gh_n, gp[2 * H + j]));
-                    const float hold = hs[cur][rr][j];
-                    const float hnew = fmaf(hold - n, z, n);
-                    hs[cur ^ 1][rr][j] = hnew;
-                    S.hidden[idx[q] * H + j] = hnew;
-                    if (S.gates) {
-                        float* go = S.gates + idx[q] * (4 * H) + j;
-                        go[0] = r; go[H] = z; go[2 * H] = n; go[3 * H] = gh_n;
-                    }
-                }
-                idx[q] += N;
-            }
-            cur ^= 1;
-        }
-        cp_async_wait<0>();
-        group_sync_w<H>(bar_id);
-        if (S.h_last) {
-#pragma unroll
-            for (int q = 0; q < OWN; ++q)
-                if (own[q]) S.h_last[(long long)srow[ks + KS * q] * H + j] = hs[cur][ks + KS * q][j];
-        }
-    }
-}
-
-template <int H, bool SEP>
-__global__ void __launch_bounds__(GruWidth<H>::T * GruWidth<H>::kGroups) gru_unroll_fwd_kernel_w(GruFwdArgs a) {
-    using W = GruWidth<H>;
-    pdl_enter();
-    extern __shared__ __align__(16) float gru_smem[];
-    const int grp = threadIdx.x / W::T;
-    const int chain = blockIdx.y * W::kGroups + grp;
-    if (chain >= a.n_chains) return;
-    float* smem = gru_smem + grp * (gru_fwd_smem_w<H>(W::kMaxRows) / sizeof(float));
-    int begin = 0;
-    for (int i = 0; i < (int)blockIdx.x; ++i) begin += a.rows_of[chain][i];
-    const int count = a.rows_of[chain][blockIdx.x];
-    for (int off = 0, n = 0; off < count; off += SEP ? n : W::kMaxRows) {
-        n = gru_pass_rows_w<H, SEP>(begin + off, count - off, a.B);
-        if (n == 1) gru_chain_fwd_w<H, 1, SEP>(a, chain, begin + off, n, smem, 1 + grp);
-        else if (n == 2 || W::kMaxRows == 2) gru_chain_fwd_w<H, 2, SEP>(a, chain, begin + off, n, smem, 1 + grp);
-        else if (n <= 4) gru_chain_fwd_w<H, (W::kMaxRows < 4 ? 2 : 4), SEP>(a, chain, begin + off, n, smem, 1 + grp);
-        else gru_chain_fwd_w<H, W::kMaxRows, SEP>(a, chain, begin + off, n, smem, 1 + grp);
-        group_sync_w<H>(1 + grp);
-    }
-}
-
-template <int H>
-constexpr size_t gru_bwd_smem_w(int R) { return (size_t)(2 * R * 3 * H + bwd_depth(R) * R * 7 * H) * sizeof(float); }
-
-template <int H, int R, bool SEP>
-__device__ __forceinline__ void gru_rows_bwd_w(const GruBwdArgs& a, int row0, int nrows, float* gru_smem) {
-    using W = GruWidth<H>;
-    constexpr int KS = W::KS, T = W::T, G = W::G, SLOT = 7 * H, CPR = SLOT / 4;
-    constexpr int D = bwd_depth(R);
-    float (*sg)[R][G] = reinterpret_cast<float (*)[R][G]>(gru_smem);                          // [2][R][3H]
-    float (*ring)[R][SLOT] = reinterpret_cast<float (*)[R][SLOT]>(gru_smem + 2 * R * G);     // [D][R][7H]
-    const int tid = threadIdx.x, ks = tid % KS, j = tid / KS;
-    const int L = a.L, N = a.N;
-    __shared__ int srow[W::kMaxRows];
-    if (tid < R) srow[tid] = (a.row_order && tid < nrows) ? __ldg(a.row_order + row0 + tid) : gru_position_row<SEP>(row0 + tid, a.B, N);
-    __syncthreads();
-    constexpr int OWN = (R + KS - 1) / KS;
-    bool own[OWN]; long long base[OWN]; float dh_carry[OWN];
-#pragma unroll
-    for (int q = 0; q < OWN; ++q) {
-        const int rr = ks + KS * q;
-        own[q] = rr < nrows;
-        const int row = own[q] ? srow[rr] : 0;
-        base[q] = own[q] ? ((long long)(row / N) * L * N + (row % N)) : 0;
-        dh_carry[q] = 0.0f;
-    }
-    // column j of W_hh, rows m = 4 (KS i + ks) + c, i = 0..23
-    const float* w_hh = a.w_hh + (SEP ? (long long)(row0 / a.B) * a.agent_stride : 0);
-    f32x2 wt[48];
-#pragma unroll
-    for (int i = 0; i < 24; ++i)
-#pragma unroll
-        for (int c = 0; c < 2; ++c)
             wt[2 * i + c] = pack2(__ldg(w_hh + (long long)(4 * (KS * i + ks) + 2 * c) * H + j),
                                   __ldg(w_hh + (long long)(4 * (KS * i + ks) + 2 * c + 1) * H + j));
-    // cp.async work list, per row and step 7H/4 chunks of 16 B: gates (H chunks), h_prev, dh_ext, dh_ext2 (H/4 each).  The
-    // chunk's source is recomputed per step from (row, kind, column): a list of pointers would not fit 128 registers at H = 128.
+    // cp.async work list: per row CPR chunks of 16 B (H of gates, H / 4 each of h_prev, dh_ext, dh_ext2).  The per-chunk source
+    // pointer at t = 0 and its per-step stride are fixed, so they are computed once -- which takes ~35 registers a thread: a
+    // 512-thread group, left with 128 registers a thread, recomputes each chunk's source per step instead.
+    constexpr bool kChunkList = T < 512;
+    constexpr int NCH = (R * CPR + T - 1) / T;
+    const float* csrc[NCH]; int cstride[NCH], cdst[NCH], ckind[NCH];
+    if constexpr (kChunkList) {
+#pragma unroll
+        for (int l = 0; l < NCH; ++l) {
+            const int c = tid + l * T, rr = c / CPR, ch = c % CPR, row = row_at(rr);
+            csrc[l] = nullptr; cstride[l] = 0; cdst[l] = rr * SLOT + ch * 4; ckind[l] = 0;
+            if (c < R * CPR && rr < nrows) {
+                const long long idx0 = (long long)(row / N) * L * N + (row % N);
+                if (ch < H) { csrc[l] = a.gates + idx0 * (4 * H) + ch * 4; cstride[l] = N * 4 * H; }
+                else if (ch < H + H / 4) { csrc[l] = a.hidden + (idx0 - N) * H + (ch - H) * 4; cstride[l] = N * H; ckind[l] = 1;
+                                           if (a.h0) ckind[l] = 2; }
+                else if (ch < H + H / 2) { if (a.dh_ext) { csrc[l] = a.dh_ext + idx0 * H + (ch - H - H / 4) * 4; cstride[l] = N * H; } }
+                else { if (a.dh_ext2) { csrc[l] = a.dh_ext2 + idx0 * H + (ch - H - H / 2) * 4; cstride[l] = N * H; } }
+            }
+        }
+    }
     auto issue = [&](int t) {
         if (t >= 0) {
             float* slot = &ring[t % D][0][0];
-            for (int c = tid; c < nrows * CPR; c += T) {
-                const int rr = c / CPR, ch = c % CPR, row = srow[rr];
-                const long long idx = ((long long)(row / N) * L + t) * N + (row % N);
-                const float* src = nullptr;
-                if (ch < H) src = a.gates + idx * (4 * H) + ch * 4;
-                else if (ch < H + H / 4) {
-                    if (t > 0) src = a.hidden + (idx - N) * H + (ch - H) * 4;
-                    else if (a.h0) src = a.h0 + (long long)row * H + (ch - H) * 4;     // (zeros without h0: the consumer)
-                } else if (ch < H + H / 2) { if (a.dh_ext) src = a.dh_ext + idx * H + (ch - H - H / 4) * 4; }
-                else if (a.dh_ext2) src = a.dh_ext2 + idx * H + (ch - H - H / 2) * 4;
-                if (src) cp_async16(slot + rr * SLOT + ch * 4, src);
+            if constexpr (kChunkList) {
+#pragma unroll
+                for (int l = 0; l < NCH; ++l) {
+                    if (!csrc[l]) continue;
+                    if (ckind[l] != 0 && t == 0) {      // h_prev of the first step: h0 (or zeros, handled by the consumer)
+                        if (ckind[l] == 2) cp_async16(slot + cdst[l], a.h0 + (long long)row_at(cdst[l] / SLOT) * H + (cdst[l] % SLOT - 4 * H));
+                        continue;
+                    }
+                    cp_async16(slot + cdst[l], csrc[l] + (long long)t * cstride[l]);
+                }
+            } else {
+                for (int c = tid; c < nrows * CPR; c += T) {
+                    const int rr = c / CPR, ch = c % CPR, row = row_at(rr);
+                    const long long idx = ((long long)(row / N) * L + t) * N + (row % N);
+                    const float* src = nullptr;
+                    if (ch < H) src = a.gates + idx * (4 * H) + ch * 4;
+                    else if (ch < H + H / 4) {
+                        if (t > 0) src = a.hidden + (idx - N) * H + (ch - H) * 4;
+                        else if (a.h0) src = a.h0 + (long long)row * H + (ch - H) * 4;     // (zeros without h0: the consumer)
+                    } else if (ch < H + H / 2) { if (a.dh_ext) src = a.dh_ext + idx * H + (ch - H - H / 4) * 4; }
+                    else if (a.dh_ext2) src = a.dh_ext2 + idx * H + (ch - H - H / 2) * 4;
+                    if (src) cp_async16(slot + rr * SLOT + ch * 4, src);
+                }
             }
         }
         cp_async_commit();
     };
     for (int idx = tid; idx < 2 * R * G; idx += T) (&sg[0][0][0])[idx] = 0.0f;
+    // per-step output pointers of the rows this lane owns, walked backwards one time step (N rows) per iteration
     float* pi_[OWN]; float* ph_[OWN];
 #pragma unroll
     for (int q = 0; q < OWN; ++q) {
@@ -791,14 +500,16 @@ __device__ __forceinline__ void gru_rows_bwd_w(const GruBwdArgs& a, int row0, in
         ph_[q] = a.dgh + (base[q] + (long long)(L - 1) * N) * G + j;
     }
     const long long ostep = (long long)N * G;
+    // early exit (SURVEY 8(f) N3): behind the longest episode of this pass every upstream gradient is masked to zero, so the
+    // chain would only produce zeros there -- they are written directly and the chain starts at that episode's last step
     int Lp = L;
     if (a.ep_len) {
         Lp = 1;
-        for (int rr = 0; rr < nrows; ++rr) Lp = max(Lp, min(L, __ldg(a.ep_len + srow[rr] / N)));
+        for (int rr = 0; rr < nrows; ++rr) Lp = max(Lp, min(L, __ldg(a.ep_len + row_at(rr) / N)));
         const int tail = L - Lp;
         for (int idx = tid; idx < tail * nrows * (G / 4); idx += T) {
             const int c4 = idx % (G / 4), rr = (idx / (G / 4)) % nrows, t = Lp + idx / ((G / 4) * nrows);
-            const int row = srow[rr];
+            const int row = row_at(rr);
             const long long off = (((long long)(row / N) * L + t) * N + (row % N)) * G + 4 * c4;
             *reinterpret_cast<float4*>(a.dgi + off) = make_float4(0.f, 0.f, 0.f, 0.f);
             *reinterpret_cast<float4*>(a.dgh + off) = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -824,6 +535,7 @@ __device__ __forceinline__ void gru_rows_bwd_w(const GruBwdArgs& a, int row0, in
                 float dh = dh_carry[q];
                 if (a.dh_ext) dh += sl[5 * H + j];
                 if (a.dh_ext2) dh += sl[6 * H + j];
+                // h' = (h - n) z + n ; n = tanh(gi_n + r (W_hn h + b_hn)) ; r, z = sigmoid(gi + gh)
                 const float dn_pre = dh * (1.0f - g_z) * (1.0f - g_n * g_n);
                 const float dz_pre = dh * (hprev - g_n) * g_z * (1.0f - g_z);
                 const float dr_pre = dn_pre * g_hn * g_r * (1.0f - g_r);
@@ -837,11 +549,14 @@ __device__ __forceinline__ void gru_rows_bwd_w(const GruBwdArgs& a, int row0, in
             }
             pi_[q] -= ostep; ph_[q] -= ostep;
         }
-        issue(t - (D - 1));
-        cp_async_wait<D - 2>();
+        // the refill of the slot of step t+1 (consumed before the previous barrier): early when many rows keep the CTA
+        // throughput-bound, behind the FMAs (see the forward kernel) when the chain is latency-bound and the registers allow
+        constexpr bool kLateIssue = R <= 2 && T < 512;
+        if (!kLateIssue) { issue(t - (D - 1)); cp_async_wait<D - 2>(); }
+        else cp_async_wait<D - 3>();     // only D-2 groups are pending here: step t-1 has landed
         __syncthreads();                 // dgh of step t visible; ring[t-1] visible
         float part[R];
-        f32x2 pab[R], pcd[R];
+        f32x2 pab[R], pcd[R];                   // four partial sums per row in two packed accumulators: short dependent chains
 #pragma unroll
         for (int rr = 0; rr < R; ++rr) { pab[rr] = 0ull; pcd[rr] = 0ull; }
 #pragma unroll
@@ -852,6 +567,7 @@ __device__ __forceinline__ void gru_rows_bwd_w(const GruBwdArgs& a, int row0, in
                 pab[rr] = ffma2(wt[2 * i], v.x, pab[rr]);
                 pcd[rr] = ffma2(wt[2 * i + 1], v.y, pcd[rr]);
             }
+        if (kLateIssue) issue(t - (D - 1));
 #pragma unroll
         for (int rr = 0; rr < R; ++rr) {
             float pa, pb, pc, pd;
@@ -866,18 +582,28 @@ __device__ __forceinline__ void gru_rows_bwd_w(const GruBwdArgs& a, int row0, in
     if (a.dh0) {
 #pragma unroll
         for (int q = 0; q < OWN; ++q)
-            if (own[q]) a.dh0[(long long)srow[ks + KS * q] * H + j] = dh_carry[q];
+            if (own[q]) a.dh0[(long long)row_at(ks + KS * q) * H + j] = dh_carry[q];
     }
     __syncthreads();
 }
 
+#ifndef MARL_GRU_BWD_CTAS
+#define MARL_GRU_BWD_CTAS 2
+#endif
+constexpr int kGruBwdCtasPerSm = MARL_GRU_BWD_CTAS;      // H = 64: 254 registers x 128 threads and ~55 KB of shared memory: two CTAs fit an SM
+// up to two rows per SM: one CTA per row (see marl_agent_unroll_bwd); the same CTA count at every width, so that the row deal
+// marl_agent_unroll_fwd plans for it (row_order_bwd) holds
+static int gru_bwd_ctas(int rows) { return rows <= kGruBwdCtasPerSm * kNumSMs ? rows : kNumSMs; }
+// the largest pass's shared memory (the ring is shallower at 8 rows, so the 4-row pass may need more)
 template <int H>
-constexpr size_t gru_bwd_smem_max_w() {
-    return gru_bwd_smem_w<H>(GruWidth<H>::kMaxRows) > gru_bwd_smem_w<H>(2) ? gru_bwd_smem_w<H>(GruWidth<H>::kMaxRows) : gru_bwd_smem_w<H>(2);
+constexpr size_t gru_bwd_smem_max() {
+    size_t m = 0;
+    for (int R = 1; R <= GruWidth<H>::kMaxRows; R *= 2) m = gru_bwd_smem<H>(R) > m ? gru_bwd_smem<H>(R) : m;
+    return m;
 }
 
 template <int H, bool SEP>
-__global__ void __launch_bounds__(GruWidth<H>::T) gru_unroll_bwd_kernel_w(GruBwdArgs a) {
+__global__ void __launch_bounds__(GruWidth<H>::T) gru_unroll_bwd_kernel(GruBwdArgs a) {
     using W = GruWidth<H>;
     pdl_enter();
     extern __shared__ __align__(16) float gru_smem[];
@@ -885,41 +611,41 @@ __global__ void __launch_bounds__(GruWidth<H>::T) gru_unroll_bwd_kernel_w(GruBwd
     if (SEP) cta_rows_by_agent(a.B, a.N, begin, count);
     else cta_rows(a.B * a.N, 0, begin, count);
     for (int off = 0, n = 0; off < count; off += SEP ? n : W::kMaxRows) {
-        n = gru_pass_rows_w<H, SEP>(begin + off, count - off, a.B);
-        if (n == 1) gru_rows_bwd_w<H, 1, SEP>(a, begin + off, n, gru_smem);
-        else if (n == 2 || W::kMaxRows == 2) gru_rows_bwd_w<H, 2, SEP>(a, begin + off, n, gru_smem);
-        else if (n <= 4) gru_rows_bwd_w<H, (W::kMaxRows < 4 ? 2 : 4), SEP>(a, begin + off, n, gru_smem);
-        else gru_rows_bwd_w<H, W::kMaxRows, SEP>(a, begin + off, n, gru_smem);
+        n = gru_pass_rows<H, SEP>(begin + off, count - off, a.B);
+        if (n == 1) gru_rows_bwd<H, 1, SEP>(a, begin + off, n, gru_smem);
+        else if (W::kMaxRows == 2 || n == 2) gru_rows_bwd<H, 2, SEP>(a, begin + off, n, gru_smem);
+        else if (W::kMaxRows == 4 || n <= 4) gru_rows_bwd<H, W::rows(4), SEP>(a, begin + off, n, gru_smem);
+        else gru_rows_bwd<H, W::rows(8), SEP>(a, begin + off, n, gru_smem);
     }
 }
 
-// Launches of the H = 32 / 128 recurrence.  Forward: the H = 64 grid (one CTA per SM and chain group), a group per chain.
-// Backward: the H = 64 CTA count, so that the row deal marl_agent_unroll_fwd plans for it (row_order_bwd) holds.
+// Forward launch: one CTA per SM and chain group, a thread group per chain.  `smem` (0: what the kernel needs) may ask for more,
+// so that the launch has its SMs to itself (gru_fwd_launch_solo); the kernel's opt-in is raised to the largest size asked for.
 template <int H>
-static void gru_fwd_launch_w(const GruFwdArgs& ga, int n_ctas, bool sep, cudaStream_t st) {
+static void gru_fwd_launch(const GruFwdArgs& ga, int n_ctas, bool sep, cudaStream_t st, size_t smem = 0) {
     using W = GruWidth<H>;
-    const size_t sm = W::kGroups * gru_fwd_smem_w<H>(W::kMaxRows);
-    static bool attr_set = false;
-    if (!attr_set) {
-        cudaFuncSetAttribute(gru_unroll_fwd_kernel_w<H, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-        cudaFuncSetAttribute(gru_unroll_fwd_kernel_w<H, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-        attr_set = true;
+    if (!smem) smem = W::kGroups * gru_fwd_smem<H>(W::kMaxRows);
+    static size_t opt_in = 0;
+    if (smem > opt_in) {
+        cudaFuncSetAttribute(gru_unroll_fwd_kernel<H, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaFuncSetAttribute(gru_unroll_fwd_kernel<H, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        opt_in = smem;
     }
     const dim3 grid(n_ctas, (ga.n_chains + W::kGroups - 1) / W::kGroups);
-    launch_pdl_prio(kGruPrio, sep ? gru_unroll_fwd_kernel_w<H, true> : gru_unroll_fwd_kernel_w<H, false>, grid,
-                    dim3(W::T * W::kGroups), sm, st, ga);
+    launch_pdl_prio(kGruPrio, sep ? gru_unroll_fwd_kernel<H, true> : gru_unroll_fwd_kernel<H, false>, grid,
+                    dim3(W::T * W::kGroups), smem, st, ga);
 }
 
 template <int H>
-static void gru_bwd_launch_w(const GruBwdArgs& ga, int rows, bool sep, cudaStream_t st) {
-    const size_t sm = gru_bwd_smem_max_w<H>();
+static void gru_bwd_launch(const GruBwdArgs& ga, int rows, bool sep, cudaStream_t st) {
+    constexpr size_t sm = gru_bwd_smem_max<H>();
     static bool attr_set = false;
     if (!attr_set) {
-        cudaFuncSetAttribute(gru_unroll_bwd_kernel_w<H, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-        cudaFuncSetAttribute(gru_unroll_bwd_kernel_w<H, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+        cudaFuncSetAttribute(gru_unroll_bwd_kernel<H, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+        cudaFuncSetAttribute(gru_unroll_bwd_kernel<H, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
         attr_set = true;
     }
-    launch_pdl_prio(kGruPrio, sep ? gru_unroll_bwd_kernel_w<H, true> : gru_unroll_bwd_kernel_w<H, false>, dim3(gru_bwd_ctas(rows)),
+    launch_pdl_prio(kGruPrio, sep ? gru_unroll_bwd_kernel<H, true> : gru_unroll_bwd_kernel<H, false>, dim3(gru_bwd_ctas(rows)),
                     dim3(GruWidth<H>::T), sm, st, ga);
 }
 
@@ -981,6 +707,7 @@ static void plan_rows(GruFwdArgs& ga, int rows, int n_ctas, int agents) {
 constexpr int kMaxOrderCtas = 2 * kNumSMs;      // the BPTT kernel runs up to two one-row CTAs per SM
 constexpr int kMaxOrderEpisodes = 1024;          // (larger batches keep the index order: the ranking below is O(B^2 / 256) per block)
 constexpr int kOrderWarps = 8;
+constexpr int kOrderRows = GruWidth<MARL_H>::kMaxRows;   // rows of a pass level (the H = 64 pass, at every width)
 template <int C>
 struct OrderPlan {
     int n_ctas;                 // 0: unused
@@ -1030,18 +757,18 @@ __global__ void __launch_bounds__(kOrderWarps * 32) row_order_kernel(const __gri
     for (int o = lane; o < c; o += 32) begin += cnt[o];
     begin = (int)warp_sum((float)begin);            // (exact: < 2^24 rows)
     int level_start = 0;                            // sorted position of the first row of pass level p
-    for (int p = 0; p * kGruMaxRows < mine; ++p) {
+    for (int p = 0; p * kOrderRows < mine; ++p) {
         int before = 0, width = 0;                  // rows of level p dealt before this CTA's / in the whole level
         for (int o = lane; o < n_ctas; o += 32) {
-            const int w = min(max((int)cnt[o] - kGruMaxRows * p, 0), kGruMaxRows);
+            const int w = min(max((int)cnt[o] - kOrderRows * p, 0), kOrderRows);
             width += w;
             if ((p & 1) ? pos[o] > mypos : pos[o] < mypos) before += w;        // the deal runs backwards on odd levels
         }
         before = (int)warp_sum((float)before); width = (int)warp_sum((float)width);
-        const int w = min(mine - kGruMaxRows * p, kGruMaxRows);
+        const int w = min(mine - kOrderRows * p, kOrderRows);
         if (lane < w) {
             const int sorted = level_start + before + lane;
-            out[begin + kGruMaxRows * p + lane] = (int)ep_of_rank[sorted / N] * N + sorted % N;
+            out[begin + kOrderRows * p + lane] = (int)ep_of_rank[sorted / N] * N + sorted % N;
         }
         level_start += width;
     }
@@ -1243,15 +970,6 @@ static GruFwdArgs single_chain(const marl_dims* d, const marl_unroll_stream& u, 
     return g;
 }
 
-// the dynamic shared memory the H = 64 forward kernel may be launched with: raised to the largest size asked for so far
-static void gru_fwd_smem_attr(size_t bytes) {
-    static size_t cur = 0;
-    if (bytes <= cur) return;
-    cudaFuncSetAttribute(gru_unroll_fwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-    cudaFuncSetAttribute(gru_unroll_fwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-    cur = bytes;
-}
-
 // A recurrence launch of the split forward: it reserves the whole of the SM's shared memory, so that nothing runs beside it
 static void gru_fwd_launch_solo(const GruFwdArgs& ga, int n_ctas, bool pdl, cudaStream_t st) {
     static size_t solo = 0;
@@ -1260,15 +978,13 @@ static void gru_fwd_launch_solo(const GruFwdArgs& ga, int n_ctas, bool pdl, cuda
         cudaGetDevice(&dev);
         cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
         cudaFuncAttributes fa{};
-        cudaFuncGetAttributes(&fa, gru_unroll_fwd_kernel<false>);
+        cudaFuncGetAttributes(&fa, gru_unroll_fwd_kernel<MARL_H, false>);
         solo = (size_t)optin - fa.sharedSizeBytes;
     }
-    gru_fwd_smem_attr(solo);
     ProfScope ps_("gru_unroll_fwd_kernel", st);
     const bool keep_ = pdl_small_problem();
     pdl_small_problem() = keep_ && pdl;
-    launch_pdl_prio(kGruPrio, gru_unroll_fwd_kernel<false>, dim3(n_ctas, (ga.n_chains + kGruGroups - 1) / kGruGroups),
-                    dim3(kGruThreads * kGruGroups), solo, st, ga);
+    gru_fwd_launch<MARL_H>(ga, n_ctas, false, st, solo);
     pdl_small_problem() = keep_;
 }
 
@@ -1512,16 +1228,10 @@ extern "C" int marl_agent_unroll_fwd(const marl_dims* d, const marl_unroll_strea
         ProfScope ps_("gru_unroll_fwd_kernel", st);
         ga.trace = trace_buffer();
         if (order_lane) order_lane->join();
-        if (H == MARL_H) {
-            const size_t sm = kGruGroups * gru_fwd_smem(kGruMaxRows);
-            gru_fwd_smem_attr(sm);
-            dim3 grid(n_ctas, (ga.n_chains + kGruGroups - 1) / kGruGroups);
-            launch_pdl_prio(kGruPrio, sep ? gru_unroll_fwd_kernel<true> : gru_unroll_fwd_kernel<false>, grid,
-                            dim3(kGruThreads * kGruGroups), sm, st, ga);
-        } else if (H == 32) {
-            gru_fwd_launch_w<32>(ga, n_ctas, sep, st);
-        } else {
-            gru_fwd_launch_w<128>(ga, n_ctas, sep, st);
+        switch (H) {
+        case 32: gru_fwd_launch<32>(ga, n_ctas, sep, st); break;
+        case 64: gru_fwd_launch<64>(ga, n_ctas, sep, st); break;
+        default: gru_fwd_launch<128>(ga, n_ctas, sep, st); break;
         }
     }
     MARL_LAUNCH_CHECK();
@@ -1574,24 +1284,17 @@ extern "C" int marl_agent_unroll_bwd(const marl_dims* d, const marl_unroll_bwd* 
     const int rows = d->B * d->N;
     {
         ProfScope ps_("gru_unroll_bwd_kernel", st);
-        static bool attr_set = false;
-        if (!attr_set) {
-            cudaFuncSetAttribute(gru_unroll_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gru_bwd_smem_max());
-            cudaFuncSetAttribute(gru_unroll_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gru_bwd_smem_max());
-            attr_set = true;
-        }
         const bool keep_ = pdl_small_problem();
         // measured: launched programmatically the 148 recurrence CTAs come up while the producer still runs and the
         // step gets 10-27 us slower on every config; a plain launch here, PDL for its consumers
         pdl_small_problem() = false;
         // up to two rows per SM: one CTA per row -- two co-resident one-row CTAs overlap each other's latency, where one CTA with two
         // rows serialises 2 x 96 packed FMAs per thread on the dependent chain (the 12 two-row CTAs of config 2 ended the kernel)
-        const int n_ctas = gru_bwd_ctas(rows);
-        if (H == MARL_H)
-            launch_pdl_prio(kGruPrio, sep ? gru_unroll_bwd_kernel<true> : gru_unroll_bwd_kernel<false>, dim3(n_ctas),
-                            dim3(kGruThreads), gru_bwd_smem_max(), st, ga);
-        else if (H == 32) gru_bwd_launch_w<32>(ga, rows, sep, st);
-        else gru_bwd_launch_w<128>(ga, rows, sep, st);
+        switch (H) {
+        case 32: gru_bwd_launch<32>(ga, rows, sep, st); break;
+        case 64: gru_bwd_launch<64>(ga, rows, sep, st); break;
+        default: gru_bwd_launch<128>(ga, rows, sep, st); break;
+        }
         pdl_small_problem() = keep_;
     }
     MARL_LAUNCH_CHECK();
